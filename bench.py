@@ -2,6 +2,7 @@
 """Benchmark of the hot path: streamed audio-seconds per second through fbank -> CMVN -> encoder -> adapter.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload stream|latency|offline]
+                    [--dump-outputs DIR]
 
 One "step" = every session of the batch advances one 160 ms chunk (int16 PCM in, LLM-space embeddings out).
 Workload at N=1 is BASELINE.json configs[1]: 64 concurrent sessions, synthetic 16 kHz audio, streaming chunks with
@@ -381,6 +382,25 @@ def parity_spot_check(eng, cfg, n_sessions, steps=3, sampled=(0, 1)):
                     "%s weights" % (n_sessions, steps, list(oracle), "bf16-rounded" if eng.dtype == torch.bfloat16 else "fp32")}
 
 
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each (sessions, ...) output as out_dir/<name>.npy in float32 so that two builds can be compared output for
+    output.  Past DUMP_LIMIT bytes in all, the same seeded sample of session rows is kept of every array and its row
+    numbers are written as out_dir/session_index.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    host = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    n = len(next(iter(host.values())))
+    row_bytes = sum(a[0].nbytes for a in host.values())
+    if n * row_bytes > DUMP_LIMIT:
+        rows = np.sort(np.random.RandomState(0).choice(n, DUMP_LIMIT // row_bytes, replace=False))
+        host = {k: a[rows] for k, a in host.items()}
+        np.save(os.path.join(out_dir, "session_index.npy"), rows.astype(np.float64))
+    for k, a in host.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 def ncu_traffic():
     """dram__bytes_read+write per GEMM launch of a 64-session step from the committed ncu capture of THIS round's build
     (profiles/r02_ncu_gemm_dram_traffic_stream64.json written by tools/ncu_summary.py); None when absent."""
@@ -416,7 +436,11 @@ def main():
     ap.add_argument("--debug-skip", type=int, default=0, help="timing attribution only: bitmask of kernel classes to skip")
     ap.add_argument("--quick", action="store_true", help="device-resident timing only")
     ap.add_argument("--opt", action="append", default=[], help="library option name=value (fo_set_option), repeatable")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (adapter_out, float32) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.workload in ("ragged", "offline")):
+        ap.error("--dump-outputs covers the streaming path (--impl ours, --workload stream or latency)")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.workload == "latency":
@@ -549,6 +573,8 @@ def main():
     ms = timed(K, False, W)
     launches = eng.stats()["kernel_launches"] - l0
     value = world * S * CHUNK_SEC * K / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"adapter_out": y_dev})      # y_dev holds the last timed step's embeddings
     if args.quick:
         sampler.stop_flag = True
         if rank == 0:

@@ -12,9 +12,15 @@ harness shims of SURVEY 8c:
   2. Tensor.to('cuda') is mapped to a no-op on this GPU-less host (transformer.py:279);
   3. sys.argv is cleared before construction (encoder.py:54-56 parses the process argv).
 Weights are the seeded state dict of freeze_omni_b200/weights.py loaded with strict=True.
-/root/reference does not exist on the GPU box, so nothing else imports this file.
+Nothing in the test suite imports this file: it needs a checkout of the reference.
+
+Every stored file stays under 1 MB.  Inputs that are a function of a seed (synthetic audio, random features) are not
+stored: tests/conftest.py rebuilds them with the same seeds.  The streaming fbank features of those streams are stored
+only as the SHA-256 of the reference's values, which the features rebuilt from the audio must match bit for bit.  The
+widest outputs keep a seeded sample of their last axis, with the sampled indices stored as <name>_cols.
 """
 import argparse
+import hashlib
 import os
 import sys
 import wave
@@ -25,9 +31,23 @@ import torch
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.dirname(HERE))
 
+from conftest import synth_audio  # noqa: E402
 from freeze_omni_b200.config import load_yaml, path_config_from_dict  # noqa: E402
 from freeze_omni_b200.weights import make_adapter_state, make_encoder_state  # noqa: E402
+
+
+def feats_digest(feats):
+    return np.array(hashlib.sha256(np.ascontiguousarray(feats, np.float32).tobytes()).hexdigest())
+
+
+def sample_last_axis(arrs, name, n, keys):
+    """Keep the same seeded n indices of the last axis of every array in keys; store them as <name>_cols."""
+    cols = np.sort(np.random.RandomState(0).choice(arrs[keys[0]].shape[-1], n, replace=False))
+    arrs[name + "_cols"] = cols
+    for k in keys:
+        arrs[k] = arrs[k][..., cols]
 
 
 def import_reference(ref_root):
@@ -68,16 +88,6 @@ def build_reference(mods, yaml_cfg, cfg, seed):
                                      mc["activation_func"], mc["norm"])
     adp.load_state_dict(adp_sd, strict=True)
     return enc.eval(), adp.eval()
-
-
-def synth_audio(seed, n):
-    """SURVEY 8d config 2: 0.1*N(0,1) band-limited, 200 ms silent gaps, int16-quantised."""
-    g = torch.Generator().manual_seed(seed)
-    x = 0.1 * torch.randn(n + 8, generator=g)
-    x = torch.nn.functional.avg_pool1d(x.view(1, 1, -1), 5, 1).view(-1)[:n] * 2.0
-    t = torch.arange(n)
-    x = x * ((t // 3200) % 5 != 4).float()
-    return torch.clamp((x * 32768.0).round(), -32768, 32767).to(torch.int16)
 
 
 def stream_reference(enc, adp, feats_seq, layers_to_keep=(0,)):
@@ -257,10 +267,12 @@ def main():
                 off["adp_c%d_L%d" % (c, L)] = y.numpy()
                 off["mask_c%d_L%d" % (c, L)] = m.numpy()
                 off["amask_c%d_L%d" % (c, L)] = ym.numpy()
-        save("tiny", seed=np.int64(3), stream_pcm=np.stack(pcm_b), stream_feats=torch.stack(feats_seq).numpy(),
-             **{"stream_" + k: v for k, v in st.items()},
-             t7_feats=torch.stack(feats32).numpy(), **{"t7_" + k: v for k, v in st7.items()},
-             off_feats=xs.numpy(), off_ilens=ilens.numpy(), **{"off_" + k: v for k, v in off.items()})
+        arrs = dict(seed=np.int64(3), stream_feats_sha256=feats_digest(torch.stack(feats_seq).numpy()),
+                    **{"stream_" + k: v for k, v in st.items()},
+                    **{"t7_" + k: st7[k] for k in ("enc_out", "adapter_out", "pe_index")},
+                    off_ilens=ilens.numpy(), **{"off_" + k: v for k, v in off.items()})
+        sample_last_axis(arrs, "kv", 16, ["stream_k_cache_l0", "stream_v_cache_l0", "stream_k_cache_l1", "stream_v_cache_l1"])
+        save("tiny", **arrs)
 
     # ---------------- conv1d-linear positionwise variant (Conv1dLinear, attention.py:198-266) ----------
     # Only `forward` can be executed in the reference for this variant (its streaming wiring is broken, SURVEY 2.3):
@@ -406,15 +418,22 @@ def main():
         # config 1: question.wav, 13 chunks, 1 session
         fq = feats_from_pcm(pcm_pad)
         st = stream_reference(enc, adp, fq, layers_to_keep=(0, 23))
-        save("shipped_question", seed=np.int64(0), pcm=pcm_pad, feats=torch.stack(fq).numpy(),
-             **{k: v for k, v in st.items()})
+        arrs = dict(seed=np.int64(0), pcm=pcm_pad, feats_sha256=feats_digest(torch.stack(fq).numpy()), **st)
+        sample_last_axis(arrs, "enc", 512, ["enc_out"])
+        sample_last_axis(arrs, "adp", 1024, ["adapter_out"])
+        sample_last_axis(arrs, "kv", 32, ["k_cache_l0", "v_cache_l0", "k_cache_l23", "v_cache_l23"])
+        save("shipped_question", **arrs)
         # 2 lock-step sessions x 20 chunks: crosses the 17-chunk cache saturation (SURVEY 2.4-1)
         pcm_b = [synth_audio(1000 + b, 2560 * 20).numpy() for b in range(2)]
         per = [feats_from_pcm(p) for p in pcm_b]
         feats_seq = [torch.cat([per[b][i] for b in range(2)], 0) for i in range(20)]
         st2 = stream_reference(enc, adp, feats_seq, layers_to_keep=(0, 23))
-        save("shipped_b2", seed=np.int64(0), pcm=np.stack(pcm_b), feats=torch.stack(feats_seq).numpy(),
-             **{k: v for k, v in st2.items()})
+        arrs = dict(seed=np.int64(0), feats_sha256=feats_digest(torch.stack(feats_seq).numpy()),
+                    enc_out=st2["enc_out"], adapter_out=st2["adapter_out"], k_cache_l23=st2["k_cache_l23"])
+        sample_last_axis(arrs, "enc", 512, ["enc_out"])
+        sample_last_axis(arrs, "adp", 1024, ["adapter_out"])
+        sample_last_axis(arrs, "kv", 32, ["k_cache_l23"])
+        save("shipped_b2", **arrs)
         # the reference's own bf16 regime (models/pipeline.py:67-68 runs it under autocast bf16; on this
         # GPU-less host the CPU autocast is the executable stand-in): its distance from its fp32 outputs
         # is the noise floor quoted next to the bf16 parity numbers.

@@ -46,7 +46,7 @@ def test_checkpoint_split_and_audit(tmp_path):
     import shutil
     import yaml
     from freeze_omni_b200.config import load_yaml
-    shutil.copy(os.path.join(os.path.dirname(__file__), "..", "configs", "tiny.yaml"), tmp_path / "final.yaml")
+    shutil.copyfile(os.path.join(os.path.dirname(__file__), "..", "configs", "tiny.yaml"), tmp_path / "final.yaml")
     torch.save(ckpt, tmp_path / "final.pt")
     cfg2, e2, a2 = load_trained(str(tmp_path), role="system")
     assert cfg2.d_model == cfg.d_model and torch.equal(e2[k], enc[k] * 2.0) and set(a2) == set(adp)
@@ -84,9 +84,9 @@ def test_absent_model_conf_keys_take_the_reference_defaults(tmp_path):
     ckpt["adpter.bn2.num_batches_tracked"] = torch.tensor(7)
     import shutil
     torch.save(ckpt, tmp_path / "final.pt")
-    shutil.copy(os.path.join(os.path.dirname(__file__), "..", "configs", "tiny.yaml"), tmp_path / "final.yaml")
+    shutil.copyfile(os.path.join(os.path.dirname(__file__), "..", "configs", "tiny.yaml"), tmp_path / "final.yaml")
     with pytest.raises(ValueError, match="does not use"):
         load_trained(str(tmp_path))
-    shutil.copy(os.path.join(os.path.dirname(__file__), "..", "configs", "tiny_bn.yaml"), tmp_path / "final.yaml")
+    shutil.copyfile(os.path.join(os.path.dirname(__file__), "..", "configs", "tiny_bn.yaml"), tmp_path / "final.yaml")
     cfg2, _, a2 = load_trained(str(tmp_path))                              # num_batches_tracked rides along with a BatchNorm
     assert cfg2.adapter_norm == "batch" and "bn2.running_var" in a2

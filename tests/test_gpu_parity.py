@@ -2,8 +2,6 @@
 against the golden vectors produced by the reference modules and against the CPU oracle on seeded inputs.
 Tolerances are the north star's: fbank 1e-5 relative (fp32), encoder/adapter 1e-4 max-abs in fp32 and
 2e-2 max-abs in bf16, masks / cache indexing / position bookkeeping bit-exact."""
-import os
-
 import numpy as np
 import pytest
 import torch
@@ -137,12 +135,13 @@ def test_tiny_stream_fp32(golden, tiny32):
             for b in range(3):
                 nf, pe = eng.state(int(ids[b]))
                 assert nf == 4 * (i + 1) and pe == int(g["stream_pe_index"][i])       # bit-exact bookkeeping
+        kv = g["kv_cols"]                                          # the golden keeps a sample of the head dimension
         for li in (0, 1):
             k = torch.cat([eng.export_kv(int(s), li)[0] for s in ids])
             v = torch.cat([eng.export_kv(int(s), li)[1] for s in ids])
-            assert k.shape == g["stream_k_cache_l%d" % li].shape
-            assert maxabs(k, g["stream_k_cache_l%d" % li]) < FP32_TOL
-            assert maxabs(v, g["stream_v_cache_l%d" % li]) < FP32_TOL
+            assert k.shape == g["stream_k_cache_l%d" % li].shape[:-1] + (cfg.d_k,)
+            assert maxabs(k[..., kv], g["stream_k_cache_l%d" % li]) < FP32_TOL
+            assert maxabs(v[..., kv], g["stream_v_cache_l%d" % li]) < FP32_TOL
         ac = torch.cat([eng.export_adapter_cache(int(s)) for s in ids])
         assert maxabs(ac, g["stream_adapter_cache"]) < FP32_TOL
     finally:
@@ -323,36 +322,52 @@ def test_gemm_simt_vs_torch(tiny32):
 # shipped config
 # ------------------------------------------------------------------------------------------------
 def test_shipped_question_fp32(golden, shipped32):
-    """BASELINE.json config 1 on the GPU path: question.wav, 13 chunks, PCM in."""
+    """BASELINE.json config 1 on the GPU path: question.wav, 13 chunks, PCM in.  Against the reference on the seeded
+    sample of feature columns the golden keeps, and against the oracle on every column."""
     cfg, eng = shipped32
     g = golden("shipped_question")
+    sess = O.StreamSession(cfg, make_encoder_state(cfg, 0), make_adapter_state(cfg, 0))
     ids = eng.alloc(1)
     try:
         pcm = (g["pcm"].astype(np.float32) / 32768.0).reshape(13, 1, 2560)
         for i in range(13):
             enc, y = eng.stream_step(ids, torch.from_numpy(pcm[i]), 32768.0)
-            assert maxabs(enc.cpu(), g["enc_out"][i]) < FP32_TOL, i
-            assert maxabs(y.cpu(), g["adapter_out"][i]) < FP32_TOL, i
+            _, eo, yo = sess.step_pcm(torch.from_numpy(pcm[i, 0]), 32768.0)
+            assert maxabs(enc.cpu(), eo) < FP32_TOL and maxabs(y.cpu(), yo) < FP32_TOL, i
+            assert maxabs(enc.cpu()[..., g["enc_cols"]], g["enc_out"][i]) < FP32_TOL, i
+            assert maxabs(y.cpu()[..., g["adp_cols"]], g["adapter_out"][i]) < FP32_TOL, i
             assert eng.state(int(ids[0]))[1] == int(g["pe_index"][i])
+        kv = g["kv_cols"]
         for li in (0, 23):
             k, v = eng.export_kv(int(ids[0]), li)
-            assert maxabs(k, g["k_cache_l%d" % li]) < FP32_TOL and maxabs(v, g["v_cache_l%d" % li]) < FP32_TOL
+            assert maxabs(k, sess.buffer[li][0]) < FP32_TOL and maxabs(v, sess.buffer[li][1]) < FP32_TOL
+            assert maxabs(k[..., kv], g["k_cache_l%d" % li]) < FP32_TOL and maxabs(v[..., kv], g["v_cache_l%d" % li]) < FP32_TOL
         assert maxabs(eng.export_adapter_cache(int(ids[0])), g["adapter_cache"]) < FP32_TOL
     finally:
         eng.free(ids)
 
 
 def test_shipped_two_sessions_past_saturation_fp32(golden, shipped32):
+    """Against the reference on the seeded sample of feature columns the golden keeps, and against the oracle on every
+    column."""
     cfg, eng = shipped32
     g = golden("shipped_b2")
+    asd = make_adapter_state(cfg, 0)
+    orc = O.EncoderOracle(cfg, make_encoder_state(cfg, 0))
+    buf, cache, pe = orc.new_buffer(), None, 0
     ids = eng.alloc(2)
     try:
         for i in range(20):
-            enc, y = eng.encode_stream(ids, torch.from_numpy(g["feats"][i]))
-            assert maxabs(enc.cpu(), g["enc_out"][i]) < FP32_TOL, i
-            assert maxabs(y.cpu(), g["adapter_out"][i]) < FP32_TOL, i
+            x = torch.from_numpy(g["feats"][i])
+            enc, y = eng.encode_stream(ids, x)
+            eo, buf, pe = orc.infer(x, buf, pe)
+            yo, _, cache = O.adapter_forward(cfg, asd, eo, torch.ones(2, 1, 4, dtype=torch.bool), cache)
+            assert maxabs(enc.cpu(), eo) < FP32_TOL and maxabs(y.cpu(), yo) < FP32_TOL, i
+            assert maxabs(enc.cpu()[..., g["enc_cols"]], g["enc_out"][i]) < FP32_TOL, i
+            assert maxabs(y.cpu()[..., g["adp_cols"]], g["adapter_out"][i]) < FP32_TOL, i
         k, _ = eng.export_kv(int(ids[1]), 23)
-        assert maxabs(k, g["k_cache_l23"][1:2]) < FP32_TOL
+        assert maxabs(k, buf[23][0][1:2]) < FP32_TOL
+        assert maxabs(k[..., g["kv_cols"]], g["k_cache_l23"][1:2]) < FP32_TOL
     finally:
         eng.free(ids)
 
@@ -433,7 +448,8 @@ def test_shipped_stream_bf16(golden, shipped16):
             eo, buf, pe = orc.infer(x, buf, pe)
             yo, _, cache = O.adapter_forward(cfg, asd, eo, torch.ones(2, 1, 4, dtype=torch.bool), cache)
             we, wy = max(we, maxabs(enc.cpu(), eo)), max(wy, maxabs(y.cpu(), yo))
-            fe, fy = max(fe, maxabs(enc.cpu(), g["enc_out"][i])), max(fy, maxabs(y.cpu(), g["adapter_out"][i]))
+            fe = max(fe, maxabs(enc.cpu()[..., g["enc_cols"]], g["enc_out"][i]))
+            fy = max(fy, maxabs(y.cpu()[..., g["adp_cols"]], g["adapter_out"][i]))
         print("bf16 max-abs vs oracle on bf16 weights: encoder %.4g adapter %.4g; vs fp32 reference: %.4g / %.4g "
               "(reference autocast floor %.4g / %.4g)" % (we, wy, fe, fy, float(floor["ref_autocast_vs_fp32_encoder"]),
                                                           float(floor["ref_autocast_vs_fp32_adapter"])))
@@ -818,7 +834,7 @@ def test_stack_kernel_vs_oracle_one_session(shipped16):
         eng.free(ids)
 
 
-def test_stack_kernel_tiny_rows_and_frames():
+def test_stack_kernel_tiny_rows_and_frames(golden):
     """Toy widths (D = 128, FF = 256, 2 heads: CTAs with zero, one or two weight rows per phase), 12 and 16 token rows
     (two activation rows per warp pair, FFN2 activations in K chunks) and 7 encoder frames per call (fork frontend)."""
     cfg, eng = make_engine("tiny", 3, dtype=torch.bfloat16, max_sessions=16)
@@ -837,7 +853,7 @@ def test_stack_kernel_tiny_rows_and_frames():
             assert eng.get_option("stack_launches") - l0 == 20
             eng.free(ia)
             eng.free(ib)
-        golden7 = np.load(os.path.join(os.path.dirname(__file__), "golden", "tiny.npz"))
+        golden7 = golden("tiny")
         ia, ib = eng.alloc(2), eng.alloc(2)
         l0 = eng.get_option("stack_launches")
         for i in range(12):

@@ -109,9 +109,9 @@ def test_tiny_stream(golden, tiny):
     assert np.abs(eo - g["stream_enc_out"]).max() < FP32_TOL
     assert np.abs(y - g["stream_adapter_out"]).max() < FP32_TOL
     assert pes == g["stream_pe_index"].tolist()
-    for li in (0, 1):
-        assert np.abs(buf[li][0].numpy() - g["stream_k_cache_l%d" % li]).max() < FP32_TOL
-        assert np.abs(buf[li][1].numpy() - g["stream_v_cache_l%d" % li]).max() < FP32_TOL
+    for li in (0, 1):                                                # the golden keeps a sample of the head dimension
+        assert np.abs(buf[li][0].numpy()[..., g["kv_cols"]] - g["stream_k_cache_l%d" % li]).max() < FP32_TOL
+        assert np.abs(buf[li][1].numpy()[..., g["kv_cols"]] - g["stream_v_cache_l%d" % li]).max() < FP32_TOL
     assert buf[0][0].shape[2] == cfg.kv_window
     assert np.abs(cache[0].numpy() - g["stream_adapter_cache"]).max() < FP32_TOL
 
@@ -212,7 +212,8 @@ def shipped():
 
 
 def test_shipped_question_stream(golden, shipped):
-    """BASELINE.json config 1: question.wav, 13 chunks, 1 session, fp32."""
+    """BASELINE.json config 1: question.wav, 13 chunks, 1 session, fp32 (the golden keeps a seeded sample of the
+    feature columns of each output)."""
     cfg, esd, asd = shipped
     g = golden("shipped_question")
     sess = O.StreamSession(cfg, esd, asd)
@@ -220,11 +221,11 @@ def test_shipped_question_stream(golden, shipped):
     for i in range(13):
         feats, eo, y = sess.step_pcm(torch.from_numpy(pcm[i * 2560:(i + 1) * 2560]))
         assert rel_err(feats.numpy(), g["feats"][i]) < 1e-5
-        assert np.abs(eo.numpy() - g["enc_out"][i]).max() < FP32_TOL, i
-        assert np.abs(y.numpy() - g["adapter_out"][i]).max() < FP32_TOL, i
+        assert np.abs(eo.numpy()[..., g["enc_cols"]] - g["enc_out"][i]).max() < FP32_TOL, i
+        assert np.abs(y.numpy()[..., g["adp_cols"]] - g["adapter_out"][i]).max() < FP32_TOL, i
         assert sess.pe_index == int(g["pe_index"][i])
     for li in (0, 23):
-        assert np.abs(sess.buffer[li][0].numpy() - g["k_cache_l%d" % li]).max() < FP32_TOL
+        assert np.abs(sess.buffer[li][0].numpy()[..., g["kv_cols"]] - g["k_cache_l%d" % li]).max() < FP32_TOL
     assert np.abs(sess.cache[0].numpy() - g["adapter_cache"]).max() < FP32_TOL
 
 

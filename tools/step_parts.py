@@ -1,5 +1,5 @@
 import os, sys, torch
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from freeze_omni_b200.config import load_path_config
 from freeze_omni_b200.engine import Engine
 from freeze_omni_b200.weights import make_adapter_state, make_encoder_state
