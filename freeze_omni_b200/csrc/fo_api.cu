@@ -164,6 +164,9 @@ struct fo_ctx {
         int32_t* row_start = nullptr;
     } armed;
     uint8_t* onset_dev = nullptr;
+    // adapter pass of a k-chunk call (adapter_chunks): its rows are (sessions, kk, t_out); row c of chunk jj of session b goes
+    // to output block b*k + j0 + jj.  The default is the plain layout of a single-chunk call.
+    struct ChunkRows { int k = 1, kk = 1, j0 = 0; } ad_rows;
     int groups = 1;                           // session groups whose layer kernels run on parallel streams
     cudaStream_t grp_stream[MAX_GROUPS] = {nullptr};
     cudaEvent_t ev_fork = nullptr, ev_join[MAX_GROUPS] = {nullptr};
@@ -196,7 +199,7 @@ struct fo_ctx {
 namespace {
 
 enum { WS_FEATS = 0, WS_C1, WS_C2, WS_XSUB, WS_EMB, WS_X, WS_H, WS_QKV, WS_ATT, WS_FFH, WS_ENC, WS_XIN, WS_ACONV, WS_AH,
-       WS_Y, WS_MASK2, WS_ILENS, WS_ILENS2, WS_AMASK, WS_PCM, WS_TMP0, WS_TMP1, WS_TMP2, WS_TMP3, WS_Q32, WS_HC, WS_PART, WS_PCM2, WS_ENC2, WS_Y2, WS_AC1, WS_XIN2, WS_TMP4, WS_TMP5, WS_HP, WS_FP, WS_COUNT };
+       WS_Y, WS_MASK2, WS_ILENS, WS_ILENS2, WS_AMASK, WS_PCM, WS_TMP0, WS_TMP1, WS_TMP2, WS_TMP3, WS_Q32, WS_HC, WS_PART, WS_PCM2, WS_ENC2, WS_Y2, WS_AC1, WS_XIN2, WS_TMP4, WS_TMP5, WS_HP, WS_FP, WS_ENCJ, WS_COUNT };
 
 int dev_alloc(fo_ctx* c, void** p, size_t bytes) {
     *p = nullptr;
@@ -271,7 +274,7 @@ int check_ids(fo_ctx* c, const int32_t* ids, int n) {
     return 0;
 }
 
-int upload_ids(fo_ctx* c, const int32_t* ids, int n, cudaStream_t st, const uint8_t* onset = nullptr) {
+int upload_ids(fo_ctx* c, const int32_t* ids, int n, cudaStream_t st, const uint8_t* onset = nullptr, int n_onset = 0) {
     // the same sessions as in the previous step (the steady state of a server loop): the device copy is still valid
     if (!onset && st == c->ids_last_stream && (int)c->ids_last.size() == n && memcmp(c->ids_last.data(), ids, sizeof(int32_t) * n) == 0) return 0;
     c->ids_last.assign(ids, ids + n);
@@ -283,8 +286,8 @@ int upload_ids(fo_ctx* c, const int32_t* ids, int n, cudaStream_t st, const uint
     FO_CUDA(cudaMemcpyAsync(c->ids_dev, c->ids_host[k], sizeof(int32_t) * n, cudaMemcpyHostToDevice, st));
     if (onset) {                                 // second half of the pinned staging slot: the hand-off's per-session onset flags
         uint8_t* oh = reinterpret_cast<uint8_t*>(c->ids_host[k] + c->cfg.max_sessions);
-        memcpy(oh, onset, n);
-        FO_CUDA(cudaMemcpyAsync(c->onset_dev, oh, n, cudaMemcpyHostToDevice, st));
+        memcpy(oh, onset, n_onset);
+        FO_CUDA(cudaMemcpyAsync(c->onset_dev, oh, n_onset, cudaMemcpyHostToDevice, st));
     }
     FO_CUDA(cudaEventRecord(c->ids_event[k], st));
     return 0;
@@ -628,6 +631,15 @@ inline int ad_frames(const fo_ctx* c, int T) {
     return (T + c->KA - 1 - c->KA) / 2 + 1;
 }
 
+// RowMap of the adapter's last GEMM onto output blocks of `pitch` rows (fo_ctx::ad_rows); pass_rows = output rows per session
+// of this pass (kk chunks); *base_row = row of the first block
+inline void chunk_rowmap(const fo_ctx* c, int pass_rows, long long pitch, RowMap* rm, long long* base_row) {
+    const fo_ctx::ChunkRows& cr = c->ad_rows;
+    const int t_out = pass_rows / cr.kk;
+    rm->p1 = cr.kk * t_out; rm->p0 = t_out; rm->v1 = cr.kk; rm->v0 = t_out; rm->q1 = (int)(cr.k * pitch); rm->q0 = (int)pitch;
+    *base_row = (long long)cr.j0 * pitch;
+}
+
 // ---- adapter program on device buffers -----------------------------------------------------------
 // enc (B, T, D) fp32 -> y (B, t_out, E) fp32.  Slot-resident cache when ids != null.
 template <typename TA>
@@ -679,10 +691,14 @@ int adapter_program(fo_ctx* c, const float* enc, const uint8_t* mask, int B, int
         e3.c_f32 = y;
         e3.ldc = E;
         RowMap rm3;
+        long long base;
         if (c->handoff && ids_dev) {
+            chunk_rowmap(c, t_out, c->handoff_rows, &rm3, &base);
             e3.c_f32 = nullptr;
-            e3.c_act = reinterpret_cast<TA*>(c->handoff) + c->handoff_off * E;
-            rm3.p1 = t_out; rm3.p0 = t_out; rm3.v1 = 1; rm3.v0 = t_out; rm3.q1 = (int)c->handoff_rows; rm3.q0 = 0;
+            e3.c_act = reinterpret_cast<TA*>(c->handoff) + (c->handoff_off + base) * E;
+        } else if (c->ad_rows.kk != c->ad_rows.k) {              // one chunk of a chunk-by-chunk pass
+            chunk_rowmap(c, t_out, t_out, &rm3, &base);
+            e3.c_f32 = y + base * E;
         }
         if (!(c->debug_skip & 16))
             FO_TRY(gemm<TA>(c, reinterpret_cast<const TA*>(ah), plain_rows(4 * D, Mo), c->ad_proj_w, Mo, E, 4 * D, e3, rm3, st));
@@ -706,9 +722,10 @@ int adapter_program(fo_ctx* c, const float* enc, const uint8_t* mask, int B, int
         e.ldc = E;
         RowMap rml;
         if (c->handoff && ids_dev) {
+            long long base;
+            chunk_rowmap(c, T, c->handoff_rows, &rml, &base);
             e.c_f32 = nullptr;
-            e.c_act = reinterpret_cast<TA*>(c->handoff) + c->handoff_off * E;
-            rml.p1 = T; rml.p0 = T; rml.v1 = 1; rml.v0 = T; rml.q1 = (int)c->handoff_rows; rml.q0 = 0;
+            e.c_act = reinterpret_cast<TA*>(c->handoff) + (c->handoff_off + base) * E;
         }
         if (!(c->debug_skip & 16)) FO_TRY(gemm<TA>(c, a_in, plain_rows(D, M), c->ad_proj_w, M, E, D, e, rml, st));
         return 0;
@@ -737,12 +754,16 @@ int adapter_program(fo_ctx* c, const float* enc, const uint8_t* mask, int B, int
     e2.c_f32 = y;
     e2.ldc = E;
     RowMap rm2;
+    long long base;
     if (c->handoff && ids_dev) {
         // LLM hand-off (audioLLM.py:404-411): rows of session b go, as fp16, to row  b * rows_per_session + row_offset + j  of
         // the caller's inputs_embeds buffer, straight from the projection's epilogue (no fp32 copy, no cat, no .half())
+        chunk_rowmap(c, t_out, c->handoff_rows, &rm2, &base);
         e2.c_f32 = nullptr;
-        e2.c_act = reinterpret_cast<TA*>(c->handoff) + c->handoff_off * E;
-        rm2.p1 = t_out; rm2.p0 = t_out; rm2.v1 = 1; rm2.v0 = t_out; rm2.q1 = (int)c->handoff_rows; rm2.q0 = 0;
+        e2.c_act = reinterpret_cast<TA*>(c->handoff) + (c->handoff_off + base) * E;
+    } else if (c->ad_rows.kk != c->ad_rows.k) {                  // one chunk of a chunk-by-chunk pass
+        chunk_rowmap(c, t_out, t_out, &rm2, &base);
+        e2.c_f32 = y + base * E;
     }
     if (!(c->debug_skip & 16))
         FO_TRY(gemm<TA>(c, reinterpret_cast<const TA*>(ah), plain_rows(2 * D, Mo), c->ad_proj_w, Mo, E, 2 * D, e2, rm2, st));
@@ -1043,17 +1064,48 @@ int stack_program(fo_ctx* c, int n, int t, float* x, void* qkv, float* q32, void
     return 0;
 }
 
+// The adapter of a k-chunk call (rows (session, chunk, frame) in enc), equal to k sequential single-chunk calls per session.
 template <typename TA>
-int stream_program(fo_ctx* c, int n, const float* feats, int t_in, float* enc_out_dev, float* y_dev, cudaStream_t st) {
+int adapter_chunks(fo_ctx* c, const float* enc, int n, int k, int t, float* y, cudaStream_t st) {
+    struct Reset { fo_ctx* c; ~Reset() { c->ad_rows = fo_ctx::ChunkRows(); } } reset{c};
+    // LinearAdapter works per row and CNNAdapter starts from zero left context on every call (adapter.py:41-52):
+    // n*k independent blocks of t frames
+    if (c->cfg.adapter_type != 0) return adapter_program<TA>(c, enc, nullptr, n * k, t, c->ids_dev, nullptr, nullptr, y, st);
+    if (t % 2 == 0) {
+        // CNNSubsampling with even t: every chunk brings an even number of frames to the stride-2 conv, so one pass over a
+        // session's k*t frames with the carried cache gives the k sequential outputs and leaves the same cache
+        c->ad_rows.k = c->ad_rows.kk = k;
+        return adapter_program<TA>(c, enc, nullptr, n, k * t, c->ids_dev, nullptr, nullptr, y, st);
+    }
+    // odd t: the output phase of the stride-2 conv shifts between chunks (a joint pass yields other frames, and fewer), so
+    // the chunks run one by one, flipping the live half of the double-buffered cache in between as a session advance does
+    const size_t row = (size_t)t * c->D * sizeof(float);
+    void* ej;
+    FO_TRY(ws_ensure(c, WS_ENCJ, (size_t)n * row, &ej));
+    c->ad_rows.k = k;
+    c->ad_rows.kk = 1;
+    for (int j = 0; j < k; ++j) {
+        FO_CUDA(cudaMemcpy2DAsync(ej, row, reinterpret_cast<const char*>(enc) + j * row, (size_t)k * row, row, n, cudaMemcpyDeviceToDevice, st));
+        c->ad_rows.j0 = j;
+        FO_TRY(adapter_program<TA>(c, reinterpret_cast<const float*>(ej), nullptr, n, t, c->ids_dev, nullptr, nullptr, y, st));
+        if (j + 1 < k) FO_TRY(advance_sessions(c->ids_dev, n, 0, 0, 1, nullptr, nullptr, c->ad_valid, st));
+    }
+    return 0;
+}
+
+// k > 1: k consecutive chunks per session (fo_encode_stream_chunks); rows are ordered (session, chunk, frame), so every
+// per-session kernel sees a session's k*t new rows as one run
+template <typename TA>
+int stream_program(fo_ctx* c, int n, int k, const float* feats, int t_in, float* enc_out_dev, float* y_dev, cudaStream_t st) {
     const int D = c->D, FF = c->FF, H = c->H;
-    const int T1 = (t_in - 1) / 2, t = (T1 - 1) / 2, M = n * t;
+    const int T1 = (t_in - 1) / 2, t = (T1 - 1) / 2, kt = k * t, M = n * kt;
     float* x;
     if (c->step_part == 2) {
         void* xp;
         FO_TRY(ws_ensure(c, WS_X, (size_t)M * D * sizeof(float), &xp));
         x = reinterpret_cast<float*>(xp);
     } else {
-        FO_TRY(subsample_program<TA>(c, feats, n, t_in, &x, st));
+        FO_TRY(subsample_program<TA>(c, feats, n * k, t_in, &x, st));   // every block brings its own context frames
         if (c->step_part == 1) return 0;
     }
     void *h, *qkv, *att, *ffh;
@@ -1070,7 +1122,7 @@ int stream_program(fo_ctx* c, int n, const float* feats, int t_in, float* enc_ou
     // two groups' kernels overlap each other's pipeline fill, epilogue and launch gaps.  Rows of one group are
     // contiguous, so the groups just take slices of the same workspaces.
     int stacked = 1;
-    if (sizeof(TA) == 2) {
+    if (sizeof(TA) == 2 && k == 1) {                        // the stack kernel's attention is single-chunk
         stacked = stack_program(c, n, t, x, qkv, q32, att, ffh, enc_out_dev, st);
         if (stacked < 0) return stacked;
     }
@@ -1093,8 +1145,8 @@ int stream_program(fo_ctx* c, int n, const float* feats, int t_in, float* enc_ou
             if (ng <= 0) continue;
             cudaStream_t sg = g == 0 ? st : c->grp_stream[g];
             c->tc_cur = &c->tc_wsg[g];
-            const long long r0 = (long long)s0 * t;
-            const int Mg = ng * t;
+            const long long r0 = (long long)s0 * kt;
+            const int Mg = ng * kt;
             AttnStream a;
             a.ids = c->ids_dev + s0;
             a.n_frames = c->n_frames;
@@ -1102,6 +1154,8 @@ int stream_program(fo_ctx* c, int n, const float* feats, int t_in, float* enc_ou
             a.n = ng; a.t = t; a.H = H; a.ring_cap = c->ring_cap; a.window = c->window; a.full_chunk = c->full_chunk;
             a.pe_wrap = c->pe_wrap; a.pos_rows = c->pos_rows;
             a.ring_slot_stride = 2LL * H * c->ring_cap * 64;
+            a.chunks = k;
+            a.chunk_size = c->cfg.chunk_size;
             TA* hg = reinterpret_cast<TA*>(h) + r0 * D;
             TA* qkvg = reinterpret_cast<TA*>(qkv) + r0 * 3 * D;
             TA* attg = reinterpret_cast<TA*>(att) + r0 * D;
@@ -1123,7 +1177,8 @@ int stream_program(fo_ctx* c, int n, const float* feats, int t_in, float* enc_ou
                 a.prefetch = pf1(w.w1, (long long)D * FF * c->esz);                       // attention runs: FFN1's weights
             }
             int qkv_splits = 0;
-            if (r == 0) r = layer_pre<TA>(c, w, Mg, hg, qkvg, q32g, pfq, sg, &qkv_splits);
+            // the multi-chunk attention reads finished QKV rows: no split-K reduction deferred to it
+            if (r == 0) r = layer_pre<TA>(c, w, Mg, hg, qkvg, q32g, pfq, sg, k == 1 ? &qkv_splits : nullptr);
             if (qkv_splits > 0) {
                 a.part = c->tc_cur->partial;
                 a.part_bias = w.bqkv;
@@ -1136,7 +1191,7 @@ int stream_program(fo_ctx* c, int n, const float* feats, int t_in, float* enc_ou
             NextNorm nn{last ? c->after_g : c->layers[l + 1].ln1g, last ? c->after_b : c->layers[l + 1].ln1b,
                         last ? enc_out_dev + r0 * D : nullptr};
             FfnConv fc;
-            fc.B = ng; fc.T = t; fc.ids = c->ids_dev + s0; fc.layer = l;
+            fc.B = ng; fc.T = kt; fc.ids = c->ids_dev + s0; fc.layer = l;   // Conv1dLinear: one pass over k*t rows with the carry
             fc.hc = hc ? reinterpret_cast<TA*>(hc) + r0 * D : nullptr;
             if (r == 0) r = layer_post<TA>(c, w, xg, Mg, attg, hg, ffhg, nn, last ? nullptr : c->layers[l + 1].wqkv, fc, sg);
             if (r != 0) { c->tc_cur = &c->tc_wsg[0]; return r; }
@@ -1150,10 +1205,12 @@ int stream_program(fo_ctx* c, int n, const float* feats, int t_in, float* enc_ou
         }
     }
     const bool run_adapter = c->cfg.has_adapter && (y_dev || c->handoff);
-    if (run_adapter)
-        FO_TRY(adapter_program<TA>(c, enc_out_dev, nullptr, n, t, c->ids_dev, nullptr, nullptr, y_dev, st));
+    if (run_adapter) {
+        if (k == 1) FO_TRY(adapter_program<TA>(c, enc_out_dev, nullptr, n, t, c->ids_dev, nullptr, nullptr, y_dev, st));
+        else FO_TRY(adapter_chunks<TA>(c, enc_out_dev, n, k, t, y_dev, st));
+    }
     FO_TRY(advance_sessions(c->ids_dev, n, t, c->cfg.chunk_size, c->pe_wrap, c->n_frames, c->pe_index,
-                            (run_adapter && c->cfg.adapter_type == 0) ? c->ad_valid : nullptr, st));
+                            (run_adapter && c->cfg.adapter_type == 0) ? c->ad_valid : nullptr, st, k));
     return 0;
 }
 
@@ -1295,12 +1352,12 @@ int fo_create(const fo_config* cfg, int device, int dtype, fo_ctx** out) {
             c->ad_cache2 = (float*)p;
         }
         if (!r) { r = dev_alloc(c, &p, S * sizeof(int32_t)); c->ids_dev = (int32_t*)p; }
-        if (!r) { r = dev_alloc(c, &p, S); c->onset_dev = (uint8_t*)p; }
+        if (!r) { r = dev_alloc(c, &p, (size_t)S * STREAM_CHUNKS_MAX_KEYS); c->onset_dev = (uint8_t*)p; }   // one flag per block, <= 128 blocks per session
         if (!r) { r = dev_alloc(c, &p, sizeof(unsigned long long)); c->sat_counter = (unsigned long long*)p; }
         if (!r && cudaMemset(c->sat_counter, 0, sizeof(unsigned long long)) != cudaSuccess) r = FO_ERR_CUDA;
     }
     for (int k = 0; k < fo_ctx::NSTAGE && !r; ++k) {
-        if (cudaMallocHost((void**)&c->ids_host[k], 2 * S * sizeof(int32_t)) != cudaSuccess ||
+        if (cudaMallocHost((void**)&c->ids_host[k], S * sizeof(int32_t) + (size_t)S * STREAM_CHUNKS_MAX_KEYS) != cudaSuccess ||
             cudaEventCreateWithFlags(&c->ids_event[k], cudaEventDisableTiming) != cudaSuccess) {
             set_error("fo_create: pinned staging allocation failed");
             r = FO_ERR_NOMEM;
@@ -1668,6 +1725,7 @@ int fo_fbank_offline(fo_ctx* c, const void* pcm, int pcm_dtype, int B, int64_t n
 // captures.  A workspace that moves (ws_epoch) invalidates the graphs.
 struct StepArgs {
     int n, t_in;
+    int k;                     // consecutive chunks per session (fo_encode_stream_chunks; 1 otherwise)
     bool with_fbank, want_y;
     int pcm_is_i16;
     float scale;
@@ -1681,17 +1739,18 @@ static int step_body(fo_ctx* c, const StepArgs& a, cudaStream_t st) {
     void *dfeats, *denc, *dy = nullptr;
     const int T1 = (a.t_in - 1) / 2, t = (T1 - 1) / 2;
     const int km1 = c->KA - 1, t_out = ad_frames(c, t);
-    FO_TRY(ws_ensure(c, WS_FEATS, (size_t)a.n * a.t_in * c->F * sizeof(float), &dfeats));
-    FO_TRY(ws_ensure(c, ws_enc(a.buf), (size_t)a.n * t * c->D * sizeof(float), &denc));
-    if (a.want_y) FO_TRY(ws_ensure(c, ws_y(a.buf), (size_t)a.n * t_out * c->E * sizeof(float), &dy));
+    const size_t blocks = (size_t)a.n * a.k;
+    FO_TRY(ws_ensure(c, WS_FEATS, blocks * a.t_in * c->F * sizeof(float), &dfeats));
+    FO_TRY(ws_ensure(c, ws_enc(a.buf), blocks * t * c->D * sizeof(float), &denc));
+    if (a.want_y) FO_TRY(ws_ensure(c, ws_y(a.buf), blocks * t_out * c->E * sizeof(float), &dy));
     if (a.with_fbank && c->step_part != 2) {
         void* dp;
         FO_TRY(ws_ensure(c, ws_pcm(a.buf), (size_t)a.n * c->chunk_samples * 4, &dp));
         FO_TRY(fbank_stream(fbank_params(c), c->ids_dev, a.n, dp, a.pcm_is_i16, a.scale, c->cfg.frames_per_chunk,
                             c->cfg.context_frames, c->samples, c->feat_ring, (float*)dfeats, st));
     }
-    return c->dtype == FO_BF16 ? stream_program<act16>(c, a.n, (const float*)dfeats, a.t_in, (float*)denc, (float*)dy, st)
-                               : stream_program<float>(c, a.n, (const float*)dfeats, a.t_in, (float*)denc, (float*)dy, st);
+    return c->dtype == FO_BF16 ? stream_program<act16>(c, a.n, a.k, (const float*)dfeats, a.t_in, (float*)denc, (float*)dy, st)
+                               : stream_program<float>(c, a.n, a.k, (const float*)dfeats, a.t_in, (float*)denc, (float*)dy, st);
 }
 
 static int run_step(fo_ctx* c, const StepArgs& a, cudaStream_t st) {
@@ -1705,7 +1764,7 @@ static int run_step(fo_ctx* c, const StepArgs& a, cudaStream_t st) {
     char key[192];
     uint32_t sbits;
     memcpy(&sbits, &a.scale, 4);
-    snprintf(key, sizeof(key), "%d/%p/%lld/%lld/%d/%d/%d/%d/%d/%08x/%d/%d/%d/%d-%d", a.buf, c->handoff, c->handoff_rows, c->handoff_off, a.n, a.t_in, (int)a.with_fbank, (int)a.want_y, a.pcm_is_i16, sbits,
+    snprintf(key, sizeof(key), "%d/%p/%lld/%lld/%d/%d/%d/%d/%d/%d/%08x/%d/%d/%d/%d-%d", a.buf, c->handoff, c->handoff_rows, c->handoff_off, a.n, a.k, a.t_in, (int)a.with_fbank, (int)a.want_y, a.pcm_is_i16, sbits,
              c->gemm_backend, c->groups, (((c->debug_skip * 2 + c->defer_reduce) * 2 + c->fuse_ln) * 4 + c->use_prefetch) * 64 + c->stack_rows,
              ((c->use_prefetch & 2) ? c->pf_slot_lo * 2 + g_use_pdl : g_use_pdl), (c->use_prefetch & 2) ? c->pf_slot_hi : 0);   // the prefetch range is baked into the graph
     if (c->graphs.size() > 256 && c->graphs.find(key) == c->graphs.end()) {
@@ -1751,7 +1810,8 @@ static int run_step(fo_ctx* c, const StepArgs& a, cudaStream_t st) {
 }
 
 // copies between the caller's buffers and the context's staging buffers, then the step
-static int stream_common(fo_ctx* c, const int32_t* ids, int n, const void* pcm, int pcm_dtype, float scale,
+// k > 1 (fo_encode_stream_chunks, feats only): k consecutive chunk blocks per session, feats (n, k, t_in, F)
+static int stream_common(fo_ctx* c, const int32_t* ids, int n, int k, const void* pcm, int pcm_dtype, float scale,
                          const float* feats, int t_in, float* enc_out, float* adapter_out, cudaStream_t st) {
     const int T1 = (t_in - 1) / 2, t = (T1 - 1) / 2;
     FO_CHECK(t >= 1 && t <= c->max_t, "streaming call of %d feature frames gives %d encoder frames; context allows 1..%d",
@@ -1760,8 +1820,8 @@ static int stream_common(fo_ctx* c, const int32_t* ids, int n, const void* pcm, 
     FO_CHECK(!c->KM, "this context's positionwise layer is MultiLayeredConv1d, which has no streaming form (the reference module has no infer(), "
                      "models/encoder/attention.py:145-196); use fo_encode_offline");
     const int km1 = c->KA - 1, t_out = ad_frames(c, t);
-    const size_t enc_bytes = (size_t)n * t * c->D * sizeof(float);
-    const size_t y_bytes = (size_t)n * t_out * c->E * sizeof(float);
+    const size_t enc_bytes = (size_t)n * k * t * c->D * sizeof(float);
+    const size_t y_bytes = (size_t)n * k * t_out * c->E * sizeof(float);
     if (c->copy_stream && c->async_ticket > 0) {
         // a synchronous call after pipelined ones reuses staging set 0 (and the shared intermediates): let the read-backs of
         // the steps still in flight on the copy stream finish first
@@ -1771,7 +1831,8 @@ static int stream_common(fo_ctx* c, const int32_t* ids, int n, const void* pcm, 
     fo_ctx::Armed armed = c->armed;              // consumed by this call, whatever its outcome
     c->armed.on = false;
     if (armed.on) {
-        FO_CHECK(armed.n == n, "fo_handoff_arm was armed for %d sessions, this call advances %d", armed.n, n);
+        FO_CHECK(armed.n == n * k, "fo_handoff_arm was armed for %d blocks, this call advances %d sessions x %d chunks", armed.n, n, k);
+        FO_CHECK(armed.rows * k < (1LL << 31), "hand-off: %d chunks of %lld rows per session are too many rows", k, armed.rows);
         FO_CHECK(!adapter_out && !c->handoff, "an armed hand-off replaces adapter_out: pass NULL");
         FO_CHECK(armed.rows >= armed.prefix + t_out, "hand-off: %d adapter rows behind a %lld-row prefix do not fit %lld rows per session",
                  t_out, armed.prefix, armed.rows);
@@ -1780,17 +1841,17 @@ static int stream_common(fo_ctx* c, const int32_t* ids, int n, const void* pcm, 
         c->handoff_off = armed.prefix;
     }
     struct HandoffReset { fo_ctx* c; bool on; ~HandoffReset() { if (on) { c->handoff = nullptr; c->handoff_rows = c->handoff_off = 0; } } } hreset{c, armed.on};
-    FO_TRY(upload_ids(c, ids, n, st, armed.on ? armed.onset.data() : nullptr));
+    FO_TRY(upload_ids(c, ids, n, st, armed.on ? armed.onset.data() : nullptr, n * k));
     c->pf_slot_lo = c->pf_slot_hi = ids[0];
     for (int i = 1; i < n; ++i) { c->pf_slot_lo = std::min(c->pf_slot_lo, (int)ids[i]); c->pf_slot_hi = std::max(c->pf_slot_hi, (int)ids[i]); }
-    StepArgs a{n, t_in, pcm != nullptr, adapter_out != nullptr, pcm_dtype == FO_I16, scale, 0};
+    StepArgs a{n, t_in, k, pcm != nullptr, adapter_out != nullptr, pcm_dtype == FO_I16, scale, 0};
     void* stage;
     if (pcm) {
         const size_t in_bytes = (size_t)n * c->chunk_samples * (pcm_dtype == FO_I16 ? 2 : 4);
         FO_TRY(ws_ensure(c, WS_PCM, (size_t)n * c->chunk_samples * 4, &stage));
         FO_CUDA(cudaMemcpyAsync(stage, pcm, in_bytes, cudaMemcpyDefault, st));
     } else if (feats) {
-        const size_t in_bytes = (size_t)n * t_in * c->F * sizeof(float);
+        const size_t in_bytes = (size_t)n * k * t_in * c->F * sizeof(float);
         FO_TRY(ws_ensure(c, WS_FEATS, in_bytes, &stage));
         FO_CUDA(cudaMemcpyAsync(stage, feats, in_bytes, cudaMemcpyDefault, st));
     } else {
@@ -1802,13 +1863,13 @@ static int stream_common(fo_ctx* c, const int32_t* ids, int n, const void* pcm, 
     }
     FO_TRY(run_step(c, a, st));
     if (armed.on && armed.attn_mask)
-        FO_TRY(handoff_mask(c->onset_dev, armed.prefix_mask, n, (int)armed.prefix, t_out, (int)armed.rows, armed.attn_mask, armed.row_start, st));
+        FO_TRY(handoff_mask(c->onset_dev, armed.prefix_mask, n * k, (int)armed.prefix, t_out, (int)armed.rows, armed.attn_mask, armed.row_start, st));
     if (enc_out) FO_CUDA(cudaMemcpyAsync(enc_out, c->ws[WS_ENC].p, enc_bytes, cudaMemcpyDefault, st));
     if (adapter_out) FO_CUDA(cudaMemcpyAsync(adapter_out, c->ws[WS_Y].p, y_bytes, cudaMemcpyDefault, st));
     if (!c->ev_sync) FO_CUDA(cudaEventCreateWithFlags(&c->ev_sync, cudaEventDisableTiming));
     FO_CUDA(cudaEventRecord(c->ev_sync, st));
     c->stats.stream_steps += 1;
-    c->stats.session_chunks += n;
+    c->stats.session_chunks += (long long)n * k;
     return 0;
 }
 
@@ -1819,14 +1880,33 @@ int fo_encode_stream(fo_ctx* c, const int32_t* ids, int n, const float* feats, i
     FO_CUDA(cudaSetDevice(c->device));
     if (feats) FO_CHECK(t_in >= 7, "fo_encode_stream: need at least 7 feature frames");
     else t_in = c->cfg.context_frames + c->cfg.frames_per_chunk;
-    return stream_common(c, ids, n, nullptr, FO_F32, 1.0f, feats, t_in, enc_out, adapter_out, (cudaStream_t)stream);
+    return stream_common(c, ids, n, 1, nullptr, FO_F32, 1.0f, feats, t_in, enc_out, adapter_out, (cudaStream_t)stream);
+}
+
+int fo_encode_stream_chunks(fo_ctx* c, const int32_t* ids, int n, int k, const float* feats, int t_in, float* enc_out,
+                            float* adapter_out, void* stream) {
+    FO_CHECK(c && c->finalized && c->cfg.has_encoder, "fo_encode_stream_chunks: context has no finalized encoder");
+    FO_CHECK(feats, "fo_encode_stream_chunks: feats must not be NULL (the feature ring holds one block per session)");
+    FO_CHECK(k >= 1, "fo_encode_stream_chunks: k must be >= 1");
+    FO_CHECK(t_in >= 7, "fo_encode_stream_chunks: need at least 7 feature frames per chunk");
+    FO_TRY(check_ids(c, ids, n));
+    const int t = ((t_in - 1) / 2 - 1) / 2;
+    if (k > 1 && t >= 1 && t <= c->max_t) {
+        const int kmax = std::max(1, (STREAM_CHUNKS_MAX_KEYS - c->window) / t);
+        FO_CHECK(c->window + k * t <= STREAM_CHUNKS_MAX_KEYS,
+                 "fo_encode_stream_chunks: the attention window (%d frames) + %d chunks x %d frames exceeds %d keys; the largest k is %d",
+                 c->window, k, t, STREAM_CHUNKS_MAX_KEYS, kmax);
+    }
+    FO_CUDA(cudaSetDevice(c->device));
+    return stream_common(c, ids, n, k, nullptr, FO_F32, 1.0f, feats, t_in, enc_out, adapter_out, (cudaStream_t)stream);
 }
 
 int fo_handoff_arm(fo_ctx* c, int n, void* embeds_f16, int64_t rows_per_session, int64_t prefix_len, const uint8_t* onset,
                    const uint8_t* prefix_mask, uint8_t* attn_mask, int32_t* row_start) {
     FO_CHECK(c && c->finalized && c->cfg.has_encoder && c->cfg.has_adapter, "fo_handoff_arm: context needs a finalized encoder + adapter");
     FO_CHECK(c->dtype == FO_BF16, "fo_handoff_arm: the fp16 hand-off is built for bf16 contexts");
-    FO_CHECK(n > 0 && n <= c->cfg.max_sessions && embeds_f16 && onset, "fo_handoff_arm: bad argument");
+    // n blocks: one per session, or per (session, chunk) for fo_encode_stream_chunks
+    FO_CHECK(n > 0 && n <= c->cfg.max_sessions * STREAM_CHUNKS_MAX_KEYS && embeds_f16 && onset, "fo_handoff_arm: bad argument");
     FO_CHECK(prefix_len >= 0 && rows_per_session > prefix_len && rows_per_session < (1LL << 31), "fo_handoff_arm: bad row counts");
     cudaPointerAttributes pa;
     FO_CHECK(cudaPointerGetAttributes(&pa, embeds_f16) == cudaSuccess && pa.type == cudaMemoryTypeDevice && pa.device == c->device,
@@ -1864,7 +1944,7 @@ int fo_stream_step_embeds(fo_ctx* c, const int32_t* ids, int n, const void* pcm,
     c->handoff = embeds_f16;
     c->handoff_rows = rows_per_session;
     c->handoff_off = row_offset;
-    const int r = stream_common(c, ids, n, pcm, pcm_dtype, scale, nullptr, t_in, enc_out, nullptr, (cudaStream_t)stream);
+    const int r = stream_common(c, ids, n, 1, pcm, pcm_dtype, scale, nullptr, t_in, enc_out, nullptr, (cudaStream_t)stream);
     c->handoff = nullptr;
     c->handoff_rows = c->handoff_off = 0;
     return r;
@@ -1894,7 +1974,7 @@ int fo_stream_step_async(fo_ctx* c, const int32_t* ids, int n, const void* pcm, 
     FO_TRY(upload_ids(c, ids, n, st));
     c->pf_slot_lo = c->pf_slot_hi = ids[0];
     for (int i = 1; i < n; ++i) { c->pf_slot_lo = std::min(c->pf_slot_lo, (int)ids[i]); c->pf_slot_hi = std::max(c->pf_slot_hi, (int)ids[i]); }
-    StepArgs a{n, t_in, true, adapter_out != nullptr, pcm_dtype == FO_I16, scale, buf};
+    StepArgs a{n, t_in, 1, true, adapter_out != nullptr, pcm_dtype == FO_I16, scale, buf};
     // inputs: copy stream, once the step that last read this PCM buffer (two tickets ago) is done
     void* stage;
     FO_TRY(ws_ensure(c, ws_pcm(buf), (size_t)n * c->chunk_samples * 4, &stage));
@@ -1932,7 +2012,7 @@ int fo_stream_step(fo_ctx* c, const int32_t* ids, int n, const void* pcm, int pc
     FO_CHECK(pcm && (pcm_dtype == FO_F32 || pcm_dtype == FO_I16), "fo_stream_step: pcm must be FO_F32 or FO_I16");
     FO_TRY(check_ids(c, ids, n));
     FO_CUDA(cudaSetDevice(c->device));
-    return stream_common(c, ids, n, pcm, pcm_dtype, scale, nullptr, c->cfg.context_frames + c->cfg.frames_per_chunk, enc_out,
+    return stream_common(c, ids, n, 1, pcm, pcm_dtype, scale, nullptr, c->cfg.context_frames + c->cfg.frames_per_chunk, enc_out,
                          adapter_out, (cudaStream_t)stream);
 }
 

@@ -603,6 +603,321 @@ attention_stream_mma_kernel(AttnStream a, const __half* __restrict__ qkv, const 
 }
 
 // ---------------------------------------------------------------------------------------------
+// Several consecutive chunks of every session in one call (AttnStream::chunks = k, fo_encode_stream_chunks).  One CTA per
+// (session, head) stages the keys once -- the ring window of frames [first, nf) (first = nf - min(nf, window)) by bulk
+// copy, then the call's own k*t rows -- and walks the k query chunks in order.  Chunk j sees exactly what the j-th
+// sequential single-chunk call would see:
+//     nf_j = nf + j*t,  keys = frames [nf_j - min(nf_j, window), nf_j + t)   (a contiguous run of the staged rows)
+//     pe_j = pe_index stepped j times by pe = pe % wrap + chunk_size,  rel-pos rows P[max(0, pe_j % wrap - full_chunk) + m]
+// The rel-pos window moves (and may wrap) with pe_j, so it is re-staged per chunk.  The new rows go to the ring only after
+// the staged copy of the old window has landed: the ring holds window + max_t rows, fewer than the call's keys, so a later
+// chunk's rows would overwrite frames an earlier chunk still needs.  Layouts (fp16 chunk swizzle of K/V by frame and of P
+// by position, q swizzled by query row) are those of the single-chunk kernels.
+__device__ __forceinline__ int chunk_pe(int pe, int j, const AttnStream& a) {
+    for (int i = 0; i < j; ++i) pe = pe % a.pe_wrap + a.chunk_size;
+    return pe % a.pe_wrap;
+}
+
+// stage the call's new K/V rows (smem rows cl + r, frame nf + r) and, once the ring window has landed, append them to the
+// ring (only the last `cap` of them when the call brings more frames than the ring holds)
+template <typename TA, int NCH, bool SWZ>
+__device__ __forceinline__ void chunks_stage_new(const AttnStream& a, const TA* qkv, TA* Ks, TA* Vs, int b, int h, int nf, int cl,
+                                                 int kt) {
+    constexpr int EPC = 16 / sizeof(TA);
+    const int D = a.H * DK;
+    for (int i = threadIdx.x; i < kt * NCH * 2; i += ATT_THREADS) {
+        const int which = i / (kt * NCH), r = (i / NCH) % kt, c = i % NCH;
+        const int pc = SWZ ? (c ^ ((nf + r) & 7)) : c;
+        *reinterpret_cast<uint4*>((which ? Vs : Ks) + (cl + r) * DK + pc * EPC) =
+            *reinterpret_cast<const uint4*>(qkv + (long long)(b * kt + r) * 3 * D + (which + 1) * D + h * DK + c * EPC);
+    }
+}
+template <typename TA, int NCH>
+__device__ __forceinline__ void chunks_append_ring(const AttnStream& a, const TA* Ks, const TA* Vs, TA* ringK, TA* ringV, int nf,
+                                                   int cl, int kt) {
+    constexpr int EPC = 16 / sizeof(TA);
+    const int r0 = max(0, kt - a.ring_cap);
+    for (int i = threadIdx.x; i < (kt - r0) * NCH * 2; i += ATT_THREADS) {
+        const int which = i / ((kt - r0) * NCH), r = r0 + (i / NCH) % (kt - r0), c = i % NCH;
+        *reinterpret_cast<uint4*>((which ? ringV : ringK) + (long long)((nf + r) % a.ring_cap) * DK + c * EPC) =
+            *reinterpret_cast<const uint4*>((which ? Vs : Ks) + (cl + r) * DK + c * EPC);
+    }
+}
+__device__ __forceinline__ void chunks_start_ring_copy(const void* ringK, const void* ringV, void* Ks, void* Vs, int first, int cl,
+                                                       int cap, uint32_t rowb, uint64_t* bar) {
+    mbar_init(bar, 1);
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    const int p0 = first % cap;
+    const int len1 = min(cl, cap - p0), len2 = cl - len1;
+    mbar_expect_tx(bar, 2u * cl * rowb);
+    if (len1 > 0) {
+        bulk_g2s(Ks, (const char*)ringK + (long long)p0 * rowb, len1 * rowb, bar);
+        bulk_g2s(Vs, (const char*)ringV + (long long)p0 * rowb, len1 * rowb, bar);
+    }
+    if (len2 > 0) {
+        bulk_g2s((char*)Ks + len1 * rowb, ringK, len2 * rowb, bar);
+        bulk_g2s((char*)Vs + len1 * rowb, ringV, len2 * rowb, bar);
+    }
+}
+
+// fp32 (parity) form: scalar FFMA contractions as in attention_stream_kernel
+template <typename TA>
+__global__ void __launch_bounds__(ATT_THREADS)
+attention_chunks_kernel(AttnStream a, const TA* __restrict__ qkv, const float* __restrict__ q32, TA* __restrict__ ring,
+                        const TA* __restrict__ ptab_h, const float* __restrict__ pos_u, const float* __restrict__ pos_v,
+                        TA* __restrict__ out) {
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    constexpr int EPC = Chunk<TA>::EPC, NCH = Chunk<TA>::NCH;
+    FO_PDL_TRIGGER();
+    FO_PDL_WAIT();
+    const int cap = a.ring_cap, t = a.t, kt = a.chunks * t, D = a.H * DK;
+    const int rows = a.window + kt, prow = a.window + t;
+    TA* Ks = reinterpret_cast<TA*>(smem_raw);
+    TA* Vs = Ks + rows * DK;
+    TA* Ps = Vs + rows * DK;
+    float* qu = reinterpret_cast<float*>(Ps + prow * DK);
+    float* qv = qu + t * DK;
+    float* prob = qv + t * DK;                      // t x prow
+    __shared__ __align__(8) uint64_t bar;
+
+    const int b = blockIdx.x, h = blockIdx.y;
+    const int slot = a.ids[b];
+    const int nf = a.n_frames[slot];
+    const int cl = min(nf, a.window), first = nf - cl;
+    TA* ringK = ring + (long long)slot * a.ring_slot_stride + (long long)h * cap * DK;
+    TA* ringV = ringK + (long long)a.H * cap * DK;
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    if (tid == 0) chunks_start_ring_copy(ringK, ringV, Ks, Vs, first, cl, cap, DK * sizeof(TA), &bar);
+    chunks_stage_new<TA, NCH, false>(a, qkv, Ks, Vs, b, h, nf, cl, kt);
+    __syncthreads();
+    mbar_wait(&bar, 0);
+    chunks_append_ring<TA, NCH>(a, Ks, Vs, ringK, ringV, nf, cl, kt);
+
+    const int pe0 = a.pe_index[slot];
+    for (int j = 0; j < a.chunks; ++j) {
+        const int nfj = nf + j * t, clj = min(nfj, a.window);
+        const int o = nfj - clj - first;            // staged row of this chunk's first key
+        const int nk = clj + t;
+        const int start = max(0, chunk_pe(pe0, j, a) - a.full_chunk);
+        for (int i = tid; i < nk * NCH; i += ATT_THREADS) {        // positions past the table end repeat its last row
+            const int r = i / NCH, c = i % NCH, pos = min(start + r, a.pos_rows - 1);
+            *reinterpret_cast<uint4*>(Ps + r * DK + c * EPC) = *reinterpret_cast<const uint4*>(ptab_h + ((long long)h * a.pos_rows + pos) * DK + c * EPC);
+        }
+        for (int i = tid; i < t * DK; i += ATT_THREADS) {
+            const int r = i / DK, d = i % DK;
+            const float q = q32[(long long)(b * kt + j * t + r) * 3 * D + h * DK + d];
+            qu[i] = q + pos_u[h * DK + d];
+            qv[i] = q + pos_v[h * DK + d];
+        }
+        __syncthreads();
+        constexpr int KPL = 4;                        // keys per lane: nk <= window + t <= STREAM_CHUNKS_MAX_KEYS
+        for (int i = warp; i < t; i += ATT_THREADS / 32) {
+            const float* qui = qu + i * DK;
+            const float* qvi = qv + i * DK;
+            float sc[KPL];
+#pragma unroll
+            for (int k = 0; k < KPL; ++k) sc[k] = 0.f;
+            for (int c = 0; c < NCH; ++c) {
+                const int cc = (c + lane) & (NCH - 1);
+#pragma unroll
+                for (int k = 0; k < KPL; ++k) {
+                    const int jj = lane + 32 * k;
+                    if (jj < nk) {
+                        float kv[EPC], pp[EPC];
+                        Chunk<TA>::load(Ks + (o + jj) * DK + cc * EPC, kv);
+                        Chunk<TA>::load(Ps + jj * DK + cc * EPC, pp);
+                        float s = sc[k];
+#pragma unroll
+                        for (int e = 0; e < EPC; ++e) s = fmaf(qui[cc * EPC + e], kv[e], fmaf(qvi[cc * EPC + e], pp[e], s));
+                        sc[k] = s;
+                    }
+                }
+            }
+            float m = -INFINITY;
+#pragma unroll
+            for (int k = 0; k < KPL; ++k) {
+                sc[k] = (lane + 32 * k < nk) ? sc[k] * 0.125f : -INFINITY;
+                m = fmaxf(m, sc[k]);
+            }
+            m = warp_max(m);
+            float ssum = 0.f;
+            float* pr = prob + i * prow;
+#pragma unroll
+            for (int k = 0; k < KPL; ++k) {
+                const int jj = lane + 32 * k;
+                if (jj < nk) {
+                    const float e = __expf(sc[k] - m);
+                    pr[jj] = e;
+                    ssum += e;
+                }
+            }
+            ssum = warp_sum(ssum);
+            __syncwarp();
+            const float inv = 1.f / ssum;
+            float o0 = 0.f, o1 = 0.f;
+            for (int jj = 0; jj < nk; ++jj) {
+                const float p = pr[jj];
+                o0 = fmaf(p, to_f(Vs[(o + jj) * DK + 2 * lane]), o0);
+                o1 = fmaf(p, to_f(Vs[(o + jj) * DK + 2 * lane + 1]), o1);
+            }
+            TA* op = out + (long long)(b * kt + j * t + i) * D + h * DK + 2 * lane;
+            op[0] = from_f<TA>(o0 * inv);
+            op[1] = from_f<TA>(o1 * inv);
+        }
+        __syncthreads();                              // Ps / qu / prob are restaged by the next chunk
+    }
+}
+
+// fp16 form: the two contractions on mma.sync as in attention_stream_mma_kernel, per query chunk (t <= 8 = the MMA's N)
+__global__ void __launch_bounds__(ATT_THREADS)
+attention_chunks_mma_kernel(AttnStream a, const __half* __restrict__ qkv, const float* __restrict__ q32, __half* __restrict__ ring,
+                            const __half* __restrict__ ptab_h, const float* __restrict__ pos_u, const float* __restrict__ pos_v,
+                            __half* __restrict__ out) {
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    typedef __half TA;
+    constexpr int EPC = 8, NCH = 8;
+    FO_PDL_TRIGGER();
+    FO_PDL_WAIT();
+    const int cap = a.ring_cap, t = a.t, kt = a.chunks * t, D = a.H * DK;
+    const int rows = a.window + kt;
+    const int krows = ((rows + 15) & ~15) + 16;     // a chunk's last key tile may read up to 15 rows past the staged keys
+    const int vrows = (a.window + t + 15) & ~15;    // rel-pos rows / probability columns of one chunk
+    TA* Ks = reinterpret_cast<TA*>(smem_raw);
+    TA* Vs = Ks + krows * DK;
+    TA* Ps = Vs + krows * DK;
+    TA* quh = Ps + vrows * DK;
+    TA* qvh = quh + t * DK;
+    TA* ph = qvh + t * DK;                          // t x vrows
+    float* sc = reinterpret_cast<float*>(ph + t * vrows);   // t x max(vrows, 64)
+    __shared__ __align__(8) uint64_t bar;
+
+    const int b = blockIdx.x, h = blockIdx.y;
+    const int slot = a.ids[b];
+    const int nf = a.n_frames[slot];
+    const int cl = min(nf, a.window), first = nf - cl;
+    const int nk_all = cl + kt;
+    TA* ringK = ring + (long long)slot * a.ring_slot_stride + (long long)h * cap * DK;
+    TA* ringV = ringK + (long long)a.H * cap * DK;
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    if (tid == 0) chunks_start_ring_copy(ringK, ringV, Ks, Vs, first, cl, cap, DK * sizeof(TA), &bar);
+    chunks_stage_new<TA, NCH, true>(a, qkv, Ks, Vs, b, h, nf, cl, kt);
+    // rows behind the last key: K is masked there, V enters the PV MMAs with probability 0 and must be finite
+    for (int i = tid; i < (krows - nk_all) * NCH; i += ATT_THREADS) {
+        *reinterpret_cast<uint4*>(Ks + (nk_all + i / NCH) * DK + (i % NCH) * EPC) = make_uint4(0, 0, 0, 0);
+        *reinterpret_cast<uint4*>(Vs + (nk_all + i / NCH) * DK + (i % NCH) * EPC) = make_uint4(0, 0, 0, 0);
+    }
+    __syncthreads();
+    mbar_wait(&bar, 0);
+    chunks_append_ring<TA, NCH>(a, Ks, Vs, ringK, ringV, nf, cl, kt);
+
+    const int g = lane >> 2, c = lane & 3;
+    const int pe0 = a.pe_index[slot];
+    for (int j = 0; j < a.chunks; ++j) {
+        const int nfj = nf + j * t, clj = min(nfj, a.window);
+        const int o = nfj - clj - first;
+        const int nk = clj + t;
+        const int start = max(0, chunk_pe(pe0, j, a) - a.full_chunk);
+        for (int i = tid; i < nk * NCH; i += ATT_THREADS) {        // row r = position start + r, swizzled by that position
+            const int r = i / NCH, cc = i % NCH, pos = min(start + r, a.pos_rows - 1);
+            *reinterpret_cast<uint4*>(Ps + r * DK + ((cc ^ ((start + r) & 7)) * EPC)) =
+                *reinterpret_cast<const uint4*>(ptab_h + ((long long)h * a.pos_rows + pos) * DK + ((cc ^ (pos & 7)) * EPC));
+        }
+        for (int i = tid; i < t * DK; i += ATT_THREADS) {
+            const int r = i / DK, d = i % DK;
+            const float q = q32[(long long)(b * kt + j * t + r) * 3 * D + h * DK + d];
+            const int sw = r * DK + (((d >> 3) ^ (r & 7)) << 3) + (d & 7);
+            quh[sw] = from_f<TA>(q + pos_u[h * DK + d]);
+            qvh[sw] = from_f<TA>(q + pos_v[h * DK + d]);
+        }
+        __syncthreads();
+        for (int k0 = warp * 16; k0 < nk; k0 += 16 * (ATT_THREADS / 32)) {
+            float d[4] = {0.f, 0.f, 0.f, 0.f};
+            const int kk0 = (first + o + k0 + g) & 7, kk1 = (first + o + k0 + g + 8) & 7;
+            const int kp0 = (start + k0 + g) & 7, kp1 = (start + k0 + g + 8) & 7;
+            const TA* kr0 = Ks + (o + k0 + g) * DK + c * 2;
+            const TA* kr1 = Ks + (o + k0 + g + 8) * DK + c * 2;
+            const TA* pr0 = Ps + (k0 + g) * DK + c * 2;
+            const TA* pr1 = Ps + (k0 + g + 8) * DK + c * 2;
+#pragma unroll
+            for (int ks = 0; ks < DK / 16; ++ks) {
+                const int c0 = ks * 2, c1 = ks * 2 + 1;
+                uint32_t af[4], bf[2];
+                af[0] = lds32(kr0 + ((c0 ^ kk0) << 3));
+                af[1] = lds32(kr1 + ((c0 ^ kk1) << 3));
+                af[2] = lds32(kr0 + ((c1 ^ kk0) << 3));
+                af[3] = lds32(kr1 + ((c1 ^ kk1) << 3));
+                bf[0] = g < t ? lds32(quh + g * DK + ((c0 ^ g) << 3) + c * 2) : 0u;
+                bf[1] = g < t ? lds32(quh + g * DK + ((c1 ^ g) << 3) + c * 2) : 0u;
+                mma16816(d, af, bf);
+                af[0] = lds32(pr0 + ((c0 ^ kp0) << 3));
+                af[1] = lds32(pr1 + ((c0 ^ kp1) << 3));
+                af[2] = lds32(pr0 + ((c1 ^ kp0) << 3));
+                af[3] = lds32(pr1 + ((c1 ^ kp1) << 3));
+                bf[0] = g < t ? lds32(qvh + g * DK + ((c0 ^ g) << 3) + c * 2) : 0u;
+                bf[1] = g < t ? lds32(qvh + g * DK + ((c1 ^ g) << 3) + c * 2) : 0u;
+                mma16816(d, af, bf);
+            }
+            const int q0 = c * 2;
+            if (q0 < t) { sc[q0 * vrows + k0 + g] = d[0] * 0.125f; sc[q0 * vrows + k0 + g + 8] = d[2] * 0.125f; }
+            if (q0 + 1 < t) { sc[(q0 + 1) * vrows + k0 + g] = d[1] * 0.125f; sc[(q0 + 1) * vrows + k0 + g + 8] = d[3] * 0.125f; }
+        }
+        __syncthreads();
+        for (int i = warp; i < t; i += ATT_THREADS / 32) {
+            float sv[4];
+            float m = -INFINITY;
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+                const int jj = lane + 32 * k;
+                sv[k] = jj < nk ? sc[i * vrows + jj] : -INFINITY;
+                m = fmaxf(m, sv[k]);
+            }
+            m = warp_max(m);
+            float ssum = 0.f;
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+                sv[k] = (lane + 32 * k < nk) ? __expf(sv[k] - m) : 0.f;
+                ssum += sv[k];
+            }
+            ssum = warp_sum(ssum);
+            const float inv = 1.f / ssum;
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+                const int jj = lane + 32 * k;
+                if (jj < vrows) ph[i * vrows + jj] = __float2half_rn(sv[k] * inv);
+            }
+        }
+        __syncthreads();
+        {
+            float d[4] = {0.f, 0.f, 0.f, 0.f};
+            const int dim0 = warp * 16;
+            const int mi = lane >> 3, r = lane & 7;
+            for (int key0 = 0; key0 < nk; key0 += 16) {
+                uint32_t af[4], bf[2];
+                const int vrow = o + key0 + r + ((mi & 2) ? 8 : 0);
+                const TA* ap = Vs + vrow * DK + ((((dim0 >> 3) + (mi & 1)) ^ ((first + vrow) & 7)) << 3);
+                const uint32_t saddr = smem_u32(ap);
+                asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0,%1,%2,%3}, [%4];"
+                             : "=r"(af[0]), "=r"(af[1]), "=r"(af[2]), "=r"(af[3])
+                             : "r"(saddr));
+                bf[0] = g < t ? lds32(ph + g * vrows + key0 + c * 2) : 0u;
+                bf[1] = g < t ? lds32(ph + g * vrows + key0 + 8 + c * 2) : 0u;
+                mma16816(d, af, bf);
+            }
+            const int q0 = c * 2;
+            if (q0 < t) { sc[q0 * DK + dim0 + g] = d[0]; sc[q0 * DK + dim0 + g + 8] = d[2]; }
+            if (q0 + 1 < t) { sc[(q0 + 1) * DK + dim0 + g] = d[1]; sc[(q0 + 1) * DK + dim0 + g + 8] = d[3]; }
+        }
+        __syncthreads();
+        for (int i = tid; i < t * (DK / 2); i += ATT_THREADS) {
+            const int q = i / (DK / 2), pr = i % (DK / 2);
+            *reinterpret_cast<uint32_t*>(out + (long long)(b * kt + j * t + q) * D + h * DK + 2 * pr) =
+                pack2<__half>(sc[q * DK + 2 * pr], sc[q * DK + 2 * pr + 1]);
+        }
+        __syncthreads();                              // Ps / quh / ph / sc are restaged by the next chunk
+    }
+}
+
+// ---------------------------------------------------------------------------------------------
 constexpr int KT = 96;          // key tile: the shipped band of a 32-query block (64 left + 32 own keys) in one pass
 constexpr int QB = 32;          // query rows per CTA
 constexpr int QPW = QB / (ATT_THREADS / 32);   // queries per warp
@@ -1043,17 +1358,56 @@ attention_offline_fa_kernel(const __half* __restrict__ qkv, const float* __restr
 }
 
 __global__ void advance_sessions_kernel(const int32_t* __restrict__ ids, int n, int t, int chunk_size, int pe_wrap,
-                                        int32_t* n_frames, int32_t* pe_index, int32_t* adapter_valid) {
+                                        int32_t* n_frames, int32_t* pe_index, int32_t* adapter_valid, int chunks) {
     FO_PDL_TRIGGER();
     FO_PDL_WAIT();
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= n) return;
     const int s = ids[b];
     if (n_frames) {
-        n_frames[s] += t;
-        pe_index[s] = pe_index[s] % pe_wrap + chunk_size;   // attention.py:107,120 (+chunk_size, not +t)
+        n_frames[s] += chunks * t;
+        int pe = pe_index[s];
+        for (int j = 0; j < chunks; ++j) pe = pe % pe_wrap + chunk_size;   // attention.py:107,120 (+chunk_size, not +t)
+        pe_index[s] = pe;
     }
     if (adapter_valid) adapter_valid[s] = adapter_valid[s] == 1 ? 2 : 1;
+}
+
+// launcher of the multi-chunk kernels (AttnStream::chunks > 1)
+template <typename TA>
+int attention_stream_chunks(const AttnStream& a, const TA* qkv, const float* q32, TA* ring, const TA* ptab_h,
+                            const float* pos_u, const float* pos_v, TA* out, cudaStream_t st) {
+    const int kt = a.chunks * a.t, rows = a.window + kt, prow = a.window + a.t;
+    FO_CHECK(a.t <= TQ_MAX, "attention_stream: %d frames per chunk exceeds %d", a.t, TQ_MAX);
+    FO_CHECK(rows <= STREAM_CHUNKS_MAX_KEYS, "attention_stream: window %d + %d chunks x %d frames exceeds %d keys", a.window,
+             a.chunks, a.t, STREAM_CHUNKS_MAX_KEYS);
+    dim3 grid(a.n, a.H);
+    static bool attr_set[2] = {false, false};
+    size_t smem;
+    if constexpr (sizeof(TA) == 2) {
+        const int krows = ((rows + 15) & ~15) + 16, vrows = (prow + 15) & ~15;
+        smem = (size_t)(2 * krows + vrows) * DK * 2 + (size_t)2 * a.t * DK * 2 + (size_t)a.t * vrows * 2 +
+               (size_t)a.t * std::max(vrows, DK) * 4;
+        if (!attr_set[1]) {
+            FO_CUDA(cudaFuncSetAttribute(attention_chunks_mma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
+            attr_set[1] = true;
+        }
+        FO_CHECK(smem <= 160 * 1024, "attention_stream: multi-chunk call too large for shared memory");
+        FO_CUDA(launch_pdl(attention_chunks_mma_kernel, grid, dim3(ATT_THREADS), smem, st, a, reinterpret_cast<const __half*>(qkv), q32,
+                           reinterpret_cast<__half*>(ring), reinterpret_cast<const __half*>(ptab_h), pos_u, pos_v,
+                           reinterpret_cast<__half*>(out)));
+    } else {
+        smem = (size_t)(2 * rows + prow) * DK * sizeof(TA) + (size_t)2 * a.t * DK * sizeof(float) + (size_t)a.t * prow * sizeof(float);
+        if (!attr_set[0]) {
+            FO_CUDA(cudaFuncSetAttribute(attention_chunks_kernel<TA>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
+            attr_set[0] = true;
+        }
+        FO_CHECK(smem <= 160 * 1024, "attention_stream: multi-chunk call too large for shared memory");
+        FO_CUDA(launch_pdl(attention_chunks_kernel<TA>, grid, dim3(ATT_THREADS), smem, st, a, qkv, q32, ring, ptab_h, pos_u, pos_v, out));
+    }
+    FO_LAUNCHED();
+    FO_CUDA(cudaGetLastError());
+    return 0;
 }
 
 }  // namespace
@@ -1062,6 +1416,7 @@ template <typename TA>
 int attention_stream(const AttnStream& a, const TA* qkv, const float* q32, TA* ring, const TA* ptab_h,
                      const float* pos_u, const float* pos_v, TA* out, cudaStream_t st) {
     if (a.n <= 0) return 0;
+    if (a.chunks > 1) return attention_stream_chunks<TA>(a, qkv, q32, ring, ptab_h, pos_u, pos_v, out, st);
     FO_CHECK(a.t <= TQ_MAX, "attention_stream: %d frames per call exceeds %d", a.t, TQ_MAX);
     FO_CHECK(a.ring_cap >= a.window + a.t, "attention_stream: ring capacity %d < window %d + %d", a.ring_cap, a.window, a.t);
     const int rows = a.window + a.t;
@@ -1171,9 +1526,10 @@ template int attention_offline<bf16>(const bf16*, const float*, int, int, int, c
 template int attention_offline<__half>(const __half*, const float*, int, int, int, const int32_t*, int, int, const float*, const __half*, int, const float*, const float*, __half*, cudaStream_t);
 
 int advance_sessions(const int32_t* ids, int n, int t, int chunk_size, int pe_wrap, int32_t* n_frames,
-                      int32_t* pe_index, int32_t* adapter_valid, cudaStream_t st) {
+                      int32_t* pe_index, int32_t* adapter_valid, cudaStream_t st, int chunks) {
     if (n <= 0) return 0;
-    FO_CUDA(launch_pdl(advance_sessions_kernel, dim3(cdiv(n, 128)), dim3(128), 0, st, ids, n, t, chunk_size, pe_wrap, n_frames, pe_index, adapter_valid));
+    FO_CUDA(launch_pdl(advance_sessions_kernel, dim3(cdiv(n, 128)), dim3(128), 0, st, ids, n, t, chunk_size, pe_wrap, n_frames, pe_index, adapter_valid,
+                       chunks));
     FO_LAUNCHED();
     FO_CUDA(cudaGetLastError());
     return 0;

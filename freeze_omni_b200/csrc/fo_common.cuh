@@ -368,7 +368,13 @@ struct AttnStream {
     const float* part_bias = nullptr;
     int nsplit = 0;
     long long part_stride = 0;
+    // consecutive chunks per session in this call (fo_encode_stream_chunks): rows are (session, chunk, frame), n*chunks*t
+    // of them; chunk j of a session is attended exactly as the j-th of `chunks` sequential calls (chunk_size: pe_index step)
+    int chunks = 1;
+    int chunk_size = 0;
 };
+// staged keys of the multi-chunk attention (window + chunks * t at most): bounds the chunks of one call
+constexpr int STREAM_CHUNKS_MAX_KEYS = 128;
 // qkv (n*t, 3*D) activation type (K and V columns are read from it); q32 (n*t, 3*D) fp32 whose first D
 // columns hold Q (the QKV GEMM keeps Q in fp32, Epilogue::split_col); ring = this layer's
 // (slot, 2, H, ring_cap, 64); ptab (pos_rows, D) fp32; out (n*t, D).  Appends the new K/V rows to the ring.
@@ -384,9 +390,10 @@ int attention_offline(const TA* qkv, const float* q32, int B, int T, int H, cons
                       const float* ptab, const TA* ptab_h, int pos_rows, const float* pos_u, const float* pos_v, TA* out,
                       cudaStream_t st);
 // end of a streaming step: n_frames += t, pe_index = pe_index % wrap + chunk_size (attention.py:107,120),
-// and flip the live half of the double-buffered adapter cache.  Either group may be null.
+// and flip the live half of the double-buffered adapter cache.  Either group may be null.  chunks > 1: the session
+// advanced by that many chunks of t frames (pe_index stepped `chunks` times; the adapter cache still flips once).
 int advance_sessions(const int32_t* ids, int n, int t, int chunk_size, int pe_wrap, int32_t* n_frames,
-                     int32_t* pe_index, int32_t* adapter_valid, cudaStream_t st);
+                     int32_t* pe_index, int32_t* adapter_valid, cudaStream_t st, int chunks = 1);
 
 // ---- weight-streaming layer stack for a handful of sessions (fo_stack.cu) ---------------------------
 // All transformer layers of a streaming step in ONE cooperative launch when the step has at most 16 token rows (1-4

@@ -355,10 +355,10 @@ template <typename TA>
 __global__ void __launch_bounds__(256)
 depthwise_conv_kernel(const TA* __restrict__ x, int T, int C, int k, const float* __restrict__ w,
                       const float* __restrict__ bias, const int32_t* __restrict__ ids, float* slot_cache,
-                      long long slot_stride, TA* __restrict__ y) {
+                      long long slot_stride, TA* __restrict__ y, int row0) {
     FO_PDL_TRIGGER();
     FO_PDL_WAIT();
-    const int b = blockIdx.y, r0 = blockIdx.x * DW_TB;
+    const int b = blockIdx.y, r0 = row0 + blockIdx.x * DW_TB;
     const int nr = min(DW_TB, T - r0);
     const int km1 = k - 1;
     float* cache = ids ? slot_cache + (long long)ids[b] * slot_stride : nullptr;
@@ -393,7 +393,8 @@ depthwise_conv_kernel(const TA* __restrict__ x, int T, int C, int k, const float
         }
         // streaming: the CTA that owns the last rows writes the new context (single CTA per session when T <= DW_TB;
         // for longer calls the old context is only read by the first CTA and written by the last one, after a
-        // kernel-wide ordering that a second launch provides: the host rejects streaming calls with T > DW_TB)
+        // kernel-wide ordering that a second launch provides: the host runs streaming calls with T > DW_TB as one launch
+        // per DW_TB rows)
         if (cache && r0 + nr == T) {
             for (int q = 0; q < km1; ++q) cache[(long long)q * C + c] = win[q];
         }
@@ -655,9 +656,17 @@ int depthwise_conv(const TA* x, int B, int T, int C, int k, const float* w, cons
                    float* slot_cache, long long slot_stride, TA* y, cudaStream_t st) {
     if (B <= 0 || T <= 0) return 0;
     FO_CHECK(k >= 2 && k <= DW_KMAX, "depthwise_conv: kernel size %d outside 2..%d", k, DW_KMAX);
-    FO_CHECK(!ids || T <= DW_TB, "depthwise_conv: a streaming call may carry at most %d frames", DW_TB);
+    if (ids && T > DW_TB) {
+        // streaming, several chunks per session (fo_encode_stream_chunks): the first rows read the carried context and the
+        // last ones replace it, so the row blocks run in order, one launch each
+        for (int r0 = 0; r0 < T; r0 += DW_TB) {
+            FO_CUDA(launch_pdl(depthwise_conv_kernel<TA>, dim3(1, B), dim3(256), 0, st, x, T, C, k, w, bias, ids, slot_cache, slot_stride, y, r0));
+            FO_LAUNCHED();
+        }
+        return 0;
+    }
     dim3 grid(cdiv(T, DW_TB), B);
-    FO_CUDA(launch_pdl(depthwise_conv_kernel<TA>, grid, dim3(256), 0, st, x, T, C, k, w, bias, ids, slot_cache, slot_stride, y));
+    FO_CUDA(launch_pdl(depthwise_conv_kernel<TA>, grid, dim3(256), 0, st, x, T, C, k, w, bias, ids, slot_cache, slot_stride, y, 0));
     FO_LAUNCHED();
     return 0;
 }

@@ -283,6 +283,24 @@ class Engine:
                                              _ptr(adapter_out) if want_adapter else None, self._stream()))
         return enc_out, (adapter_out if want_adapter else None)
 
+    def encode_stream_chunks(self, ids, feats: ArrayLike, want_adapter: Optional[bool] = None,
+                             enc_out: Optional[torch.Tensor] = None, adapter_out: Optional[torch.Tensor] = None):
+        """n sessions advance k consecutive chunks in one step, with the results of k single-chunk encode_stream calls.
+        feats (n, k, t_in, F): every block with its own context frames.  Returns enc (n, k, t, D) and adapter (n, k, t_out, E)."""
+        ids = _ids(ids)
+        n = len(ids)
+        assert feats is not None and feats.ndim == 4, "feats must be (n, k, t_in, F)"
+        k, t_in = int(feats.shape[1]), int(feats.shape[2])
+        assert tuple(feats.shape) == (n, k, t_in, self.cfg.feat_dim) and feats.dtype in (torch.float32, np.dtype(np.float32))
+        t, t_out = self.out_frames(t_in)
+        want_adapter = self.has_adapter if want_adapter is None else want_adapter
+        enc_out = self._out(enc_out, (n, k, t, self.cfg.d_model))
+        if want_adapter:
+            adapter_out = self._out(adapter_out, (n, k, t_out, self.cfg.llm_dim))
+        _lib.check(self.lib.fo_encode_stream_chunks(self._h, _i32p(ids), n, k, _ptr(feats), t_in, _ptr(enc_out),
+                                                    _ptr(adapter_out) if want_adapter else None, self._stream()))
+        return enc_out, (adapter_out if want_adapter else None)
+
     def stream_step(self, ids, pcm: ArrayLike, scale: Optional[float] = None, enc_out: Optional[torch.Tensor] = None,
                     adapter_out: Optional[torch.Tensor] = None, want_enc: bool = True):
         """PCM in, encoder frames + LLM-space embeddings out, one library call."""

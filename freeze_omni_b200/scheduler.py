@@ -16,6 +16,9 @@ on the device and drains the per-session feature queues with batched encoder+ada
 
 Per drain round the head block of every session with a non-empty queue forms one batch; the batch is padded to a
 multiple of `bucket` with scratch sessions so that a handful of captured CUDA graphs serve every active-set size.
+With `max_chunks` > 1 a round takes up to that many queued blocks of a session at once (Engine.encode_stream_chunks, same
+results as one block per call): an onset tick then costs one call for the sessions with one block and one for those
+replaying their history, instead of 1 + onset_chunks calls.
 State (KV rings, adapter cache, sample carry, feature ring, history ring, queued blocks) never leaves the device.
 """
 from collections import deque
@@ -79,14 +82,46 @@ def plan_rounds(queue_lens: Dict[Hashable, int], max_batch: int) -> List[List[Ha
             left[k] -= 1
 
 
+def plan_chunk_calls(queue_lens: Dict[Hashable, int], max_chunks: int, max_batch: int) -> List[Tuple[int, List[Hashable]]]:
+    """Drain order when one call may advance a session by up to `max_chunks` consecutive queued blocks: every round takes
+    k = min(blocks left, max_chunks) blocks of each session that still has some; sessions with the same k share a call
+    (smaller k first, sessions in queue order, `max_batch` sessions per call).  A session appears at most once per round and
+    rounds run in order, so its blocks stay in stream order.  Returns [(k, sessions)]; max_chunks = 1 is plan_rounds.
+    Pure function of the queue lengths -> testable without a GPU."""
+    assert max_chunks >= 1
+    left = dict(queue_lens)
+    calls: List[Tuple[int, List[Hashable]]] = []
+    while True:
+        ready = [key for key, n in left.items() if n > 0]
+        if not ready:
+            return calls
+        by_k: Dict[int, List[Hashable]] = {}
+        for key in ready:
+            by_k.setdefault(min(left[key], max_chunks), []).append(key)
+        for k in sorted(by_k):
+            group = by_k[k]
+            for i in range(0, len(group), max_batch):
+                calls.append((k, group[i:i + max_batch]))
+        for key in ready:
+            left[key] -= min(left[key], max_chunks)
+
+
 def bucket_size(n: int, bucket: int) -> int:
     return (n + bucket - 1) // bucket * bucket
 
 
+def chunk_bucket_size(n: int, k: int, bucket: int) -> int:
+    """Sessions of a call of n sessions x k chunks after padding.  The padding is counted in blocks (token rows), not in
+    sessions: sessions are padded to a multiple of max(1, bucket // k), so it adds fewer than `bucket` blocks, as the padding
+    of a single-chunk call does (2 onset sessions x 7 chunks stay 2 sessions with bucket 16, not 16 x 7 blocks)."""
+    return bucket_size(n, max(1, bucket // k))
+
+
 class StreamScheduler:
     def __init__(self, engine, history_chunks: int = 10, onset_chunks: int = 6, bucket: int = 16,
-                 max_batch: Optional[int] = None, max_sessions: Optional[int] = None):
-        assert 0 <= onset_chunks <= history_chunks
+                 max_batch: Optional[int] = None, max_sessions: Optional[int] = None, max_chunks: int = 1):
+        assert 0 <= onset_chunks <= history_chunks and max_chunks >= 1
+        self.max_chunks = int(max_chunks)
         self.eng, self.cfg = engine, engine.cfg
         self.history_chunks, self.onset_chunks, self.bucket = history_chunks, onset_chunks, max(1, bucket)
         self.max_batch = max_batch or 1 << 30
@@ -176,6 +211,8 @@ class StreamScheduler:
                     self.block_log.extend((k, b, lab) for b, lab in labelled)
             self.pending.clear()
         cursor = 0
+        if self.max_chunks > 1:
+            return self._drain_chunks(out, handoff)
         for batch in plan_rounds({k: len(q) for k, q in self.queues.items()}, self.max_batch):
             heads = [self.queues[k].popleft() for k in batch]
             blocks = [h[0] for h in heads]
@@ -208,6 +245,48 @@ class StreamScheduler:
             for i, k in enumerate(batch):
                 out.setdefault(k, []).append(Block(enc[i], emb[i] if emb is not None else None, heads[i][1]))
         return out
+
+    def _drain_chunks(self, out: Dict[Hashable, List[Block]], handoff: Optional[Handoff]) -> Dict[Hashable, List[Block]]:
+        """The drain of tick() with up to max_chunks blocks of a session per call (plan_chunk_calls)."""
+        cursor = 0
+        for k, batch in plan_chunk_calls({s: len(q) for s, q in self.queues.items()}, self.max_chunks, self.max_batch):
+            heads = [[self.queues[s].popleft() for _ in range(k)] for s in batch]
+            n = len(batch)
+            pad = chunk_bucket_size(n, k, self.bucket) - n
+            ids = np.concatenate([np.array([self.keys[s] for s in batch], np.int32), self.scratch[:pad]]).astype(np.int32)
+            x = torch.stack([h[0] for hs in heads + [heads[0]] * pad for h in hs])
+            x = x.view(n + pad, k, *x.shape[1:])                                                  # (n + pad, k, t_in, F)
+            self.stats["encode_calls"] += 1
+            self.stats["session_steps"] += n * k
+            self.stats["padded_steps"] += pad * k
+            if handoff is not None:
+                # block i*k + j of the armed call is chunk j of session i
+                n_blocks = (n + pad) * k
+                if cursor + n_blocks > handoff.embeds.shape[0]:
+                    raise RuntimeError("Handoff capacity %d exceeded in one tick" % handoff.embeds.shape[0])
+                onset = [h[1] == IPU_START for hs in heads for h in hs] + [False] * (pad * k)
+                self.eng.handoff_arm(n_blocks, handoff.embeds[cursor:], handoff.prefix_len, onset, handoff.prefix_mask,
+                                     handoff.attn_mask[cursor:], handoff.row_start[cursor:])
+                enc, _ = self._encode(ids, x, k, want_adapter=False)
+                for i, s in enumerate(batch):
+                    for j, h in enumerate(heads[i]):
+                        row = cursor + i * k + j
+                        st0 = 0 if h[1] == IPU_START else handoff.prefix_len
+                        out.setdefault(s, []).append(Block(enc[i, j], handoff.embeds[row, st0:], h[1], handoff.attn_mask[row, st0:]))
+                cursor += n_blocks
+                continue
+            enc, emb = self._encode(ids, x, k)
+            for i, s in enumerate(batch):
+                for j, h in enumerate(heads[i]):
+                    out.setdefault(s, []).append(Block(enc[i, j], emb[i, j] if emb is not None else None, h[1]))
+        return out
+
+    def _encode(self, ids, x, k, **kw):
+        """(n, k, ...) results of one call: a single-chunk call keeps the engine's one-chunk entry point."""
+        if k == 1:
+            enc, emb = self.eng.encode_stream(ids, x[:, 0], **kw)
+            return enc.unsqueeze(1), (emb.unsqueeze(1) if emb is not None else None)
+        return self.eng.encode_stream_chunks(ids, x, **kw)
 
     def history(self, key: Hashable) -> torch.Tensor:
         return self._hist[self.rows[key]]

@@ -88,8 +88,8 @@ typedef struct fo_config {
 } fo_config;
 
 typedef struct fo_stats_t {
-    int64_t stream_steps;      /* fo_encode_stream / fo_stream_step calls */
-    int64_t session_chunks;    /* sum over steps of sessions advanced */
+    int64_t stream_steps;      /* fo_encode_stream / fo_encode_stream_chunks / fo_stream_step calls */
+    int64_t session_chunks;    /* sum over steps of sessions x chunks advanced */
     int64_t offline_calls;
     int64_t offline_frames;    /* encoder frames produced offline */
     int64_t kernel_launches;   /* kernels of this library enqueued so far (graph replays count their nodes) */
@@ -159,6 +159,16 @@ int fo_fbank_offline(fo_ctx* ctx, const void* pcm, int pcm_dtype, int B, int64_t
  * t = ((t_in-1)/2-1)/2; t_out = (t + kernel-1 - kernel)/2 + 1. */
 int fo_encode_stream(fo_ctx* ctx, const int32_t* ids, int n, const float* feats, int t_in,
                      float* enc_out, float* adapter_out, void* stream);
+/* k consecutive chunks per session in one call, equal to k successive fo_encode_stream calls of one chunk each
+ * (speechEncoder.infer + CNNSubsampling.forward(cache) k times, models/audioLLM.py:380-387): speech-onset replay and
+ * catch-up encoding stream the weights once for n*k*t token rows instead of k times.
+ * feats (n, k, t_in, feat_dim), required: every chunk block carries its own context frames, as fo_fbank_stream returns them.
+ * enc_out (n, k, t, d_model), adapter_out (n, k, t_out, llm_dim): either may be NULL.  A session's state advances by k chunks.
+ * window + k*t keys must fit the multi-chunk attention (128: k <= 16 with the shipped chunking); beyond that FO_ERR_ARG
+ * names the largest k.  An armed hand-off (fo_handoff_arm) applies when armed for n*k blocks: block i*k + j is chunk j of
+ * session i (onset flag, embedding rows, mask row and row_start per block).  Counts as one stream step and n*k session chunks. */
+int fo_encode_stream_chunks(fo_ctx* ctx, const int32_t* ids, int n, int k, const float* feats, int t_in,
+                            float* enc_out, float* adapter_out, void* stream);
 /* fbank + encode in one call (one captured graph): PCM in, embeddings out */
 int fo_stream_step(fo_ctx* ctx, const int32_t* ids, int n, const void* pcm, int pcm_dtype, float scale,
                    float* enc_out, float* adapter_out, void* stream);
