@@ -428,7 +428,29 @@ int finalize_t(fo_ctx* c) {
         }
         // positional table (fp32 sin/cos built on the host exactly as attention.py:13-30 does)
         const HostTensor* pe;
-        FO_TRY(need(c, "pos.table", {c->pos_rows, D}, &pe));
+        FO_TRY(need(c, "pos.table", {g.pos_max_len, D}, &pe));
+        // rows past pos_max_len (streaming positions of left_chunks <= 0 contexts, fo_create): the same fp32 operations as the
+        // table, pos * exp(2i * -(ln 10000 / D)) then sin / cos.  The host's expf may differ from torch's by one ulp in a few
+        // columns, i.e. ~1e-4 in the argument at position 5000 -- the size of the fp32 rounding of the argument itself.
+        const float* pe_rows = pe->d;
+        struct TmpBuf { void* p = nullptr; ~TmpBuf() { if (p) cudaFree(p); } } pe_ext;
+        if (c->pos_rows > g.pos_max_len) {
+            const int extra = c->pos_rows - g.pos_max_len;
+            std::vector<float> hx((size_t)extra * D);
+            const float s = (float)(-(log(10000.0) / D));
+            for (int i = 0; i < D / 2; ++i) {
+                const float dt = expf((float)(2 * i) * s);
+                for (int r = 0; r < extra; ++r) {
+                    const float a = (float)(g.pos_max_len + r) * dt;
+                    hx[(size_t)r * D + 2 * i] = sinf(a);
+                    hx[(size_t)r * D + 2 * i + 1] = cosf(a);
+                }
+            }
+            FO_CUDA(cudaMalloc(&pe_ext.p, (size_t)c->pos_rows * D * sizeof(float)));
+            FO_CUDA(cudaMemcpy(pe_ext.p, pe->d, (size_t)g.pos_max_len * D * sizeof(float), cudaMemcpyDeviceToDevice));
+            FO_CUDA(cudaMemcpy((float*)pe_ext.p + (size_t)g.pos_max_len * D, hx.data(), hx.size() * sizeof(float), cudaMemcpyHostToDevice));
+            pe_rows = (const float*)pe_ext.p;
+        }
         c->layers.resize(L);
         for (int l = 0; l < L; ++l) {
             LayerW& w = c->layers[l];
@@ -508,7 +530,7 @@ int finalize_t(fo_ctx* c) {
                 Epilogue ep;
                 ep.c_f32 = w.ptab;
                 ep.ldc = D;
-                r = gemm_simt<float, float>(pe->d, plain_rows(D, c->pos_rows), wpos, c->pos_rows, D, D, ep, RowMap(), 0);
+                r = gemm_simt<float, float>(pe_rows, plain_rows(D, c->pos_rows), wpos, c->pos_rows, D, D, ep, RowMap(), 0);
             }
             if (r == 0) r = dev_alloc(c, &w.ptab_h, (size_t)c->pos_rows * D * (sizeof(TW) == 2 ? 2 : 4));
             if (r == 0) {
@@ -1312,12 +1334,19 @@ int fo_create(const fo_config* cfg, int device, int dtype, fo_ctx** out) {
     const bool streaming = cfg->chunk_size > 0 && cfg->left_chunks > 0;
     c->window = streaming ? cfg->chunk_size * cfg->left_chunks : 1;                  // attention.py:290-295
     c->full_chunk = (cfg->left_chunks + 1) * cfg->chunk_size;                         // attention.py:83
-    c->pos_rows = cfg->pos_max_len;
     c->pe_wrap = cfg->chunk_size > 0 ? cfg->chunk_size * (cfg->pos_max_len / cfg->chunk_size) - c->full_chunk : cfg->pos_max_len;
     const int msf = cfg->max_stream_frames > 0 ? cfg->max_stream_frames : cfg->frames_per_chunk + cfg->context_frames;
     c->max_t = (((msf - 1) / 2) - 1) / 2;
     if (c->max_t < 1) c->max_t = 1;
+    if (c->max_t > STREAM_MAX_T) c->max_t = STREAM_MAX_T;      // the streaming attention takes at most 8 frames per chunk
     c->ring_cap = ((c->window + c->max_t + 7) / 8) * 8;
+    // Rel-pos rows the streaming kernels may read: a call at pe_index % pe_wrap = pe sees positions
+    // max(0, pe - full_chunk) + [0, window + t).  With left_chunks <= 0 (full_chunk 0, pe_wrap = pos_max_len) that runs up to
+    // pe_wrap + t - 1, past the reference's max_len rows; its RelPositionalEncoding.infer evaluates the sinusoid there
+    // (attention.py:111-117), so the tables get real rows up to the last reachable position (fo_finalize_weights).
+    c->pos_rows = cfg->pos_max_len;
+    if (cfg->chunk_size > 0)
+        c->pos_rows = std::max(c->pos_rows, std::max(0, c->pe_wrap - 1 - c->full_chunk) + c->window + c->max_t);
     c->carry = cfg->frame_len - cfg->frame_shift;
     c->chunk_samples = cfg->frame_shift * cfg->frames_per_chunk;
     c->fft = 1;
@@ -1809,13 +1838,27 @@ static int run_step(fo_ctx* c, const StepArgs& a, cudaStream_t st) {
     return 0;
 }
 
+// What every streaming entry checks before it enqueues anything, so that a refused call leaves the sessions as they were:
+// chunk_size > 0 (with chunk_size <= 0 pe_index would step backwards into negative values, attention.py:107,120), at most
+// max_t (<= STREAM_MAX_T) encoder frames per chunk, and window + t keys within the 128 the streaming attention stages.
+static int stream_geometry(const fo_ctx* c, int t_in) {
+    const int t = ((t_in - 1) / 2 - 1) / 2;
+    FO_CHECK(c->cfg.chunk_size > 0, "streaming needs transformer-chunk_size > 0 (got %d); chunk_size <= 0 is full attention, "
+                                    "use fo_encode_offline", c->cfg.chunk_size);
+    FO_CHECK(t >= 1 && t <= c->max_t, "streaming call of %d feature frames gives %d encoder frames; context allows 1..%d",
+             t_in, t, c->max_t);
+    FO_CHECK(c->window + t <= STREAM_CHUNKS_MAX_KEYS,
+             "streaming call: the attention window (%d frames) + %d new frames exceeds the %d keys of the streaming attention",
+             c->window, t, STREAM_CHUNKS_MAX_KEYS);
+    return 0;
+}
+
 // copies between the caller's buffers and the context's staging buffers, then the step
 // k > 1 (fo_encode_stream_chunks, feats only): k consecutive chunk blocks per session, feats (n, k, t_in, F)
 static int stream_common(fo_ctx* c, const int32_t* ids, int n, int k, const void* pcm, int pcm_dtype, float scale,
                          const float* feats, int t_in, float* enc_out, float* adapter_out, cudaStream_t st) {
     const int T1 = (t_in - 1) / 2, t = (T1 - 1) / 2;
-    FO_CHECK(t >= 1 && t <= c->max_t, "streaming call of %d feature frames gives %d encoder frames; context allows 1..%d",
-             t_in, t, c->max_t);
+    FO_TRY(stream_geometry(c, t_in));
     if (adapter_out) FO_CHECK(c->cfg.has_adapter, "adapter_out requested but the context has no adapter");
     FO_CHECK(!c->KM, "this context's positionwise layer is MultiLayeredConv1d, which has no streaming form (the reference module has no infer(), "
                      "models/encoder/attention.py:145-196); use fo_encode_offline");
@@ -1890,8 +1933,9 @@ int fo_encode_stream_chunks(fo_ctx* c, const int32_t* ids, int n, int k, const f
     FO_CHECK(k >= 1, "fo_encode_stream_chunks: k must be >= 1");
     FO_CHECK(t_in >= 7, "fo_encode_stream_chunks: need at least 7 feature frames per chunk");
     FO_TRY(check_ids(c, ids, n));
+    FO_TRY(stream_geometry(c, t_in));
     const int t = ((t_in - 1) / 2 - 1) / 2;
-    if (k > 1 && t >= 1 && t <= c->max_t) {
+    if (k > 1) {
         const int kmax = std::max(1, (STREAM_CHUNKS_MAX_KEYS - c->window) / t);
         FO_CHECK(c->window + k * t <= STREAM_CHUNKS_MAX_KEYS,
                  "fo_encode_stream_chunks: the attention window (%d frames) + %d chunks x %d frames exceeds %d keys; the largest k is %d",
@@ -1957,6 +2001,7 @@ int fo_stream_step_async(fo_ctx* c, const int32_t* ids, int n, const void* pcm, 
     FO_CHECK(!c->KM, "fo_stream_step_async: MultiLayeredConv1d has no streaming form; use fo_encode_offline");
     if (adapter_out) FO_CHECK(c->cfg.has_adapter, "adapter_out requested but the context has no adapter");
     FO_TRY(check_ids(c, ids, n));
+    FO_TRY(stream_geometry(c, c->cfg.context_frames + c->cfg.frames_per_chunk));
     FO_CUDA(cudaSetDevice(c->device));
     cudaStream_t st = (cudaStream_t)stream;
     if (!c->copy_stream) {
@@ -2022,7 +2067,7 @@ int fo_encode_offline(fo_ctx* c, const float* feats, const int32_t* ilens, int B
     FO_CHECK(c && c->finalized && c->cfg.has_encoder, "fo_encode_offline: context has no finalized encoder");
     FO_CHECK(feats && ilens && B > 0 && T >= 7, "fo_encode_offline: need feats, ilens and T >= 7");
     const int T1 = (T - 1) / 2, T2 = (T1 - 1) / 2;
-    FO_CHECK(T2 <= c->pos_rows, "fo_encode_offline: %d encoder frames exceed the positional table (%d)", T2, c->pos_rows);
+    FO_CHECK(T2 <= c->cfg.pos_max_len, "fo_encode_offline: %d encoder frames exceed the positional table (%d)", T2, c->cfg.pos_max_len);
     FO_CUDA(cudaSetDevice(c->device));
     cudaStream_t st = (cudaStream_t)stream;
     const void *dfeats, *dil;

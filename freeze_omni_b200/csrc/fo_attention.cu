@@ -18,7 +18,7 @@ namespace fo {
 namespace {
 
 constexpr int DK = 64;
-constexpr int TQ_MAX = 8;          // query rows per CTA (streaming chunk: 4, fork: 7)
+constexpr int TQ_MAX = STREAM_MAX_T;   // query rows per CTA (streaming chunk: 4, fork: 7)
 constexpr int ATT_THREADS = 128;
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -211,7 +211,7 @@ attention_stream_kernel(AttnStream a, const TA* __restrict__ qkv, const float* _
         *reinterpret_cast<uint4*>((which ? Vs : Ks) + (cl + r) * DK + c * EPC) = val;
         *reinterpret_cast<uint4*>((which ? ringV : ringK) + (long long)((nf + r) % cap) * DK + c * EPC) = val;
     }
-    // positions past the end of the table repeat its last row (unreachable with the reference's pe_index wrap)
+    // the table holds every position a call can reach (fo_create sizes pos_rows): this clamp only keeps reads in bounds
     for (int i = tid + np * (DK / 8); i < nk * (DK / 8); i += ATT_THREADS) {
         const int j = i / (DK / 8), c = i % (DK / 8);
         const TA* src = ptab_h + ((long long)h * a.pos_rows + a.pos_rows - 1) * DK + c * 8;
@@ -479,7 +479,7 @@ attention_stream_mma_kernel(AttnStream a, const __half* __restrict__ qkv, const 
     // zero rows of V behind the last key (they enter the PV MMAs with probability 0: they must be finite)
     for (int i = tid; i < (vrows - nk) * NCH; i += ATT_THREADS)
         *reinterpret_cast<uint4*>(Vs + (nk + i / NCH) * DK + (i % NCH) * EPC) = make_uint4(0, 0, 0, 0);
-    for (int i = tid + np * NCH; i < nk * NCH; i += ATT_THREADS) {       // positions past the table end repeat its last row
+    for (int i = tid + np * NCH; i < nk * NCH; i += ATT_THREADS) {       // in-bounds clamp only: pos_rows covers every reachable position
         const int j = i / NCH, c = i % NCH;
         *reinterpret_cast<uint4*>(Ps + j * DK + (c ^ ((start + j) & 7)) * EPC) =
             *reinterpret_cast<const uint4*>(ptab_h + ((long long)h * a.pos_rows + a.pos_rows - 1) * DK + (c ^ ((a.pos_rows - 1) & 7)) * EPC);
@@ -699,7 +699,7 @@ attention_chunks_kernel(AttnStream a, const TA* __restrict__ qkv, const float* _
         const int o = nfj - clj - first;            // staged row of this chunk's first key
         const int nk = clj + t;
         const int start = max(0, chunk_pe(pe0, j, a) - a.full_chunk);
-        for (int i = tid; i < nk * NCH; i += ATT_THREADS) {        // positions past the table end repeat its last row
+        for (int i = tid; i < nk * NCH; i += ATT_THREADS) {        // the min() keeps reads in bounds; pos_rows covers every reachable position
             const int r = i / NCH, c = i % NCH, pos = min(start + r, a.pos_rows - 1);
             *reinterpret_cast<uint4*>(Ps + r * DK + c * EPC) = *reinterpret_cast<const uint4*>(ptab_h + ((long long)h * a.pos_rows + pos) * DK + c * EPC);
         }
@@ -1434,6 +1434,14 @@ int attention_stream(const AttnStream& a, const TA* qkv, const float* q32, TA* r
             const int vrows = (rows + 15) & ~15;
             const size_t sm = (size_t)(2 * rows + vrows) * DK * 2 + (size_t)2 * a.t * DK * 2 + (size_t)a.t * vrows * 2 +
                               (size_t)a.t * std::max(vrows, DK) * 4;
+            // past 48 KB (window + t > ~115 keys, e.g. left_chunks 31) the launch needs the opt-in
+            static bool mma_attr_set = false;
+            if (!mma_attr_set) {
+                FO_CUDA(cudaFuncSetAttribute(attention_stream_mma_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
+                FO_CUDA(cudaFuncSetAttribute(attention_stream_mma_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
+                mma_attr_set = true;
+            }
+            FO_CHECK(sm <= 160 * 1024, "attention_stream: window too large for shared memory");
             if (a.nsplit > 0)
                 FO_CUDA(launch_pdl(attention_stream_mma_kernel<true>, grid, dim3(ATT_THREADS), sm, st, a, reinterpret_cast<const __half*>(qkv), q32,
                                    reinterpret_cast<__half*>(ring), reinterpret_cast<const __half*>(ptab_h), pos_u, pos_v,

@@ -26,6 +26,7 @@ void set_error(const char* fmt, ...);
         cudaError_t _e = (expr);                                                                  \
         if (_e != cudaSuccess) {                                                                  \
             fo::set_error("%s failed: %s (%s:%d)", #expr, cudaGetErrorString(_e), __FILE__, __LINE__); \
+            (void)cudaGetLastError();   /* a refused launch must not fail the next call's checks */ \
             return -2;                                                                            \
         }                                                                                         \
     } while (0)
@@ -375,6 +376,8 @@ struct AttnStream {
 };
 // staged keys of the multi-chunk attention (window + chunks * t at most): bounds the chunks of one call
 constexpr int STREAM_CHUNKS_MAX_KEYS = 128;
+// encoder frames of one streaming chunk (query rows of an attention CTA, the MMA's N); fo_create caps the context's max_t here
+constexpr int STREAM_MAX_T = 8;
 // qkv (n*t, 3*D) activation type (K and V columns are read from it); q32 (n*t, 3*D) fp32 whose first D
 // columns hold Q (the QKV GEMM keeps Q in fp32, Epilogue::split_col); ring = this layer's
 // (slot, 2, H, ring_cap, 64); ptab (pos_rows, D) fp32; out (n*t, D).  Appends the new K/V rows to the ring.

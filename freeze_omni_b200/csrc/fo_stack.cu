@@ -420,7 +420,7 @@ __device__ __forceinline__ void attn_unit(const StackArgs& p, const AttnGeom& ge
     }
     for (int i = tid; i < (vrows - nk) * 8; i += ST_THREADS)          // zero V rows behind the last key (probability 0 x finite)
         *reinterpret_cast<uint4*>(Vs + (nk + (i >> 3)) * DK + (i & 7) * 8) = make_uint4(0, 0, 0, 0);
-    for (int i = tid + np * 8; i < nk * 8; i += ST_THREADS) {          // positions past the table end repeat its last row
+    for (int i = tid + np * 8; i < nk * 8; i += ST_THREADS) {          // in-bounds clamp only: pos_rows covers every reachable position
         const int j = i >> 3, c = i & 7;
         *reinterpret_cast<uint4*>(Ps + j * DK + (c ^ ((start + j) & 7)) * 8) =
             *reinterpret_cast<const uint4*>(w.ptab_h + ((long long)h * a.pos_rows + a.pos_rows - 1) * DK + (c ^ ((a.pos_rows - 1) & 7)) * 8);

@@ -56,7 +56,6 @@ class Engine:
         self.has_encoder, self.has_adapter = enc_state is not None, adp_state is not None
         self.max_sessions = int(max_sessions)
         msf = max_stream_frames or max(cfg.chunk_feat_frames, 39)
-        self.max_t = PathConfig.sub_len(msf)
         c = _lib.FoConfig(
             feat_dim=cfg.feat_dim, d_model=cfg.d_model, n_heads=cfg.n_heads, ffn_dim=cfg.ffn_dim,
             n_layers=cfg.n_layers, chunk_size=cfg.chunk_size, left_chunks=cfg.left_chunks,
@@ -74,6 +73,7 @@ class Engine:
         _lib.check(self.lib.fo_create(C.byref(c), self.device, _lib.FO_BF16 if dtype == torch.bfloat16 else _lib.FO_F32,
                                       C.byref(h)))
         self._h = h
+        self.max_t = self.get_option("max_t")      # encoder frames per streaming chunk, capped at 8 by the library
         try:
             if self.has_encoder:
                 exp = encoder_param_shapes(cfg)

@@ -59,7 +59,8 @@ typedef struct fo_config {
     int32_t context_frames;    /* 3 */
     /* capacity */
     int32_t max_sessions;      /* session slots resident in HBM */
-    int32_t max_stream_frames; /* largest fbank-frame count of one streaming call (>= context+frames_per_chunk) */
+    int32_t max_stream_frames; /* largest fbank-frame count of one streaming call (>= context+frames_per_chunk); the encoder
+                                * frames per chunk it gives are capped at 8 (35 feature frames), what the streaming attention takes */
     /* positionwise layer: 0 or 1 = PositionwiseFeedForward (models/encoder/attention.py:122-143);
      * k >= 2 = Conv1dLinear with kernel_size k (models/encoder/attention.py:198-266): causal depthwise conv over
      * time (left context carried per session and layer) + 1x1 conv + ReLU + Linear */
@@ -156,7 +157,9 @@ int fo_fbank_offline(fo_ctx* ctx, const void* pcm, int pcm_dtype, int B, int64_t
  * starred calls of AudioLLM.recognize (models/audioLLM.py:380-387), for n sessions at once.
  * feats (n, t_in, feat_dim) or NULL = the block left in the sessions by fo_fbank_stream.
  * enc_out (n, t, d_model), adapter_out (n, t_out, llm_dim): either may be NULL.
- * t = ((t_in-1)/2-1)/2; t_out = (t + kernel-1 - kernel)/2 + 1. */
+ * t = ((t_in-1)/2-1)/2; t_out = (t + kernel-1 - kernel)/2 + 1.
+ * Every streaming entry refuses (FO_ERR_ARG, nothing enqueued, no session advanced) a context with chunk_size <= 0 (full
+ * attention: fo_encode_offline only), t beyond the context's max_t (<= 8), and window + t > 128 keys (e.g. left_chunks 32). */
 int fo_encode_stream(fo_ctx* ctx, const int32_t* ids, int n, const float* feats, int t_in,
                      float* enc_out, float* adapter_out, void* stream);
 /* k consecutive chunks per session in one call, equal to k successive fo_encode_stream calls of one chunk each

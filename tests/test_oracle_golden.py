@@ -1,5 +1,7 @@
 """Pin the CPU oracle to the vectors produced by the reference modules (tests/golden/make_golden.py).
 These run without a GPU."""
+import dataclasses
+
 import numpy as np
 import pytest
 import torch
@@ -165,6 +167,30 @@ def test_tiny_stream_equals_offline_until_saturation(golden, tiny):
     diff = (xs[0, :n].reshape(-1, 4, cfg.d_model) - st).abs().amax(dim=(1, 2))
     assert float(diff[:17].max()) < 1e-4
     assert float(diff[17:].max()) > 1e-4
+
+
+@pytest.mark.parametrize("C,L", [(4, 16), (4, 2), (3, 1), (3, 5), (2, 8), (1, 16), (8, 8), (4, 31)])
+def test_tiny_stream_equals_offline_until_saturation_other_chunkings(tiny, C, L):
+    """The property above at every chunking the streaming GPU tests run, on seeded features: chunk i is the block
+    F[4C*i : 4C*i + 4C + 3] (t_in = 4C + 3 gives t = C frames, offline frames [C*i, C*i + C)).  Streaming equals
+    forward(C, L) for chunks 0..L, while the cache fills; from chunk L+1 on the rel-pos rows start one chunk behind the
+    keys (SURVEY 2.4-1) and every chunk differs."""
+    base, esd, _ = tiny
+    cfg = dataclasses.replace(base, chunk_size=C, left_chunks=L)
+    n_chunks = L + 4
+    g = torch.Generator().manual_seed(100 * C + L)
+    feats = 9.0 + 3.0 * torch.randn(1, 4 * C * n_chunks + 3, cfg.feat_dim, generator=g)
+    enc = O.EncoderOracle(cfg, esd)
+    xs, _ = enc.forward(feats, torch.tensor([feats.size(1)]), C, L)
+    assert xs.size(1) >= C * n_chunks
+    buf, pe = enc.new_buffer(), 0
+    diff = []
+    for i in range(n_chunks):
+        out, buf, pe = enc.infer(feats[:, 4 * C * i:4 * C * i + 4 * C + 3], buf, pe)
+        assert out.shape == (1, C, cfg.d_model)
+        diff.append(float((out[0] - xs[0, C * i:C * (i + 1)]).abs().max()))
+    assert max(diff[:L + 1]) < 1e-4, diff
+    assert min(diff[L + 1:]) > 1e-4, diff
 
 
 # ---- conv1d-linear positionwise variant (Conv1dLinear, attention.py:198-266) -------------------------------------
