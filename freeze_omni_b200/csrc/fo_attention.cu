@@ -3,141 +3,45 @@
 //     score[i][j] = ((q_i + u) . K_j + (q_i + v) . P[pos_j]) / sqrt(d_k),   softmax over j,   out = sum_j p_ij V_j
 // d_k is 64.  Streaming: one CTA per (session, head); the cached K/V rows come from the session's ring in
 // HBM with cp.async.bulk (TMA bulk copy, mbarrier completion) while the chunk's own rows arrive from the
-// fused QKV GEMM output and are appended to the ring in the same pass.  Offline: one CTA per
-// (utterance, head, 4 query rows); the band [start,end) of models/masks.py:50-56 and the pad mask are
-// evaluated arithmetically, never materialised; key tiles + online softmax cover unbounded left context.
+// fused QKV GEMM output and are appended to the ring.  The four streaming kernels (one chunk or several, fp16 or fp32)
+// differ in how they stage the rows; the per-chunk math is attn_chunk_mma / attn_chunk_ffma (fo_attn_core.cuh).
+// Offline: one CTA per (utterance, head, query block); the band [start,end) of models/masks.py:50-56 and the pad mask
+// are evaluated arithmetically, never materialised; key tiles + online softmax cover unbounded left context.
 #include <stdlib.h>
 
 #include <algorithm>
+#include <array>
 
-#include "fo_common.cuh"
+#include "fo_attn_core.cuh"
 
 namespace fo {
 
 
 namespace {
 
-constexpr int DK = 64;
-constexpr int TQ_MAX = STREAM_MAX_T;   // query rows per CTA (streaming chunk: 4, fork: 7)
 constexpr int ATT_THREADS = 128;
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* bar, int count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "WAIT_LOOP:\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-        "@p bra DONE;\n\t"
-        "bra WAIT_LOOP;\n\t"
-        "DONE:\n\t}" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(void* dst, const void* src, uint32_t bytes, uint64_t* bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                     smem_u32(dst)),
-                 "l"(src), "r"(bytes), "r"(smem_u32(bar))
-                 : "memory");
-}
-
-template <typename TA> struct Chunk;        // one 16-byte slice of a 64-wide row
-template <> struct Chunk<float> {
-    static constexpr int EPC = 4, NCH = 16;
-    static __device__ __forceinline__ void load(const float* p, float (&v)[4]) {
-        float4 t = *reinterpret_cast<const float4*>(p);
-        v[0] = t.x; v[1] = t.y; v[2] = t.z; v[3] = t.w;
-    }
-};
-template <> struct Chunk<__half> {
-    static constexpr int EPC = 8, NCH = 8;
-    static __device__ __forceinline__ void load(const __half* p, float (&v)[8]) {
-        uint4 t = *reinterpret_cast<const uint4*>(p);
-        const __half2* h = reinterpret_cast<const __half2*>(&t);
-#pragma unroll
-        for (int i = 0; i < 4; ++i) { const float2 f = __half22float2(h[i]); v[2 * i] = f.x; v[2 * i + 1] = f.y; }
-    }
-};
-template <> struct Chunk<bf16> {
-    static constexpr int EPC = 8, NCH = 8;
-    static __device__ __forceinline__ void load(const bf16* p, float (&v)[8]) {
-        uint4 t = *reinterpret_cast<const uint4*>(p);
-        const __nv_bfloat162* h = reinterpret_cast<const __nv_bfloat162*>(&t);
-#pragma unroll
-        for (int i = 0; i < 4; ++i) { v[2 * i] = __low2float(h[i]); v[2 * i + 1] = __high2float(h[i]); }
-    }
-};
-
-// scores of key row j (smem) against nq query rows; chunk order is rotated by j so that the 8 lanes of
-// one shared-memory phase touch 8 different 16-byte bank groups (rows are 128 B / 256 B apart).
-template <typename TA>
-__device__ __forceinline__ void score_row(const TA* Krow, const TA* Prow, const float* qu, const float* qv, int nq,
-                                          int rot, float (&acc)[TQ_MAX]) {
-    constexpr int EPC = Chunk<TA>::EPC, NCH = Chunk<TA>::NCH;
-#pragma unroll
-    for (int i = 0; i < TQ_MAX; ++i) acc[i] = 0.f;
-#pragma unroll 2
-    for (int c = 0; c < NCH; ++c) {
-        const int cc = (c + rot) & (NCH - 1);
-        float kv[EPC], pv[EPC];
-        Chunk<TA>::load(Krow + cc * EPC, kv);
-        Chunk<TA>::load(Prow + cc * EPC, pv);
-#pragma unroll
-        for (int i = 0; i < TQ_MAX; ++i) {
-            if (i < nq) {
-                const float* a = qu + i * DK + cc * EPC;
-                const float* b = qv + i * DK + cc * EPC;
-                float s = acc[i];
-#pragma unroll
-                for (int e = 0; e < EPC; ++e) s = fmaf(a[e], kv[e], fmaf(b[e], pv[e], s));
-                acc[i] = s;
-            }
-        }
-    }
-}
-
-__device__ __forceinline__ float warp_max(float v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
-    return v;
-}
-__device__ __forceinline__ float warp_sum(float v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
-}
-
 // ---------------------------------------------------------------------------------------------
-// Streaming chunk attention (fp32 contexts; the fp16 variant below runs the contractions on mma.sync), one CTA per
-// (session, head), 4 warps.  Steady state: 64 cached + 4 new keys, 4 queries.
-//   load   thread 0 starts the bulk copies of the ring's K/V rows (HBM -> smem, mbarrier); meanwhile every thread
-//          fetches its share of the chunk's own K/V rows (appended to the ring in the same pass), the rel-pos rows
-//          P_l[start + j] and Q, all issued before the first use so that one memory latency covers them
-//   score  warp = query row, lane = keys lane, lane+32, lane+64: ((q+u).K_j + (q+v).P_j)/8 with the 16-byte chunks
-//          of a row visited in a lane-rotated order (conflict-free); scores stay in registers
-//   soft   warp-shuffle max / sum in fp32, probabilities to a 1 KB smem strip
-//   PV     lane = output dims (2*lane, 2*lane+1), loop over the keys
-// smem rows are sized by window + t (68), not by the ring capacity, so 7 CTAs fit per SM and the 1024 CTAs of a
-// 64-session layer are ONE wave.
-template <typename TA>
+// Single-chunk streaming attention of fp32 contexts (k = 1), one CTA per (session, head), 4 warps.  Steady state: 64 cached
+// + 4 new keys, 4 queries.  Staging: thread 0 starts the bulk copies of the ring window and of the rel-pos rows
+// P_l[start .. start+nk) (HBM -> smem, mbarrier); meanwhile every thread fetches its share of the chunk's own K/V rows
+// (appended to the ring in the same pass) and Q, all issued before the first use so that one memory latency covers them.
+// smem rows are sized by window + t (68), not by the ring capacity.
 __global__ void __launch_bounds__(ATT_THREADS, 7)
-attention_stream_kernel(AttnStream a, const TA* __restrict__ qkv, const float* __restrict__ q32, TA* __restrict__ ring,
-                        const TA* __restrict__ ptab_h, const float* __restrict__ pos_u, const float* __restrict__ pos_v,
-                        TA* __restrict__ out) {
+attention_stream_kernel(AttnStream a, const float* __restrict__ qkv, const float* __restrict__ q32, float* __restrict__ ring,
+                        const float* __restrict__ ptab_h, const float* __restrict__ pos_u, const float* __restrict__ pos_v,
+                        float* __restrict__ out) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
-    constexpr int EPC = Chunk<TA>::EPC, NCH = Chunk<TA>::NCH;
+    constexpr int EPC = 4, NCH = DK / EPC;
     FO_PDL_TRIGGER();
     FO_PDL_WAIT();
     const int cap = a.ring_cap;
     const int t = a.t, D = a.H * DK;
     const int rows = a.window + t;                  // most keys a call can see
-    TA* Ks = reinterpret_cast<TA*>(smem_raw);
-    TA* Vs = Ks + rows * DK;
-    TA* Ps = Vs + rows * DK;                        // rel-pos rows, rounded from the fp32 table to the activation type
-    float* qu = reinterpret_cast<float*>(Ps + rows * DK);
+    float* Ks = reinterpret_cast<float*>(smem_raw);
+    float* Vs = Ks + rows * DK;
+    float* Ps = Vs + rows * DK;
+    float* qu = Ps + rows * DK;
     float* qv = qu + t * DK;
     float* prob = qv + t * DK;                      // t x rows
     __shared__ __align__(8) uint64_t bar;
@@ -150,35 +54,23 @@ attention_stream_kernel(AttnStream a, const TA* __restrict__ qkv, const float* _
     const int nk = cl + t;
     const int pe = a.pe_index[slot] % a.pe_wrap;
     const int start = max(0, pe - a.full_chunk);     // attention.py:112-114
-    TA* ringK = ring + (long long)slot * a.ring_slot_stride + (long long)h * cap * DK;
-    TA* ringV = ringK + (long long)a.H * cap * DK;
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    float* ringK = ring + (long long)slot * a.ring_slot_stride + (long long)h * cap * DK;
+    float* ringV = ringK + (long long)a.H * cap * DK;
+    const int tid = threadIdx.x;
 
     // rel-pos rows P_l[start .. start+nk) of this head are contiguous in the head-major table: one bulk copy
     const int np = min(nk, a.pos_rows - start);
     if (tid == 0) {
         mbar_init(&bar, 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        const int p0 = first % cap;
-        const int len1 = min(cl, cap - p0), len2 = cl - len1;
-        const uint32_t rowb = DK * sizeof(TA);
-        mbar_expect_tx(&bar, (2u * cl + np) * rowb);
-        bulk_g2s(Ps, ptab_h + ((long long)h * a.pos_rows + start) * DK, np * rowb, &bar);
-        if (len1 > 0) {
-            bulk_g2s(Ks, ringK + (long long)p0 * DK, len1 * rowb, &bar);
-            bulk_g2s(Vs, ringV + (long long)p0 * DK, len1 * rowb, &bar);
-        }
-        if (len2 > 0) {
-            bulk_g2s(Ks + len1 * DK, ringK, len2 * rowb, &bar);
-            bulk_g2s(Vs + len1 * DK, ringV, len2 * rowb, &bar);
-        }
+        ring_window_copy(ringK, ringV, cap, first, cl, Ks, Vs, ptab_h + ((long long)h * a.pos_rows + start) * DK, Ps, np, &bar);
     }
     // ---- loads into registers (no dependent use before they are all issued) ----
     // (a) chunk's own K/V rows: t rows x NCH chunks x {K,V}
     const int n_new = t * NCH * 2;
     uint4 newv = make_uint4(0, 0, 0, 0);
     int new_which = 0, new_r = 0, new_c = 0;
-    const bool has_new = tid < n_new;                // t <= 8, NCH <= 16: n_new <= 256 -> second slot below
+    const bool has_new = tid < n_new;                // t <= 4: one slot per thread, more rows in the loop below
     if (has_new) {
         new_which = tid / (t * NCH);
         new_r = (tid / NCH) % t;
@@ -200,12 +92,12 @@ attention_stream_kernel(AttnStream a, const TA* __restrict__ qkv, const float* _
     l2_prefetch_slice(a.prefetch, blockIdx.y * gridDim.x + blockIdx.x, gridDim.x * gridDim.y, tid, ATT_THREADS);
     // ---- registers -> smem / ring ----
     if (has_new) {
-        TA* sdst = (new_which ? Vs : Ks) + (cl + new_r) * DK + new_c * EPC;
+        float* sdst = (new_which ? Vs : Ks) + (cl + new_r) * DK + new_c * EPC;
         *reinterpret_cast<uint4*>(sdst) = newv;
-        TA* gdst = (new_which ? ringV : ringK) + (long long)((nf + new_r) % cap) * DK + new_c * EPC;
+        float* gdst = (new_which ? ringV : ringK) + (long long)((nf + new_r) % cap) * DK + new_c * EPC;
         *reinterpret_cast<uint4*>(gdst) = newv;
     }
-    for (int i = tid + ATT_THREADS; i < n_new; i += ATT_THREADS) {      // only when t*NCH*2 > 128 (fp32 context or t > 8)
+    for (int i = tid + ATT_THREADS; i < n_new; i += ATT_THREADS) {      // only when t > 4
         const int which = i / (t * NCH), r = (i / NCH) % t, c = i % NCH;
         const uint4 val = *reinterpret_cast<const uint4*>(qkv + (long long)(b * t + r) * 3 * D + (which + 1) * D + h * DK + c * EPC);
         *reinterpret_cast<uint4*>((which ? Vs : Ks) + (cl + r) * DK + c * EPC) = val;
@@ -214,7 +106,7 @@ attention_stream_kernel(AttnStream a, const TA* __restrict__ qkv, const float* _
     // the table holds every position a call can reach (fo_create sizes pos_rows): this clamp only keeps reads in bounds
     for (int i = tid + np * (DK / 8); i < nk * (DK / 8); i += ATT_THREADS) {
         const int j = i / (DK / 8), c = i % (DK / 8);
-        const TA* src = ptab_h + ((long long)h * a.pos_rows + a.pos_rows - 1) * DK + c * 8;
+        const float* src = ptab_h + ((long long)h * a.pos_rows + a.pos_rows - 1) * DK + c * 8;
 #pragma unroll
         for (int e = 0; e < 8; ++e) Ps[j * DK + c * 8 + e] = src[e];
     }
@@ -231,105 +123,9 @@ attention_stream_kernel(AttnStream a, const TA* __restrict__ qkv, const float* _
     }
     __syncthreads();
     mbar_wait(&bar, 0);
-
-    // ---- scores + softmax + PV: warp = query row ----
-    constexpr int KPL = 4;                                // keys per lane (<= 128 keys per call)
-    for (int i = warp; i < t; i += ATT_THREADS / 32) {
-        const float* qui = qu + i * DK;
-        const float* qvi = qv + i * DK;
-        float sc[KPL];
-#pragma unroll
-        for (int k = 0; k < KPL; ++k) sc[k] = 0.f;
-#pragma unroll 2
-        for (int c = 0; c < NCH; ++c) {
-            const int cc = (c + lane) & (NCH - 1);
-            float au[EPC], av[EPC];
-#pragma unroll
-            for (int e = 0; e < EPC; e += 4) {
-                const float4 x = *reinterpret_cast<const float4*>(qui + cc * EPC + e);
-                const float4 y = *reinterpret_cast<const float4*>(qvi + cc * EPC + e);
-                au[e] = x.x; au[e + 1] = x.y; au[e + 2] = x.z; au[e + 3] = x.w;
-                av[e] = y.x; av[e + 1] = y.y; av[e + 2] = y.z; av[e + 3] = y.w;
-            }
-#pragma unroll
-            for (int k = 0; k < KPL; ++k) {
-                const int j = lane + 32 * k;
-                if (j < nk) {
-                    float kv[EPC], pp[EPC];
-                    Chunk<TA>::load(Ks + j * DK + cc * EPC, kv);
-                    Chunk<TA>::load(Ps + j * DK + cc * EPC, pp);
-                    float s = sc[k];
-#pragma unroll
-                    for (int e = 0; e < EPC; ++e) s = fmaf(au[e], kv[e], fmaf(av[e], pp[e], s));
-                    sc[k] = s;
-                }
-            }
-        }
-        float m = -INFINITY;
-#pragma unroll
-        for (int k = 0; k < KPL; ++k) {
-            sc[k] = (lane + 32 * k < nk) ? sc[k] * 0.125f : -INFINITY;
-            m = fmaxf(m, sc[k]);
-        }
-        m = warp_max(m);
-        float ssum = 0.f;
-        float* pr = prob + i * rows;
-#pragma unroll
-        for (int k = 0; k < KPL; ++k) {
-            const int j = lane + 32 * k;
-            if (j < nk) {
-                const float e = __expf(sc[k] - m);
-                pr[j] = e;
-                ssum += e;
-            }
-        }
-        for (int j = lane + 32 * KPL; j < nk; j += 32) pr[j] = 0.f;      // unreachable for nk <= 128 (checked on the host)
-        ssum = warp_sum(ssum);
-        __syncwarp();
-        const float inv = 1.f / ssum;
-        float o0 = 0.f, o1 = 0.f;
-        if constexpr (sizeof(TA) == 2) {
-            const uint32_t* vp = reinterpret_cast<const uint32_t*>(Vs) + lane;
-#pragma unroll 4
-            for (int j = 0; j < nk; ++j) {
-                const float p = pr[j];
-                const float2 vv = unpack2<TA>(vp[j * (DK / 2)]);
-                o0 = fmaf(p, vv.x, o0);
-                o1 = fmaf(p, vv.y, o1);
-            }
-        } else {
-#pragma unroll 4
-            for (int j = 0; j < nk; ++j) {
-                const float p = pr[j];
-                o0 = fmaf(p, to_f(Vs[j * DK + 2 * lane]), o0);
-                o1 = fmaf(p, to_f(Vs[j * DK + 2 * lane + 1]), o1);
-            }
-        }
-        TA* o = out + (long long)(b * t + i) * D + h * DK + 2 * lane;
-        if constexpr (sizeof(TA) == 2) {
-            *reinterpret_cast<uint32_t*>(o) = pack2<TA>(o0 * inv, o1 * inv);
-        } else {
-            o[0] = from_f<TA>(o0 * inv);
-            o[1] = from_f<TA>(o1 * inv);
-        }
-    }
+    attn_chunk_ffma(Ks, Vs, Ps, qu, qv, prob, rows, nk, t, out + (long long)b * t * D + h * DK, D);
 }
 
-// ---------------------------------------------------------------------------------------------
-// fp16 variant of the streaming kernel with the two small contractions on the legacy tensor-core path
-// (mma.sync.m16n8k16, fp32 accumulate; the attention core is 1 % of the FLOPs, far too small for tcgen05):
-//   S^T (keys x queries) = K (keys x 64) . (q+u)^T  +  P (keys x 64) . (q+v)^T     key tiles of 16 over the 4 warps
-//   O^T (64 x queries)   = V^T (64 x keys) . prob^T                                   one 16-dim tile per warp
-// With 4 query rows the scalar kernel spends ~13 k FMA/convert instructions per CTA on these; here they are ~60 MMAs.
-// Loads, ring append, masking, fp32 softmax and the outputs are as in attention_stream_kernel.  (q+u), (q+v) and the
-// normalised probabilities are rounded to fp16 for the MMAs.
-__device__ __forceinline__ void mma16816(float (&d)[4], const uint32_t (&a)[4], const uint32_t (&b)[2]) {
-    asm volatile(
-        "mma.sync.aligned.m16n8k16.row.col.f32.f16.f16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-        : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
-        : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b[0]), "r"(b[1]));
-}
-__device__ __forceinline__ uint32_t lds32(const __half* p) { return *reinterpret_cast<const uint32_t*>(p); }
 #ifdef FO_TC_TRACE_BUILD
 __device__ unsigned long long g_attn_trace[16];
 #define AT_TRACE(slot)                                                                                   \
@@ -344,7 +140,14 @@ __device__ unsigned long long g_attn_trace[16];
 #define AT_TRACE(slot) do { } while (0)
 #endif
 
-template <bool DEFER>            // DEFER: q / k / v of the chunk are summed from the QKV GEMM's split-K partials (AttnStream::part)
+// ---------------------------------------------------------------------------------------------
+// Single-chunk streaming attention of fp16 contexts (k = 1), the contractions on mma.sync (attn_chunk_mma).  With 4 query
+// rows the scalar form spends ~13 k FMA/convert instructions per CTA on them; here they are ~60 MMAs.  Staging: the ring
+// window and rel-pos bulk copies are issued BEFORE the dependency wait, the chunk's own K/V rows are appended to the ring
+// in the same pass, and with DEFER q / k / v are summed from the QKV GEMM's split-K partials (AttnStream::part).  Shared
+// memory is sized by window + t (mma_unit_layout: 30,592 B at 64 + 4 keys), so 7 CTAs fit per SM and the 1024 CTAs of a
+// 64-session layer are ONE wave.  (q+u), (q+v) are rounded to fp16 for the MMAs.
+template <bool DEFER>
 __global__ void __launch_bounds__(ATT_THREADS, 7)
 attention_stream_mma_kernel(AttnStream a, const __half* __restrict__ qkv, const float* __restrict__ q32,
                             __half* __restrict__ ring, const __half* __restrict__ ptab_h, const float* __restrict__ pos_u,
@@ -363,15 +166,15 @@ attention_stream_mma_kernel(AttnStream a, const __half* __restrict__ qkv, const 
     AT_TRACE(1);
     const int cap = a.ring_cap;
     const int t = a.t, D = a.H * DK;
-    const int rows = a.window + t;                  // K / P rows held; a partial last key tile reads on into the next
-    const int vrows = (rows + 15) & ~15;            // array (finite or masked); V is padded with zero rows instead
+    const MmaUnitLayout lay = mma_unit_layout(a.window, t);
+    const int vrows = lay.vrows;
     TA* Ks = reinterpret_cast<TA*>(smem_raw);
-    TA* Ps = Ks + rows * DK;
-    TA* Vs = Ps + rows * DK;
-    TA* quh = Vs + vrows * DK;                      // (q+u), (q+v) as fp16, t x 64 each
-    TA* qvh = quh + t * DK;
-    TA* ph = qvh + t * DK;                          // normalised probabilities, t x vrows
-    float* sc = reinterpret_cast<float*>(ph + t * vrows);   // scores t x vrows (fp32); later the output tile t x 64
+    TA* Ps = reinterpret_cast<TA*>(smem_raw + lay.p);
+    TA* Vs = reinterpret_cast<TA*>(smem_raw + lay.v);
+    TA* quh = reinterpret_cast<TA*>(smem_raw + lay.qu);
+    TA* qvh = reinterpret_cast<TA*>(smem_raw + lay.qv);
+    TA* ph = reinterpret_cast<TA*>(smem_raw + lay.ph);
+    float* sc = reinterpret_cast<float*>(smem_raw + lay.sc);
     __shared__ __align__(8) uint64_t bar;
 
     const int b = blockIdx.x, h = blockIdx.y;
@@ -384,37 +187,18 @@ attention_stream_mma_kernel(AttnStream a, const __half* __restrict__ qkv, const 
     const int start = max(0, pe - a.full_chunk);     // attention.py:112-114
     TA* ringK = ring + (long long)slot * a.ring_slot_stride + (long long)h * cap * DK;
     TA* ringV = ringK + (long long)a.H * cap * DK;
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const int tid = threadIdx.x;
 
     const int np = min(nk, a.pos_rows - start);
     AT_TRACE(2);
     if (tid == 0) {
         mbar_init(&bar, 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        const int p0 = first % cap;
-        const int len1 = min(cl, cap - p0), len2 = cl - len1;
-        const uint32_t rowb = DK * sizeof(TA);
-        mbar_expect_tx(&bar, (2u * cl + np) * rowb);
-        bulk_g2s(Ps, ptab_h + ((long long)h * a.pos_rows + start) * DK, np * rowb, &bar);
-        if (len1 > 0) {
-            bulk_g2s(Ks, ringK + (long long)p0 * DK, len1 * rowb, &bar);
-            bulk_g2s(Vs, ringV + (long long)p0 * DK, len1 * rowb, &bar);
-        }
-        if (len2 > 0) {
-            bulk_g2s(Ks + len1 * DK, ringK, len2 * rowb, &bar);
-            bulk_g2s(Vs + len1 * DK, ringV, len2 * rowb, &bar);
-        }
+        ring_window_copy(ringK, ringV, cap, first, cl, Ks, Vs, ptab_h + ((long long)h * a.pos_rows + start) * DK, Ps, np, &bar);
     }
     AT_TRACE(3);
-    float ureg[4], vreg[4];
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-        const int i = tid + k * ATT_THREADS;
-        if (i < t * DK) {
-            ureg[k] = pos_u[h * DK + i % DK];
-            vreg[k] = pos_v[h * DK + i % DK];
-        }
-    }
+    // bias of dimension tid % 64: the same for every Q element this thread stages below (ATT_THREADS is a multiple of 64)
+    const float ub = pos_u[h * DK + tid % DK], vb = pos_v[h * DK + tid % DK];
     FO_PDL_WAIT();                                  // from here on: the QKV GEMM's output
     if (threadIdx.x == 0) FO_TR_STAMP(1);
     // chunk's own K/V rows -> registers
@@ -452,9 +236,9 @@ attention_stream_mma_kernel(AttnStream a, const __half* __restrict__ qkv, const 
         new_c = tid % NCH;
         newv = load_new(new_which, new_r, new_c);
     }
-    float qreg[4];
+    float qreg[2];                                  // Q of t <= 4 rows; more rows are loaded where they are stored
 #pragma unroll
-    for (int k = 0; k < 4; ++k) {
+    for (int k = 0; k < 2; ++k) {
         const int i = tid + k * ATT_THREADS;
         if (i < t * DK) {
             const int r = i / DK, d = i % DK;
@@ -485,16 +269,16 @@ attention_stream_mma_kernel(AttnStream a, const __half* __restrict__ qkv, const 
             *reinterpret_cast<const uint4*>(ptab_h + ((long long)h * a.pos_rows + a.pos_rows - 1) * DK + (c ^ ((a.pos_rows - 1) & 7)) * EPC);
     }
 #pragma unroll
-    for (int k = 0; k < 4; ++k) {
+    for (int k = 0; k < 2; ++k) {
         const int i = tid + k * ATT_THREADS;
         if (i < t * DK) {
             const int r = i / DK, d = i % DK;
             const int o = r * DK + (((d >> 3) ^ (r & 7)) << 3) + (d & 7);      // same chunk swizzle, keyed by the query row
-            quh[o] = from_f<TA>(qreg[k] + ureg[k]);
-            qvh[o] = from_f<TA>(qreg[k] + vreg[k]);
+            quh[o] = from_f<TA>(qreg[k] + ub);
+            qvh[o] = from_f<TA>(qreg[k] + vb);
         }
     }
-    for (int i = tid + 4 * ATT_THREADS; i < t * DK; i += ATT_THREADS) {
+    for (int i = tid + 2 * ATT_THREADS; i < t * DK; i += ATT_THREADS) {
         const int r = i / DK, d = i % DK;
         const float q = load_q(r, d);
         const int o = r * DK + (((d >> 3) ^ (r & 7)) << 3) + (d & 7);
@@ -506,98 +290,7 @@ attention_stream_mma_kernel(AttnStream a, const __half* __restrict__ qkv, const 
     mbar_wait(&bar, 0);
     AT_TRACE(5);
     if (threadIdx.x == 0) FO_TR_STAMP(2);
-
-    const int g = lane >> 2, c = lane & 3;
-    // ---- scores: S^T tile (16 keys x 8 queries) per MMA chain ----
-    for (int k0 = warp * 16; k0 < nk; k0 += 16 * (ATT_THREADS / 32)) {
-        float d[4] = {0.f, 0.f, 0.f, 0.f};
-        // swizzle keys of the rows this lane reads: K rows by frame number, P rows by position, q rows by query index
-        const int kk0 = (first + k0 + g) & 7, kk1 = (first + k0 + g + 8) & 7;
-        const int kp0 = (start + k0 + g) & 7, kp1 = (start + k0 + g + 8) & 7;
-        const TA* kr0 = Ks + (k0 + g) * DK + c * 2;
-        const TA* kr1 = Ks + (k0 + g + 8) * DK + c * 2;
-        const TA* pr0 = Ps + (k0 + g) * DK + c * 2;
-        const TA* pr1 = Ps + (k0 + g + 8) * DK + c * 2;
-#pragma unroll
-        for (int ks = 0; ks < DK / 16; ++ks) {
-            const int c0 = ks * 2, c1 = ks * 2 + 1;                 // the two 16-byte chunks of this k step
-            uint32_t af[4], bf[2];
-            af[0] = lds32(kr0 + ((c0 ^ kk0) << 3));
-            af[1] = lds32(kr1 + ((c0 ^ kk1) << 3));
-            af[2] = lds32(kr0 + ((c1 ^ kk0) << 3));
-            af[3] = lds32(kr1 + ((c1 ^ kk1) << 3));
-            bf[0] = g < t ? lds32(quh + g * DK + ((c0 ^ g) << 3) + c * 2) : 0u;
-            bf[1] = g < t ? lds32(quh + g * DK + ((c1 ^ g) << 3) + c * 2) : 0u;
-            mma16816(d, af, bf);
-            af[0] = lds32(pr0 + ((c0 ^ kp0) << 3));
-            af[1] = lds32(pr1 + ((c0 ^ kp1) << 3));
-            af[2] = lds32(pr0 + ((c1 ^ kp0) << 3));
-            af[3] = lds32(pr1 + ((c1 ^ kp1) << 3));
-            bf[0] = g < t ? lds32(qvh + g * DK + ((c0 ^ g) << 3) + c * 2) : 0u;
-            bf[1] = g < t ? lds32(qvh + g * DK + ((c1 ^ g) << 3) + c * 2) : 0u;
-            mma16816(d, af, bf);
-        }
-        const int q0 = c * 2;
-        if (q0 < t) { sc[q0 * vrows + k0 + g] = d[0] * 0.125f; sc[q0 * vrows + k0 + g + 8] = d[2] * 0.125f; }
-        if (q0 + 1 < t) { sc[(q0 + 1) * vrows + k0 + g] = d[1] * 0.125f; sc[(q0 + 1) * vrows + k0 + g + 8] = d[3] * 0.125f; }
-    }
-    __syncthreads();
-    AT_TRACE(6);
-    // ---- softmax (fp32), probabilities normalised and rounded to fp16 ----
-    for (int i = warp; i < t; i += ATT_THREADS / 32) {
-        float sv[4];
-        float m = -INFINITY;
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            const int j = lane + 32 * k;
-            sv[k] = j < nk ? sc[i * vrows + j] : -INFINITY;
-            m = fmaxf(m, sv[k]);
-        }
-        m = warp_max(m);
-        float ssum = 0.f;
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            sv[k] = (lane + 32 * k < nk) ? __expf(sv[k] - m) : 0.f;
-            ssum += sv[k];
-        }
-        ssum = warp_sum(ssum);
-        const float inv = 1.f / ssum;
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            const int j = lane + 32 * k;
-            if (j < vrows) ph[i * vrows + j] = __float2half_rn(sv[k] * inv);
-        }
-    }
-    __syncthreads();
-    AT_TRACE(7);
-    // ---- PV: O^T tile (16 dims x 8 queries) per warp ----
-    {
-        float d[4] = {0.f, 0.f, 0.f, 0.f};
-        const int dim0 = warp * 16;
-        const int mi = lane >> 3, r = lane & 7;
-        for (int key0 = 0; key0 < nk; key0 += 16) {
-            uint32_t af[4], bf[2];
-            const int vrow = key0 + r + ((mi & 2) ? 8 : 0);
-            const TA* ap = Vs + vrow * DK + ((((dim0 >> 3) + (mi & 1)) ^ ((first + vrow) & 7)) << 3);
-            const uint32_t saddr = smem_u32(ap);
-            asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0,%1,%2,%3}, [%4];"
-                         : "=r"(af[0]), "=r"(af[1]), "=r"(af[2]), "=r"(af[3])
-                         : "r"(saddr));
-            bf[0] = g < t ? lds32(ph + g * vrows + key0 + c * 2) : 0u;
-            bf[1] = g < t ? lds32(ph + g * vrows + key0 + 8 + c * 2) : 0u;
-            mma16816(d, af, bf);
-        }
-        const int q0 = c * 2;
-        if (q0 < t) { sc[q0 * DK + dim0 + g] = d[0]; sc[q0 * DK + dim0 + g + 8] = d[2]; }
-        if (q0 + 1 < t) { sc[(q0 + 1) * DK + dim0 + g] = d[1]; sc[(q0 + 1) * DK + dim0 + g + 8] = d[3]; }
-    }
-    __syncthreads();
-    AT_TRACE(8);
-    for (int i = tid; i < t * (DK / 2); i += ATT_THREADS) {
-        const int q = i / (DK / 2), pr = i % (DK / 2);
-        *reinterpret_cast<uint32_t*>(out + (long long)(b * t + q) * D + h * DK + 2 * pr) =
-            pack2<__half>(sc[q * DK + 2 * pr], sc[q * DK + 2 * pr + 1]);
-    }
+    attn_chunk_mma<ATT_THREADS / 32>(Ks, Vs, first, Ps, start, quh, qvh, ph, sc, vrows, nk, t, out + (long long)b * t * D + h * DK, D);
     AT_TRACE(9);
     if (threadIdx.x == 0) { FO_TR_STAMP(3); FO_TR_STAMP(4); FO_TR_FLUSH(2, 0); }
 }
@@ -643,39 +336,23 @@ __device__ __forceinline__ void chunks_append_ring(const AttnStream& a, const TA
             *reinterpret_cast<const uint4*>((which ? Vs : Ks) + (cl + r) * DK + c * EPC);
     }
 }
-__device__ __forceinline__ void chunks_start_ring_copy(const void* ringK, const void* ringV, void* Ks, void* Vs, int first, int cl,
-                                                       int cap, uint32_t rowb, uint64_t* bar) {
-    mbar_init(bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    const int p0 = first % cap;
-    const int len1 = min(cl, cap - p0), len2 = cl - len1;
-    mbar_expect_tx(bar, 2u * cl * rowb);
-    if (len1 > 0) {
-        bulk_g2s(Ks, (const char*)ringK + (long long)p0 * rowb, len1 * rowb, bar);
-        bulk_g2s(Vs, (const char*)ringV + (long long)p0 * rowb, len1 * rowb, bar);
-    }
-    if (len2 > 0) {
-        bulk_g2s((char*)Ks + len1 * rowb, ringK, len2 * rowb, bar);
-        bulk_g2s((char*)Vs + len1 * rowb, ringV, len2 * rowb, bar);
-    }
-}
 
-// fp32 (parity) form: scalar FFMA contractions as in attention_stream_kernel
-template <typename TA>
+// Multi-chunk streaming attention of fp32 contexts.  Staging: the ring window and the call's k*t new rows once, the ring
+// append after the window has landed, the rel-pos rows and Q of every chunk re-staged before its core (attn_chunk_ffma).
 __global__ void __launch_bounds__(ATT_THREADS)
-attention_chunks_kernel(AttnStream a, const TA* __restrict__ qkv, const float* __restrict__ q32, TA* __restrict__ ring,
-                        const TA* __restrict__ ptab_h, const float* __restrict__ pos_u, const float* __restrict__ pos_v,
-                        TA* __restrict__ out) {
+attention_chunks_kernel(AttnStream a, const float* __restrict__ qkv, const float* __restrict__ q32, float* __restrict__ ring,
+                        const float* __restrict__ ptab_h, const float* __restrict__ pos_u, const float* __restrict__ pos_v,
+                        float* __restrict__ out) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
-    constexpr int EPC = Chunk<TA>::EPC, NCH = Chunk<TA>::NCH;
+    constexpr int EPC = 4, NCH = DK / EPC;
     FO_PDL_TRIGGER();
     FO_PDL_WAIT();
     const int cap = a.ring_cap, t = a.t, kt = a.chunks * t, D = a.H * DK;
     const int rows = a.window + kt, prow = a.window + t;
-    TA* Ks = reinterpret_cast<TA*>(smem_raw);
-    TA* Vs = Ks + rows * DK;
-    TA* Ps = Vs + rows * DK;
-    float* qu = reinterpret_cast<float*>(Ps + prow * DK);
+    float* Ks = reinterpret_cast<float*>(smem_raw);
+    float* Vs = Ks + rows * DK;
+    float* Ps = Vs + rows * DK;
+    float* qu = Ps + prow * DK;
     float* qv = qu + t * DK;
     float* prob = qv + t * DK;                      // t x prow
     __shared__ __align__(8) uint64_t bar;
@@ -684,14 +361,18 @@ attention_chunks_kernel(AttnStream a, const TA* __restrict__ qkv, const float* _
     const int slot = a.ids[b];
     const int nf = a.n_frames[slot];
     const int cl = min(nf, a.window), first = nf - cl;
-    TA* ringK = ring + (long long)slot * a.ring_slot_stride + (long long)h * cap * DK;
-    TA* ringV = ringK + (long long)a.H * cap * DK;
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    if (tid == 0) chunks_start_ring_copy(ringK, ringV, Ks, Vs, first, cl, cap, DK * sizeof(TA), &bar);
-    chunks_stage_new<TA, NCH, false>(a, qkv, Ks, Vs, b, h, nf, cl, kt);
+    float* ringK = ring + (long long)slot * a.ring_slot_stride + (long long)h * cap * DK;
+    float* ringV = ringK + (long long)a.H * cap * DK;
+    const int tid = threadIdx.x;
+    if (tid == 0) {
+        mbar_init(&bar, 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        ring_window_copy<float>(ringK, ringV, cap, first, cl, Ks, Vs, nullptr, nullptr, 0, &bar);
+    }
+    chunks_stage_new<float, NCH, false>(a, qkv, Ks, Vs, b, h, nf, cl, kt);
     __syncthreads();
     mbar_wait(&bar, 0);
-    chunks_append_ring<TA, NCH>(a, Ks, Vs, ringK, ringV, nf, cl, kt);
+    chunks_append_ring<float, NCH>(a, Ks, Vs, ringK, ringV, nf, cl, kt);
 
     const int pe0 = a.pe_index[slot];
     for (int j = 0; j < a.chunks; ++j) {
@@ -710,65 +391,13 @@ attention_chunks_kernel(AttnStream a, const TA* __restrict__ qkv, const float* _
             qv[i] = q + pos_v[h * DK + d];
         }
         __syncthreads();
-        constexpr int KPL = 4;                        // keys per lane: nk <= window + t <= STREAM_CHUNKS_MAX_KEYS
-        for (int i = warp; i < t; i += ATT_THREADS / 32) {
-            const float* qui = qu + i * DK;
-            const float* qvi = qv + i * DK;
-            float sc[KPL];
-#pragma unroll
-            for (int k = 0; k < KPL; ++k) sc[k] = 0.f;
-            for (int c = 0; c < NCH; ++c) {
-                const int cc = (c + lane) & (NCH - 1);
-#pragma unroll
-                for (int k = 0; k < KPL; ++k) {
-                    const int jj = lane + 32 * k;
-                    if (jj < nk) {
-                        float kv[EPC], pp[EPC];
-                        Chunk<TA>::load(Ks + (o + jj) * DK + cc * EPC, kv);
-                        Chunk<TA>::load(Ps + jj * DK + cc * EPC, pp);
-                        float s = sc[k];
-#pragma unroll
-                        for (int e = 0; e < EPC; ++e) s = fmaf(qui[cc * EPC + e], kv[e], fmaf(qvi[cc * EPC + e], pp[e], s));
-                        sc[k] = s;
-                    }
-                }
-            }
-            float m = -INFINITY;
-#pragma unroll
-            for (int k = 0; k < KPL; ++k) {
-                sc[k] = (lane + 32 * k < nk) ? sc[k] * 0.125f : -INFINITY;
-                m = fmaxf(m, sc[k]);
-            }
-            m = warp_max(m);
-            float ssum = 0.f;
-            float* pr = prob + i * prow;
-#pragma unroll
-            for (int k = 0; k < KPL; ++k) {
-                const int jj = lane + 32 * k;
-                if (jj < nk) {
-                    const float e = __expf(sc[k] - m);
-                    pr[jj] = e;
-                    ssum += e;
-                }
-            }
-            ssum = warp_sum(ssum);
-            __syncwarp();
-            const float inv = 1.f / ssum;
-            float o0 = 0.f, o1 = 0.f;
-            for (int jj = 0; jj < nk; ++jj) {
-                const float p = pr[jj];
-                o0 = fmaf(p, to_f(Vs[(o + jj) * DK + 2 * lane]), o0);
-                o1 = fmaf(p, to_f(Vs[(o + jj) * DK + 2 * lane + 1]), o1);
-            }
-            TA* op = out + (long long)(b * kt + j * t + i) * D + h * DK + 2 * lane;
-            op[0] = from_f<TA>(o0 * inv);
-            op[1] = from_f<TA>(o1 * inv);
-        }
+        attn_chunk_ffma(Ks + o * DK, Vs + o * DK, Ps, qu, qv, prob, prow, nk, t, out + (long long)(b * kt + j * t) * D + h * DK, D);
         __syncthreads();                              // Ps / qu / prob are restaged by the next chunk
     }
 }
 
-// fp16 form: the two contractions on mma.sync as in attention_stream_mma_kernel, per query chunk (t <= 8 = the MMA's N)
+// Multi-chunk streaming attention of fp16 contexts (t <= 8 = the MMA's N).  Staging as in attention_chunks_kernel, with the
+// K/V rows swizzled by frame and padded past the last staged key; each chunk's core is attn_chunk_mma.
 __global__ void __launch_bounds__(ATT_THREADS)
 attention_chunks_mma_kernel(AttnStream a, const __half* __restrict__ qkv, const float* __restrict__ q32, __half* __restrict__ ring,
                             const __half* __restrict__ ptab_h, const float* __restrict__ pos_u, const float* __restrict__ pos_v,
@@ -798,8 +427,12 @@ attention_chunks_mma_kernel(AttnStream a, const __half* __restrict__ qkv, const 
     const int nk_all = cl + kt;
     TA* ringK = ring + (long long)slot * a.ring_slot_stride + (long long)h * cap * DK;
     TA* ringV = ringK + (long long)a.H * cap * DK;
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    if (tid == 0) chunks_start_ring_copy(ringK, ringV, Ks, Vs, first, cl, cap, DK * sizeof(TA), &bar);
+    const int tid = threadIdx.x;
+    if (tid == 0) {
+        mbar_init(&bar, 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        ring_window_copy<TA>(ringK, ringV, cap, first, cl, Ks, Vs, nullptr, nullptr, 0, &bar);
+    }
     chunks_stage_new<TA, NCH, true>(a, qkv, Ks, Vs, b, h, nf, cl, kt);
     // rows behind the last key: K is masked there, V enters the PV MMAs with probability 0 and must be finite
     for (int i = tid; i < (krows - nk_all) * NCH; i += ATT_THREADS) {
@@ -810,11 +443,10 @@ attention_chunks_mma_kernel(AttnStream a, const __half* __restrict__ qkv, const 
     mbar_wait(&bar, 0);
     chunks_append_ring<TA, NCH>(a, Ks, Vs, ringK, ringV, nf, cl, kt);
 
-    const int g = lane >> 2, c = lane & 3;
     const int pe0 = a.pe_index[slot];
     for (int j = 0; j < a.chunks; ++j) {
         const int nfj = nf + j * t, clj = min(nfj, a.window);
-        const int o = nfj - clj - first;
+        const int o = nfj - clj - first;            // staged row of this chunk's first key
         const int nk = clj + t;
         const int start = max(0, chunk_pe(pe0, j, a) - a.full_chunk);
         for (int i = tid; i < nk * NCH; i += ATT_THREADS) {        // row r = position start + r, swizzled by that position
@@ -830,93 +462,11 @@ attention_chunks_mma_kernel(AttnStream a, const __half* __restrict__ qkv, const 
             qvh[sw] = from_f<TA>(q + pos_v[h * DK + d]);
         }
         __syncthreads();
-        for (int k0 = warp * 16; k0 < nk; k0 += 16 * (ATT_THREADS / 32)) {
-            float d[4] = {0.f, 0.f, 0.f, 0.f};
-            const int kk0 = (first + o + k0 + g) & 7, kk1 = (first + o + k0 + g + 8) & 7;
-            const int kp0 = (start + k0 + g) & 7, kp1 = (start + k0 + g + 8) & 7;
-            const TA* kr0 = Ks + (o + k0 + g) * DK + c * 2;
-            const TA* kr1 = Ks + (o + k0 + g + 8) * DK + c * 2;
-            const TA* pr0 = Ps + (k0 + g) * DK + c * 2;
-            const TA* pr1 = Ps + (k0 + g + 8) * DK + c * 2;
-#pragma unroll
-            for (int ks = 0; ks < DK / 16; ++ks) {
-                const int c0 = ks * 2, c1 = ks * 2 + 1;
-                uint32_t af[4], bf[2];
-                af[0] = lds32(kr0 + ((c0 ^ kk0) << 3));
-                af[1] = lds32(kr1 + ((c0 ^ kk1) << 3));
-                af[2] = lds32(kr0 + ((c1 ^ kk0) << 3));
-                af[3] = lds32(kr1 + ((c1 ^ kk1) << 3));
-                bf[0] = g < t ? lds32(quh + g * DK + ((c0 ^ g) << 3) + c * 2) : 0u;
-                bf[1] = g < t ? lds32(quh + g * DK + ((c1 ^ g) << 3) + c * 2) : 0u;
-                mma16816(d, af, bf);
-                af[0] = lds32(pr0 + ((c0 ^ kp0) << 3));
-                af[1] = lds32(pr1 + ((c0 ^ kp1) << 3));
-                af[2] = lds32(pr0 + ((c1 ^ kp0) << 3));
-                af[3] = lds32(pr1 + ((c1 ^ kp1) << 3));
-                bf[0] = g < t ? lds32(qvh + g * DK + ((c0 ^ g) << 3) + c * 2) : 0u;
-                bf[1] = g < t ? lds32(qvh + g * DK + ((c1 ^ g) << 3) + c * 2) : 0u;
-                mma16816(d, af, bf);
-            }
-            const int q0 = c * 2;
-            if (q0 < t) { sc[q0 * vrows + k0 + g] = d[0] * 0.125f; sc[q0 * vrows + k0 + g + 8] = d[2] * 0.125f; }
-            if (q0 + 1 < t) { sc[(q0 + 1) * vrows + k0 + g] = d[1] * 0.125f; sc[(q0 + 1) * vrows + k0 + g + 8] = d[3] * 0.125f; }
-        }
-        __syncthreads();
-        for (int i = warp; i < t; i += ATT_THREADS / 32) {
-            float sv[4];
-            float m = -INFINITY;
-#pragma unroll
-            for (int k = 0; k < 4; ++k) {
-                const int jj = lane + 32 * k;
-                sv[k] = jj < nk ? sc[i * vrows + jj] : -INFINITY;
-                m = fmaxf(m, sv[k]);
-            }
-            m = warp_max(m);
-            float ssum = 0.f;
-#pragma unroll
-            for (int k = 0; k < 4; ++k) {
-                sv[k] = (lane + 32 * k < nk) ? __expf(sv[k] - m) : 0.f;
-                ssum += sv[k];
-            }
-            ssum = warp_sum(ssum);
-            const float inv = 1.f / ssum;
-#pragma unroll
-            for (int k = 0; k < 4; ++k) {
-                const int jj = lane + 32 * k;
-                if (jj < vrows) ph[i * vrows + jj] = __float2half_rn(sv[k] * inv);
-            }
-        }
-        __syncthreads();
-        {
-            float d[4] = {0.f, 0.f, 0.f, 0.f};
-            const int dim0 = warp * 16;
-            const int mi = lane >> 3, r = lane & 7;
-            for (int key0 = 0; key0 < nk; key0 += 16) {
-                uint32_t af[4], bf[2];
-                const int vrow = o + key0 + r + ((mi & 2) ? 8 : 0);
-                const TA* ap = Vs + vrow * DK + ((((dim0 >> 3) + (mi & 1)) ^ ((first + vrow) & 7)) << 3);
-                const uint32_t saddr = smem_u32(ap);
-                asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0,%1,%2,%3}, [%4];"
-                             : "=r"(af[0]), "=r"(af[1]), "=r"(af[2]), "=r"(af[3])
-                             : "r"(saddr));
-                bf[0] = g < t ? lds32(ph + g * vrows + key0 + c * 2) : 0u;
-                bf[1] = g < t ? lds32(ph + g * vrows + key0 + 8 + c * 2) : 0u;
-                mma16816(d, af, bf);
-            }
-            const int q0 = c * 2;
-            if (q0 < t) { sc[q0 * DK + dim0 + g] = d[0]; sc[q0 * DK + dim0 + g + 8] = d[2]; }
-            if (q0 + 1 < t) { sc[(q0 + 1) * DK + dim0 + g] = d[1]; sc[(q0 + 1) * DK + dim0 + g + 8] = d[3]; }
-        }
-        __syncthreads();
-        for (int i = tid; i < t * (DK / 2); i += ATT_THREADS) {
-            const int q = i / (DK / 2), pr = i % (DK / 2);
-            *reinterpret_cast<uint32_t*>(out + (long long)(b * kt + j * t + q) * D + h * DK + 2 * pr) =
-                pack2<__half>(sc[q * DK + 2 * pr], sc[q * DK + 2 * pr + 1]);
-        }
+        attn_chunk_mma<ATT_THREADS / 32>(Ks + o * DK, Vs + o * DK, first + o, Ps, start, quh, qvh, ph, sc, vrows, nk, t,
+                                         out + (long long)(b * kt + j * t) * D + h * DK, D);
         __syncthreads();                              // Ps / quh / ph / sc are restaged by the next chunk
     }
 }
-
 // ---------------------------------------------------------------------------------------------
 constexpr int KT = 96;          // key tile: the shipped band of a 32-query block (64 left + 32 own keys) in one pass
 constexpr int QB = 32;          // query rows per CTA
@@ -929,20 +479,19 @@ constexpr int QPW = QB / (ATT_THREADS / 32);   // queries per warp
 // from shared memory feeds four dot products and the query chunks are warp-wide broadcasts.  Window [start,end) of
 // masks.py:50-56 and the pad mask (masks.py:110-120) are applied arithmetically; online softmax across tiles
 // (unbounded left context works); PV with lane = output dims.  A row whose whole window is masked yields zeros
-// (attention.py:396-397).
-template <typename TA>
+// (attention.py:396-397).  fp32 contexts; fp16 contexts run attention_offline_fa_kernel below.
 __global__ void __launch_bounds__(ATT_THREADS)
-attention_offline_kernel(const TA* __restrict__ qkv, const float* __restrict__ q32, int T, int H,
+attention_offline_kernel(const float* __restrict__ qkv, const float* __restrict__ q32, int T, int H,
                          const int32_t* __restrict__ ilens, int chunk, int left, const float* __restrict__ ptab,
-                         const float* __restrict__ pos_u, const float* __restrict__ pos_v, TA* __restrict__ out) {
+                         const float* __restrict__ pos_u, const float* __restrict__ pos_v, float* __restrict__ out) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
-    constexpr int EPC = Chunk<TA>::EPC, NCH = Chunk<TA>::NCH;
+    constexpr int EPC = 4, NCH = DK / EPC;
     constexpr int DKP = DK + EPC;                          // padded row (16 B): conflict-free 16-byte row reads
     constexpr int QG = 4;                                  // queries per register block
-    TA* Ks = reinterpret_cast<TA*>(smem_raw);
-    TA* Vs = Ks + KT * DKP;
-    TA* Ps = Vs + KT * DKP;
-    float* qu = reinterpret_cast<float*>(Ps + KT * DKP);   // QB x 64
+    float* Ks = reinterpret_cast<float*>(smem_raw);
+    float* Vs = Ks + KT * DKP;
+    float* Ps = Vs + KT * DKP;
+    float* qu = Ps + KT * DKP;                             // QB x 64
     float* qv = qu + QB * DK;
     float* prob = qv + QB * DK;                            // warps x KT
     __shared__ int win[QB][2];
@@ -993,22 +542,14 @@ attention_offline_kernel(const TA* __restrict__ qkv, const float* __restrict__ q
         for (int i = tid; i < nk * NCH * 2; i += ATT_THREADS) {
             const int which = i / (nk * NCH);              // 0 K, 1 V
             const int j = (i / NCH) % nk, c = i % NCH;
-            const TA* src = qkv + ((long long)b * T + kt + j) * 3 * D + (which + 1) * D + h * DK + c * EPC;
-            TA* dst = (which == 0 ? Ks : Vs) + j * DKP + c * EPC;
+            const float* src = qkv + ((long long)b * T + kt + j) * 3 * D + (which + 1) * D + h * DK + c * EPC;
+            float* dst = (which == 0 ? Ks : Vs) + j * DKP + c * EPC;
             *reinterpret_cast<uint4*>(dst) = *reinterpret_cast<const uint4*>(src);
         }
         for (int i = tid; i < nk * (DK / 4); i += ATT_THREADS) {
             const int j = i / (DK / 4), c = i % (DK / 4);
             const float4 v4 = *reinterpret_cast<const float4*>(ptab + (long long)(kt + j) * D + h * DK + c * 4);
-            TA* d = Ps + j * DKP + c * 4;
-            if constexpr (sizeof(TA) == 2) {
-                uint2 hh;
-                hh.x = pack2<TA>(v4.x, v4.y);
-                hh.y = pack2<TA>(v4.z, v4.w);
-                *reinterpret_cast<uint2*>(d) = hh;
-            } else {
-                *reinterpret_cast<float4*>(d) = v4;
-            }
+            *reinterpret_cast<float4*>(Ps + j * DKP + c * 4) = v4;
         }
         __syncthreads();
 #pragma unroll
@@ -1038,8 +579,8 @@ attention_offline_kernel(const TA* __restrict__ qkv, const float* __restrict__ q
                     const int j = lane + 32 * k;
                     if (j < nk) {
                         float kv[EPC], pp[EPC];
-                        Chunk<TA>::load(Ks + j * DKP + c * EPC, kv);
-                        Chunk<TA>::load(Ps + j * DKP + c * EPC, pp);
+                        ld4(Ks + j * DKP + c * EPC, kv);
+                        ld4(Ps + j * DKP + c * EPC, pp);
 #pragma unroll
                         for (int q = 0; q < QG; ++q) {
                             float s = sc[q][k];
@@ -1082,22 +623,11 @@ attention_offline_kernel(const TA* __restrict__ qkv, const float* __restrict__ q
                 l_run[qi] = l_run[qi] * corr + ssum;
                 float a0 = o0[qi] * corr, a1 = o1[qi] * corr;
                 const int j0 = max(lo - kt, 0), j1 = min(hi - kt, nk);
-                if constexpr (sizeof(TA) == 2) {
-                    const uint32_t* vp = reinterpret_cast<const uint32_t*>(Vs) + lane;
 #pragma unroll 4
-                    for (int j = j0; j < j1; ++j) {
-                        const float2 vv = unpack2<TA>(vp[j * (DKP / 2)]);
-                        const float p = pr[j];
-                        a0 = fmaf(p, vv.x, a0);
-                        a1 = fmaf(p, vv.y, a1);
-                    }
-                } else {
-#pragma unroll 4
-                    for (int j = j0; j < j1; ++j) {
-                        const float p = pr[j];
-                        a0 = fmaf(p, to_f(Vs[j * DKP + 2 * lane]), a0);
-                        a1 = fmaf(p, to_f(Vs[j * DKP + 2 * lane + 1]), a1);
-                    }
+                for (int j = j0; j < j1; ++j) {
+                    const float p = pr[j];
+                    a0 = fmaf(p, Vs[j * DKP + 2 * lane], a0);
+                    a1 = fmaf(p, Vs[j * DKP + 2 * lane + 1], a1);
                 }
                 o0[qi] = a0;
                 o1[qi] = a1;
@@ -1110,13 +640,9 @@ attention_offline_kernel(const TA* __restrict__ qkv, const float* __restrict__ q
         const int r = warp * QPW + qi;
         if (r < nq) {
             const float inv = l_run[qi] > 0.f ? 1.f / l_run[qi] : 0.f;
-            TA* o = out + ((long long)b * T + q0 + r) * D + h * DK + 2 * lane;
-            if constexpr (sizeof(TA) == 2) {
-                *reinterpret_cast<uint32_t*>(o) = pack2<TA>(o0[qi] * inv, o1[qi] * inv);
-            } else {
-                o[0] = from_f<TA>(o0[qi] * inv);
-                o[1] = from_f<TA>(o1[qi] * inv);
-            }
+            float* o = out + ((long long)b * T + q0 + r) * D + h * DK + 2 * lane;
+            o[0] = o0[qi] * inv;
+            o[1] = o1[qi] * inv;
         }
     }
 }
@@ -1373,98 +899,50 @@ __global__ void advance_sessions_kernel(const int32_t* __restrict__ ids, int n, 
     if (adapter_valid) adapter_valid[s] = adapter_valid[s] == 1 ? 2 : 1;
 }
 
-// launcher of the multi-chunk kernels (AttnStream::chunks > 1)
-template <typename TA>
-int attention_stream_chunks(const AttnStream& a, const TA* qkv, const float* q32, TA* ring, const TA* ptab_h,
-                            const float* pos_u, const float* pos_v, TA* out, cudaStream_t st) {
-    const int kt = a.chunks * a.t, rows = a.window + kt, prow = a.window + a.t;
-    FO_CHECK(a.t <= TQ_MAX, "attention_stream: %d frames per chunk exceeds %d", a.t, TQ_MAX);
-    FO_CHECK(rows <= STREAM_CHUNKS_MAX_KEYS, "attention_stream: window %d + %d chunks x %d frames exceeds %d keys", a.window,
-             a.chunks, a.t, STREAM_CHUNKS_MAX_KEYS);
-    dim3 grid(a.n, a.H);
-    static bool attr_set[2] = {false, false};
-    size_t smem;
-    if constexpr (sizeof(TA) == 2) {
-        const int krows = ((rows + 15) & ~15) + 16, vrows = (prow + 15) & ~15;
-        smem = (size_t)(2 * krows + vrows) * DK * 2 + (size_t)2 * a.t * DK * 2 + (size_t)a.t * vrows * 2 +
-               (size_t)a.t * std::max(vrows, DK) * 4;
-        if (!attr_set[1]) {
-            FO_CUDA(cudaFuncSetAttribute(attention_chunks_mma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
-            attr_set[1] = true;
-        }
-        FO_CHECK(smem <= 160 * 1024, "attention_stream: multi-chunk call too large for shared memory");
-        FO_CUDA(launch_pdl(attention_chunks_mma_kernel, grid, dim3(ATT_THREADS), smem, st, a, reinterpret_cast<const __half*>(qkv), q32,
-                           reinterpret_cast<__half*>(ring), reinterpret_cast<const __half*>(ptab_h), pos_u, pos_v,
-                           reinterpret_cast<__half*>(out)));
-    } else {
-        smem = (size_t)(2 * rows + prow) * DK * sizeof(TA) + (size_t)2 * a.t * DK * sizeof(float) + (size_t)a.t * prow * sizeof(float);
-        if (!attr_set[0]) {
-            FO_CUDA(cudaFuncSetAttribute(attention_chunks_kernel<TA>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
-            attr_set[0] = true;
-        }
-        FO_CHECK(smem <= 160 * 1024, "attention_stream: multi-chunk call too large for shared memory");
-        FO_CUDA(launch_pdl(attention_chunks_kernel<TA>, grid, dim3(ATT_THREADS), smem, st, a, qkv, q32, ring, ptab_h, pos_u, pos_v, out));
-    }
-    FO_LAUNCHED();
-    FO_CUDA(cudaGetLastError());
-    return 0;
-}
-
 }  // namespace
 
 template <typename TA>
 int attention_stream(const AttnStream& a, const TA* qkv, const float* q32, TA* ring, const TA* ptab_h,
                      const float* pos_u, const float* pos_v, TA* out, cudaStream_t st) {
     if (a.n <= 0) return 0;
-    if (a.chunks > 1) return attention_stream_chunks<TA>(a, qkv, q32, ring, ptab_h, pos_u, pos_v, out, st);
-    FO_CHECK(a.t <= TQ_MAX, "attention_stream: %d frames per call exceeds %d", a.t, TQ_MAX);
-    FO_CHECK(a.ring_cap >= a.window + a.t, "attention_stream: ring capacity %d < window %d + %d", a.ring_cap, a.window, a.t);
-    const int rows = a.window + a.t;
-    FO_CHECK(rows <= 128, "attention_stream: window + frames per call (%d) exceeds 128 keys", rows);
-    const size_t smem = (size_t)3 * rows * DK * sizeof(TA) + (size_t)2 * a.t * DK * sizeof(float) +
-                        (size_t)a.t * rows * sizeof(float);
-    static bool attr_set[2] = {false, false};
-    if (!attr_set[sizeof(TA) == 2]) {
-        FO_CUDA(cudaFuncSetAttribute(attention_stream_kernel<TA>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
-        attr_set[sizeof(TA) == 2] = true;
+    const int t = a.t, rows = a.window + a.chunks * t, prow = a.window + t;     // staged keys, keys of one chunk
+    FO_CHECK(t <= STREAM_MAX_T, "attention_stream: %d frames per chunk exceeds %d", t, STREAM_MAX_T);
+    FO_CHECK(a.ring_cap >= prow, "attention_stream: ring capacity %d < window %d + %d", a.ring_cap, a.window, t);
+    FO_CHECK(rows <= STREAM_CHUNKS_MAX_KEYS, "attention_stream: window %d + %d chunks x %d frames exceeds %d keys", a.window,
+             a.chunks, t, STREAM_CHUNKS_MAX_KEYS);
+    using Kernel = void (*)(AttnStream, const TA*, const float*, TA*, const TA*, const float*, const float*, TA*);
+    // [0] one chunk, [1] one chunk summed from the QKV GEMM's split-K partials (fp16 only), [2] several chunks
+    std::array<Kernel, 3> kernels;
+    size_t smem;
+    if constexpr (sizeof(TA) == 2) {
+        kernels = {attention_stream_mma_kernel<false>, attention_stream_mma_kernel<true>, attention_chunks_mma_kernel};
+        const int krows = ((rows + 15) & ~15) + 16, vrows = (prow + 15) & ~15;
+        smem = a.chunks > 1 ? (size_t)(2 * krows + vrows) * DK * 2 + (size_t)2 * t * DK * 2 + (size_t)t * vrows * 2 +
+                                  (size_t)t * std::max(vrows, DK) * 4
+                            : (size_t)mma_unit_layout(a.window, t).bytes;
+    } else {
+        kernels = {attention_stream_kernel, attention_stream_kernel, attention_chunks_kernel};
+        smem = (size_t)(2 * rows + prow) * DK * 4 + (size_t)2 * t * DK * 4 + (size_t)t * prow * 4;
     }
     FO_CHECK(smem <= 160 * 1024, "attention_stream: window too large for shared memory");
-    dim3 grid(a.n, a.H);
-    if constexpr (sizeof(TA) == 2) {
-            const int vrows = (rows + 15) & ~15;
-            const size_t sm = (size_t)(2 * rows + vrows) * DK * 2 + (size_t)2 * a.t * DK * 2 + (size_t)a.t * vrows * 2 +
-                              (size_t)a.t * std::max(vrows, DK) * 4;
-            // past 48 KB (window + t > ~115 keys, e.g. left_chunks 31) the launch needs the opt-in
-            static bool mma_attr_set = false;
-            if (!mma_attr_set) {
-                FO_CUDA(cudaFuncSetAttribute(attention_stream_mma_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
-                FO_CUDA(cudaFuncSetAttribute(attention_stream_mma_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
-                mma_attr_set = true;
-            }
-            FO_CHECK(sm <= 160 * 1024, "attention_stream: window too large for shared memory");
-            if (a.nsplit > 0)
-                FO_CUDA(launch_pdl(attention_stream_mma_kernel<true>, grid, dim3(ATT_THREADS), sm, st, a, reinterpret_cast<const __half*>(qkv), q32,
-                                   reinterpret_cast<__half*>(ring), reinterpret_cast<const __half*>(ptab_h), pos_u, pos_v,
-                                   reinterpret_cast<__half*>(out)));
-            else
-                FO_CUDA(launch_pdl(attention_stream_mma_kernel<false>, grid, dim3(ATT_THREADS), sm, st, a, reinterpret_cast<const __half*>(qkv), q32,
-                                   reinterpret_cast<__half*>(ring), reinterpret_cast<const __half*>(ptab_h), pos_u, pos_v,
-                                   reinterpret_cast<__half*>(out)));
-            FO_LAUNCHED();
-#ifdef FO_TC_TRACE_BUILD
-            if (getenv("FO_TC_TRACE") && st == nullptr) {
-                cudaStreamSynchronize(st);
-                unsigned long long hb[16];
-                cudaMemcpyFromSymbol(hb, g_attn_trace, sizeof(hb));
-                fprintf(stderr, "attn_trace n=%d:", a.n);
-                for (int i = 1; i <= 9; ++i) fprintf(stderr, " t%d=%lld", i, (long long)(hb[i] - hb[0]));
-                fprintf(stderr, " ns\n");
-            }
-#endif
-    } else {
-        FO_CUDA(launch_pdl(attention_stream_kernel<TA>, grid, dim3(ATT_THREADS), smem, st, a, qkv, q32, ring, ptab_h, pos_u, pos_v, out));
-        FO_LAUNCHED();
+    static bool opted_in = false;      // past 48 KB (window + t > ~115 keys, e.g. left_chunks 31) a launch needs the opt-in
+    if (!opted_in) {
+        for (Kernel k : kernels) FO_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
+        opted_in = true;
     }
+    const Kernel kern = kernels[a.chunks > 1 ? 2 : a.nsplit > 0 ? 1 : 0];
+    FO_CUDA(launch_pdl(kern, dim3(a.n, a.H), dim3(ATT_THREADS), smem, st, a, qkv, q32, ring, ptab_h, pos_u, pos_v, out));
+    FO_LAUNCHED();
+#ifdef FO_TC_TRACE_BUILD
+    if (sizeof(TA) == 2 && a.chunks == 1 && getenv("FO_TC_TRACE") && st == nullptr) {
+        cudaStreamSynchronize(st);
+        unsigned long long hb[16];
+        cudaMemcpyFromSymbol(hb, g_attn_trace, sizeof(hb));
+        fprintf(stderr, "attn_trace n=%d:", a.n);
+        for (int i : {1, 2, 3, 4, 5, 9}) fprintf(stderr, " t%d=%lld", i, (long long)(hb[i] - hb[0]));
+        fprintf(stderr, " ns\n");
+    }
+#endif
     FO_CUDA(cudaGetLastError());
     return 0;
 }
@@ -1498,39 +976,31 @@ int attention_offline(const TA* qkv, const float* q32, int B, int T, int H, cons
                       const float* ptab, const TA* ptab_h, int pos_rows, const float* pos_u, const float* pos_v, TA* out,
                       cudaStream_t st) {
     if (B <= 0 || T <= 0) return 0;
-    dim3 grid(cdiv(T, QB), H, B);
-    const size_t smem = (size_t)3 * KT * (DK + 16 / sizeof(TA)) * sizeof(TA) + (size_t)2 * QB * DK * sizeof(float) +
-                        (size_t)(ATT_THREADS / 32) * KT * sizeof(float);
-    static bool attr_set[2] = {false, false};
-    if (!attr_set[sizeof(TA) == 2]) {
-        FO_CUDA(cudaFuncSetAttribute(attention_offline_kernel<TA>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
-        attr_set[sizeof(TA) == 2] = true;
-    }
     if constexpr (sizeof(TA) == 2) {
         if (!ptab_h || T > pos_rows) return 1;
-        {
-            const size_t smf = (size_t)2 * 3 * FK * DK * 2;      // 48 KB: double-buffered K | P | V tiles
-            static bool attr3 = false;
-            if (!attr3) {
-                FO_CUDA(cudaFuncSetAttribute(attention_offline_fa_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
-                attr3 = true;
-            }
-            attention_offline_fa_kernel<<<dim3(cdiv(T, FQ), H, B), ATT_THREADS, smf, st>>>(
-                reinterpret_cast<const __half*>(qkv), q32, T, H, ilens, chunk, left, reinterpret_cast<const __half*>(ptab_h), pos_rows,
-                pos_u, pos_v, reinterpret_cast<__half*>(out));
-            FO_LAUNCHED();
-            FO_CUDA(cudaGetLastError());
-            return 0;
+        const size_t smem = (size_t)2 * 3 * FK * DK * 2;      // 48 KB: double-buffered K | P | V tiles
+        static bool attr_set = false;
+        if (!attr_set) {
+            FO_CUDA(cudaFuncSetAttribute(attention_offline_fa_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
+            attr_set = true;
         }
+        attention_offline_fa_kernel<<<dim3(cdiv(T, FQ), H, B), ATT_THREADS, smem, st>>>(qkv, q32, T, H, ilens, chunk, left, ptab_h,
+                                                                                         pos_rows, pos_u, pos_v, out);
     } else {
-        attention_offline_kernel<TA><<<grid, ATT_THREADS, smem, st>>>(qkv, q32, T, H, ilens, chunk, left, ptab, pos_u, pos_v, out);
+        const size_t smem = (size_t)3 * KT * (DK + 4) * 4 + (size_t)2 * QB * DK * 4 + (size_t)(ATT_THREADS / 32) * KT * 4;
+        static bool attr_set = false;
+        if (!attr_set) {
+            FO_CUDA(cudaFuncSetAttribute(attention_offline_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
+            attr_set = true;
+        }
+        attention_offline_kernel<<<dim3(cdiv(T, QB), H, B), ATT_THREADS, smem, st>>>(qkv, q32, T, H, ilens, chunk, left, ptab, pos_u,
+                                                                                    pos_v, out);
     }
     FO_LAUNCHED();
     FO_CUDA(cudaGetLastError());
     return 0;
 }
 template int attention_offline<float>(const float*, const float*, int, int, int, const int32_t*, int, int, const float*, const float*, int, const float*, const float*, float*, cudaStream_t);
-template int attention_offline<bf16>(const bf16*, const float*, int, int, int, const int32_t*, int, int, const float*, const bf16*, int, const float*, const float*, bf16*, cudaStream_t);
 template int attention_offline<__half>(const __half*, const float*, int, int, int, const int32_t*, int, int, const float*, const __half*, int, const float*, const float*, __half*, cudaStream_t);
 
 int advance_sessions(const int32_t* ids, int n, int t, int chunk_size, int pe_wrap, int32_t* n_frames,

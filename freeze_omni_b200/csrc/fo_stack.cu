@@ -33,12 +33,11 @@
 
 #include <algorithm>
 
-#include "fo_common.cuh"
+#include "fo_attn_core.cuh"
 
 namespace fo {
 namespace {
 
-constexpr int DK = 64;
 constexpr int ST_THREADS = 256;
 constexpr int ST_WARPS = ST_THREADS / 32;
 constexpr int BAR_COUNTER = 512;          // counter word of the barrier buffer (the words below it are the per-CTA records)
@@ -53,48 +52,9 @@ struct StackLayout {                       // byte offsets into the dynamic shar
     int dbg;                               // development (FO_STACK_DBG, results invalid): 1 = no epilogue stores
 };
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* bar, int count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "WAIT_LOOP:\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-        "@p bra DONE;\n\t"
-        "bra WAIT_LOOP;\n\t"
-        "DONE:\n\t}" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(void* dst, const void* src, uint32_t bytes, uint64_t* bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                     smem_u32(dst)),
-                 "l"(src), "r"(bytes), "r"(smem_u32(bar))
-                 : "memory");
-}
-__device__ __forceinline__ void mma16816(float (&d)[4], const uint32_t (&a)[4], const uint32_t (&b)[2]) {
-    asm volatile(
-        "mma.sync.aligned.m16n8k16.row.col.f32.f16.f16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-        : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
-        : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b[0]), "r"(b[1]));
-}
-__device__ __forceinline__ uint32_t lds32(const __half* p) { return *reinterpret_cast<const uint32_t*>(p); }
 __device__ __forceinline__ uint32_t lds32s(uint32_t addr) {        // explicit shared-space load (inside non-inlined code the
     uint32_t v;                                                    // compiler only sees generic pointers)
     asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(addr));
-    return v;
-}
-__device__ __forceinline__ float warp_max(float v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
-    return v;
-}
-__device__ __forceinline__ float warp_sum(float v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
     return v;
 }
 __device__ __forceinline__ unsigned long long gtime() {
@@ -374,39 +334,30 @@ __device__ __forceinline__ AttnGeom attn_geom(const AttnStream& a, int b) {
     g.np = min(g.nk, a.pos_rows - g.start);
     return g;
 }
-// thread 0, one phase early: cached K / V rows of the ring and the rel-pos rows of this head -> shared memory
-__device__ __forceinline__ void attn_issue(const AttnStream& a, const AttnGeom& g, const StackLayer& w, int h, __half* Ks, __half* Ps,
-                                           __half* Vs, uint64_t* bar) {
-    const int cap = a.ring_cap;
-    const __half* ringK = w.ring + (long long)g.slot * a.ring_slot_stride + (long long)h * cap * DK;
-    const __half* ringV = ringK + (long long)a.H * cap * DK;
-    const int p0 = g.first % cap;
-    const int len1 = min(g.cl, cap - p0), len2 = g.cl - len1;
-    const uint32_t rowb = DK * sizeof(__half);
-    mbar_expect_tx(bar, (2u * g.cl + g.np) * rowb);
-    bulk_g2s(Ps, w.ptab_h + ((long long)h * a.pos_rows + g.start) * DK, g.np * rowb, bar);
-    if (len1 > 0) {
-        bulk_g2s(Ks, ringK + (long long)p0 * DK, len1 * rowb, bar);
-        bulk_g2s(Vs, ringV + (long long)p0 * DK, len1 * rowb, bar);
-    }
-    if (len2 > 0) {
-        bulk_g2s(Ks + len1 * DK, ringK, len2 * rowb, bar);
-        bulk_g2s(Vs + len1 * DK, ringV, len2 * rowb, bar);
-    }
+// thread 0, one phase early: cached K / V rows of the ring and the rel-pos rows of this head -> the unit's shared memory
+__device__ __forceinline__ void attn_issue(const AttnStream& a, const AttnGeom& g, const StackLayer& w, int h, unsigned char* region,
+                                           uint64_t* bar) {
+    const MmaUnitLayout lay = mma_unit_layout(a.window, a.t);
+    const __half* ringK = w.ring + (long long)g.slot * a.ring_slot_stride + (long long)h * a.ring_cap * DK;
+    const __half* ringV = ringK + (long long)a.H * a.ring_cap * DK;
+    ring_window_copy(ringK, ringV, a.ring_cap, g.first, g.cl, reinterpret_cast<__half*>(region), reinterpret_cast<__half*>(region + lay.v),
+                     w.ptab_h + ((long long)h * a.pos_rows + g.start) * DK, reinterpret_cast<__half*>(region + lay.p), g.np, bar);
 }
+// Staging of the stack kernel's attention phase: the chunk's own K / V rows from p.kv and Q from p.q32 (written by other CTAs in
+// this launch, hence __ldcg), appended to the ring in the same pass; the ring window and rel-pos rows were issued a phase early
+// (attn_issue).  The core is attn_chunk_mma over all ST_WARPS warps.
 __device__ __forceinline__ void attn_unit(const StackArgs& p, const AttnGeom& ge, const StackLayer& w, int b, int h, unsigned char* region,
-                                          uint64_t* bar, uint32_t parity, int tid, int warp, int lane) {
+                                          uint64_t* bar, uint32_t parity, int tid) {
     const AttnStream& a = p.a;
     const int t = a.t, D = a.H * DK, cap = a.ring_cap;
-    const int rows = a.window + t, vrows = (rows + 15) & ~15;
+    const MmaUnitLayout lay = mma_unit_layout(a.window, t);
+    const int vrows = lay.vrows;
     __half* Ks = reinterpret_cast<__half*>(region);
-    __half* Ps = Ks + rows * DK;
-    __half* Vs = Ps + rows * DK;
-    __half* quh = Vs + vrows * DK;
-    __half* qvh = quh + t * DK;
-    __half* ph = qvh + t * DK;
-    float* sc = reinterpret_cast<float*>(ph + t * vrows);
-    const int nf = ge.nf, cl = ge.cl, first = ge.first, nk = ge.nk, start = ge.start, np = ge.np;
+    __half* Ps = reinterpret_cast<__half*>(region + lay.p);
+    __half* Vs = reinterpret_cast<__half*>(region + lay.v);
+    __half* quh = reinterpret_cast<__half*>(region + lay.qu);
+    __half* qvh = reinterpret_cast<__half*>(region + lay.qv);
+    const int nf = ge.nf, cl = ge.cl, nk = ge.nk, start = ge.start, np = ge.np;
     __half* ringK = w.ring + (long long)ge.slot * a.ring_slot_stride + (long long)h * cap * DK;
     __half* ringV = ringK + (long long)a.H * cap * DK;
     // the chunk's own K / V rows: into the tile and appended to the ring.  16-byte chunk c of the row of frame f lives at
@@ -434,92 +385,8 @@ __device__ __forceinline__ void attn_unit(const StackArgs& p, const AttnGeom& ge
     }
     __syncthreads();
     mbar_wait(bar, parity);
-    const int g = lane >> 2, c = lane & 3;
-    // scores: S^T tile (16 keys x 8 queries) per MMA chain
-    for (int k0 = warp * 16; k0 < nk; k0 += 16 * ST_WARPS) {
-        float d[4] = {0.f, 0.f, 0.f, 0.f};
-        const int kk0 = (first + k0 + g) & 7, kk1 = (first + k0 + g + 8) & 7;
-        const int kp0 = (start + k0 + g) & 7, kp1 = (start + k0 + g + 8) & 7;
-        const __half* kr0 = Ks + (k0 + g) * DK + c * 2;
-        const __half* kr1 = Ks + (k0 + g + 8) * DK + c * 2;
-        const __half* pr0 = Ps + (k0 + g) * DK + c * 2;
-        const __half* pr1 = Ps + (k0 + g + 8) * DK + c * 2;
-#pragma unroll
-        for (int ks = 0; ks < DK / 16; ++ks) {
-            const int c0 = ks * 2, c1 = ks * 2 + 1;
-            uint32_t af[4], bf[2];
-            af[0] = lds32(kr0 + ((c0 ^ kk0) << 3));
-            af[1] = lds32(kr1 + ((c0 ^ kk1) << 3));
-            af[2] = lds32(kr0 + ((c1 ^ kk0) << 3));
-            af[3] = lds32(kr1 + ((c1 ^ kk1) << 3));
-            bf[0] = g < t ? lds32(quh + g * DK + ((c0 ^ g) << 3) + c * 2) : 0u;
-            bf[1] = g < t ? lds32(quh + g * DK + ((c1 ^ g) << 3) + c * 2) : 0u;
-            mma16816(d, af, bf);
-            af[0] = lds32(pr0 + ((c0 ^ kp0) << 3));
-            af[1] = lds32(pr1 + ((c0 ^ kp1) << 3));
-            af[2] = lds32(pr0 + ((c1 ^ kp0) << 3));
-            af[3] = lds32(pr1 + ((c1 ^ kp1) << 3));
-            bf[0] = g < t ? lds32(qvh + g * DK + ((c0 ^ g) << 3) + c * 2) : 0u;
-            bf[1] = g < t ? lds32(qvh + g * DK + ((c1 ^ g) << 3) + c * 2) : 0u;
-            mma16816(d, af, bf);
-        }
-        const int q0 = c * 2;
-        if (q0 < t) { sc[q0 * vrows + k0 + g] = d[0] * 0.125f; sc[q0 * vrows + k0 + g + 8] = d[2] * 0.125f; }
-        if (q0 + 1 < t) { sc[(q0 + 1) * vrows + k0 + g] = d[1] * 0.125f; sc[(q0 + 1) * vrows + k0 + g + 8] = d[3] * 0.125f; }
-    }
-    __syncthreads();
-    // softmax (fp32), probabilities normalised and rounded to fp16
-    for (int i = warp; i < t; i += ST_WARPS) {
-        float sv[4];
-        float m = -INFINITY;
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            const int j = lane + 32 * k;
-            sv[k] = j < nk ? sc[i * vrows + j] : -INFINITY;
-            m = fmaxf(m, sv[k]);
-        }
-        m = warp_max(m);
-        float ssum = 0.f;
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            sv[k] = (lane + 32 * k < nk) ? __expf(sv[k] - m) : 0.f;
-            ssum += sv[k];
-        }
-        ssum = warp_sum(ssum);
-        const float inv = 1.f / ssum;
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            const int j = lane + 32 * k;
-            if (j < vrows) ph[i * vrows + j] = __float2half_rn(sv[k] * inv);
-        }
-    }
-    __syncthreads();
-    // PV: O^T tile (16 dims x 8 queries) per warp, warps 0-3
-    if (warp < DK / 16) {
-        float d[4] = {0.f, 0.f, 0.f, 0.f};
-        const int dim0 = warp * 16;
-        const int mi = lane >> 3, r = lane & 7;
-        for (int key0 = 0; key0 < nk; key0 += 16) {
-            uint32_t af[4], bf[2];
-            const int vrow = key0 + r + ((mi & 2) ? 8 : 0);
-            const __half* ap = Vs + vrow * DK + ((((dim0 >> 3) + (mi & 1)) ^ ((first + vrow) & 7)) << 3);
-            asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0,%1,%2,%3}, [%4];"
-                         : "=r"(af[0]), "=r"(af[1]), "=r"(af[2]), "=r"(af[3])
-                         : "r"(smem_u32(ap)));
-            bf[0] = g < t ? lds32(ph + g * vrows + key0 + c * 2) : 0u;
-            bf[1] = g < t ? lds32(ph + g * vrows + key0 + 8 + c * 2) : 0u;
-            mma16816(d, af, bf);
-        }
-        const int q0 = c * 2;
-        if (q0 < t) { sc[q0 * DK + dim0 + g] = d[0]; sc[q0 * DK + dim0 + g + 8] = d[2]; }
-        if (q0 + 1 < t) { sc[(q0 + 1) * DK + dim0 + g] = d[1]; sc[(q0 + 1) * DK + dim0 + g + 8] = d[3]; }
-    }
-    __syncthreads();
-    for (int i = tid; i < t * (DK / 2); i += ST_THREADS) {
-        const int q = i / (DK / 2), pr = i % (DK / 2);
-        *reinterpret_cast<uint32_t*>(p.att + (long long)(b * t + q) * D + h * DK + 2 * pr) =
-            pack2<__half>(sc[q * DK + 2 * pr], sc[q * DK + 2 * pr + 1]);
-    }
+    attn_chunk_mma<ST_WARPS>(Ks, Vs, ge.first, Ps, start, quh, qvh, reinterpret_cast<__half*>(region + lay.ph),
+                             reinterpret_cast<float*>(region + lay.sc), vrows, nk, t, p.att + (long long)b * t * D + h * DK, D);
 }
 
 // development stamps inside a phase (CTA 0, thread 0): trace[5L + 2 + 6 * phase + k]
@@ -549,10 +416,6 @@ stream_stack_kernel(const __grid_constant__ StackArgs p, const __grid_constant__
     const int fr0 = (int)((long long)cta * FF / G), fn = (int)((long long)(cta + 1) * FF / G) - fr0;
     const bool has_attn = cta < p.a.n * H;
     const int ab = cta / H, ah = cta % H;
-    const int att_rows = p.a.window + t;
-    __half* aKs = reinterpret_cast<__half*>(ATT);
-    __half* aPs = aKs + att_rows * DK;
-    __half* aVs = aPs + att_rows * DK;
     uint32_t par1 = 0, par2 = 0, par3 = 0, para = 0;
     unsigned int epoch = 0;
     const unsigned int base = p.bar[cta];                 // barriers this CTA has passed in earlier launches (see grid_barrier)
@@ -570,7 +433,7 @@ stream_stack_kernel(const __grid_constant__ StackArgs p, const __grid_constant__
             load_rows(S1, w0.wqkv, qr0, qn, D, &bars[0]);
             load_rows(S3, w0.wo, or0, on, D, &bars[2]);
             load_rows(S2, w0.w2, or0, on, FF, &bars[1]);
-            if (has_attn) attn_issue(p.a, ge, w0, ah, aKs, aPs, aVs, &bars[3]);
+            if (has_attn) attn_issue(p.a, ge, w0, ah, ATT, &bars[3]);
         }
         prefetch_small(w0, D, FF, cta, tid);
     }
@@ -615,7 +478,7 @@ stream_stack_kernel(const __grid_constant__ StackArgs p, const __grid_constant__
         if (p.trace && cta == 0 && tid == 0) p.trace[epoch] = gtime();
         // ---------------- attention units on the first n*H CTAs ----------------
         if (has_attn) {
-            attn_unit(p, ge, w, ab, ah, ATT, &bars[3], para, tid, warp, lane);
+            attn_unit(p, ge, w, ab, ah, ATT, &bars[3], para, tid);
             para ^= 1;
         } else if (more) {
             prefetch_small(p.layers[l + 1], D, FF, cta - p.a.n * H, tid);
@@ -701,7 +564,7 @@ stream_stack_kernel(const __grid_constant__ StackArgs p, const __grid_constant__
         }
         grid_barrier(p.bar, base + ++epoch, G, [&] {
             if (!more || lane != 0) return;
-            if (has_attn) attn_issue(p.a, ge, p.layers[l + 1], ah, aKs, aPs, aVs, &bars[3]);   // next layer's ring / rel-pos rows
+            if (has_attn) attn_issue(p.a, ge, p.layers[l + 1], ah, ATT, &bars[3]);   // next layer's ring / rel-pos rows
         }, arr ? arr + 2 * G * 4 : nullptr);
         if (p.trace && cta == 0 && tid == 0) p.trace[epoch] = gtime();
     }
@@ -768,8 +631,7 @@ static bool stack_layout(int D, int FF, int H, int n, int t, int window, int L, 
     lay->act_bytes = std::max(lay->act_bytes, M * (kc * 2 + 16));
     lay->act = take(lay->act_bytes);
     lay->red = take(ST_WARPS * MAXG * 128 * 4);
-    const int rows = window + t, vrows = (rows + 15) & ~15;
-    lay->attn = take((2 * rows + vrows) * DK * 2 + 2 * t * DK * 2 + t * vrows * 2 + t * std::max(vrows, DK) * 4);
+    lay->attn = take(mma_unit_layout(window, t).bytes);
     *smem = off;
     return off <= smem_max;
 }

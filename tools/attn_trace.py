@@ -1,7 +1,8 @@
 #!/usr/bin/env python
 """Timeline of one CTA of the fp16 streaming attention kernel (library built with FO_TC_TRACE_BUILD=1).
 t1 after the dependency wait, t2 session state read, t3 bulk copies issued, t4 registers staged to smem, t5 all rows
-landed, t6 scores done, t7 softmax done, t8 PV done, t9 output stored (ns from kernel entry)."""
+landed, t9 output stored (ns from kernel entry).  t9 - t5 is the shared chunk core (scores, softmax, PV, store:
+attn_chunk_mma in csrc/fo_attn_core.cuh)."""
 import os
 import sys
 
