@@ -90,22 +90,30 @@ struct fo_ctx {
     float *conv2_b = nullptr, *sub_b = nullptr, *emb_b = nullptr, *emb_g = nullptr, *emb_beta = nullptr;
     std::vector<LayerW> layers;
     float *after_g = nullptr, *after_b = nullptr;
-    void *ad_conv_w = nullptr, *ad_proj_w = nullptr;
-    float *ad_conv_b = nullptr, *ad_ln_g = nullptr, *ad_ln_b = nullptr, *ad_proj_b = nullptr;
-    // two-conv adapters (CNNAdapter, adapter.py:10-57; CNNSubsampling with 4 * enc_out_dim < llm_embed_dim, adapter.py:84-96):
-    // first conv C -> 2C and its folded eval-BatchNorm; the second conv (2C -> 4C) reuses ad_conv_* / ad_ln_* above
-    void* ad_conv1_w = nullptr;
-    float *ad_conv1_b = nullptr, *ad_bn1_s = nullptr, *ad_bn1_t = nullptr;
-    bool ad_two = false;                      // two convolutions
-    int ad_stride2 = 2;                       // stride of the LAST conv (CNNAdapter: 1)
-    float* ad_cache2 = nullptr;               // [slot][2][k-1][2C] fp32: left context of the second conv (reference cache[0])
+    // adapter: ad_nst causal convolutions (0 LinearAdapter, 1 CNNSubsampling, 2 CNNAdapter and CNNSubsampling with
+    // 4 * enc_out_dim < llm_embed_dim, adapter.py:10-57,83-96), then a norm of the last conv's rows (ad_ln_*: LayerNorm
+    // or folded BatchNorm, then ReLU or GELU) and the projection to llm_dim
+    struct AdStage {
+        void* w = nullptr;                    // [cout][KA * cin] (implicit GEMM over the staged rows)
+        float* b = nullptr;
+        int cin = 0, cout = 0, stride = 1;
+        float *in_scale = nullptr, *in_shift = nullptr;   // folded BatchNorm of the previous conv: conv_stage feeds
+                                                          // ReLU(x * scale + shift) to this one
+        float* cache = nullptr;               // [slot][2][k-1][cin] fp32, double buffered by ad_valid (carried caches only)
+    } ad_st[2];
+    int ad_nst = 0;
+    bool ad_carry = false;                    // CNNSubsampling carries the caches; CNNAdapter starts from zeros every call
+    float ad_ln_eps = 1e-3f;                  // < 0: folded BatchNorm (affine only)
+    int ad_ln_act = 1;                        // 1 ReLU, 2 GELU
+    void* ad_proj_w = nullptr;
+    float *ad_ln_g = nullptr, *ad_ln_b = nullptr, *ad_proj_b = nullptr;
     float *fb_window = nullptr, *fb_mel = nullptr;
     int *fb_lo = nullptr, *fb_hi = nullptr;
 
     // sessions
     void* ring = nullptr;                     // [L][S][2][H][cap][64]
     int32_t *n_frames = nullptr, *pe_index = nullptr, *ad_valid = nullptr;
-    float *ad_cache = nullptr, *samples = nullptr, *feat_ring = nullptr;
+    float *samples = nullptr, *feat_ring = nullptr;
     std::vector<uint8_t> slot_used;
     std::vector<int32_t> free_slots;
     long long sessions_in_use = 0;
@@ -164,9 +172,6 @@ struct fo_ctx {
         int32_t* row_start = nullptr;
     } armed;
     uint8_t* onset_dev = nullptr;
-    // adapter pass of a k-chunk call (adapter_chunks): its rows are (sessions, kk, t_out); row c of chunk jj of session b goes
-    // to output block b*k + j0 + jj.  The default is the plain layout of a single-chunk call.
-    struct ChunkRows { int k = 1, kk = 1, j0 = 0; } ad_rows;
     int groups = 1;                           // session groups whose layer kernels run on parallel streams
     cudaStream_t grp_stream[MAX_GROUPS] = {nullptr};
     cudaEvent_t ev_fork = nullptr, ev_join[MAX_GROUPS] = {nullptr};
@@ -570,19 +575,19 @@ int finalize_t(fo_ctx* c) {
             c->fb_hi = reinterpret_cast<int*>(dhi);
         }
     }
-    if (g.has_adapter && g.adapter_type == 1) {
-        FO_TRY(keep_w<TW>(c, "adapter.adpter.weight", {E, D}, &c->ad_proj_w));
-        FO_TRY(keep_f32(c, "adapter.adpter.bias", {E}, &c->ad_proj_b));
-    } else if (g.has_adapter) {
+    if (g.has_adapter) {
         // eval-mode BatchNorm1d(eps 1e-3) as a per-channel affine map of the running statistics (adapter.py:25-26,87,92,100-101):
         // y = (x - mean) / sqrt(var + 1e-3) * gamma + beta = x * s + (beta - mean * s); folded once, in double
-        auto fold_bn = [&](const std::string& name, int n, float* gam_d, float* bet_d) -> int {
+        auto keep_bn = [&](const std::string& name, int n, float** gam_d, float** bet_d, bool fold) -> int {
+            FO_TRY(keep_f32(c, "adapter." + name + ".weight", {n}, gam_d));
+            FO_TRY(keep_f32(c, "adapter." + name + ".bias", {n}, bet_d));
+            if (!fold) return 0;
             const HostTensor *rm, *rv;
             FO_TRY(need(c, "adapter." + name + ".running_mean", {n}, &rm));
             FO_TRY(need(c, "adapter." + name + ".running_var", {n}, &rv));
             std::vector<float> gam(n), bet(n), mean(n), var(n);
-            FO_CUDA(cudaMemcpy(gam.data(), gam_d, n * sizeof(float), cudaMemcpyDeviceToHost));
-            FO_CUDA(cudaMemcpy(bet.data(), bet_d, n * sizeof(float), cudaMemcpyDeviceToHost));
+            FO_CUDA(cudaMemcpy(gam.data(), *gam_d, n * sizeof(float), cudaMemcpyDeviceToHost));
+            FO_CUDA(cudaMemcpy(bet.data(), *bet_d, n * sizeof(float), cudaMemcpyDeviceToHost));
             FO_CUDA(cudaMemcpy(mean.data(), rm->d, n * sizeof(float), cudaMemcpyDeviceToHost));
             FO_CUDA(cudaMemcpy(var.data(), rv->d, n * sizeof(float), cudaMemcpyDeviceToHost));
             for (int i = 0; i < n; ++i) {
@@ -590,41 +595,30 @@ int finalize_t(fo_ctx* c) {
                 gam[i] = (float)sc;
                 bet[i] = (float)((double)bet[i] - (double)mean[i] * sc);
             }
-            FO_CUDA(cudaMemcpy(gam_d, gam.data(), n * sizeof(float), cudaMemcpyHostToDevice));
-            FO_CUDA(cudaMemcpy(bet_d, bet.data(), n * sizeof(float), cudaMemcpyHostToDevice));
+            FO_CUDA(cudaMemcpy(*gam_d, gam.data(), n * sizeof(float), cudaMemcpyHostToDevice));
+            FO_CUDA(cudaMemcpy(*bet_d, bet.data(), n * sizeof(float), cudaMemcpyHostToDevice));
             return 0;
         };
-        const HostTensor* t;
-        if (c->ad_two) {
-            // conv1d1 (C -> 2C, stride 1) + bn1 + ReLU; conv1d2 (2C -> 4C) + bn2 + ReLU; project (4C -> E).  This branch ignores
-            // activation_func / norm: the modules are BatchNorm1d and ReLU by construction (adapter.py:20-29, 84-95)
-            FO_TRY(need(c, "adapter.conv1d1.weight", {2 * D, D, KA}, &t));
-            FO_TRY(dev_alloc(c, &c->ad_conv1_w, (size_t)2 * D * D * KA * sizeof(TW)));
-            FO_TRY(repack_adapter_conv<TW>(t->d, 2 * D, D, KA, reinterpret_cast<TW*>(c->ad_conv1_w), 0));
-            FO_TRY(keep_f32(c, "adapter.conv1d1.bias", {2 * D}, &c->ad_conv1_b));
-            FO_TRY(keep_f32(c, "adapter.bn1.weight", {2 * D}, &c->ad_bn1_s));
-            FO_TRY(keep_f32(c, "adapter.bn1.bias", {2 * D}, &c->ad_bn1_t));
-            FO_TRY(fold_bn("bn1", 2 * D, c->ad_bn1_s, c->ad_bn1_t));
-            FO_TRY(need(c, "adapter.conv1d2.weight", {4 * D, 2 * D, KA}, &t));
-            FO_TRY(dev_alloc(c, &c->ad_conv_w, (size_t)4 * D * 2 * D * KA * sizeof(TW)));
-            FO_TRY(repack_adapter_conv<TW>(t->d, 4 * D, 2 * D, KA, reinterpret_cast<TW*>(c->ad_conv_w), 0));
-            FO_TRY(keep_f32(c, "adapter.conv1d2.bias", {4 * D}, &c->ad_conv_b));
-            FO_TRY(keep_f32(c, "adapter.bn2.weight", {4 * D}, &c->ad_ln_g));
-            FO_TRY(keep_f32(c, "adapter.bn2.bias", {4 * D}, &c->ad_ln_b));
-            FO_TRY(fold_bn("bn2", 4 * D, c->ad_ln_g, c->ad_ln_b));
-            FO_TRY(keep_w<TW>(c, "adapter.project.weight", {E, 4 * D}, &c->ad_proj_w));
-            FO_TRY(keep_f32(c, "adapter.project.bias", {E}, &c->ad_proj_b));
-        } else {
-            FO_TRY(need(c, "adapter.conv1d2.weight", {2 * D, D, KA}, &t));
-            FO_TRY(dev_alloc(c, &c->ad_conv_w, (size_t)2 * D * D * KA * sizeof(TW)));
-            FO_TRY(repack_adapter_conv<TW>(t->d, 2 * D, D, KA, reinterpret_cast<TW*>(c->ad_conv_w), 0));
-            FO_TRY(keep_f32(c, "adapter.conv1d2.bias", {2 * D}, &c->ad_conv_b));
-            FO_TRY(keep_f32(c, "adapter.bn2.weight", {2 * D}, &c->ad_ln_g));
-            FO_TRY(keep_f32(c, "adapter.bn2.bias", {2 * D}, &c->ad_ln_b));
-            if (g.adapter_batchnorm) FO_TRY(fold_bn("bn2", 2 * D, c->ad_ln_g, c->ad_ln_b));
-            FO_TRY(keep_w<TW>(c, "adapter.project.weight", {E, 2 * D}, &c->ad_proj_w));
-            FO_TRY(keep_f32(c, "adapter.project.bias", {E}, &c->ad_proj_b));
+        auto keep_conv = [&](const std::string& name, fo_ctx::AdStage& s) -> int {
+            const HostTensor* t;
+            FO_TRY(need(c, "adapter." + name + ".weight", {s.cout, s.cin, KA}, &t));
+            FO_TRY(dev_alloc(c, &s.w, (size_t)s.cout * s.cin * KA * sizeof(TW)));
+            FO_TRY(repack_adapter_conv<TW>(t->d, s.cout, s.cin, KA, reinterpret_cast<TW*>(s.w), 0));
+            return keep_f32(c, "adapter." + name + ".bias", {s.cout}, &s.b);
+        };
+        // two convs: conv1d1 + bn1 + ReLU, then conv1d2 + bn2 + ReLU; one conv: conv1d2 + bn2 (LayerNorm or BatchNorm)
+        const int ns = c->ad_nst;
+        if (ns == 2) {
+            FO_TRY(keep_conv("conv1d1", c->ad_st[0]));
+            FO_TRY(keep_bn("bn1", c->ad_st[1].cin, &c->ad_st[1].in_scale, &c->ad_st[1].in_shift, true));
         }
+        if (ns > 0) {
+            FO_TRY(keep_conv("conv1d2", c->ad_st[ns - 1]));
+            FO_TRY(keep_bn("bn2", c->ad_st[ns - 1].cout, &c->ad_ln_g, &c->ad_ln_b, c->ad_ln_eps < 0.f));
+        }
+        const std::string proj = ns > 0 ? "adapter.project" : "adapter.adpter";    // LinearAdapter's module name, spelt as such
+        FO_TRY(keep_w<TW>(c, proj + ".weight", {E, ns > 0 ? c->ad_st[ns - 1].cout : D}, &c->ad_proj_w));
+        FO_TRY(keep_f32(c, proj + ".bias", {E}, &c->ad_proj_b));
     }
     FO_CUDA(cudaDeviceSynchronize());
     for (auto& kv : c->staged) cudaFree(kv.second.d);
@@ -646,149 +640,78 @@ FbankParams fbank_params(fo_ctx* c) {
     return p;
 }
 
-// frames the adapter emits for T encoder frames: CNNSubsampling = causal conv(k, stride 2) over k-1 cached / padded frames
-// (adapter.py:137-144); LinearAdapter keeps the frame rate (adapter.py:69-70)
-inline int ad_frames(const fo_ctx* c, int T) {
-    if (c->cfg.adapter_type == 1 || c->cfg.adapter_type == 2) return T;      // LinearAdapter / CNNAdapter: stride 1 throughout
-    return (T + c->KA - 1 - c->KA) / 2 + 1;
+// frames out of the first n adapter convolutions (default: all) for T encoder frames.  A causal conv over k-1 cached / padded
+// frames maps T frames to (T - 1) / stride + 1 (adapter.py:137-144); LinearAdapter keeps the frame rate (adapter.py:69-70).
+inline int ad_frames(const fo_ctx* c, int T, int n = -1) {
+    for (int i = 0; i < (n < 0 ? c->ad_nst : n); ++i) T = (T - 1) / c->ad_st[i].stride + 1;
+    return T;
 }
 
-// RowMap of the adapter's last GEMM onto output blocks of `pitch` rows (fo_ctx::ad_rows); pass_rows = output rows per session
-// of this pass (kk chunks); *base_row = row of the first block
-inline void chunk_rowmap(const fo_ctx* c, int pass_rows, long long pitch, RowMap* rm, long long* base_row) {
-    const fo_ctx::ChunkRows& cr = c->ad_rows;
-    const int t_out = pass_rows / cr.kk;
-    rm->p1 = cr.kk * t_out; rm->p0 = t_out; rm->v1 = cr.kk; rm->v0 = t_out; rm->q1 = (int)(cr.k * pitch); rm->q0 = (int)pitch;
-    *base_row = (long long)cr.j0 * pitch;
+// Where the adapter's projection writes: fp32 rows of y, or fp16 rows of an LLM hand-off buffer (audioLLM.py:404-411), base
+// past the prefix.  The rows of a pass are (session, kk chunks, t_out frames); row r of chunk jj of session b goes to row r of
+// output block b * k + j0 + jj, blocks `pitch` rows apart.  A pass into y with kk == k is plain row-major.
+struct AdOut {
+    float* y = nullptr;
+    void* h16 = nullptr;      // instead of y
+    long long pitch = 0;      // rows per output block
+    int k = 1, kk = 1, j0 = 0;
+};
+
+// RowMap of the projection onto o's blocks, t_out rows per chunk; returns the row of the first block
+inline long long chunk_rowmap(const AdOut& o, int t_out, RowMap* rm) {
+    rm->p1 = o.kk * t_out; rm->p0 = t_out; rm->v1 = o.kk; rm->v0 = t_out; rm->q1 = (int)(o.k * o.pitch); rm->q0 = (int)o.pitch;
+    return (long long)o.j0 * o.pitch;
 }
 
 // ---- adapter program on device buffers -----------------------------------------------------------
-// enc (B, T, D) fp32 -> y (B, t_out, E) fp32.  Slot-resident cache when ids != null.
+// enc (B, T, D) fp32 -> B * t_out rows of E at `out`.  Each conv: conv_stage builds its A operand from [left context | input
+// rows] (the mask on the first conv's input, the previous conv's folded BatchNorm + ReLU on a later one), then an implicit
+// GEMM into fp32; the last conv's rows are normalised and projected.  LinearAdapter projects the encoder rows as they are
+// (the reference does not even apply the pad mask).  Left context: the slot caches of ids_dev when the adapter carries them,
+// else per stage cache_in[i] (reference layout (B, C, k-1); null = zeros), the new one to cache_out[i] if given.
 template <typename TA>
 int adapter_program(fo_ctx* c, const float* enc, const uint8_t* mask, int B, int T, const int32_t* ids_dev,
-                    const float* cache_in, float* cache_out, float* y, cudaStream_t st,
-                    const float* cache2_in = nullptr, float* cache2_out = nullptr) {
-    const int D = c->D, E = c->E, KA = c->KA, km1 = KA - 1;
-    if (c->ad_two) {
-        // CNNAdapter (adapter.py:33-57) / two-conv CNNSubsampling (adapter.py:112-157 with cnn_num == 2):
-        //   stage(x | cache1) -> conv1d1 (stride 1) -> [bn1 + ReLU fused into the next staging] -> stage(. | cache0) -> conv1d2
-        //   (stride 1 or 2) -> bn2 + ReLU -> project.  Both convolutions are implicit GEMMs off the staged rows.
-        const bool cached = c->cfg.adapter_type == 0;             // CNNAdapter carries no cache: zero left context every call
-        const int s2 = c->ad_stride2;
-        const int t_out = s2 == 1 ? T : (T - 1) / 2 + 1;
-        const int Mo = B * t_out;
-        void *xin, *c1out, *xin2, *aconv, *ah;
-        AGather ga1, ga2;
-        RowMap rm1, rm2;
-        conv1d_gather(B, T, D, KA, &ga1, &rm1);
-        if (s2 == 1) conv1d_gather(B, T, 2 * D, KA, &ga2, &rm2);
-        else adapter_gather(B, T, 2 * D, KA, &ga2, &rm2);
-        FO_TRY(ws_ensure(c, WS_XIN, (size_t)ga1.rows * D * sizeof(TA), &xin));
-        FO_TRY(ws_ensure(c, WS_AC1, (size_t)B * T * 2 * D * sizeof(float), &c1out));
-        FO_TRY(ws_ensure(c, WS_XIN2, (size_t)ga2.planes * ga2.rows * 2 * D * sizeof(TA), &xin2));
-        FO_TRY(ws_ensure(c, WS_ACONV, (size_t)Mo * 4 * D * sizeof(float), &aconv));
-        FO_TRY(ws_ensure(c, WS_AH, (size_t)Mo * 4 * D * sizeof(TA), &ah));
-        const int32_t* ids1 = cached ? ids_dev : nullptr;
-        FO_TRY(conv_stage<TA>(enc, mask, B, T, D, km1, 1, nullptr, nullptr, ids1, c->ad_cache, c->ad_valid,
-                              cached ? cache_in : nullptr, cached ? cache_out : nullptr, reinterpret_cast<TA*>(xin), st));
-        Epilogue e1;
-        e1.bias = c->ad_conv1_b;
-        e1.c_f32 = reinterpret_cast<float*>(c1out);
-        e1.ldc = 2 * D;
-        if (!(c->debug_skip & 16))
-            FO_TRY(gemm<TA>(c, reinterpret_cast<const TA*>(xin), ga1, c->ad_conv1_w, (int)ga1.rows, 2 * D, KA * D, e1, rm1, st));
-        FO_TRY(conv_stage<TA>(reinterpret_cast<const float*>(c1out), nullptr, B, T, 2 * D, km1, s2, c->ad_bn1_s, c->ad_bn1_t, ids1,
-                              c->ad_cache2, c->ad_valid, cached ? cache2_in : nullptr, cached ? cache2_out : nullptr,
-                              reinterpret_cast<TA*>(xin2), st));
-        Epilogue e2;
-        e2.bias = c->ad_conv_b;
-        e2.c_f32 = reinterpret_cast<float*>(aconv);
-        e2.ldc = 4 * D;
-        if (!(c->debug_skip & 16))
-            FO_TRY(gemm<TA>(c, reinterpret_cast<const TA*>(xin2), ga2, c->ad_conv_w, (int)ga2.rows, 4 * D, KA * 2 * D, e2, rm2, st));
-        FO_TRY(layer_norm<TA>(reinterpret_cast<const float*>(aconv), Mo, 4 * D, c->ad_ln_g, c->ad_ln_b, -1.0f /* folded BatchNorm */,
-                              1 /* ReLU */, 1.0f, reinterpret_cast<TA*>(ah), nullptr, st));
-        Epilogue e3;
-        e3.bias = c->ad_proj_b;
-        e3.c_f32 = y;
-        e3.ldc = E;
-        RowMap rm3;
-        long long base;
-        if (c->handoff && ids_dev) {
-            chunk_rowmap(c, t_out, c->handoff_rows, &rm3, &base);
-            e3.c_f32 = nullptr;
-            e3.c_act = reinterpret_cast<TA*>(c->handoff) + (c->handoff_off + base) * E;
-        } else if (c->ad_rows.kk != c->ad_rows.k) {              // one chunk of a chunk-by-chunk pass
-            chunk_rowmap(c, t_out, t_out, &rm3, &base);
-            e3.c_f32 = y + base * E;
-        }
-        if (!(c->debug_skip & 16))
-            FO_TRY(gemm<TA>(c, reinterpret_cast<const TA*>(ah), plain_rows(4 * D, Mo), c->ad_proj_w, Mo, E, 4 * D, e3, rm3, st));
-        return 0;
-    }
-    if (c->cfg.adapter_type == 1) {
-        // LinearAdapter: one GEMM over the encoder frames as they are (the reference does not even apply the pad mask)
-        const int M = B * T;
-        void* xin;
-        FO_TRY(ws_ensure(c, WS_XIN, (size_t)M * D * sizeof(TA), &xin));
-        const TA* a_in;
-        if (sizeof(TA) == 2) {
-            FO_TRY(f32_to_act16(enc, reinterpret_cast<act16*>(xin), (long long)M * D, st));
-            a_in = reinterpret_cast<const TA*>(xin);
-        } else {
-            a_in = reinterpret_cast<const TA*>(enc);
-        }
+                    const float* const* cache_in, float* const* cache_out, const AdOut& out, cudaStream_t st) {
+    const int D = c->D, E = c->E, KA = c->KA, ns = c->ad_nst, t_out = ad_frames(c, T), M = B * t_out;
+    const bool run_gemm = !(c->debug_skip & 16);
+    const float* x = enc;
+    for (int i = 0; i < ns; ++i) {
+        const fo_ctx::AdStage& s = c->ad_st[i];
+        const int Ti = ad_frames(c, T, i);
+        AGather ga;
+        RowMap rm;
+        if (s.stride == 1) conv1d_gather(B, Ti, s.cin, KA, &ga, &rm);
+        else adapter_gather(B, Ti, s.cin, KA, &ga, &rm);
+        void *xin, *conv;
+        FO_TRY(ws_ensure(c, i == 0 ? WS_XIN : WS_XIN2, (size_t)ga.planes * ga.rows * s.cin * sizeof(TA), &xin));
+        FO_TRY(ws_ensure(c, i + 1 == ns ? WS_ACONV : WS_AC1, (size_t)B * ad_frames(c, T, i + 1) * s.cout * sizeof(float), &conv));
+        FO_TRY(conv_stage<TA>(x, i == 0 ? mask : nullptr, B, Ti, s.cin, KA - 1, s.stride, s.in_scale, s.in_shift,
+                              c->ad_carry ? ids_dev : nullptr, s.cache, c->ad_valid, cache_in ? cache_in[i] : nullptr,
+                              cache_out ? cache_out[i] : nullptr, reinterpret_cast<TA*>(xin), st));
         Epilogue e;
-        e.bias = c->ad_proj_b;
-        e.c_f32 = y;
-        e.ldc = E;
-        RowMap rml;
-        if (c->handoff && ids_dev) {
-            long long base;
-            chunk_rowmap(c, T, c->handoff_rows, &rml, &base);
-            e.c_f32 = nullptr;
-            e.c_act = reinterpret_cast<TA*>(c->handoff) + (c->handoff_off + base) * E;
-        }
-        if (!(c->debug_skip & 16)) FO_TRY(gemm<TA>(c, a_in, plain_rows(D, M), c->ad_proj_w, M, E, D, e, rml, st));
-        return 0;
+        e.bias = s.b;
+        e.c_f32 = reinterpret_cast<float*>(conv);
+        e.ldc = s.cout;
+        if (run_gemm) FO_TRY(gemm<TA>(c, reinterpret_cast<const TA*>(xin), ga, s.w, (int)ga.rows, s.cout, KA * s.cin, e, rm, st));
+        x = reinterpret_cast<const float*>(conv);
     }
-    const int t_out = (T + km1 - KA) / 2 + 1;
-    const int Mo = B * t_out;
-    void *xin, *aconv, *ah;
-    AGather ga;
+    const int K = ns > 0 ? c->ad_st[ns - 1].cout : D;
+    const TA* a = reinterpret_cast<const TA*>(enc);
+    if (ns > 0 || sizeof(TA) == 2) {                 // the projection's operand in the activation type
+        void* ah;
+        FO_TRY(ws_ensure(c, ns > 0 ? WS_AH : WS_XIN, (size_t)M * K * sizeof(TA), &ah));
+        if (ns > 0) FO_TRY(layer_norm<TA>(x, M, K, c->ad_ln_g, c->ad_ln_b, c->ad_ln_eps, c->ad_ln_act, 1.0f, reinterpret_cast<TA*>(ah), nullptr, st));
+        else FO_TRY(f32_to_act16(enc, reinterpret_cast<act16*>(ah), (long long)M * D, st));
+        a = reinterpret_cast<const TA*>(ah);
+    }
+    Epilogue e;
+    e.bias = c->ad_proj_b;
+    e.ldc = E;
     RowMap rm;
-    adapter_gather(B, T, D, KA, &ga, &rm);
-    FO_TRY(ws_ensure(c, WS_XIN, (size_t)2 * ga.rows * D * sizeof(TA), &xin));
-    FO_TRY(ws_ensure(c, WS_ACONV, (size_t)Mo * 2 * D * sizeof(float), &aconv));
-    FO_TRY(ws_ensure(c, WS_AH, (size_t)Mo * 2 * D * sizeof(TA), &ah));
-    FO_TRY(adapter_stage<TA>(enc, mask, B, T, D, km1, ids_dev, c->ad_cache, c->ad_valid, cache_in, cache_out,
-                             reinterpret_cast<TA*>(xin), st));
-    Epilogue e1;
-    e1.bias = c->ad_conv_b;
-    e1.c_f32 = reinterpret_cast<float*>(aconv);
-    e1.ldc = 2 * D;
-    if (!(c->debug_skip & 16)) FO_TRY(gemm<TA>(c, reinterpret_cast<const TA*>(xin), ga, c->ad_conv_w, (int)ga.rows, 2 * D, KA * D, e1, rm, st));
-    FO_TRY(layer_norm<TA>(reinterpret_cast<const float*>(aconv), Mo, 2 * D, c->ad_ln_g, c->ad_ln_b,
-                          c->cfg.adapter_batchnorm ? -1.0f : 1e-3f,      // eps < 0: affine only (folded BatchNorm)
-                          c->cfg.adapter_gelu ? 2 : 1, 1.0f, reinterpret_cast<TA*>(ah), nullptr, st));
-    Epilogue e2;
-    e2.bias = c->ad_proj_b;
-    e2.c_f32 = y;
-    e2.ldc = E;
-    RowMap rm2;
-    long long base;
-    if (c->handoff && ids_dev) {
-        // LLM hand-off (audioLLM.py:404-411): rows of session b go, as fp16, to row  b * rows_per_session + row_offset + j  of
-        // the caller's inputs_embeds buffer, straight from the projection's epilogue (no fp32 copy, no cat, no .half())
-        chunk_rowmap(c, t_out, c->handoff_rows, &rm2, &base);
-        e2.c_f32 = nullptr;
-        e2.c_act = reinterpret_cast<TA*>(c->handoff) + (c->handoff_off + base) * E;
-    } else if (c->ad_rows.kk != c->ad_rows.k) {                  // one chunk of a chunk-by-chunk pass
-        chunk_rowmap(c, t_out, t_out, &rm2, &base);
-        e2.c_f32 = y + base * E;
-    }
-    if (!(c->debug_skip & 16))
-        FO_TRY(gemm<TA>(c, reinterpret_cast<const TA*>(ah), plain_rows(2 * D, Mo), c->ad_proj_w, Mo, E, 2 * D, e2, rm2, st));
+    const long long base = (out.h16 || out.kk != out.k) ? chunk_rowmap(out, t_out / out.kk, &rm) : 0;
+    if (out.h16) e.c_act = reinterpret_cast<TA*>(out.h16) + base * E;   // straight from the epilogue: no fp32 copy, no .half()
+    else e.c_f32 = out.y + base * E;
+    if (run_gemm) FO_TRY(gemm<TA>(c, a, plain_rows(K, M), c->ad_proj_w, M, E, K, e, rm, st));
     return 0;
 }
 
@@ -1087,29 +1010,28 @@ int stack_program(fo_ctx* c, int n, int t, float* x, void* qkv, float* q32, void
 }
 
 // The adapter of a k-chunk call (rows (session, chunk, frame) in enc), equal to k sequential single-chunk calls per session.
+// `out` names one output block per (session, chunk); this function sets its chunk mapping.
 template <typename TA>
-int adapter_chunks(fo_ctx* c, const float* enc, int n, int k, int t, float* y, cudaStream_t st) {
-    struct Reset { fo_ctx* c; ~Reset() { c->ad_rows = fo_ctx::ChunkRows(); } } reset{c};
+int adapter_chunks(fo_ctx* c, const float* enc, int n, int k, int t, AdOut out, cudaStream_t st) {
     // LinearAdapter works per row and CNNAdapter starts from zero left context on every call (adapter.py:41-52):
     // n*k independent blocks of t frames
-    if (c->cfg.adapter_type != 0) return adapter_program<TA>(c, enc, nullptr, n * k, t, c->ids_dev, nullptr, nullptr, y, st);
+    if (!c->ad_carry) return adapter_program<TA>(c, enc, nullptr, n * k, t, c->ids_dev, nullptr, nullptr, out, st);
+    out.k = k;
     if (t % 2 == 0) {
         // CNNSubsampling with even t: every chunk brings an even number of frames to the stride-2 conv, so one pass over a
         // session's k*t frames with the carried cache gives the k sequential outputs and leaves the same cache
-        c->ad_rows.k = c->ad_rows.kk = k;
-        return adapter_program<TA>(c, enc, nullptr, n, k * t, c->ids_dev, nullptr, nullptr, y, st);
+        out.kk = k;
+        return adapter_program<TA>(c, enc, nullptr, n, k * t, c->ids_dev, nullptr, nullptr, out, st);
     }
     // odd t: the output phase of the stride-2 conv shifts between chunks (a joint pass yields other frames, and fewer), so
     // the chunks run one by one, flipping the live half of the double-buffered cache in between as a session advance does
     const size_t row = (size_t)t * c->D * sizeof(float);
     void* ej;
     FO_TRY(ws_ensure(c, WS_ENCJ, (size_t)n * row, &ej));
-    c->ad_rows.k = k;
-    c->ad_rows.kk = 1;
     for (int j = 0; j < k; ++j) {
         FO_CUDA(cudaMemcpy2DAsync(ej, row, reinterpret_cast<const char*>(enc) + j * row, (size_t)k * row, row, n, cudaMemcpyDeviceToDevice, st));
-        c->ad_rows.j0 = j;
-        FO_TRY(adapter_program<TA>(c, reinterpret_cast<const float*>(ej), nullptr, n, t, c->ids_dev, nullptr, nullptr, y, st));
+        out.j0 = j;
+        FO_TRY(adapter_program<TA>(c, reinterpret_cast<const float*>(ej), nullptr, n, t, c->ids_dev, nullptr, nullptr, out, st));
         if (j + 1 < k) FO_TRY(advance_sessions(c->ids_dev, n, 0, 0, 1, nullptr, nullptr, c->ad_valid, st));
     }
     return 0;
@@ -1228,11 +1150,19 @@ int stream_program(fo_ctx* c, int n, int k, const float* feats, int t_in, float*
     }
     const bool run_adapter = c->cfg.has_adapter && (y_dev || c->handoff);
     if (run_adapter) {
-        if (k == 1) FO_TRY(adapter_program<TA>(c, enc_out_dev, nullptr, n, t, c->ids_dev, nullptr, nullptr, y_dev, st));
-        else FO_TRY(adapter_chunks<TA>(c, enc_out_dev, n, k, t, y_dev, st));
+        AdOut out;
+        if (c->handoff) {
+            out.h16 = reinterpret_cast<TA*>(c->handoff) + c->handoff_off * c->E;
+            out.pitch = c->handoff_rows;
+        } else {
+            out.y = y_dev;
+            out.pitch = ad_frames(c, t);
+        }
+        if (k == 1) FO_TRY(adapter_program<TA>(c, enc_out_dev, nullptr, n, t, c->ids_dev, nullptr, nullptr, out, st));
+        else FO_TRY(adapter_chunks<TA>(c, enc_out_dev, n, k, t, out, st));
     }
     FO_TRY(advance_sessions(c->ids_dev, n, t, c->cfg.chunk_size, c->pe_wrap, c->n_frames, c->pe_index,
-                            (run_adapter && c->cfg.adapter_type == 0) ? c->ad_valid : nullptr, st, k));
+                            (run_adapter && c->ad_carry) ? c->ad_valid : nullptr, st, k));
     return 0;
 }
 
@@ -1276,8 +1206,11 @@ int offline_program(fo_ctx* c, const float* feats, const int32_t* ilens_dev, int
         fc.B = B; fc.T = T2; fc.ids = nullptr; fc.layer = l; fc.hc = hc; fc.hp = hp; fc.fp = fp;
         FO_TRY(layer_post<TA>(c, w, x, M, reinterpret_cast<TA*>(att), reinterpret_cast<TA*>(h), reinterpret_cast<TA*>(ffh), nn, nullptr, fc, st));
     }
-    if (c->cfg.has_adapter && y_dev)
-        FO_TRY(adapter_program<TA>(c, enc_out_dev, mask2, B, T2, nullptr, nullptr, nullptr, y_dev, st));
+    if (c->cfg.has_adapter && y_dev) {
+        AdOut out;
+        out.y = y_dev;
+        FO_TRY(adapter_program<TA>(c, enc_out_dev, mask2, B, T2, nullptr, nullptr, nullptr, out, st));
+    }
     return 0;
 }
 
@@ -1325,10 +1258,24 @@ int fo_create(const fo_config* cfg, int device, int dtype, fo_ctx** out) {
     c->F = cfg->feat_dim; c->F1 = (c->F - 1) / 2; c->F2 = (c->F1 - 1) / 2;
     c->D = cfg->d_model; c->H = cfg->n_heads; c->FF = cfg->ffn_dim; c->L = cfg->n_layers; c->E = cfg->llm_dim;
     c->KA = cfg->adapter_kernel;
-    // adapter module: 0 CNNSubsampling (two convolutions when 4 * enc_out_dim < llm_embed_dim, adapter.py:83), 1 LinearAdapter,
-    // 2 CNNAdapter (two stride-1 convolutions, no cache)
-    c->ad_two = cfg->has_adapter && (cfg->adapter_type == 2 || (cfg->adapter_type == 0 && 4 * cfg->d_model < cfg->llm_dim));
-    c->ad_stride2 = cfg->adapter_type == 2 ? 1 : 2;
+    // adapter module: 0 CNNSubsampling, conv(C -> 2C, stride 2), or with 4 * enc_out_dim < llm_embed_dim (adapter.py:83)
+    // conv(C -> 2C) then conv(2C -> 4C, stride 2); 1 LinearAdapter, no conv; 2 CNNAdapter, the two convs at stride 1, no cache
+    if (cfg->has_adapter && cfg->adapter_type != 1) {
+        const bool two = cfg->adapter_type == 2 || 4 * cfg->d_model < cfg->llm_dim;
+        c->ad_nst = two ? 2 : 1;
+        c->ad_st[0].cin = c->D;
+        c->ad_st[0].cout = 2 * c->D;
+        c->ad_st[0].stride = two ? 1 : 2;
+        if (two) {
+            c->ad_st[1].cin = 2 * c->D;
+            c->ad_st[1].cout = 4 * c->D;
+            c->ad_st[1].stride = cfg->adapter_type == 2 ? 1 : 2;
+        }
+        c->ad_carry = cfg->adapter_type == 0;
+        // the two-conv modules are BatchNorm1d and ReLU by construction, whatever activation_func / norm say (adapter.py:20-29,84-95)
+        c->ad_ln_eps = two || cfg->adapter_batchnorm ? -1.0f : 1e-3f;
+        c->ad_ln_act = !two && cfg->adapter_gelu ? 2 : 1;
+    }
     c->KF = (cfg->ffn_conv_kernel >= 2 && !cfg->ffn_multi_conv) ? cfg->ffn_conv_kernel : 0;
     c->KM = cfg->ffn_multi_conv ? cfg->ffn_conv_kernel : 0;
     const bool streaming = cfg->chunk_size > 0 && cfg->left_chunks > 0;
@@ -1375,10 +1322,9 @@ int fo_create(const fo_config* cfg, int device, int dtype, fo_ctx** out) {
     {
         void* p = nullptr;
         if (!r) { r = dev_alloc(c, &p, S * sizeof(int32_t)); c->ad_valid = (int32_t*)p; }
-        if (!r) { r = dev_alloc(c, &p, (size_t)S * 2 * (c->KA - 1) * c->D * sizeof(float)); c->ad_cache = (float*)p; }
-        if (!r && c->ad_two && cfg->adapter_type == 0) {
-            r = dev_alloc(c, &p, (size_t)S * 2 * (c->KA - 1) * 2 * c->D * sizeof(float));
-            c->ad_cache2 = (float*)p;
+        for (int i = 0; i < c->ad_nst && c->ad_carry && !r; ++i) {
+            r = dev_alloc(c, &p, (size_t)S * 2 * (c->KA - 1) * c->ad_st[i].cin * sizeof(float));
+            c->ad_st[i].cache = (float*)p;
         }
         if (!r) { r = dev_alloc(c, &p, S * sizeof(int32_t)); c->ids_dev = (int32_t*)p; }
         if (!r) { r = dev_alloc(c, &p, (size_t)S * STREAM_CHUNKS_MAX_KEYS); c->onset_dev = (uint8_t*)p; }   // one flag per block, <= 128 blocks per session
@@ -1621,18 +1567,18 @@ int fo_session_import_kv(fo_ctx* c, int32_t id, int layer, const float* K, const
     return 0;
 }
 
-// reference cache list entry `which` of the configured adapter: single-conv CNNSubsampling has one entry (d_model channels);
-// the two-conv branch has cache[0] = second conv's input (2 * d_model channels) and cache[1] = first conv's input (d_model)
+// Entry `which` of the reference's cache list (adapter.py:123-143) is the left context of conv ad_nst - 1 - which: single-conv
+// CNNSubsampling has one entry (d_model channels); the two-conv branch has cache[0] = second conv's input (2 * d_model channels)
+// and cache[1] = first conv's input (d_model)
+inline int ad_stage_of_entry(const fo_ctx* c, int which) { return c->ad_nst - 1 - which; }
+
 static int ad_cache_of(fo_ctx* c, int which, float** base, int* C) {
-    FO_CHECK(c && c->ad_cache && c->cfg.adapter_type == 0, "context's adapter carries no cache");
-    if (!c->ad_two) {
-        FO_CHECK(which == 0, "single-conv CNNSubsampling has one cache entry (which = 0)");
-        *base = c->ad_cache; *C = c->D;
-    } else {
-        FO_CHECK(which == 0 || which == 1, "two-conv CNNSubsampling has cache entries 0 and 1");
-        *base = which == 0 ? c->ad_cache2 : c->ad_cache;
-        *C = which == 0 ? 2 * c->D : c->D;
-    }
+    FO_CHECK(c && c->ad_carry, "context's adapter carries no cache");
+    if (c->ad_nst == 1) FO_CHECK(which == 0, "single-conv CNNSubsampling has one cache entry (which = 0)");
+    else FO_CHECK(which == 0 || which == 1, "two-conv CNNSubsampling has cache entries 0 and 1");
+    const fo_ctx::AdStage& s = c->ad_st[ad_stage_of_entry(c, which)];
+    *base = s.cache;
+    *C = s.cin;
     return 0;
 }
 
@@ -1767,7 +1713,7 @@ inline int ws_y(int buf) { return buf ? WS_Y2 : WS_Y; }
 static int step_body(fo_ctx* c, const StepArgs& a, cudaStream_t st) {
     void *dfeats, *denc, *dy = nullptr;
     const int T1 = (a.t_in - 1) / 2, t = (T1 - 1) / 2;
-    const int km1 = c->KA - 1, t_out = ad_frames(c, t);
+    const int t_out = ad_frames(c, t);
     const size_t blocks = (size_t)a.n * a.k;
     FO_TRY(ws_ensure(c, WS_FEATS, blocks * a.t_in * c->F * sizeof(float), &dfeats));
     FO_TRY(ws_ensure(c, ws_enc(a.buf), blocks * t * c->D * sizeof(float), &denc));
@@ -1862,7 +1808,7 @@ static int stream_common(fo_ctx* c, const int32_t* ids, int n, int k, const void
     if (adapter_out) FO_CHECK(c->cfg.has_adapter, "adapter_out requested but the context has no adapter");
     FO_CHECK(!c->KM, "this context's positionwise layer is MultiLayeredConv1d, which has no streaming form (the reference module has no infer(), "
                      "models/encoder/attention.py:145-196); use fo_encode_offline");
-    const int km1 = c->KA - 1, t_out = ad_frames(c, t);
+    const int t_out = ad_frames(c, t);
     const size_t enc_bytes = (size_t)n * k * t * c->D * sizeof(float);
     const size_t y_bytes = (size_t)n * k * t_out * c->E * sizeof(float);
     if (c->copy_stream && c->async_ticket > 0) {
@@ -2073,7 +2019,7 @@ int fo_encode_offline(fo_ctx* c, const float* feats, const int32_t* ilens, int B
     const void *dfeats, *dil;
     FO_TRY(in_dev(c, feats, (size_t)B * T * c->F * sizeof(float), WS_FEATS, st, &dfeats));
     FO_TRY(in_dev(c, ilens, (size_t)B * sizeof(int32_t), WS_ILENS, st, &dil));
-    const int km1 = c->KA - 1, t_out = ad_frames(c, T2);
+    const int t_out = ad_frames(c, T2);
     const size_t enc_bytes = (size_t)B * T2 * c->D * sizeof(float), y_bytes = (size_t)B * t_out * c->E * sizeof(float);
     void *denc, *dy = nullptr, *dmask, *dil2, *damask = nullptr;
     FO_TRY(out_dev(c, enc_out, enc_bytes, WS_ENC, &denc));
@@ -2109,40 +2055,44 @@ int fo_adapter_forward2(fo_ctx* c, const float* x, const uint8_t* mask, int B, i
     cudaStream_t st = (cudaStream_t)stream;
     const int km1 = c->KA - 1, t_out = ad_frames(c, T);
     FO_CHECK(t_out >= 1, "fo_adapter_forward: input too short");
-    const bool cached = c->cfg.adapter_type == 0;
-    if (!cached) FO_CHECK(!cache0_in && !cache0_out && !cache1_in && !cache1_out, "fo_adapter_forward: this adapter carries no cache");
-    if (!c->ad_two) FO_CHECK(!cache1_in && !cache1_out, "fo_adapter_forward: single-conv CNNSubsampling has one cache entry");
-    // entry 0 / 1 of the reference's cache list (adapter.py:123-143): channels 2C / C with two convolutions, C with one
-    const int C0 = c->ad_two ? 2 * c->D : c->D, C1 = c->D;
-    const void *dx, *dm = nullptr, *dc0 = nullptr, *dc1 = nullptr;
+    if (!c->ad_carry) FO_CHECK(!cache0_in && !cache0_out && !cache1_in && !cache1_out, "fo_adapter_forward: this adapter carries no cache");
+    if (c->ad_nst < 2) FO_CHECK(!cache1_in && !cache1_out, "fo_adapter_forward: single-conv CNNSubsampling has one cache entry");
+    const void *dx, *dm = nullptr;
     FO_TRY(in_dev(c, x, (size_t)B * T * c->D * sizeof(float), WS_ENC, st, &dx));
     if (mask) FO_TRY(in_dev(c, mask, (size_t)B * T, WS_MASK2, st, &dm));
-    const size_t b0 = (size_t)B * C0 * km1 * sizeof(float), b1 = (size_t)B * C1 * km1 * sizeof(float);
-    if (cache0_in) FO_TRY(in_dev(c, cache0_in, b0, WS_TMP0, st, &dc0));
-    if (cache1_in) FO_TRY(in_dev(c, cache1_in, b1, WS_TMP4, st, &dc1));
-    void *do0 = nullptr, *do1 = nullptr, *dy;
-    if (cache0_out) FO_TRY(out_dev(c, cache0_out, b0, WS_TMP1, &do0));
-    if (cache1_out) FO_TRY(out_dev(c, cache1_out, b1, WS_TMP5, &do1));
+    // user_*[which]: the reference's cache list order; stage_*[i]: conv i's left context
+    const float* user_in[2] = {cache0_in, cache1_in};
+    float* user_out[2] = {cache0_out, cache1_out};
+    const float* stage_in[2] = {nullptr, nullptr};
+    float* stage_out[2] = {nullptr, nullptr};
+    void* dev_out[2] = {nullptr, nullptr};
+    size_t bytes[2] = {0, 0};
+    for (int w = 0; w < c->ad_nst; ++w) {
+        const int i = ad_stage_of_entry(c, w);
+        bytes[w] = (size_t)B * c->ad_st[i].cin * km1 * sizeof(float);
+        const void* din = nullptr;
+        if (user_in[w]) FO_TRY(in_dev(c, user_in[w], bytes[w], w ? WS_TMP4 : WS_TMP0, st, &din));
+        if (user_out[w]) FO_TRY(out_dev(c, user_out[w], bytes[w], w ? WS_TMP5 : WS_TMP1, &dev_out[w]));
+        stage_in[i] = (const float*)din;
+        stage_out[i] = (float*)dev_out[w];
+    }
+    void* dy;
     const size_t y_bytes = (size_t)B * t_out * c->E * sizeof(float);
     FO_TRY(out_dev(c, y, y_bytes, WS_Y, &dy));
-    // adapter_program: (cache_in, cache_out) = the FIRST conv's input cache, (cache2_*) = the second conv's
-    const float* first_in = (const float*)(c->ad_two ? dc1 : dc0);
-    float* first_out = (float*)(c->ad_two ? do1 : do0);
-    const float* second_in = (const float*)(c->ad_two ? dc0 : nullptr);
-    float* second_out = (float*)(c->ad_two ? do0 : nullptr);
-    int r = c->dtype == FO_BF16
-                ? adapter_program<act16>(c, (const float*)dx, (const uint8_t*)dm, B, T, nullptr, first_in, first_out, (float*)dy, st, second_in, second_out)
-                : adapter_program<float>(c, (const float*)dx, (const uint8_t*)dm, B, T, nullptr, first_in, first_out, (float*)dy, st, second_in, second_out);
+    AdOut out;
+    out.y = (float*)dy;
+    int r = c->dtype == FO_BF16 ? adapter_program<act16>(c, (const float*)dx, (const uint8_t*)dm, B, T, nullptr, stage_in, stage_out, out, st)
+                                : adapter_program<float>(c, (const float*)dx, (const uint8_t*)dm, B, T, nullptr, stage_in, stage_out, out, st);
     FO_TRY(r);
-    if (cache0_out) FO_TRY(out_done(cache0_out, do0, b0, st));
-    if (cache1_out) FO_TRY(out_done(cache1_out, do1, b1, st));
+    for (int w = 0; w < 2; ++w)
+        if (user_out[w]) FO_TRY(out_done(user_out[w], dev_out[w], bytes[w], st));
     FO_TRY(out_done(y, dy, y_bytes, st));
     return 0;
 }
 
 int fo_adapter_forward(fo_ctx* c, const float* x, const uint8_t* mask, int B, int T, const float* cache_in,
                        float* cache_out, float* y, void* stream) {
-    FO_CHECK(c && !(c->ad_two && c->cfg.adapter_type == 0 && (cache_in || cache_out)),
+    FO_CHECK(c && !(c->ad_carry && c->ad_nst == 2 && (cache_in || cache_out)),
              "fo_adapter_forward: the two-conv CNNSubsampling carries two caches; use fo_adapter_forward2");
     return fo_adapter_forward2(c, x, mask, B, T, cache_in, nullptr, cache_out, nullptr, y, stream);
 }

@@ -162,7 +162,7 @@ template <> __device__ __forceinline__ float2 unpack2<__half>(uint32_t v) { retu
 //     A[(plane[s] * rows + r + rowoff[s]) * seg_len + k % seg_len]
 // i.e. every k-segment is a plain 2-D box of one plane shifted by a row offset -- exactly what one TMA
 // box load fetches.  The producers write their outputs in this layout (cmvn_conv1: 6 planes indexed by
-// (kernel row, column parity); adapter_stage: 2 planes indexed by time parity), so neither convolution
+// (kernel row, column parity); conv_stage at stride 2: 2 planes indexed by time parity), so neither convolution
 // ever materialises im2col.  GEMM rows then run over a PADDED row grid; RowMap drops the padding rows
 // and compacts the rest on the way out.  Plain row-major A is the case n_seg = 1.
 struct AGather {
@@ -324,16 +324,10 @@ int layer_norm_reduce(float* x, const float* partial, int nsplit, const float* b
                       const float* beta, float eps, TA* y_act, float* y_f32, cudaStream_t st);
 // scale-copy (input-layer "none"): y = x * s
 int scale_rows(const float* x, float* y, long long n, float s, cudaStream_t st);
-// adapter staging: virtual rows x[b][0..k-2] = cache (or 0), x[b][k-1+i] = enc_out[b][i] (zeroed where
-// mask==0), stored parity-split as xin[time&1][b*RP + time/2][D] (adapter_gather);
-// new_cache = last k-1 rows (fp32).  cache layout (slot, k-1, D) time-major.
-template <typename TA>
-int adapter_stage(const float* enc_out, const uint8_t* mask, int B, int T, int D, int km1,
-                  const int32_t* ids, float* slot_cache, int32_t* slot_valid,       // slot-resident (ids != null)
-                  const float* cache_in, float* cache_out,                          // explicit (B, D, km1) layout
-                  TA* xin, cudaStream_t st);
-// generalised causal-conv staging for CNNAdapter / the two-conv CNNSubsampling branch (see conv_stage_kernel); C channels,
-// stride 1 (conv1d_gather layout) or 2 (adapter_gather layout); scale/shift != null: rows = ReLU(in * scale + shift)
+// staging of an adapter conv (see conv_stage_kernel): virtual rows x[b][0..k-2] = left context (cache or 0),
+// x[b][k-1+i] = in[b][i] (zeroed where mask == 0, or ReLU(in * scale + shift) when scale != null), C channels, stride 1
+// (conv1d_gather layout) or 2 (adapter_gather layout); new cache = last k-1 rows (fp32), slot-resident (ids != null,
+// (slot, 2, k-1, C) time-major) or explicit (B, C, k-1)
 template <typename TA>
 int conv_stage(const float* in, const uint8_t* mask, int B, int T, int C, int km1, int stride, const float* scale,
                const float* shift, const int32_t* ids, float* slot_cache, int32_t* slot_valid, const float* cache_in,

@@ -264,53 +264,16 @@ __global__ void scale_rows_kernel(const float* __restrict__ x, float* __restrict
     if (i < n) y[i] = x[i] * s;
 }
 
-// ---- adapter staging (adapter.py:120-143) ---------------------------------------------------------
-// grid (B, km1 + T); thread = channel.  Rows [0,km1): old cache or zeros; rows [km1, km1+T): masked
-// encoder output.  The new cache is the last km1 rows of that virtual concatenation.  Slot-resident
-// caches are double-buffered per slot: slot_valid = 0 (None), 1 (half 0 live), 2 (half 1 live); the
-// new rows go to the other half and advance_sessions() flips the flag after every block has read it.
-template <typename TA>
-__global__ void adapter_stage_kernel(const float* __restrict__ enc_out, const uint8_t* __restrict__ mask, int T, int D,
-                                     int km1, const int32_t* __restrict__ ids, float* slot_cache,
-                                     const int32_t* __restrict__ slot_valid, const float* __restrict__ cache_in,
-                                     float* cache_out, TA* __restrict__ xin) {
-    FO_PDL_TRIGGER();
-    FO_PDL_WAIT();
-    const int b = blockIdx.x, r = blockIdx.y;          // r in [0, km1 + T)
-    const int slot = ids ? ids[b] : -1;
-    const int live = ids ? slot_valid[slot] : 0;
-    const bool have_old = ids ? (live != 0) : (cache_in != nullptr);
-    const float* old_half = ids ? slot_cache + ((long long)slot * 2 + (live == 2 ? 1 : 0)) * km1 * D : nullptr;
-    float* new_half = ids ? slot_cache + ((long long)slot * 2 + (live == 1 ? 1 : 0)) * km1 * D : nullptr;
-    const int RP = (km1 + T + 1) >> 1;                 // rows per plane and batch entry (adapter_gather)
-    for (int c = threadIdx.x; c < D; c += blockDim.x) {
-        float v;
-        if (r < km1) {
-            if (!have_old) v = 0.f;
-            else if (ids) v = old_half[(long long)r * D + c];
-            else v = cache_in[((long long)b * D + c) * km1 + r];
-        } else {
-            int t = r - km1;
-            v = enc_out[((long long)b * T + t) * D + c];
-            if (mask && !mask[(long long)b * T + t]) v = 0.f;
-        }
-        xin[(((long long)(r & 1) * gridDim.x + b) * RP + (r >> 1)) * D + c] = from_f<TA>(v);
-        int cr = r - T;                                  // row of the new cache this element becomes
-        if (cr >= 0) {
-            if (ids) new_half[(long long)cr * D + c] = v;
-            else if (cache_out) cache_out[((long long)b * D + c) * km1 + cr] = v;
-        }
-    }
-}
-
-// ---- generalised causal-conv staging (CNNAdapter adapter.py:33-52; two-conv CNNSubsampling adapter.py:123-143) ---------
-// Builds the A operand of a causal Conv1d(C -> *, k, stride) run as an implicit GEMM from fp32 rows `in` (B, T, C):
+// ---- causal-conv staging of the adapter (CNNSubsampling adapter.py:120-143; CNNAdapter adapter.py:33-52) ---------------
+// grid (B, km1 + T); thread = channel.  Builds the A operand of a causal Conv1d(C -> *, k, stride) run as an implicit GEMM
+// from fp32 rows `in` (B, T, C):
 //   virtual rows [0, km1) = left context (old cache, or zeros), rows [km1, km1 + T) = f(in) with
 //   f(v) = v (masked to 0 where mask == 0)                         when scale == nullptr  (first conv: the module's input)
 //   f(v) = max(v * scale[c] + shift[c], 0)                         otherwise             (second conv: ReLU(BatchNorm_eval(conv1)))
 // stride 1: one plane, xin[b * (km1 + T) + r][C] (conv1d_gather);  stride 2: two planes by row parity (adapter_gather).
-// The new cache = the last km1 virtual rows, fp32, time-major (slot caches double-buffered exactly as in adapter_stage_kernel;
-// explicit caches in the reference layout (B, C, km1)).
+// The new cache = the last km1 virtual rows, fp32: explicit caches in the reference layout (B, C, km1); slot-resident caches
+// time-major and double-buffered per slot: slot_valid = 0 (None), 1 (half 0 live), 2 (half 1 live); the new rows go to the
+// other half and advance_sessions() flips the flag after every block has read it.
 template <typename TA>
 __global__ void conv_stage_kernel(const float* __restrict__ in, const uint8_t* __restrict__ mask, int T, int C, int km1, int stride,
                                   const float* __restrict__ scale, const float* __restrict__ shift,
@@ -585,22 +548,6 @@ int scale_rows(const float* x, float* y, long long n, float s, cudaStream_t st) 
     FO_CUDA(cudaGetLastError());
     return 0;
 }
-
-template <typename TA>
-int adapter_stage(const float* enc_out, const uint8_t* mask, int B, int T, int D, int km1, const int32_t* ids,
-                  float* slot_cache, int32_t* slot_valid, const float* cache_in, float* cache_out, TA* xin,
-                  cudaStream_t st) {
-    if (B <= 0) return 0;
-    dim3 grid(B, km1 + T);
-    FO_CUDA(launch_pdl(adapter_stage_kernel<TA>, grid, dim3(256), 0, st, enc_out, mask, T, D, km1, ids, slot_cache,
-                       (const int32_t*)slot_valid, cache_in, cache_out, xin));
-    FO_LAUNCHED();
-    FO_CUDA(cudaGetLastError());
-    return 0;
-}
-template int adapter_stage<float>(const float*, const uint8_t*, int, int, int, int, const int32_t*, float*, int32_t*, const float*, float*, float*, cudaStream_t);
-template int adapter_stage<bf16>(const float*, const uint8_t*, int, int, int, int, const int32_t*, float*, int32_t*, const float*, float*, bf16*, cudaStream_t);
-template int adapter_stage<__half>(const float*, const uint8_t*, int, int, int, int, const int32_t*, float*, int32_t*, const float*, float*, __half*, cudaStream_t);
 
 // rows of B sequences (B, T, C) copied into zero-padded sequences (B, lead + T + trail, C): the A operand of a Conv1d with
 // symmetric padding run as an implicit GEMM (MultiLayeredConv1d, attention.py:171-184); 16-byte chunks

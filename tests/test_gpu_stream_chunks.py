@@ -150,6 +150,42 @@ def test_variants_vs_sequential_single_chunk_calls(name):
         eng.close()
 
 
+@pytest.mark.parametrize("name", ["tiny_linear", "cnn", "two", "tiny_bn", "fork_t7"])
+def test_handoff_through_every_adapter_variant(name):
+    """The fp16 LLM hand-off of every adapter variant on a bf16 engine, k = 1 then 3: an armed call writes, behind the prefix of
+    each (session, chunk) block, the adapter rows that twin sessions get as fp32, rounded to fp16 bit for bit; the prefix and
+    trailing rows keep what they held; both sets of sessions end in the same state.  fork_t7 (t = 7): the CNNSubsampling adapter
+    runs chunk by chunk, so its later chunks land in blocks j0 > 0 of a session."""
+    cfg = _variant(name)
+    t_in = 32 if name == "fork_t7" else cfg.chunk_feat_frames
+    eng = engine(cfg, adapter_seed=5 if name in ("cnn", "two") else 3, dtype=torch.bfloat16, max_sessions=4)
+    try:
+        a, b = eng.alloc(2), eng.alloc(2)
+        feats = feats_for(cfg, 2, 4, 21, t_in)
+        _, t_out = eng.out_frames(t_in)
+        P = 3
+        g = torch.Generator().manual_seed(22)
+        c0 = 0
+        for k in (1, 3):
+            f = feats[:, c0:c0 + k].contiguous()
+            emb = torch.randn(2 * k, P + t_out + 2, cfg.llm_dim, generator=g).half().cuda()
+            before = emb.clone()
+            eng.handoff_arm(2 * k, emb, P, [1, 0] * k)
+            eng.encode_stream_chunks(a, f, want_adapter=False)
+            _, y = eng.encode_stream_chunks(b, f)
+            torch.cuda.synchronize()
+            assert torch.equal(emb[:, P:P + t_out], y.reshape(2 * k, t_out, cfg.llm_dim).half()), k
+            assert torch.equal(emb[:, :P], before[:, :P]) and torch.equal(emb[:, P + t_out:], before[:, P + t_out:]), k
+            for s, r in zip(a, b):
+                assert eng.state(int(s)) == eng.state(int(r))
+                if cfg.adapter_type == "subsampling":
+                    for w in range(2 if cfg.adapter_two_conv else 1):
+                        assert torch.equal(eng.export_adapter_cache(int(s), w), eng.export_adapter_cache(int(r), w)), (k, w)
+            c0 += k
+    finally:
+        eng.close()
+
+
 def test_shipped_bf16_vs_oracle_on_bf16_weights(shipped16):
     cfg, eng = shipped16
     esd, asd = bf16_weights(make_encoder_state(cfg, 0)), bf16_weights(make_adapter_state(cfg, 0))
