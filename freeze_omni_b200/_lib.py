@@ -51,6 +51,9 @@ SYMBOLS = {
     "fo_session_export_adapter_cache_n": (C.c_int, [_P, C.c_int32, C.c_int, _P, _I32P]),
     "fo_session_import_adapter_cache_n": (C.c_int, [_P, C.c_int32, C.c_int, _P, C.c_int32]),
     "fo_session_export_ffn_cache": (C.c_int, [_P, C.c_int32, C.c_int, _P]),
+    "fo_session_snapshot_bytes": (C.c_int, [_P, _I64P]),
+    "fo_session_save": (C.c_int, [_P, _I32P, C.c_int, _P, _P]),
+    "fo_session_restore": (C.c_int, [_P, _I32P, C.c_int, _P, _P]),
     "fo_fbank_stream": (C.c_int, [_P, _I32P, C.c_int, _P, C.c_int, C.c_float, _P, _P]),
     "fo_fbank_offline": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int64, C.c_float, _P, _P]),
     "fo_encode_stream": (C.c_int, [_P, _I32P, C.c_int, _P, C.c_int, _P, _P, _P]),

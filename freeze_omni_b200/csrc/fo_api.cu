@@ -194,6 +194,14 @@ struct fo_ctx {
     };
     std::map<std::string, StepGraph> graphs;
     long long ws_epoch = 0;
+    // session snapshots (fo_session_save / fo_session_restore): buffers of their own, allocated at the first use, so that a
+    // snapshot between two graph-replayed steps neither grows a step workspace nor invalidates the captured graphs
+    int32_t* snap_ids_dev = nullptr;
+    int32_t* snap_ids_host = nullptr;         // pinned; reused once snap_ids_event (its last upload) has completed
+    cudaEvent_t snap_ids_event = nullptr;
+    int32_t* snap_hdr_host = nullptr;         // pinned [max_sessions][SNAP_HDR_WORDS]: headers of a device buffer, read back
+    char* snap_stage = nullptr;               // device staging of host buffers, snap_stage_n records
+    int snap_stage_n = 0;
     cudaStream_t cap_stream = nullptr;        // capture happens here (the caller's stream may be the legacy
                                               // default stream, which cannot be captured); replay on the caller's
     // stats
@@ -1378,6 +1386,9 @@ int fo_destroy(fo_ctx* c) {
     }
     if (c->ev_fork) cudaEventDestroy(c->ev_fork);
     if (c->ev_sync) cudaEventDestroy(c->ev_sync);
+    if (c->snap_ids_event) cudaEventDestroy(c->snap_ids_event);
+    if (c->snap_ids_host) cudaFreeHost(c->snap_ids_host);
+    if (c->snap_hdr_host) cudaFreeHost(c->snap_hdr_host);
     for (void* p : c->owned) if (p) cudaFree(p);
     for (int k = 0; k < fo_ctx::NSTAGE; ++k) {
         if (c->ids_host[k]) cudaFreeHost(c->ids_host[k]);
@@ -1648,6 +1659,218 @@ int fo_session_export_ffn_cache(fo_ctx* c, int32_t id, int layer, float* cache) 
     for (int r = 0; r < km1; ++r)
         for (int ch = 0; ch < D; ++ch) out[(size_t)ch * km1 + r] = tm[(size_t)r * D + ch];    // (D, k-1) as attention.py:258
     FO_CUDA(cudaMemcpy(cache, out.data(), out.size() * 4, cudaMemcpyDefault));
+    return 0;
+}
+
+// ---- session snapshots ------------------------------------------------------------------------------
+// Record of one session (fo_session_save), `bytes` per context, sections at multiples of 256 bytes:
+//   header   256 B of int32 words: [0] magic "FOSS", [1] format version, [2..3] record bytes (int64), [4..] the fingerprint
+//            below (one word per field, in that order), [56] n_frames, [57] pe_index, [58] adapter-cache valid flag (0 / 1)
+//   KV       encoder only: [L][K|V][H][window][64] in the ring's element type (fp16 for bf16 contexts, fp32 for fp32): the last
+//            min(n_frames, window) frames, oldest first, unswizzled; rows past them zero.  The window is all the streaming
+//            attention reads (single-, multi-chunk and stack kernels alike), so the record does not depend on ring_cap;
+//            restored, frame f goes to ring row f % ring_cap with the chunk swizzle c ^ (f & 7) (as ring_import_kernel)
+//   fp32     each only when the context has the part: Conv1dLinear left context [L][KF-1][D]; the live half of each carried
+//            adapter stage cache [k-1][cin] (stage order; zeros while the cache is None); fbank sample buffer [carry+chunk];
+//            feature ring [ctx+m][F]
+// The fingerprint is every setting that fixes the state's shape and meaning.  Capacities (max_sessions, max_stream_frames, hence
+// max_t and ring_cap) and run-time options are not in it: a record moves between contexts that differ in them.  Weights are not
+// in it either: restoring into a context with other weights of the same shapes is the caller's responsibility.
+namespace {
+
+constexpr int32_t SNAP_MAGIC = 0x53534F46;       // "FOSS" little-endian
+constexpr int32_t SNAP_VERSION = 1;
+constexpr int SNAP_W_FP = 4;                     // first fingerprint word
+constexpr long long SNAP_STAGE_BYTES = 64LL << 20;   // device staging of host buffers: whole records up to this size
+
+struct SnapField { const char* name; int32_t value; };
+
+std::vector<SnapField> snap_fingerprint(const fo_ctx* c) {
+    const fo_config& g = c->cfg;
+    return {{"dtype", c->dtype}, {"feat_dim", g.feat_dim}, {"d_model", g.d_model}, {"n_heads", g.n_heads}, {"ffn_dim", g.ffn_dim},
+            {"n_layers", g.n_layers}, {"chunk_size", g.chunk_size}, {"left_chunks", g.left_chunks}, {"window", c->window},
+            {"pe_wrap", c->pe_wrap}, {"ffn_conv_kernel", c->KF}, {"has_encoder", g.has_encoder != 0},
+            {"has_adapter", g.has_adapter != 0}, {"adapter_type", g.adapter_type}, {"adapter_kernel", g.adapter_kernel},
+            {"adapter_stages", c->ad_nst}, {"adapter_cin0", c->ad_st[0].cin}, {"adapter_cin1", c->ad_st[1].cin},
+            {"sample_rate", g.sample_rate}, {"frame_len", g.frame_len}, {"frame_shift", g.frame_shift},
+            {"frames_per_chunk", g.frames_per_chunk}, {"context_frames", g.context_frames}};
+}
+
+inline long long round256(long long x) { return (x + 255) & ~255LL; }
+
+// geometry of the record and of the context's state arrays; returns the record size
+long long snap_layout(fo_ctx* c, SnapArgs* a) {
+    const int S = c->cfg.max_sessions;
+    long long off = SNAP_HDR_WORDS * 4;
+    if (c->ring) {
+        a->ring = reinterpret_cast<char*>(c->ring);
+        a->L = c->L; a->S = S; a->H = c->H; a->cap = c->ring_cap; a->window = c->window; a->esz = (int)c->esz;
+        a->kv_off = off;
+        off = round256(off + (long long)c->L * 2 * c->H * c->window * 64 * c->esz);
+    }
+    a->n_frames = c->n_frames;
+    a->pe_index = c->pe_index;
+    a->ad_valid = c->ad_valid;
+    a->nseg = 0;
+    auto add = [&](void* base, long long bytes, long long stride, int half) {
+        SnapSeg& s = a->seg[a->nseg++];
+        s.base = reinterpret_cast<char*>(base); s.bytes = bytes; s.slot_stride = stride; s.rec_off = off; s.adapter_half = half;
+        off = round256(off + bytes);
+    };
+    if (c->ffn_cache) {
+        const long long b = (long long)c->L * (c->KF - 1) * c->D * 4;
+        add(c->ffn_cache, b, b, 0);
+    }
+    for (int i = 0; i < c->ad_nst && c->ad_carry; ++i) {
+        const long long b = (long long)(c->KA - 1) * c->ad_st[i].cin * 4;
+        add(c->ad_st[i].cache, b, 2 * b, 1);
+    }
+    if (c->samples) {
+        const long long b = (long long)(c->carry + c->chunk_samples) * 4;
+        add(c->samples, b, b, 0);
+        const long long f = (long long)(c->cfg.context_frames + c->cfg.frames_per_chunk) * c->F * 4;
+        add(c->feat_ring, f, f, 0);
+    }
+    memset(a->hdr, 0, sizeof(a->hdr));
+    a->hdr[0] = SNAP_MAGIC;
+    a->hdr[1] = SNAP_VERSION;
+    const long long bytes = round256(off);
+    memcpy(&a->hdr[2], &bytes, 8);
+    const std::vector<SnapField> fp = snap_fingerprint(c);
+    for (size_t i = 0; i < fp.size(); ++i) a->hdr[SNAP_W_FP + i] = fp[i].value;
+    a->rec_bytes = bytes;
+    return bytes;
+}
+
+// shared checks of save and restore and the record geometry; *on_device = buf is device memory (of this context's device: a
+// buffer of another GPU is refused, copy it over first)
+int snap_begin(fo_ctx* c, const char* fn, const int32_t* ids, int n, const void* buf, SnapArgs* a, bool* on_device) {
+    FO_CHECK(c && buf, "%s: null context or buffer", fn);
+    FO_TRY(check_ids(c, ids, n));
+    FO_CUDA(cudaSetDevice(c->device));
+    cudaPointerAttributes pa;
+    if (cudaPointerGetAttributes(&pa, buf) != cudaSuccess) { cudaGetLastError(); pa.type = cudaMemoryTypeUnregistered; }
+    *on_device = pa.type == cudaMemoryTypeDevice || pa.type == cudaMemoryTypeManaged;
+    FO_CHECK(!*on_device || pa.device == c->device, "%s: buf is memory of device %d, the context is on device %d", fn, pa.device,
+             c->device);
+    const int S = c->cfg.max_sessions;
+    if (!c->snap_ids_dev) {
+        void* p;
+        FO_TRY(dev_alloc(c, &p, (size_t)S * sizeof(int32_t)));
+        c->snap_ids_dev = (int32_t*)p;
+        FO_CUDA(cudaMallocHost((void**)&c->snap_ids_host, (size_t)S * sizeof(int32_t)));
+        FO_CUDA(cudaMallocHost((void**)&c->snap_hdr_host, (size_t)S * SNAP_HDR_WORDS * 4));
+        FO_CUDA(cudaEventCreateWithFlags(&c->snap_ids_event, cudaEventDisableTiming));
+    }
+    snap_layout(c, a);
+    a->n = n;
+    return 0;
+}
+
+// the ids of the call into the snapshot path's own device array (not the steps' ids_dev, which a step may reuse as it is)
+int snap_upload_ids(fo_ctx* c, const int32_t* ids, int n, cudaStream_t st, SnapArgs* a) {
+    FO_CUDA(cudaEventSynchronize(c->snap_ids_event));      // the previous call's upload has left the pinned array
+    memcpy(c->snap_ids_host, ids, sizeof(int32_t) * n);
+    FO_CUDA(cudaMemcpyAsync(c->snap_ids_dev, c->snap_ids_host, sizeof(int32_t) * n, cudaMemcpyHostToDevice, st));
+    FO_CUDA(cudaEventRecord(c->snap_ids_event, st));
+    a->ids = c->snap_ids_dev;
+    return 0;
+}
+
+// device staging for host buffers: a bounded number of whole records, reused batch after batch in stream order
+int snap_staging(fo_ctx* c, long long bytes) {
+    if (c->snap_stage) return 0;
+    c->snap_stage_n = (int)std::max(1LL, std::min((long long)c->cfg.max_sessions, SNAP_STAGE_BYTES / bytes));
+    void* p;
+    FO_TRY(dev_alloc(c, &p, (size_t)c->snap_stage_n * bytes));
+    c->snap_stage = (char*)p;
+    return 0;
+}
+
+// record i's header: 0, or FO_ERR_ARG naming the first field that does not match this context
+int snap_check_header(const fo_ctx* c, const SnapArgs& a, int i, const int32_t* h) {
+    FO_CHECK(h[0] == SNAP_MAGIC, "fo_session_restore: record %d: bad magic 0x%08x (not a session snapshot)", i, (unsigned)h[0]);
+    FO_CHECK(h[1] == SNAP_VERSION, "fo_session_restore: record %d: format version %d, this library reads version %d", i, h[1],
+             SNAP_VERSION);
+    // the fingerprint before the size, which follows from it: a record of another model names the setting that differs
+    const std::vector<SnapField> fp = snap_fingerprint(c);
+    for (size_t f = 0; f < fp.size(); ++f)
+        FO_CHECK(h[SNAP_W_FP + f] == fp[f].value, "fo_session_restore: record %d: %s is %d, this context has %d", i, fp[f].name,
+                 h[SNAP_W_FP + f], fp[f].value);
+    long long bytes;
+    memcpy(&bytes, &h[2], 8);
+    FO_CHECK(bytes == a.rec_bytes, "fo_session_restore: record %d: record size %lld bytes, this context's is %lld", i, bytes,
+             a.rec_bytes);
+    FO_CHECK(h[SNAP_W_NFRAMES] >= 0 && h[SNAP_W_PE] >= 0 && (h[SNAP_W_ADVALID] == 0 || h[SNAP_W_ADVALID] == 1),
+             "fo_session_restore: record %d: bad session state (n_frames %d, pe_index %d, adapter flag %d)", i, h[SNAP_W_NFRAMES],
+             h[SNAP_W_PE], h[SNAP_W_ADVALID]);
+    return 0;
+}
+
+}  // namespace
+
+int fo_session_snapshot_bytes(fo_ctx* c, int64_t* bytes) {
+    FO_CHECK(c && bytes, "fo_session_snapshot_bytes: bad argument");
+    SnapArgs a;
+    *bytes = snap_layout(c, &a);
+    return 0;
+}
+
+int fo_session_save(fo_ctx* c, const int32_t* ids, int n, void* buf, void* stream) {
+    const cudaStream_t st = (cudaStream_t)stream;
+    SnapArgs a;
+    bool on_device;
+    FO_TRY(snap_begin(c, "fo_session_save", ids, n, buf, &a, &on_device));
+    FO_TRY(snap_upload_ids(c, ids, n, st, &a));
+    if (on_device) {
+        a.rec = (char*)buf;
+        return session_pack(a, st);
+    }
+    FO_TRY(snap_staging(c, a.rec_bytes));
+    for (int i0 = 0; i0 < n; i0 += c->snap_stage_n) {
+        SnapArgs b = a;
+        b.ids = a.ids + i0;
+        b.n = std::min(c->snap_stage_n, n - i0);
+        b.rec = c->snap_stage;
+        FO_TRY(session_pack(b, st));
+        FO_CUDA(cudaMemcpyAsync((char*)buf + (size_t)i0 * a.rec_bytes, c->snap_stage, (size_t)b.n * a.rec_bytes,
+                                cudaMemcpyDeviceToHost, st));
+    }
+    return 0;
+}
+
+int fo_session_restore(fo_ctx* c, const int32_t* ids, int n, const void* buf, void* stream) {
+    const cudaStream_t st = (cudaStream_t)stream;
+    SnapArgs a;
+    bool on_device;
+    FO_TRY(snap_begin(c, "fo_session_restore", ids, n, buf, &a, &on_device));
+    // every header is checked before anything else is enqueued: a refused call leaves all n slots as they were.  The buffer may
+    // be the output of a save still in flight on `stream` (a host buffer included), hence the sync before the headers are read
+    const int32_t* hdr = (const int32_t*)buf;
+    long long hstride = a.rec_bytes / 4;
+    if (on_device) {
+        FO_CUDA(cudaMemcpy2DAsync(c->snap_hdr_host, SNAP_HDR_WORDS * 4, buf, (size_t)a.rec_bytes, SNAP_HDR_WORDS * 4, n,
+                                  cudaMemcpyDeviceToHost, st));
+        hdr = c->snap_hdr_host;
+        hstride = SNAP_HDR_WORDS;
+    }
+    FO_CUDA(cudaStreamSynchronize(st));
+    for (int i = 0; i < n; ++i) FO_TRY(snap_check_header(c, a, i, hdr + i * hstride));
+    FO_TRY(snap_upload_ids(c, ids, n, st, &a));
+    if (on_device) {
+        a.rec = (char*)buf;
+        return session_unpack(a, st);
+    }
+    FO_TRY(snap_staging(c, a.rec_bytes));
+    for (int i0 = 0; i0 < n; i0 += c->snap_stage_n) {
+        SnapArgs b = a;
+        b.ids = a.ids + i0;
+        b.n = std::min(c->snap_stage_n, n - i0);
+        b.rec = c->snap_stage;
+        FO_CUDA(cudaMemcpyAsync(c->snap_stage, (const char*)buf + (size_t)i0 * a.rec_bytes, (size_t)b.n * a.rec_bytes,
+                                cudaMemcpyHostToDevice, st));
+        FO_TRY(session_unpack(b, st));
+    }
     return 0;
 }
 

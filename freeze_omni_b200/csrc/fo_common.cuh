@@ -448,4 +448,35 @@ int ring_export(const TA* ring_kv, int H, int ring_cap, long long first_frame, i
 template <typename TA>
 int ring_import(TA* ring_kv, int H, int ring_cap, long long first_frame, int n, const float* in, cudaStream_t st);
 
+// ---- session snapshots (fo_session.cu; the record format is fo_api.cu's, see fo_session_save there) ------------------
+// One flat fp32 section of a record: `bytes` of each slot's state, copied as they are.
+struct SnapSeg {
+    char* base = nullptr;          // the context's array (slot 0)
+    long long slot_stride = 0;     // bytes between slots
+    long long rec_off = 0;         // byte offset inside a record
+    long long bytes = 0;
+    int adapter_half = 0;          // 1: double-buffered adapter cache, two halves of `bytes`; the live one is picked by ad_valid
+};
+constexpr int SNAP_HDR_WORDS = 64;             // header: 256 bytes of int32 words
+constexpr int SNAP_W_NFRAMES = 56, SNAP_W_PE = 57, SNAP_W_ADVALID = 58;   // per-session words; the rest is the same in every record
+constexpr int SNAP_MAX_SEGS = 5;
+struct SnapArgs {
+    const int32_t* ids = nullptr;  // (n) slots, device
+    int n = 0;
+    char* rec = nullptr;           // n records of rec_bytes
+    long long rec_bytes = 0;
+    // KV rings [L][S][K|V][H][cap][64] of esz-byte elements (16-bit rings chunk-swizzled by frame); null: no encoder
+    char* ring = nullptr;
+    int L = 0, S = 0, H = 0, cap = 0, window = 0, esz = 0;
+    long long kv_off = 0;          // record section [L][K|V][H][window][64]
+    int32_t *n_frames = nullptr, *pe_index = nullptr, *ad_valid = nullptr;
+    SnapSeg seg[SNAP_MAX_SEGS];
+    int nseg = 0;
+    int32_t hdr[SNAP_HDR_WORDS];   // pack: the header words every record starts with
+};
+// pack: slots -> records (header included); unpack: records -> slots (n_frames, pe_index, adapter flag from the headers,
+// which the caller has validated).  One launch each on `st`.
+int session_pack(const SnapArgs& a, cudaStream_t st);
+int session_unpack(const SnapArgs& a, cudaStream_t st);
+
 }  // namespace fo

@@ -216,6 +216,39 @@ class Engine:
             assert c.numel() == self._adapter_cache_channels(which) * (self.cfg.adapter_kernel - 1)
             _lib.check(self.lib.fo_session_import_adapter_cache_n(self._h, int(sid), int(which), c.data_ptr(), 1))
 
+    # ---- session snapshots ------------------------------------------------------------------------
+    @property
+    def snapshot_bytes(self) -> int:
+        """Size of one session's snapshot record (fo_session_snapshot_bytes); depends on the model, not on the capacities."""
+        b = C.c_int64()
+        _lib.check(self.lib.fo_session_snapshot_bytes(self._h, C.byref(b)))
+        return int(b.value)
+
+    def save_sessions(self, ids, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """The whole state of sessions `ids` as a uint8 tensor (n, snapshot_bytes), one record per row, on this engine's device
+        and stream; or into `out` (device, or host -- pinned keeps the copy asynchronous; a host `out` is complete on return).
+        Rows restore with restore_sessions here, on another engine of the same model, or on another GPU after
+        `blob.to(other.torch_device)`."""
+        ids = _ids(ids)
+        out = self._out(out, (len(ids), self.snapshot_bytes), torch.uint8)
+        _lib.check(self.lib.fo_session_save(self._h, _i32p(ids), len(ids), _ptr(out), self._stream()))
+        if not out.is_cuda:
+            torch.cuda.current_stream(self.torch_device).synchronize()
+        return out
+
+    def restore_sessions(self, ids, blob: torch.Tensor) -> None:
+        """Write records (n, snapshot_bytes) -- host, or on this engine's device -- into the allocated sessions `ids`; they
+        continue bit for bit as the saved sessions would have.  A record of another model configuration is refused (FoError
+        naming the field) before any session is touched."""
+        ids = _ids(ids)
+        if blob.dtype != torch.uint8 or not blob.is_contiguous() or tuple(blob.shape) != (len(ids), self.snapshot_bytes):
+            raise ValueError("blob must be a contiguous uint8 tensor (%d, %d), got %s %s"
+                             % (len(ids), self.snapshot_bytes, blob.dtype, tuple(blob.shape)))
+        if blob.is_cuda and blob.device != self.torch_device:
+            raise ValueError("blob is on %s, the engine on %s: copy it over first (blob.to(engine.torch_device))"
+                             % (blob.device, self.torch_device))
+        _lib.check(self.lib.fo_session_restore(self._h, _i32p(ids), len(ids), _ptr(blob), self._stream()))
+
     # ---- frontend ---------------------------------------------------------------------------------
     @staticmethod
     def _pcm_dtype(pcm: ArrayLike) -> int:

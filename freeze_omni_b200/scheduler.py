@@ -19,7 +19,8 @@ multiple of `bucket` with scratch sessions so that a handful of captured CUDA gr
 With `max_chunks` > 1 a round takes up to that many queued blocks of a session at once (Engine.encode_stream_chunks, same
 results as one block per call): an onset tick then costs one call for the sessions with one block and one for those
 replaying their history, instead of 1 + onset_chunks calls.
-State (KV rings, adapter cache, sample carry, feature ring, history ring, queued blocks) never leaves the device.
+State (KV rings, adapter cache, sample carry, feature ring, history ring, queued blocks) never leaves the device, unless a
+session is moved: `detach` / `attach` carry it, history rows included, to another scheduler on any GPU.
 """
 from collections import deque
 from typing import Any, Deque, Dict, Hashable, List, NamedTuple, Optional, Tuple
@@ -56,6 +57,16 @@ class Handoff:
         self.prefix_mask = None if prefix_mask is None else prefix_mask.reshape(-1).to(dev, torch.uint8).contiguous()
         self.attn_mask = torch.zeros(capacity, self.rows, dtype=torch.uint8, device=dev)
         self.row_start = torch.zeros(capacity, dtype=torch.int32, device=dev)
+
+
+class SessionSnapshot(NamedTuple):
+    """A session taken out of a scheduler (`StreamScheduler.detach`): the engine's snapshot record and the session's rows of
+    the history ring, which a speech onset after the move replays.  `to(device)` moves both, e.g. to another GPU's scheduler."""
+    record: torch.Tensor              # (snapshot_bytes,) uint8, Engine.save_sessions
+    history: torch.Tensor             # (history_chunks, t_in, F) fp32
+
+    def to(self, device) -> "SessionSnapshot":
+        return SessionSnapshot(self.record.to(device), self.history.to(device))
 
 
 def onset_statuses(n_history: int, status: str) -> List[str]:
@@ -171,6 +182,30 @@ class StreamScheduler:
         self._hist[self.rows[key]].zero_()
         self.queues[key].clear()
         self.pending.pop(key, None)
+
+    def detach(self, key: Hashable) -> SessionSnapshot:
+        """Take a session out of this scheduler between ticks (to rebalance GPUs, drain one, or restart a server): its whole
+        state as a SessionSnapshot, then the session is closed here.  `attach` continues it in any scheduler of the same model,
+        on any GPU, exactly as if it had stayed.  A chunk pushed since the last tick must be ticked first."""
+        if key in self.pending:
+            raise RuntimeError("session %r has a pushed chunk that was not ticked yet: tick before detaching it" % (key,))
+        snap = SessionSnapshot(self.eng.save_sessions([self.keys[key]])[0], self._hist[self.rows[key]].clone())
+        self.close(key)
+        return snap
+
+    def attach(self, key: Hashable, snap: SessionSnapshot) -> int:
+        """Open `key` with the state of a detached session; returns its slot in this scheduler's engine."""
+        if tuple(snap.history.shape) != tuple(self._hist.shape[1:]):
+            raise ValueError("history rows %s do not fit this scheduler's %s (history_chunks differ)"
+                             % (tuple(snap.history.shape), tuple(self._hist.shape[1:])))
+        slot = self.open(key)
+        try:
+            self.eng.restore_sessions([slot], snap.record.to(self.eng.torch_device).view(1, -1))
+        except Exception:
+            self.close(key)
+            raise
+        self._hist[self.rows[key]].copy_(snap.history)
+        return slot
 
     # ---- data path ----------------------------------------------------------------------------------
     def push(self, key: Hashable, pcm, status: Optional[str]) -> None:

@@ -141,6 +141,24 @@ int fo_session_import_adapter_cache_n(fo_ctx* ctx, int32_t id, int which, const 
 /* Conv1dLinear left context of one layer in the reference layout (models/encoder/attention.py:221,258): (d_model, k-1) */
 int fo_session_export_ffn_cache(fo_ctx* ctx, int32_t id, int layer, float* cache);
 
+/* ---- session snapshots: the whole state of n sessions -- KV window of every layer, pe_index, adapter caches, Conv1dLinear
+ * context, fbank sample carry, feature ring -- as n consecutive records of `bytes` each (one record can be sliced out), so that
+ * a conversation moves to another slot, context or GPU and continues bit for bit as if it had never moved.  The format
+ * (versioned; layout in fo_api.cu) carries a fingerprint of every setting that fixes the state's shape and meaning; capacities
+ * (max_sessions, max_stream_frames) and options are not in it, so a record moves between contexts that differ in them.
+ * Restoring into a context with other weights of the same shapes is not detected: the caller pairs records with their model.
+ * buf is host or device memory (a device buffer must be on the context's device).  Both calls are ordered on `stream` after
+ * every step enqueued there before (fo_stream_step_async included) and never synchronise the device; host buffers go through
+ * a staging buffer of their own, a few records at a time (a pinned host buffer is complete once `stream` reaches the call).
+ * Neither grows a step workspace: a snapshot between two graph-replayed steps does not force a re-capture. */
+int fo_session_snapshot_bytes(fo_ctx* ctx, int64_t* bytes);
+/* records of sessions ids[0..n) into buf (n x bytes) */
+int fo_session_save(fo_ctx* ctx, const int32_t* ids, int n, void* buf, void* stream);
+/* records of buf into the allocated slots ids[0..n) (fo_session_alloc; restoring into a second slot forks a session).  Every
+ * header is checked first -- for a device buf one small read-back and a sync of `stream`: a bad magic, version, record size or
+ * fingerprint field in any record is FO_ERR_ARG naming the first mismatching field, and none of the n slots is touched. */
+int fo_session_restore(fo_ctx* ctx, const int32_t* ids, int n, const void* buf, void* stream);
+
 /* ---- frontend: replaces audioEncoderProcessor.process (bin/inference.py:71-80) /
  * AudioFeatureGating._extract_fbank (models/AudioFeatureGating.py:54-75).
  * pcm: (n, frame_shift*frames_per_chunk) samples, FO_F32 or FO_I16; value used = sample * scale.
