@@ -123,7 +123,9 @@ struct fo_ctx {
     int32_t* ids_host[NSTAGE] = {nullptr};
     cudaEvent_t ids_event[NSTAGE] = {nullptr};
     int ids_cursor = 0;
-    int32_t* ids_dev = nullptr;
+    int32_t* ids_dev = nullptr;               // [3][max_sessions]: session ids, then cnt_dev and off_dev
+    int32_t* cnt_dev = nullptr;               // chunks per session of a multi-chunk call (fo_encode_stream_chunks[_v])
+    int32_t* off_dev = nullptr;               // first block of each session in that call (prefix sums of cnt)
     DevBuf ws[40];                            // named workspaces, see enum below
     // options
     int gemm_backend = 0, use_graph = 0, split_k = 1;
@@ -155,6 +157,7 @@ struct fo_ctx {
     cudaEvent_t ev_sync = nullptr;            // recorded after every synchronous step: the copy stream of a later async step
                                               // must not overwrite the staging buffers that step still reads
     std::vector<int32_t> ids_last;            // session ids currently in ids_dev (uploaded on ids_last_stream)
+    std::vector<int32_t> cnt_last;            // chunk counts currently in cnt_dev (empty: none uploaded with ids_last)
     cudaStream_t ids_last_stream = nullptr;
     std::vector<long long> id_stamp;          // check_ids: call number that last named each slot (duplicate detection)
     long long id_call = 0;
@@ -175,6 +178,8 @@ struct fo_ctx {
     int groups = 1;                           // session groups whose layer kernels run on parallel streams
     cudaStream_t grp_stream[MAX_GROUPS] = {nullptr};
     cudaEvent_t ev_fork = nullptr, ev_join[MAX_GROUPS] = {nullptr};
+    cudaStream_t mix_stream[MAX_GROUPS] = {nullptr};   // per group: the multi-chunk attention of a call that mixes counts
+    cudaEvent_t ev_mix_fork[MAX_GROUPS] = {nullptr}, ev_mix_join[MAX_GROUPS] = {nullptr};
     int profile_gemm = 0;                     // time every GEMM launch with a CUDA event pair (bench roofline)
     // weight-streaming layer stack (fo_stack.cu): all layers of a step of <= stack_rows token rows in one cooperative launch
     int stack_rows = 8;                       // option "stack_rows": steps of up to this many token rows take the stack kernel (<= STACK_MAX_ROWS; 0 = never)
@@ -212,7 +217,7 @@ struct fo_ctx {
 namespace {
 
 enum { WS_FEATS = 0, WS_C1, WS_C2, WS_XSUB, WS_EMB, WS_X, WS_H, WS_QKV, WS_ATT, WS_FFH, WS_ENC, WS_XIN, WS_ACONV, WS_AH,
-       WS_Y, WS_MASK2, WS_ILENS, WS_ILENS2, WS_AMASK, WS_PCM, WS_TMP0, WS_TMP1, WS_TMP2, WS_TMP3, WS_Q32, WS_HC, WS_PART, WS_PCM2, WS_ENC2, WS_Y2, WS_AC1, WS_XIN2, WS_TMP4, WS_TMP5, WS_HP, WS_FP, WS_ENCJ, WS_COUNT };
+       WS_Y, WS_MASK2, WS_ILENS, WS_ILENS2, WS_AMASK, WS_PCM, WS_TMP0, WS_TMP1, WS_TMP2, WS_TMP3, WS_Q32, WS_HC, WS_PART, WS_PCM2, WS_ENC2, WS_Y2, WS_AC1, WS_XIN2, WS_TMP4, WS_TMP5, WS_HP, WS_FP, WS_ENCJ, WS_PACK, WS_ADJ, WS_COUNT };
 
 int dev_alloc(fo_ctx* c, void** p, size_t bytes) {
     *p = nullptr;
@@ -287,18 +292,31 @@ int check_ids(fo_ctx* c, const int32_t* ids, int n) {
     return 0;
 }
 
-int upload_ids(fo_ctx* c, const int32_t* ids, int n, cudaStream_t st, const uint8_t* onset = nullptr, int n_onset = 0) {
-    // the same sessions as in the previous step (the steady state of a server loop): the device copy is still valid
-    if (!onset && st == c->ids_last_stream && (int)c->ids_last.size() == n && memcmp(c->ids_last.data(), ids, sizeof(int32_t) * n) == 0) return 0;
+// chunks (multi-chunk calls): the per-session counts, uploaded with their block offsets to cnt_dev / off_dev
+int upload_ids(fo_ctx* c, const int32_t* ids, int n, cudaStream_t st, const uint8_t* onset = nullptr, int n_onset = 0,
+               const int32_t* chunks = nullptr) {
+    // the same sessions (and counts) as in the previous step (the steady state of a server loop): the device copy is still valid
+    if (!onset && st == c->ids_last_stream && (int)c->ids_last.size() == n && memcmp(c->ids_last.data(), ids, sizeof(int32_t) * n) == 0 &&
+        (!chunks || ((int)c->cnt_last.size() == n && memcmp(c->cnt_last.data(), chunks, sizeof(int32_t) * n) == 0)))
+        return 0;
     c->ids_last.assign(ids, ids + n);
+    if (chunks) c->cnt_last.assign(chunks, chunks + n);
+    else c->cnt_last.clear();
     c->ids_last_stream = st;
-    const int k = c->ids_cursor;
+    const int k = c->ids_cursor, S = c->cfg.max_sessions;
     c->ids_cursor = (k + 1) % fo_ctx::NSTAGE;
     FO_CUDA(cudaEventSynchronize(c->ids_event[k]));
     memcpy(c->ids_host[k], ids, sizeof(int32_t) * n);
     FO_CUDA(cudaMemcpyAsync(c->ids_dev, c->ids_host[k], sizeof(int32_t) * n, cudaMemcpyHostToDevice, st));
-    if (onset) {                                 // second half of the pinned staging slot: the hand-off's per-session onset flags
-        uint8_t* oh = reinterpret_cast<uint8_t*>(c->ids_host[k] + c->cfg.max_sessions);
+    if (chunks) {
+        int32_t* ch = c->ids_host[k] + S;
+        memcpy(ch, chunks, sizeof(int32_t) * n);
+        for (int i = 0, o = 0; i < n; o += chunks[i++]) ch[S + i] = o;
+        FO_CUDA(cudaMemcpyAsync(c->cnt_dev, ch, sizeof(int32_t) * n, cudaMemcpyHostToDevice, st));
+        FO_CUDA(cudaMemcpyAsync(c->off_dev, ch + S, sizeof(int32_t) * n, cudaMemcpyHostToDevice, st));
+    }
+    if (onset) {                                 // behind the ids and the count table: the hand-off's per-block onset flags
+        uint8_t* oh = reinterpret_cast<uint8_t*>(c->ids_host[k] + 3 * S);
         memcpy(oh, onset, n_onset);
         FO_CUDA(cudaMemcpyAsync(c->onset_dev, oh, n_onset, cudaMemcpyHostToDevice, st));
     }
@@ -657,18 +675,17 @@ inline int ad_frames(const fo_ctx* c, int T, int n = -1) {
 
 // Where the adapter's projection writes: fp32 rows of y, or fp16 rows of an LLM hand-off buffer (audioLLM.py:404-411), base
 // past the prefix.  The rows of a pass are (session, kk chunks, t_out frames); row r of chunk jj of session b goes to row r of
-// output block b * k + j0 + jj, blocks `pitch` rows apart.  A pass into y with kk == k is plain row-major.
+// output block b * k + jj, blocks `pitch` rows apart.  A pass into y with kk == k is plain row-major.
 struct AdOut {
     float* y = nullptr;
     void* h16 = nullptr;      // instead of y
     long long pitch = 0;      // rows per output block
-    int k = 1, kk = 1, j0 = 0;
+    int k = 1, kk = 1;
 };
 
-// RowMap of the projection onto o's blocks, t_out rows per chunk; returns the row of the first block
-inline long long chunk_rowmap(const AdOut& o, int t_out, RowMap* rm) {
+// RowMap of the projection onto o's blocks, t_out rows per chunk
+inline void chunk_rowmap(const AdOut& o, int t_out, RowMap* rm) {
     rm->p1 = o.kk * t_out; rm->p0 = t_out; rm->v1 = o.kk; rm->v0 = t_out; rm->q1 = (int)(o.k * o.pitch); rm->q0 = (int)o.pitch;
-    return (long long)o.j0 * o.pitch;
 }
 
 // ---- adapter program on device buffers -----------------------------------------------------------
@@ -677,10 +694,25 @@ inline long long chunk_rowmap(const AdOut& o, int t_out, RowMap* rm) {
 // GEMM into fp32; the last conv's rows are normalised and projected.  LinearAdapter projects the encoder rows as they are
 // (the reference does not even apply the pad mask).  Left context: the slot caches of ids_dev when the adapter carries them,
 // else per stage cache_in[i] (reference layout (B, C, k-1); null = zeros), the new one to cache_out[i] if given.
+// mix (carried caches, sessions with different chunk counts, even t): enc holds the call's blocks packed, session b's
+// cnt[b] chunks of `unit` frames from block off[b].  The convolutions run over B sessions x T = kmax * unit rows, padded at
+// the end of each session's run (the conv is causal, so the real rows' outputs are those of the sequential calls); the
+// real output rows are packed to (block, frame) order before the norm and the projection.  pass >= 0 (odd t, chunk pass
+// `pass`): B sessions x T rows as without mix, but sessions with cnt[b] <= pass keep their caches.
+struct AdMix {
+    const int32_t* cnt;
+    const int32_t* off;
+    int kmax, unit, blocks;
+    int pass = -1;
+};
 template <typename TA>
 int adapter_program(fo_ctx* c, const float* enc, const uint8_t* mask, int B, int T, const int32_t* ids_dev,
-                    const float* const* cache_in, float* const* cache_out, const AdOut& out, cudaStream_t st) {
-    const int D = c->D, E = c->E, KA = c->KA, ns = c->ad_nst, t_out = ad_frames(c, T), M = B * t_out;
+                    const float* const* cache_in, float* const* cache_out, const AdOut& out, cudaStream_t st,
+                    const AdMix* mix = nullptr) {
+    const int D = c->D, E = c->E, KA = c->KA, ns = c->ad_nst;
+    const bool grid = mix && mix->pass < 0;                                    // per-session padded grid
+    const int t_out = grid ? ad_frames(c, mix->unit) : ad_frames(c, T);       // grid: frames out of one chunk
+    const int M = grid ? mix->blocks * t_out : B * t_out;
     const bool run_gemm = !(c->debug_skip & 16);
     const float* x = enc;
     for (int i = 0; i < ns; ++i) {
@@ -693,9 +725,18 @@ int adapter_program(fo_ctx* c, const float* enc, const uint8_t* mask, int B, int
         void *xin, *conv;
         FO_TRY(ws_ensure(c, i == 0 ? WS_XIN : WS_XIN2, (size_t)ga.planes * ga.rows * s.cin * sizeof(TA), &xin));
         FO_TRY(ws_ensure(c, i + 1 == ns ? WS_ACONV : WS_AC1, (size_t)B * ad_frames(c, T, i + 1) * s.cout * sizeof(float), &conv));
+        SessionRows sr;
+        if (mix) {
+            sr.cnt = mix->cnt;
+            sr.pass = mix->pass;
+            if (grid) {
+                sr.off = i == 0 ? mix->off : nullptr;      // the first conv reads the packed encoder rows
+                sr.unit = ad_frames(c, mix->unit, i);
+            }
+        }
         FO_TRY(conv_stage<TA>(x, i == 0 ? mask : nullptr, B, Ti, s.cin, KA - 1, s.stride, s.in_scale, s.in_shift,
                               c->ad_carry ? ids_dev : nullptr, s.cache, c->ad_valid, cache_in ? cache_in[i] : nullptr,
-                              cache_out ? cache_out[i] : nullptr, reinterpret_cast<TA*>(xin), st));
+                              cache_out ? cache_out[i] : nullptr, reinterpret_cast<TA*>(xin), st, sr));
         Epilogue e;
         e.bias = s.b;
         e.c_f32 = reinterpret_cast<float*>(conv);
@@ -704,6 +745,13 @@ int adapter_program(fo_ctx* c, const float* enc, const uint8_t* mask, int B, int
         x = reinterpret_cast<const float*>(conv);
     }
     const int K = ns > 0 ? c->ad_st[ns - 1].cout : D;
+    if (grid && ns > 0) {
+        void* pk;
+        const long long blk = (long long)t_out * K * sizeof(float);
+        FO_TRY(ws_ensure(c, WS_PACK, (size_t)M * K * sizeof(float), &pk));
+        FO_TRY(session_blocks(x, blk, pk, blk, blk, B, mix->kmax, 0, BLOCKS_PACK, mix->cnt, mix->off, st));
+        x = reinterpret_cast<const float*>(pk);
+    }
     const TA* a = reinterpret_cast<const TA*>(enc);
     if (ns > 0 || sizeof(TA) == 2) {                 // the projection's operand in the activation type
         void* ah;
@@ -716,9 +764,9 @@ int adapter_program(fo_ctx* c, const float* enc, const uint8_t* mask, int B, int
     e.bias = c->ad_proj_b;
     e.ldc = E;
     RowMap rm;
-    const long long base = (out.h16 || out.kk != out.k) ? chunk_rowmap(out, t_out / out.kk, &rm) : 0;
-    if (out.h16) e.c_act = reinterpret_cast<TA*>(out.h16) + base * E;   // straight from the epilogue: no fp32 copy, no .half()
-    else e.c_f32 = out.y + base * E;
+    if (out.h16 || out.kk != out.k) chunk_rowmap(out, grid ? t_out : t_out / out.kk, &rm);
+    if (out.h16) e.c_act = reinterpret_cast<TA*>(out.h16);     // straight from the epilogue: no fp32 copy, no .half()
+    else e.c_f32 = out.y;
     if (run_gemm) FO_TRY(gemm<TA>(c, a, plain_rows(K, M), c->ad_proj_w, M, E, K, e, rm, st));
     return 0;
 }
@@ -814,7 +862,10 @@ int layer_pre(fo_ctx* c, const LayerW& w, int M, TA* h, TA* qkv, float* q32, con
     return gemm<TA>(c, h, w.wqkv, M, 3 * D, D, e, st);
 }
 struct FfnConv {                  // Conv1dLinear only: where the rows come from
-    int B = 0, T = 0;             // rows = B * T
+    int B = 0, T = 0;             // rows = B * T (per-session counts: T = the largest session's rows)
+    const int32_t* cnt = nullptr; // streaming with per-session chunk counts (depthwise_conv)
+    const int32_t* off = nullptr;
+    int t = 0;
     const int32_t* ids = nullptr; // streaming: session slots (left context carried); offline: null (zero padding)
     int layer = 0;
     void* hc = nullptr;           // depthwise output buffer (M, D), activation type
@@ -862,7 +913,7 @@ int layer_post(fo_ctx* c, const LayerW& w, float* x, int M, TA* att, TA* h, TA* 
         const long long slot_stride = (long long)c->L * (c->KF - 1) * D;
         FO_TRY(depthwise_conv<TA>(h, fc.B, fc.T, D, c->KF, w.dw_w, w.dw_b, fc.ids,
                                   c->ffn_cache + (long long)fc.layer * (c->KF - 1) * D, slot_stride,
-                                  reinterpret_cast<TA*>(fc.hc), st));
+                                  reinterpret_cast<TA*>(fc.hc), st, fc.cnt, fc.off, fc.t));
         ffn_in = reinterpret_cast<const TA*>(fc.hc);
     }
     Epilogue e1;
@@ -1017,47 +1068,83 @@ int stack_program(fo_ctx* c, int n, int t, float* x, void* qkv, float* q32, void
     return 0;
 }
 
-// The adapter of a k-chunk call (rows (session, chunk, frame) in enc), equal to k sequential single-chunk calls per session.
-// `out` names one output block per (session, chunk); this function sets its chunk mapping.
+// Chunk counts of a streaming call: `blocks` = sum of the per-session counts (in cnt_dev / off_dev when kmax > 1), `kmax` the
+// largest, `n1` the length of the leading run of sessions with one chunk; off = host prefix sums of the counts (n + 1
+// entries), null when every session brings kmax chunks.
+struct Mix {
+    int blocks = 0, kmax = 1, n1 = 0;
+    const int32_t* off = nullptr;
+    bool uniform(int n) const { return blocks == n * kmax; }
+    int block(int i) const { return off ? off[i] : i * kmax; }
+};
+
+// The adapter of a multi-chunk call (rows (session, chunk, frame) in enc), equal to cnt[b] sequential single-chunk calls per
+// session.  `out` names one output block per (session, chunk); this function sets its chunk mapping.
 template <typename TA>
-int adapter_chunks(fo_ctx* c, const float* enc, int n, int k, int t, AdOut out, cudaStream_t st) {
+int adapter_chunks(fo_ctx* c, const float* enc, int n, const Mix& m, int t, AdOut out, cudaStream_t st) {
     // LinearAdapter works per row and CNNAdapter starts from zero left context on every call (adapter.py:41-52):
-    // n*k independent blocks of t frames
-    if (!c->ad_carry) return adapter_program<TA>(c, enc, nullptr, n * k, t, c->ids_dev, nullptr, nullptr, out, st);
-    out.k = k;
+    // independent blocks of t frames
+    if (!c->ad_carry) return adapter_program<TA>(c, enc, nullptr, m.blocks, t, c->ids_dev, nullptr, nullptr, out, st);
+    const int k = m.kmax;
     if (t % 2 == 0) {
         // CNNSubsampling with even t: every chunk brings an even number of frames to the stride-2 conv, so one pass over a
         // session's k*t frames with the carried cache gives the k sequential outputs and leaves the same cache
-        out.kk = k;
-        return adapter_program<TA>(c, enc, nullptr, n, k * t, c->ids_dev, nullptr, nullptr, out, st);
+        if (m.uniform(n)) {
+            out.k = out.kk = k;
+            return adapter_program<TA>(c, enc, nullptr, n, k * t, c->ids_dev, nullptr, nullptr, out, st);
+        }
+        // different counts: the same pass over a per-session grid of kmax*t rows, each session's padding at its end
+        const AdMix mix{c->cnt_dev, c->off_dev, k, t, m.blocks};
+        return adapter_program<TA>(c, enc, nullptr, n, k * t, c->ids_dev, nullptr, nullptr, out, st, &mix);
     }
     // odd t: the output phase of the stride-2 conv shifts between chunks (a joint pass yields other frames, and fewer), so
-    // the chunks run one by one, flipping the live half of the double-buffered cache in between as a session advance does
+    // the chunks run one by one, flipping the live half of the double-buffered cache in between as a session advance does.
+    // Pass j covers the sessions with more than j chunks (the others keep their cache and its flag); its rows are gathered
+    // from blocks off[b] + j and its output rows scattered back to them.
+    const int t_out = ad_frames(c, t);
     const size_t row = (size_t)t * c->D * sizeof(float);
-    void* ej;
+    const size_t esz = out.h16 ? sizeof(TA) : sizeof(float);
+    const long long blk = (long long)t_out * c->E * esz;
+    void *ej, *yj;
     FO_TRY(ws_ensure(c, WS_ENCJ, (size_t)n * row, &ej));
+    FO_TRY(ws_ensure(c, WS_ADJ, (size_t)n * blk, &yj));
+    AdOut oj;
+    oj.pitch = t_out;
+    if (out.h16) oj.h16 = yj;
+    else oj.y = reinterpret_cast<float*>(yj);
+    void* dst = out.h16 ? out.h16 : (void*)out.y;
     for (int j = 0; j < k; ++j) {
-        FO_CUDA(cudaMemcpy2DAsync(ej, row, reinterpret_cast<const char*>(enc) + j * row, (size_t)k * row, row, n, cudaMemcpyDeviceToDevice, st));
-        out.j0 = j;
-        FO_TRY(adapter_program<TA>(c, reinterpret_cast<const float*>(ej), nullptr, n, t, c->ids_dev, nullptr, nullptr, out, st));
-        if (j + 1 < k) FO_TRY(advance_sessions(c->ids_dev, n, 0, 0, 1, nullptr, nullptr, c->ad_valid, st));
+        FO_TRY(session_blocks(enc, (long long)row, ej, (long long)row, (long long)row, n, k, j, BLOCKS_GATHER, c->cnt_dev, c->off_dev, st));
+        const AdMix pass{c->cnt_dev, nullptr, k, t, 0, j};
+        FO_TRY(adapter_program<TA>(c, reinterpret_cast<const float*>(ej), nullptr, n, t, c->ids_dev, nullptr, nullptr, oj, st, &pass));
+        FO_TRY(session_blocks(yj, blk, dst, out.pitch * c->E * (long long)esz, blk, n, k, j, BLOCKS_SCATTER, c->cnt_dev, c->off_dev, st));
+        if (j + 1 < k) FO_TRY(advance_sessions(c->ids_dev, n, 0, 0, 1, nullptr, nullptr, c->ad_valid, st, 1, c->cnt_dev, j + 2));
     }
     return 0;
 }
 
-// k > 1: k consecutive chunks per session (fo_encode_stream_chunks); rows are ordered (session, chunk, frame), so every
-// per-session kernel sees a session's k*t new rows as one run
+// Session groups of a streaming step of n sessions (see stream_program)
+int step_groups(const fo_ctx* c, int n) {
+    int G = c->profile_gemm ? 1 : c->groups;
+    if (G > fo_ctx::MAX_GROUPS) G = fo_ctx::MAX_GROUPS;
+    while (G > 1 && n < 8 * G) --G;
+    if (c->cfg.concat_after) G = 1;                         // the concat operand is a [2][M][D] pair of planes over ALL rows
+    return G;
+}
+
+// m.kmax > 1: several consecutive chunks per session (fo_encode_stream_chunks[_v]); rows are ordered (session, chunk, frame),
+// so every per-session kernel sees a session's cnt[b]*t new rows as one run
 template <typename TA>
-int stream_program(fo_ctx* c, int n, int k, const float* feats, int t_in, float* enc_out_dev, float* y_dev, cudaStream_t st) {
+int stream_program(fo_ctx* c, int n, const Mix& m, const float* feats, int t_in, float* enc_out_dev, float* y_dev, cudaStream_t st) {
     const int D = c->D, FF = c->FF, H = c->H;
-    const int T1 = (t_in - 1) / 2, t = (T1 - 1) / 2, kt = k * t, M = n * kt;
+    const int T1 = (t_in - 1) / 2, t = (T1 - 1) / 2, M = m.blocks * t;
     float* x;
     if (c->step_part == 2) {
         void* xp;
         FO_TRY(ws_ensure(c, WS_X, (size_t)M * D * sizeof(float), &xp));
         x = reinterpret_cast<float*>(xp);
     } else {
-        FO_TRY(subsample_program<TA>(c, feats, n * k, t_in, &x, st));   // every block brings its own context frames
+        FO_TRY(subsample_program<TA>(c, feats, m.blocks, t_in, &x, st));   // every block brings its own context frames
         if (c->step_part == 1) return 0;
     }
     void *h, *qkv, *att, *ffh;
@@ -1074,15 +1161,13 @@ int stream_program(fo_ctx* c, int n, int k, const float* feats, int t_in, float*
     // two groups' kernels overlap each other's pipeline fill, epilogue and launch gaps.  Rows of one group are
     // contiguous, so the groups just take slices of the same workspaces.
     int stacked = 1;
-    if (sizeof(TA) == 2 && k == 1) {                        // the stack kernel's attention is single-chunk
+    if (sizeof(TA) == 2 && m.kmax == 1) {                   // the stack kernel's attention is single-chunk
         stacked = stack_program(c, n, t, x, qkv, q32, att, ffh, enc_out_dev, st);
         if (stacked < 0) return stacked;
     }
-    int G = c->profile_gemm ? 1 : c->groups;
-    if (stacked == 0) G = 1;
-    if (G > fo_ctx::MAX_GROUPS) G = fo_ctx::MAX_GROUPS;
-    while (G > 1 && n < 8 * G) --G;
-    if (c->cfg.concat_after) G = 1;                         // the concat operand is a [2][M][D] pair of planes over ALL rows
+    const int G = stacked == 0 ? 1 : step_groups(c, n);
+    // a call mixing one-chunk sessions (the leading n1) with multi-chunk ones: the multi-chunk attention sizes its shared
+    // memory by the largest count, so the one-chunk sessions keep the single-chunk kernel, and the two run side by side
     const long long layer_stride = (long long)c->cfg.max_sessions * 2LL * H * c->ring_cap * 64;
     if (G > 1) {
         FO_CUDA(cudaEventRecord(c->ev_fork, st));
@@ -1097,8 +1182,8 @@ int stream_program(fo_ctx* c, int n, int k, const float* feats, int t_in, float*
             if (ng <= 0) continue;
             cudaStream_t sg = g == 0 ? st : c->grp_stream[g];
             c->tc_cur = &c->tc_wsg[g];
-            const long long r0 = (long long)s0 * kt;
-            const int Mg = ng * kt;
+            const long long r0 = (long long)m.block(s0) * t;   // the group's rows: its sessions' blocks (host prefix sums)
+            const int Mg = (m.block(s0 + ng) - m.block(s0)) * t;
             AttnStream a;
             a.ids = c->ids_dev + s0;
             a.n_frames = c->n_frames;
@@ -1106,8 +1191,10 @@ int stream_program(fo_ctx* c, int n, int k, const float* feats, int t_in, float*
             a.n = ng; a.t = t; a.H = H; a.ring_cap = c->ring_cap; a.window = c->window; a.full_chunk = c->full_chunk;
             a.pe_wrap = c->pe_wrap; a.pos_rows = c->pos_rows;
             a.ring_slot_stride = 2LL * H * c->ring_cap * 64;
-            a.chunks = k;
+            a.chunks = m.kmax;
             a.chunk_size = c->cfg.chunk_size;
+            a.cnt = c->cnt_dev + s0;
+            a.off = c->off_dev + s0;
             TA* hg = reinterpret_cast<TA*>(h) + r0 * D;
             TA* qkvg = reinterpret_cast<TA*>(qkv) + r0 * 3 * D;
             TA* attg = reinterpret_cast<TA*>(att) + r0 * D;
@@ -1130,20 +1217,47 @@ int stream_program(fo_ctx* c, int n, int k, const float* feats, int t_in, float*
             }
             int qkv_splits = 0;
             // the multi-chunk attention reads finished QKV rows: no split-K reduction deferred to it
-            if (r == 0) r = layer_pre<TA>(c, w, Mg, hg, qkvg, q32g, pfq, sg, k == 1 ? &qkv_splits : nullptr);
+            if (r == 0) r = layer_pre<TA>(c, w, Mg, hg, qkvg, q32g, pfq, sg, m.kmax == 1 ? &qkv_splits : nullptr);
             if (qkv_splits > 0) {
                 a.part = c->tc_cur->partial;
                 a.part_bias = w.bqkv;
                 a.nsplit = qkv_splits;
                 a.part_stride = (long long)Mg * 3 * D;
             }
-            if (r == 0 && !(c->debug_skip & 1))
-                r = attention_stream<TA>(a, qkvg, q32g, reinterpret_cast<TA*>(c->ring) + l * layer_stride,
-                                         reinterpret_cast<const TA*>(w.ptab_h), w.pos_u, w.pos_v, attg, sg);
+            TA* ring_l = reinterpret_cast<TA*>(c->ring) + l * layer_stride;
+            const int n1g = std::min(std::max(m.n1 - s0, 0), ng);  // the group's share of the leading one-chunk run
+            if (r == 0 && !(c->debug_skip & 1) && n1g < ng) {
+                // multi-chunk sessions (rows from the end of the one-chunk run): on a forked stream when both kernels run
+                AttnStream am = a;
+                am.ids += n1g; am.cnt += n1g; am.off += n1g; am.n = ng - n1g;
+                const long long ro = (long long)n1g * t;
+                const bool fork = n1g > 0;
+                cudaStream_t sm = fork ? c->mix_stream[g] : sg;
+                if (fork) {
+                    FO_CUDA(cudaEventRecord(c->ev_mix_fork[g], sg));
+                    FO_CUDA(cudaStreamWaitEvent(sm, c->ev_mix_fork[g], 0));
+                }
+                r = attention_stream<TA>(am, qkvg + ro * 3 * D, q32g + ro * 3 * D, ring_l, reinterpret_cast<const TA*>(w.ptab_h),
+                                         w.pos_u, w.pos_v, attg + ro * D, sm);
+                if (r == 0 && n1g > 0) {
+                    AttnStream a1 = a;
+                    a1.n = n1g; a1.chunks = 1;
+                    r = attention_stream<TA>(a1, qkvg, q32g, ring_l, reinterpret_cast<const TA*>(w.ptab_h), w.pos_u, w.pos_v, attg, sg);
+                }
+                if (fork) {
+                    FO_CUDA(cudaEventRecord(c->ev_mix_join[g], sm));
+                    FO_CUDA(cudaStreamWaitEvent(sg, c->ev_mix_join[g], 0));
+                }
+            } else if (r == 0 && !(c->debug_skip & 1)) {
+                AttnStream a1 = a;
+                a1.chunks = 1;                                  // every session of the group brings one chunk
+                r = attention_stream<TA>(a1, qkvg, q32g, ring_l, reinterpret_cast<const TA*>(w.ptab_h), w.pos_u, w.pos_v, attg, sg);
+            }
             NextNorm nn{last ? c->after_g : c->layers[l + 1].ln1g, last ? c->after_b : c->layers[l + 1].ln1b,
                         last ? enc_out_dev + r0 * D : nullptr};
             FfnConv fc;
-            fc.B = ng; fc.T = kt; fc.ids = c->ids_dev + s0; fc.layer = l;   // Conv1dLinear: one pass over k*t rows with the carry
+            fc.B = ng; fc.T = m.kmax * t; fc.ids = c->ids_dev + s0; fc.layer = l;   // Conv1dLinear: one pass over each session's rows with the carry
+            if (m.kmax > 1) { fc.cnt = a.cnt; fc.off = a.off; fc.t = t; }
             fc.hc = hc ? reinterpret_cast<TA*>(hc) + r0 * D : nullptr;
             if (r == 0) r = layer_post<TA>(c, w, xg, Mg, attg, hg, ffhg, nn, last ? nullptr : c->layers[l + 1].wqkv, fc, sg);
             if (r != 0) { c->tc_cur = &c->tc_wsg[0]; return r; }
@@ -1166,11 +1280,11 @@ int stream_program(fo_ctx* c, int n, int k, const float* feats, int t_in, float*
             out.y = y_dev;
             out.pitch = ad_frames(c, t);
         }
-        if (k == 1) FO_TRY(adapter_program<TA>(c, enc_out_dev, nullptr, n, t, c->ids_dev, nullptr, nullptr, out, st));
-        else FO_TRY(adapter_chunks<TA>(c, enc_out_dev, n, k, t, out, st));
+        if (m.kmax == 1) FO_TRY(adapter_program<TA>(c, enc_out_dev, nullptr, n, t, c->ids_dev, nullptr, nullptr, out, st));
+        else FO_TRY(adapter_chunks<TA>(c, enc_out_dev, n, m, t, out, st));
     }
     FO_TRY(advance_sessions(c->ids_dev, n, t, c->cfg.chunk_size, c->pe_wrap, c->n_frames, c->pe_index,
-                            (run_adapter && c->ad_carry) ? c->ad_valid : nullptr, st, k));
+                            (run_adapter && c->ad_carry) ? c->ad_valid : nullptr, st, m.kmax, m.kmax > 1 ? c->cnt_dev : nullptr));
     return 0;
 }
 
@@ -1334,13 +1448,13 @@ int fo_create(const fo_config* cfg, int device, int dtype, fo_ctx** out) {
             r = dev_alloc(c, &p, (size_t)S * 2 * (c->KA - 1) * c->ad_st[i].cin * sizeof(float));
             c->ad_st[i].cache = (float*)p;
         }
-        if (!r) { r = dev_alloc(c, &p, S * sizeof(int32_t)); c->ids_dev = (int32_t*)p; }
+        if (!r) { r = dev_alloc(c, &p, 3 * S * sizeof(int32_t)); c->ids_dev = (int32_t*)p; c->cnt_dev = c->ids_dev + S; c->off_dev = c->ids_dev + 2 * S; }
         if (!r) { r = dev_alloc(c, &p, (size_t)S * STREAM_CHUNKS_MAX_KEYS); c->onset_dev = (uint8_t*)p; }   // one flag per block, <= 128 blocks per session
         if (!r) { r = dev_alloc(c, &p, sizeof(unsigned long long)); c->sat_counter = (unsigned long long*)p; }
         if (!r && cudaMemset(c->sat_counter, 0, sizeof(unsigned long long)) != cudaSuccess) r = FO_ERR_CUDA;
     }
     for (int k = 0; k < fo_ctx::NSTAGE && !r; ++k) {
-        if (cudaMallocHost((void**)&c->ids_host[k], S * sizeof(int32_t) + (size_t)S * STREAM_CHUNKS_MAX_KEYS) != cudaSuccess ||
+        if (cudaMallocHost((void**)&c->ids_host[k], 3 * S * sizeof(int32_t) + (size_t)S * STREAM_CHUNKS_MAX_KEYS) != cudaSuccess ||
             cudaEventCreateWithFlags(&c->ids_event[k], cudaEventDisableTiming) != cudaSuccess) {
             set_error("fo_create: pinned staging allocation failed");
             r = FO_ERR_NOMEM;
@@ -1358,6 +1472,14 @@ int fo_create(const fo_config* cfg, int device, int dtype, fo_ctx** out) {
         }
     }
     if (!r && cudaEventCreateWithFlags(&c->ev_fork, cudaEventDisableTiming) != cudaSuccess) r = FO_ERR_CUDA;
+    for (int g = 0; g < fo_ctx::MAX_GROUPS && !r; ++g) {
+        if (cudaStreamCreateWithFlags(&c->mix_stream[g], cudaStreamNonBlocking) != cudaSuccess ||
+            cudaEventCreateWithFlags(&c->ev_mix_fork[g], cudaEventDisableTiming) != cudaSuccess ||
+            cudaEventCreateWithFlags(&c->ev_mix_join[g], cudaEventDisableTiming) != cudaSuccess) {
+            set_error("fo_create: stream creation failed");
+            r = FO_ERR_CUDA;
+        }
+    }
     if (r) { fo_destroy(c); return r; }
     c->slot_used.assign(S, 0);
     c->free_slots.reserve(S);
@@ -1383,6 +1505,11 @@ int fo_destroy(fo_ctx* c) {
     for (int g = 1; g < fo_ctx::MAX_GROUPS; ++g) {
         if (c->grp_stream[g]) cudaStreamDestroy(c->grp_stream[g]);
         if (c->ev_join[g]) cudaEventDestroy(c->ev_join[g]);
+    }
+    for (int g = 0; g < fo_ctx::MAX_GROUPS; ++g) {
+        if (c->mix_stream[g]) cudaStreamDestroy(c->mix_stream[g]);
+        if (c->ev_mix_fork[g]) cudaEventDestroy(c->ev_mix_fork[g]);
+        if (c->ev_mix_join[g]) cudaEventDestroy(c->ev_mix_join[g]);
     }
     if (c->ev_fork) cudaEventDestroy(c->ev_fork);
     if (c->ev_sync) cudaEventDestroy(c->ev_sync);
@@ -1923,7 +2050,7 @@ int fo_fbank_offline(fo_ctx* c, const void* pcm, int pcm_dtype, int B, int64_t n
 // captures.  A workspace that moves (ws_epoch) invalidates the graphs.
 struct StepArgs {
     int n, t_in;
-    int k;                     // consecutive chunks per session (fo_encode_stream_chunks; 1 otherwise)
+    Mix m;                     // chunks per session (fo_encode_stream_chunks[_v]; one each otherwise)
     bool with_fbank, want_y;
     int pcm_is_i16;
     float scale;
@@ -1937,7 +2064,7 @@ static int step_body(fo_ctx* c, const StepArgs& a, cudaStream_t st) {
     void *dfeats, *denc, *dy = nullptr;
     const int T1 = (a.t_in - 1) / 2, t = (T1 - 1) / 2;
     const int t_out = ad_frames(c, t);
-    const size_t blocks = (size_t)a.n * a.k;
+    const size_t blocks = (size_t)a.m.blocks;
     FO_TRY(ws_ensure(c, WS_FEATS, blocks * a.t_in * c->F * sizeof(float), &dfeats));
     FO_TRY(ws_ensure(c, ws_enc(a.buf), blocks * t * c->D * sizeof(float), &denc));
     if (a.want_y) FO_TRY(ws_ensure(c, ws_y(a.buf), blocks * t_out * c->E * sizeof(float), &dy));
@@ -1947,8 +2074,8 @@ static int step_body(fo_ctx* c, const StepArgs& a, cudaStream_t st) {
         FO_TRY(fbank_stream(fbank_params(c), c->ids_dev, a.n, dp, a.pcm_is_i16, a.scale, c->cfg.frames_per_chunk,
                             c->cfg.context_frames, c->samples, c->feat_ring, (float*)dfeats, st));
     }
-    return c->dtype == FO_BF16 ? stream_program<act16>(c, a.n, a.k, (const float*)dfeats, a.t_in, (float*)denc, (float*)dy, st)
-                               : stream_program<float>(c, a.n, a.k, (const float*)dfeats, a.t_in, (float*)denc, (float*)dy, st);
+    return c->dtype == FO_BF16 ? stream_program<act16>(c, a.n, a.m, (const float*)dfeats, a.t_in, (float*)denc, (float*)dy, st)
+                               : stream_program<float>(c, a.n, a.m, (const float*)dfeats, a.t_in, (float*)denc, (float*)dy, st);
 }
 
 static int run_step(fo_ctx* c, const StepArgs& a, cudaStream_t st) {
@@ -1959,12 +2086,19 @@ static int run_step(fo_ctx* c, const StepArgs& a, cudaStream_t st) {
     if (pdl_min < 0) { const char* e = getenv("FO_PDL_MIN"); pdl_min = e ? atoi(e) : 1; }
     g_use_pdl = g_want_pdl && a.n >= pdl_min;
     if (!c->use_graph || c->profile_gemm) return step_body(c, a, st);
-    char key[192];
+    char key[256];
     uint32_t sbits;
     memcpy(&sbits, &a.scale, 4);
-    snprintf(key, sizeof(key), "%d/%p/%lld/%lld/%d/%d/%d/%d/%d/%d/%08x/%d/%d/%d/%d-%d", a.buf, c->handoff, c->handoff_rows, c->handoff_off, a.n, a.k, a.t_in, (int)a.with_fbank, (int)a.want_y, a.pcm_is_i16, sbits,
+    // the chunk counts enter as totals only (they are device data); the rows of session groups other than the first are
+    // baked into the graph as the block where each group starts
+    int len = snprintf(key, sizeof(key), "%d/%p/%lld/%lld/%d/%d.%d.%d/%d/%d/%d/%d/%08x/%d/%d/%d/%d-%d", a.buf, c->handoff, c->handoff_rows, c->handoff_off, a.n,
+             a.m.blocks, a.m.kmax, a.m.n1, a.t_in, (int)a.with_fbank, (int)a.want_y, a.pcm_is_i16, sbits,
              c->gemm_backend, c->groups, (((c->debug_skip * 2 + c->defer_reduce) * 2 + c->fuse_ln) * 4 + c->use_prefetch) * 64 + c->stack_rows,
              ((c->use_prefetch & 2) ? c->pf_slot_lo * 2 + g_use_pdl : g_use_pdl), (c->use_prefetch & 2) ? c->pf_slot_hi : 0);   // the prefetch range is baked into the graph
+    if (a.m.off) {
+        const int G = step_groups(c, a.n), per = (a.n + G - 1) / G;
+        for (int g = 1; g < G && g * per < a.n && len < (int)sizeof(key) - 16; ++g) len += snprintf(key + len, sizeof(key) - len, "/%d", a.m.off[g * per]);
+    }
     if (c->graphs.size() > 256 && c->graphs.find(key) == c->graphs.end()) {
         for (auto& kv : c->graphs) if (kv.second.exec) cudaGraphExecDestroy(kv.second.exec);
         c->graphs.clear();
@@ -2023,17 +2157,18 @@ static int stream_geometry(const fo_ctx* c, int t_in) {
 }
 
 // copies between the caller's buffers and the context's staging buffers, then the step
-// k > 1 (fo_encode_stream_chunks, feats only): k consecutive chunk blocks per session, feats (n, k, t_in, F)
-static int stream_common(fo_ctx* c, const int32_t* ids, int n, int k, const void* pcm, int pcm_dtype, float scale,
-                         const float* feats, int t_in, float* enc_out, float* adapter_out, cudaStream_t st) {
+// chunks (fo_encode_stream_chunks[_v], feats only; m.kmax > 1): chunks[i] consecutive chunk blocks of session i, feats
+// (m.blocks, t_in, F) in (session, chunk) order
+static int stream_common(fo_ctx* c, const int32_t* ids, int n, const int32_t* chunks, const Mix& m, const void* pcm, int pcm_dtype,
+                         float scale, const float* feats, int t_in, float* enc_out, float* adapter_out, cudaStream_t st) {
     const int T1 = (t_in - 1) / 2, t = (T1 - 1) / 2;
     FO_TRY(stream_geometry(c, t_in));
     if (adapter_out) FO_CHECK(c->cfg.has_adapter, "adapter_out requested but the context has no adapter");
     FO_CHECK(!c->KM, "this context's positionwise layer is MultiLayeredConv1d, which has no streaming form (the reference module has no infer(), "
                      "models/encoder/attention.py:145-196); use fo_encode_offline");
     const int t_out = ad_frames(c, t);
-    const size_t enc_bytes = (size_t)n * k * t * c->D * sizeof(float);
-    const size_t y_bytes = (size_t)n * k * t_out * c->E * sizeof(float);
+    const size_t enc_bytes = (size_t)m.blocks * t * c->D * sizeof(float);
+    const size_t y_bytes = (size_t)m.blocks * t_out * c->E * sizeof(float);
     if (c->copy_stream && c->async_ticket > 0) {
         // a synchronous call after pipelined ones reuses staging set 0 (and the shared intermediates): let the read-backs of
         // the steps still in flight on the copy stream finish first
@@ -2043,8 +2178,8 @@ static int stream_common(fo_ctx* c, const int32_t* ids, int n, int k, const void
     fo_ctx::Armed armed = c->armed;              // consumed by this call, whatever its outcome
     c->armed.on = false;
     if (armed.on) {
-        FO_CHECK(armed.n == n * k, "fo_handoff_arm was armed for %d blocks, this call advances %d sessions x %d chunks", armed.n, n, k);
-        FO_CHECK(armed.rows * k < (1LL << 31), "hand-off: %d chunks of %lld rows per session are too many rows", k, armed.rows);
+        FO_CHECK(armed.n == m.blocks, "fo_handoff_arm was armed for %d blocks, this call advances %d sessions by %d chunks in all", armed.n, n, m.blocks);
+        FO_CHECK(armed.rows * m.kmax < (1LL << 31), "hand-off: %d chunks of %lld rows per session are too many rows", m.kmax, armed.rows);
         FO_CHECK(!adapter_out && !c->handoff, "an armed hand-off replaces adapter_out: pass NULL");
         FO_CHECK(armed.rows >= armed.prefix + t_out, "hand-off: %d adapter rows behind a %lld-row prefix do not fit %lld rows per session",
                  t_out, armed.prefix, armed.rows);
@@ -2053,17 +2188,17 @@ static int stream_common(fo_ctx* c, const int32_t* ids, int n, int k, const void
         c->handoff_off = armed.prefix;
     }
     struct HandoffReset { fo_ctx* c; bool on; ~HandoffReset() { if (on) { c->handoff = nullptr; c->handoff_rows = c->handoff_off = 0; } } } hreset{c, armed.on};
-    FO_TRY(upload_ids(c, ids, n, st, armed.on ? armed.onset.data() : nullptr, n * k));
+    FO_TRY(upload_ids(c, ids, n, st, armed.on ? armed.onset.data() : nullptr, m.blocks, chunks));
     c->pf_slot_lo = c->pf_slot_hi = ids[0];
     for (int i = 1; i < n; ++i) { c->pf_slot_lo = std::min(c->pf_slot_lo, (int)ids[i]); c->pf_slot_hi = std::max(c->pf_slot_hi, (int)ids[i]); }
-    StepArgs a{n, t_in, k, pcm != nullptr, adapter_out != nullptr, pcm_dtype == FO_I16, scale, 0};
+    StepArgs a{n, t_in, m, pcm != nullptr, adapter_out != nullptr, pcm_dtype == FO_I16, scale, 0};
     void* stage;
     if (pcm) {
         const size_t in_bytes = (size_t)n * c->chunk_samples * (pcm_dtype == FO_I16 ? 2 : 4);
         FO_TRY(ws_ensure(c, WS_PCM, (size_t)n * c->chunk_samples * 4, &stage));
         FO_CUDA(cudaMemcpyAsync(stage, pcm, in_bytes, cudaMemcpyDefault, st));
     } else if (feats) {
-        const size_t in_bytes = (size_t)n * k * t_in * c->F * sizeof(float);
+        const size_t in_bytes = (size_t)m.blocks * t_in * c->F * sizeof(float);
         FO_TRY(ws_ensure(c, WS_FEATS, in_bytes, &stage));
         FO_CUDA(cudaMemcpyAsync(stage, feats, in_bytes, cudaMemcpyDefault, st));
     } else {
@@ -2075,13 +2210,13 @@ static int stream_common(fo_ctx* c, const int32_t* ids, int n, int k, const void
     }
     FO_TRY(run_step(c, a, st));
     if (armed.on && armed.attn_mask)
-        FO_TRY(handoff_mask(c->onset_dev, armed.prefix_mask, n * k, (int)armed.prefix, t_out, (int)armed.rows, armed.attn_mask, armed.row_start, st));
+        FO_TRY(handoff_mask(c->onset_dev, armed.prefix_mask, m.blocks, (int)armed.prefix, t_out, (int)armed.rows, armed.attn_mask, armed.row_start, st));
     if (enc_out) FO_CUDA(cudaMemcpyAsync(enc_out, c->ws[WS_ENC].p, enc_bytes, cudaMemcpyDefault, st));
     if (adapter_out) FO_CUDA(cudaMemcpyAsync(adapter_out, c->ws[WS_Y].p, y_bytes, cudaMemcpyDefault, st));
     if (!c->ev_sync) FO_CUDA(cudaEventCreateWithFlags(&c->ev_sync, cudaEventDisableTiming));
     FO_CUDA(cudaEventRecord(c->ev_sync, st));
     c->stats.stream_steps += 1;
-    c->stats.session_chunks += (long long)n * k;
+    c->stats.session_chunks += m.blocks;
     return 0;
 }
 
@@ -2092,7 +2227,9 @@ int fo_encode_stream(fo_ctx* c, const int32_t* ids, int n, const float* feats, i
     FO_CUDA(cudaSetDevice(c->device));
     if (feats) FO_CHECK(t_in >= 7, "fo_encode_stream: need at least 7 feature frames");
     else t_in = c->cfg.context_frames + c->cfg.frames_per_chunk;
-    return stream_common(c, ids, n, 1, nullptr, FO_F32, 1.0f, feats, t_in, enc_out, adapter_out, (cudaStream_t)stream);
+    Mix m;
+    m.blocks = m.n1 = n;
+    return stream_common(c, ids, n, nullptr, m, nullptr, FO_F32, 1.0f, feats, t_in, enc_out, adapter_out, (cudaStream_t)stream);
 }
 
 int fo_encode_stream_chunks(fo_ctx* c, const int32_t* ids, int n, int k, const float* feats, int t_in, float* enc_out,
@@ -2111,7 +2248,42 @@ int fo_encode_stream_chunks(fo_ctx* c, const int32_t* ids, int n, int k, const f
                  c->window, k, t, STREAM_CHUNKS_MAX_KEYS, kmax);
     }
     FO_CUDA(cudaSetDevice(c->device));
-    return stream_common(c, ids, n, k, nullptr, FO_F32, 1.0f, feats, t_in, enc_out, adapter_out, (cudaStream_t)stream);
+    // the uniform case of fo_encode_stream_chunks_v: every session brings k chunks
+    const std::vector<int32_t> chunks(n, k);
+    Mix m;
+    m.blocks = n * k;
+    m.kmax = k;
+    m.n1 = k == 1 ? n : 0;
+    return stream_common(c, ids, n, k > 1 ? chunks.data() : nullptr, m, nullptr, FO_F32, 1.0f, feats, t_in, enc_out, adapter_out,
+                         (cudaStream_t)stream);
+}
+
+int fo_encode_stream_chunks_v(fo_ctx* c, const int32_t* ids, const int32_t* chunks, int n, const float* feats, int t_in,
+                              float* enc_out, float* adapter_out, void* stream) {
+    FO_CHECK(c && c->finalized && c->cfg.has_encoder, "fo_encode_stream_chunks_v: context has no finalized encoder");
+    FO_CHECK(feats, "fo_encode_stream_chunks_v: feats must not be NULL (the feature ring holds one block per session)");
+    FO_CHECK(chunks, "fo_encode_stream_chunks_v: chunks must be a host array of n counts");
+    FO_CHECK(t_in >= 7, "fo_encode_stream_chunks_v: need at least 7 feature frames per chunk");
+    FO_TRY(check_ids(c, ids, n));
+    FO_TRY(stream_geometry(c, t_in));
+    const int t = ((t_in - 1) / 2 - 1) / 2;
+    const int kcap = std::max(1, (STREAM_CHUNKS_MAX_KEYS - c->window) / t);
+    std::vector<int32_t> off(n + 1, 0);
+    Mix m;
+    for (int i = 0; i < n; ++i) {
+        FO_CHECK(chunks[i] >= 1, "fo_encode_stream_chunks_v: session %d (id %d) has chunk count %d; counts must be >= 1", i, ids[i], chunks[i]);
+        FO_CHECK(c->window + (long long)chunks[i] * t <= STREAM_CHUNKS_MAX_KEYS,
+                 "fo_encode_stream_chunks_v: session %d (id %d): the attention window (%d frames) + %d chunks x %d frames exceeds %d keys; "
+                 "the largest count is %d", i, ids[i], c->window, chunks[i], t, STREAM_CHUNKS_MAX_KEYS, kcap);
+        off[i + 1] = off[i] + chunks[i];
+        m.kmax = std::max(m.kmax, (int)chunks[i]);
+        if (m.n1 == i && chunks[i] == 1) m.n1 = i + 1;
+    }
+    m.blocks = off[n];
+    if (!m.uniform(n)) m.off = off.data();
+    FO_CUDA(cudaSetDevice(c->device));
+    return stream_common(c, ids, n, m.kmax > 1 ? chunks : nullptr, m, nullptr, FO_F32, 1.0f, feats, t_in, enc_out, adapter_out,
+                         (cudaStream_t)stream);
 }
 
 int fo_handoff_arm(fo_ctx* c, int n, void* embeds_f16, int64_t rows_per_session, int64_t prefix_len, const uint8_t* onset,
@@ -2157,7 +2329,9 @@ int fo_stream_step_embeds(fo_ctx* c, const int32_t* ids, int n, const void* pcm,
     c->handoff = embeds_f16;
     c->handoff_rows = rows_per_session;
     c->handoff_off = row_offset;
-    const int r = stream_common(c, ids, n, 1, pcm, pcm_dtype, scale, nullptr, t_in, enc_out, nullptr, (cudaStream_t)stream);
+    Mix m;
+    m.blocks = m.n1 = n;
+    const int r = stream_common(c, ids, n, nullptr, m, pcm, pcm_dtype, scale, nullptr, t_in, enc_out, nullptr, (cudaStream_t)stream);
     c->handoff = nullptr;
     c->handoff_rows = c->handoff_off = 0;
     return r;
@@ -2188,7 +2362,9 @@ int fo_stream_step_async(fo_ctx* c, const int32_t* ids, int n, const void* pcm, 
     FO_TRY(upload_ids(c, ids, n, st));
     c->pf_slot_lo = c->pf_slot_hi = ids[0];
     for (int i = 1; i < n; ++i) { c->pf_slot_lo = std::min(c->pf_slot_lo, (int)ids[i]); c->pf_slot_hi = std::max(c->pf_slot_hi, (int)ids[i]); }
-    StepArgs a{n, t_in, 1, true, adapter_out != nullptr, pcm_dtype == FO_I16, scale, buf};
+    Mix m;
+    m.blocks = m.n1 = n;
+    StepArgs a{n, t_in, m, true, adapter_out != nullptr, pcm_dtype == FO_I16, scale, buf};
     // inputs: copy stream, once the step that last read this PCM buffer (two tickets ago) is done
     void* stage;
     FO_TRY(ws_ensure(c, ws_pcm(buf), (size_t)n * c->chunk_samples * 4, &stage));
@@ -2226,7 +2402,9 @@ int fo_stream_step(fo_ctx* c, const int32_t* ids, int n, const void* pcm, int pc
     FO_CHECK(pcm && (pcm_dtype == FO_F32 || pcm_dtype == FO_I16), "fo_stream_step: pcm must be FO_F32 or FO_I16");
     FO_TRY(check_ids(c, ids, n));
     FO_CUDA(cudaSetDevice(c->device));
-    return stream_common(c, ids, n, 1, pcm, pcm_dtype, scale, nullptr, c->cfg.context_frames + c->cfg.frames_per_chunk, enc_out,
+    Mix m;
+    m.blocks = m.n1 = n;
+    return stream_common(c, ids, n, nullptr, m, pcm, pcm_dtype, scale, nullptr, c->cfg.context_frames + c->cfg.frames_per_chunk, enc_out,
                          adapter_out, (cudaStream_t)stream);
 }
 

@@ -296,9 +296,10 @@ attention_stream_mma_kernel(AttnStream a, const __half* __restrict__ qkv, const 
 }
 
 // ---------------------------------------------------------------------------------------------
-// Several consecutive chunks of every session in one call (AttnStream::chunks = k, fo_encode_stream_chunks).  One CTA per
-// (session, head) stages the keys once -- the ring window of frames [first, nf) (first = nf - min(nf, window)) by bulk
-// copy, then the call's own k*t rows -- and walks the k query chunks in order.  Chunk j sees exactly what the j-th
+// Several consecutive chunks of every session in one call (fo_encode_stream_chunks[_v]): session b brings k = cnt[b] chunks
+// from row row0 = (off[b] - off[0]) * t.  One CTA per (session, head) stages the keys once -- the ring window of frames
+// [first, nf) (first = nf - min(nf, window)) by bulk copy, then the session's own k*t rows -- and walks the k query chunks
+// in order.  Shared memory is sized by the largest count of the call (AttnStream::chunks).  Chunk j sees exactly what the j-th
 // sequential single-chunk call would see:
 //     nf_j = nf + j*t,  keys = frames [nf_j - min(nf_j, window), nf_j + t)   (a contiguous run of the staged rows)
 //     pe_j = pe_index stepped j times by pe = pe % wrap + chunk_size,  rel-pos rows P[max(0, pe_j % wrap - full_chunk) + m]
@@ -311,10 +312,10 @@ __device__ __forceinline__ int chunk_pe(int pe, int j, const AttnStream& a) {
     return pe % a.pe_wrap;
 }
 
-// stage the call's new K/V rows (smem rows cl + r, frame nf + r) and, once the ring window has landed, append them to the
+// stage the session's new K/V rows (qkv row r -> smem row cl + r, frame nf + r) and, once the ring window has landed, append them to the
 // ring (only the last `cap` of them when the call brings more frames than the ring holds)
 template <typename TA, int NCH, bool SWZ>
-__device__ __forceinline__ void chunks_stage_new(const AttnStream& a, const TA* qkv, TA* Ks, TA* Vs, int b, int h, int nf, int cl,
+__device__ __forceinline__ void chunks_stage_new(const AttnStream& a, const TA* qkv, TA* Ks, TA* Vs, int h, int nf, int cl,
                                                  int kt) {
     constexpr int EPC = 16 / sizeof(TA);
     const int D = a.H * DK;
@@ -322,7 +323,7 @@ __device__ __forceinline__ void chunks_stage_new(const AttnStream& a, const TA* 
         const int which = i / (kt * NCH), r = (i / NCH) % kt, c = i % NCH;
         const int pc = SWZ ? (c ^ ((nf + r) & 7)) : c;
         *reinterpret_cast<uint4*>((which ? Vs : Ks) + (cl + r) * DK + pc * EPC) =
-            *reinterpret_cast<const uint4*>(qkv + (long long)(b * kt + r) * 3 * D + (which + 1) * D + h * DK + c * EPC);
+            *reinterpret_cast<const uint4*>(qkv + (long long)r * 3 * D + (which + 1) * D + h * DK + c * EPC);
     }
 }
 template <typename TA, int NCH>
@@ -347,8 +348,8 @@ attention_chunks_kernel(AttnStream a, const float* __restrict__ qkv, const float
     constexpr int EPC = 4, NCH = DK / EPC;
     FO_PDL_TRIGGER();
     FO_PDL_WAIT();
-    const int cap = a.ring_cap, t = a.t, kt = a.chunks * t, D = a.H * DK;
-    const int rows = a.window + kt, prow = a.window + t;
+    const int cap = a.ring_cap, t = a.t, D = a.H * DK;
+    const int rows = a.window + a.chunks * t, prow = a.window + t;
     float* Ks = reinterpret_cast<float*>(smem_raw);
     float* Vs = Ks + rows * DK;
     float* Ps = Vs + rows * DK;
@@ -359,6 +360,9 @@ attention_chunks_kernel(AttnStream a, const float* __restrict__ qkv, const float
 
     const int b = blockIdx.x, h = blockIdx.y;
     const int slot = a.ids[b];
+    const int k = a.cnt[b], kt = k * t;
+    const long long row0 = (long long)(a.off[b] - a.off[0]) * t;     // the session's rows: the pointers start there
+    qkv += row0 * 3 * D; q32 += row0 * 3 * D; out += row0 * D;
     const int nf = a.n_frames[slot];
     const int cl = min(nf, a.window), first = nf - cl;
     float* ringK = ring + (long long)slot * a.ring_slot_stride + (long long)h * cap * DK;
@@ -369,13 +373,13 @@ attention_chunks_kernel(AttnStream a, const float* __restrict__ qkv, const float
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
         ring_window_copy<float>(ringK, ringV, cap, first, cl, Ks, Vs, nullptr, nullptr, 0, &bar);
     }
-    chunks_stage_new<float, NCH, false>(a, qkv, Ks, Vs, b, h, nf, cl, kt);
+    chunks_stage_new<float, NCH, false>(a, qkv, Ks, Vs, h, nf, cl, kt);
     __syncthreads();
     mbar_wait(&bar, 0);
     chunks_append_ring<float, NCH>(a, Ks, Vs, ringK, ringV, nf, cl, kt);
 
     const int pe0 = a.pe_index[slot];
-    for (int j = 0; j < a.chunks; ++j) {
+    for (int j = 0; j < k; ++j) {
         const int nfj = nf + j * t, clj = min(nfj, a.window);
         const int o = nfj - clj - first;            // staged row of this chunk's first key
         const int nk = clj + t;
@@ -386,12 +390,12 @@ attention_chunks_kernel(AttnStream a, const float* __restrict__ qkv, const float
         }
         for (int i = tid; i < t * DK; i += ATT_THREADS) {
             const int r = i / DK, d = i % DK;
-            const float q = q32[(long long)(b * kt + j * t + r) * 3 * D + h * DK + d];
+            const float q = q32[(long long)(j * t + r) * 3 * D + h * DK + d];
             qu[i] = q + pos_u[h * DK + d];
             qv[i] = q + pos_v[h * DK + d];
         }
         __syncthreads();
-        attn_chunk_ffma(Ks + o * DK, Vs + o * DK, Ps, qu, qv, prob, prow, nk, t, out + (long long)(b * kt + j * t) * D + h * DK, D);
+        attn_chunk_ffma(Ks + o * DK, Vs + o * DK, Ps, qu, qv, prob, prow, nk, t, out + (long long)(j * t) * D + h * DK, D);
         __syncthreads();                              // Ps / qu / prob are restaged by the next chunk
     }
 }
@@ -407,8 +411,8 @@ attention_chunks_mma_kernel(AttnStream a, const __half* __restrict__ qkv, const 
     constexpr int EPC = 8, NCH = 8;
     FO_PDL_TRIGGER();
     FO_PDL_WAIT();
-    const int cap = a.ring_cap, t = a.t, kt = a.chunks * t, D = a.H * DK;
-    const int rows = a.window + kt;
+    const int cap = a.ring_cap, t = a.t, D = a.H * DK;
+    const int rows = a.window + a.chunks * t;
     const int krows = ((rows + 15) & ~15) + 16;     // a chunk's last key tile may read up to 15 rows past the staged keys
     const int vrows = (a.window + t + 15) & ~15;    // rel-pos rows / probability columns of one chunk
     TA* Ks = reinterpret_cast<TA*>(smem_raw);
@@ -422,6 +426,9 @@ attention_chunks_mma_kernel(AttnStream a, const __half* __restrict__ qkv, const 
 
     const int b = blockIdx.x, h = blockIdx.y;
     const int slot = a.ids[b];
+    const int k = a.cnt[b], kt = k * t;
+    const long long row0 = (long long)(a.off[b] - a.off[0]) * t;     // the session's rows: the pointers start there
+    qkv += row0 * 3 * D; q32 += row0 * 3 * D; out += row0 * D;
     const int nf = a.n_frames[slot];
     const int cl = min(nf, a.window), first = nf - cl;
     const int nk_all = cl + kt;
@@ -433,7 +440,7 @@ attention_chunks_mma_kernel(AttnStream a, const __half* __restrict__ qkv, const 
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
         ring_window_copy<TA>(ringK, ringV, cap, first, cl, Ks, Vs, nullptr, nullptr, 0, &bar);
     }
-    chunks_stage_new<TA, NCH, true>(a, qkv, Ks, Vs, b, h, nf, cl, kt);
+    chunks_stage_new<TA, NCH, true>(a, qkv, Ks, Vs, h, nf, cl, kt);
     // rows behind the last key: K is masked there, V enters the PV MMAs with probability 0 and must be finite
     for (int i = tid; i < (krows - nk_all) * NCH; i += ATT_THREADS) {
         *reinterpret_cast<uint4*>(Ks + (nk_all + i / NCH) * DK + (i % NCH) * EPC) = make_uint4(0, 0, 0, 0);
@@ -444,7 +451,7 @@ attention_chunks_mma_kernel(AttnStream a, const __half* __restrict__ qkv, const 
     chunks_append_ring<TA, NCH>(a, Ks, Vs, ringK, ringV, nf, cl, kt);
 
     const int pe0 = a.pe_index[slot];
-    for (int j = 0; j < a.chunks; ++j) {
+    for (int j = 0; j < k; ++j) {
         const int nfj = nf + j * t, clj = min(nfj, a.window);
         const int o = nfj - clj - first;            // staged row of this chunk's first key
         const int nk = clj + t;
@@ -456,14 +463,14 @@ attention_chunks_mma_kernel(AttnStream a, const __half* __restrict__ qkv, const 
         }
         for (int i = tid; i < t * DK; i += ATT_THREADS) {
             const int r = i / DK, d = i % DK;
-            const float q = q32[(long long)(b * kt + j * t + r) * 3 * D + h * DK + d];
+            const float q = q32[(long long)(j * t + r) * 3 * D + h * DK + d];
             const int sw = r * DK + (((d >> 3) ^ (r & 7)) << 3) + (d & 7);
             quh[sw] = from_f<TA>(q + pos_u[h * DK + d]);
             qvh[sw] = from_f<TA>(q + pos_v[h * DK + d]);
         }
         __syncthreads();
         attn_chunk_mma<ATT_THREADS / 32>(Ks + o * DK, Vs + o * DK, first + o, Ps, start, quh, qvh, ph, sc, vrows, nk, t,
-                                         out + (long long)(b * kt + j * t) * D + h * DK, D);
+                                         out + (long long)(j * t) * D + h * DK, D);
         __syncthreads();                              // Ps / quh / ph / sc are restaged by the next chunk
     }
 }
@@ -884,11 +891,16 @@ attention_offline_fa_kernel(const __half* __restrict__ qkv, const float* __restr
 }
 
 __global__ void advance_sessions_kernel(const int32_t* __restrict__ ids, int n, int t, int chunk_size, int pe_wrap,
-                                        int32_t* n_frames, int32_t* pe_index, int32_t* adapter_valid, int chunks) {
+                                        int32_t* n_frames, int32_t* pe_index, int32_t* adapter_valid, int chunks,
+                                        const int32_t* __restrict__ cnt, int min_cnt) {
     FO_PDL_TRIGGER();
     FO_PDL_WAIT();
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= n) return;
+    if (cnt) {
+        chunks = cnt[b];
+        if (chunks < min_cnt) return;
+    }
     const int s = ids[b];
     if (n_frames) {
         n_frames[s] += chunks * t;
@@ -1004,10 +1016,10 @@ template int attention_offline<float>(const float*, const float*, int, int, int,
 template int attention_offline<__half>(const __half*, const float*, int, int, int, const int32_t*, int, int, const float*, const __half*, int, const float*, const float*, __half*, cudaStream_t);
 
 int advance_sessions(const int32_t* ids, int n, int t, int chunk_size, int pe_wrap, int32_t* n_frames,
-                      int32_t* pe_index, int32_t* adapter_valid, cudaStream_t st, int chunks) {
+                      int32_t* pe_index, int32_t* adapter_valid, cudaStream_t st, int chunks, const int32_t* cnt, int min_cnt) {
     if (n <= 0) return 0;
     FO_CUDA(launch_pdl(advance_sessions_kernel, dim3(cdiv(n, 128)), dim3(128), 0, st, ids, n, t, chunk_size, pe_wrap, n_frames, pe_index, adapter_valid,
-                       chunks));
+                       chunks, cnt, min_cnt));
     FO_LAUNCHED();
     FO_CUDA(cudaGetLastError());
     return 0;

@@ -328,10 +328,29 @@ int scale_rows(const float* x, float* y, long long n, float s, cudaStream_t st);
 // x[b][k-1+i] = in[b][i] (zeroed where mask == 0, or ReLU(in * scale + shift) when scale != null), C channels, stride 1
 // (conv1d_gather layout) or 2 (adapter_gather layout); new cache = last k-1 rows (fp32), slot-resident (ids != null,
 // (slot, 2, k-1, C) time-major) or explicit (B, C, k-1)
+// Per-session rows of a call whose sessions bring different chunk counts (fo_encode_stream_chunks_v); cnt == null: every
+// session has the T rows of the uniform layout.
+//   pass < 0 (even t): session b's real input is its first cnt[b] * unit of T padded rows; with `off` non-null, `in` is
+//            packed instead, session b's rows starting at row off[b] * unit.  The new cache comes from the real rows.
+//   pass >= 0 (odd t, chunk pass `pass`): sessions with cnt[b] <= pass have no chunk in this pass and keep their cache.
+struct SessionRows {
+    const int32_t* cnt = nullptr;
+    const int32_t* off = nullptr;
+    int unit = 0;
+    int pass = -1;
+};
 template <typename TA>
 int conv_stage(const float* in, const uint8_t* mask, int B, int T, int C, int km1, int stride, const float* scale,
                const float* shift, const int32_t* ids, float* slot_cache, int32_t* slot_valid, const float* cache_in,
-               float* cache_out, TA* xin, cudaStream_t st);
+               float* cache_out, TA* xin, cudaStream_t st, const SessionRows& sr = SessionRows());
+// Moves blocks of `bytes` between per-session and packed (block) layouts, session b owning blocks [off[b], off[b] + cnt[b]):
+//   PACK:    grid (n, kmax), src block b * kmax + j (j < cnt[b]) -> dst block off[b] + j
+//   GATHER:  src block off[b] + min(j, cnt[b] - 1) -> dst block b
+//   SCATTER: src block b -> dst block off[b] + j, only where cnt[b] > j
+// Block i of src / dst starts at byte i * src_stride / i * dst_stride.
+enum { BLOCKS_PACK = 0, BLOCKS_GATHER = 1, BLOCKS_SCATTER = 2 };
+int session_blocks(const void* src, long long src_stride, void* dst, long long dst_stride, long long bytes, int n, int kmax,
+                   int j, int mode, const int32_t* cnt, const int32_t* off, cudaStream_t st);
 void conv1d_gather(int B, int T, int C, int k, AGather* ga, RowMap* rm);
 // (B, T, C) -> zero-padded (B, lead + T + trail, C) in the activation type
 template <typename TA>
@@ -339,10 +358,12 @@ int pad_rows(const TA* in, int B, int T, int C, int lead, int trail, TA* out, cu
 // Conv1dLinear's causal depthwise Conv1d over time (attention.py:217-224,251): y[r][c] = b[c] + sum_tau w[c][tau] *
 // xin[r + tau][c], xin = [left context (k-1 rows) | x].  Streaming (ids != null): x is (n, t, C), the left context of
 // session ids[b] lives in slot_cache (fp32, (k-1, C) per slot, stride slot_stride) and is replaced by the last k-1 rows
-// of xin.  Offline (ids == null): x is (B, T, C) with zero left padding per utterance.
+// of xin.  Offline (ids == null): x is (B, T, C) with zero left padding per utterance.  cnt / off (streaming, per-session
+// chunk counts): session b's rows are the cnt[b] * t rows from row (off[b] - off[0]) * t; T is then the largest of them.
 template <typename TA>
 int depthwise_conv(const TA* x, int B, int T, int C, int k, const float* w, const float* bias, const int32_t* ids,
-                   float* slot_cache, long long slot_stride, TA* y, cudaStream_t st);
+                   float* slot_cache, long long slot_stride, TA* y, cudaStream_t st, const int32_t* cnt = nullptr,
+                   const int32_t* off = nullptr, int t = 0);
 int subsample_mask(const int32_t* ilens, int B, int T, int T2, uint8_t* mask2, int32_t* ilens2, cudaStream_t st);
 // attention-mask rows + input start rows of the LLM hand-off (audioLLM.py:404-411); device pointers
 int handoff_mask(const uint8_t* onset, const uint8_t* prefix_mask, int n, int P, int t_out, int rows, uint8_t* attn_mask,
@@ -363,10 +384,14 @@ struct AttnStream {
     const float* part_bias = nullptr;
     int nsplit = 0;
     long long part_stride = 0;
-    // consecutive chunks per session in this call (fo_encode_stream_chunks): rows are (session, chunk, frame), n*chunks*t
-    // of them; chunk j of a session is attended exactly as the j-th of `chunks` sequential calls (chunk_size: pe_index step)
+    // consecutive chunks per session in this call (fo_encode_stream_chunks[_v]): rows are (session, chunk, frame); session b
+    // brings cnt[b] chunks and its rows start at row (off[b] - off[0]) * t; chunk j of a session is attended exactly as the
+    // j-th of cnt[b] sequential calls (chunk_size: pe_index step).  `chunks` is the largest count (it sizes shared memory);
+    // chunks == 1 is the single-chunk kernel, which reads rows b * t and no table.
     int chunks = 1;
     int chunk_size = 0;
+    const int32_t* cnt = nullptr;
+    const int32_t* off = nullptr;
 };
 // staged keys of the multi-chunk attention (window + chunks * t at most): bounds the chunks of one call
 constexpr int STREAM_CHUNKS_MAX_KEYS = 128;
@@ -388,9 +413,11 @@ int attention_offline(const TA* qkv, const float* q32, int B, int T, int H, cons
                       cudaStream_t st);
 // end of a streaming step: n_frames += t, pe_index = pe_index % wrap + chunk_size (attention.py:107,120),
 // and flip the live half of the double-buffered adapter cache.  Either group may be null.  chunks > 1: the session
-// advanced by that many chunks of t frames (pe_index stepped `chunks` times; the adapter cache still flips once).
+// advanced by that many chunks of t frames (pe_index stepped `chunks` times; the adapter cache still flips once).  cnt
+// non-null: session b's own count cnt[b] replaces `chunks`, and sessions with cnt[b] < min_cnt are left as they are.
 int advance_sessions(const int32_t* ids, int n, int t, int chunk_size, int pe_wrap, int32_t* n_frames,
-                     int32_t* pe_index, int32_t* adapter_valid, cudaStream_t st, int chunks = 1);
+                     int32_t* pe_index, int32_t* adapter_valid, cudaStream_t st, int chunks = 1,
+                     const int32_t* cnt = nullptr, int min_cnt = 0);
 
 // ---- weight-streaming layer stack for a handful of sessions (fo_stack.cu) ---------------------------
 // All transformer layers of a streaming step in ONE cooperative launch when the step has at most 16 token rows (1-4

@@ -273,15 +273,28 @@ __global__ void scale_rows_kernel(const float* __restrict__ x, float* __restrict
 // stride 1: one plane, xin[b * (km1 + T) + r][C] (conv1d_gather);  stride 2: two planes by row parity (adapter_gather).
 // The new cache = the last km1 virtual rows, fp32: explicit caches in the reference layout (B, C, km1); slot-resident caches
 // time-major and double-buffered per slot: slot_valid = 0 (None), 1 (half 0 live), 2 (half 1 live); the new rows go to the
-// other half and advance_sessions() flips the flag after every block has read it.
+// other half and advance_sessions() flips the flag after every block has read it.  SessionRows: rows of a session past its
+// real length Tb are padding (0, no cache), and the cache comes from its last real rows; a session without a chunk in an odd-t
+// pass writes no cache.
 template <typename TA>
 __global__ void conv_stage_kernel(const float* __restrict__ in, const uint8_t* __restrict__ mask, int T, int C, int km1, int stride,
                                   const float* __restrict__ scale, const float* __restrict__ shift,
                                   const int32_t* __restrict__ ids, float* slot_cache, const int32_t* __restrict__ slot_valid,
-                                  const float* __restrict__ cache_in, float* cache_out, TA* __restrict__ xin) {
+                                  const float* __restrict__ cache_in, float* cache_out, TA* __restrict__ xin, SessionRows sr) {
     FO_PDL_TRIGGER();
     FO_PDL_WAIT();
     const int b = blockIdx.x, r = blockIdx.y;          // r in [0, km1 + T)
+    int Tb = T;
+    long long in0 = (long long)b * T;                  // input row of the session's first frame
+    bool keep_cache = false;
+    if (sr.cnt) {
+        if (sr.pass >= 0) {
+            keep_cache = sr.cnt[b] <= sr.pass;
+        } else {
+            Tb = sr.cnt[b] * sr.unit;
+            if (sr.off) in0 = (long long)sr.off[b] * sr.unit;
+        }
+    }
     const int slot = ids ? ids[b] : -1;
     const int live = ids ? slot_valid[slot] : 0;
     const bool have_old = ids ? (live != 0) : (cache_in != nullptr);
@@ -294,16 +307,18 @@ __global__ void conv_stage_kernel(const float* __restrict__ in, const uint8_t* _
             if (!have_old) v = 0.f;
             else if (ids) v = old_half[(long long)r * C + c];
             else v = cache_in[((long long)b * C + c) * km1 + r];
-        } else {
+        } else if (r - km1 < Tb) {
             const int t = r - km1;
-            v = in[((long long)b * T + t) * C + c];
+            v = in[(in0 + t) * C + c];
             if (scale) v = fmaxf(v * scale[c] + shift[c], 0.f);
             else if (mask && !mask[(long long)b * T + t]) v = 0.f;
+        } else {
+            v = 0.f;                                     // padding behind a session's real rows (causal: no real output reads it)
         }
         if (stride == 1) xin[((long long)b * R1 + r) * C + c] = from_f<TA>(v);
         else xin[(((long long)(r & 1) * gridDim.x + b) * RP + (r >> 1)) * C + c] = from_f<TA>(v);
-        const int cr = r - T;                            // row of the new cache this element becomes
-        if (cr >= 0) {
+        const int cr = r - Tb;                           // row of the new cache this element becomes
+        if (cr >= 0 && cr < km1 && !keep_cache) {
             if (ids) new_half[(long long)cr * C + c] = v;
             else if (cache_out) cache_out[((long long)b * C + c) * km1 + cr] = v;
         }
@@ -318,10 +333,17 @@ template <typename TA>
 __global__ void __launch_bounds__(256)
 depthwise_conv_kernel(const TA* __restrict__ x, int T, int C, int k, const float* __restrict__ w,
                       const float* __restrict__ bias, const int32_t* __restrict__ ids, float* slot_cache,
-                      long long slot_stride, TA* __restrict__ y, int row0) {
+                      long long slot_stride, TA* __restrict__ y, int row0, const int32_t* __restrict__ cnt,
+                      const int32_t* __restrict__ off, int t) {
     FO_PDL_TRIGGER();
     FO_PDL_WAIT();
     const int b = blockIdx.y, r0 = row0 + blockIdx.x * DW_TB;
+    long long base = (long long)b * T;                 // the session's first row
+    if (cnt) {                                         // per-session counts: cnt[b] * t rows from block off[b] - off[0]
+        base = (long long)(off[b] - off[0]) * t;
+        T = cnt[b] * t;
+        if (r0 >= T) return;
+    }
     const int nr = min(DW_TB, T - r0);
     const int km1 = k - 1;
     float* cache = ids ? slot_cache + (long long)ids[b] * slot_stride : nullptr;
@@ -336,19 +358,19 @@ depthwise_conv_kernel(const TA* __restrict__ x, int T, int C, int k, const float
             if (q < km1) {
                 const int r = r0 - km1 + q;
                 float v = 0.f;
-                if (r >= 0) v = to_f(x[((long long)b * T + r) * C + c]);
+                if (r >= 0) v = to_f(x[(base + r) * C + c]);
                 else if (cache) v = cache[(long long)(km1 + r) * C + c];        // row r of the old context, r in [-km1, -1]
                 win[q] = v;
             }
         }
         for (int i = 0; i < nr; ++i) {
-            const float cur = to_f(x[((long long)b * T + r0 + i) * C + c]);
+            const float cur = to_f(x[(base + r0 + i) * C + c]);
             float acc = bv;
 #pragma unroll
             for (int q = 0; q < DW_KMAX - 1; ++q)
                 if (q < km1) acc = fmaf(wv[q], win[q], acc);
             acc = fmaf(wv[km1], cur, acc);
-            y[((long long)b * T + r0 + i) * C + c] = from_f<TA>(acc);
+            y[(base + r0 + i) * C + c] = from_f<TA>(acc);
 #pragma unroll
             for (int q = 0; q < DW_KMAX - 2; ++q)
                 if (q < km1 - 1) win[q] = win[q + 1];
@@ -577,18 +599,56 @@ template int pad_rows<__half>(const __half*, int, int, int, int, int, __half*, c
 template <typename TA>
 int conv_stage(const float* in, const uint8_t* mask, int B, int T, int C, int km1, int stride, const float* scale,
                const float* shift, const int32_t* ids, float* slot_cache, int32_t* slot_valid, const float* cache_in,
-               float* cache_out, TA* xin, cudaStream_t st) {
+               float* cache_out, TA* xin, cudaStream_t st, const SessionRows& sr) {
     if (B <= 0) return 0;
     FO_CHECK(stride == 1 || stride == 2, "conv_stage: stride must be 1 or 2");
     dim3 grid(B, km1 + T);
     FO_CUDA(launch_pdl(conv_stage_kernel<TA>, grid, dim3(256), 0, st, in, mask, T, C, km1, stride, scale, shift, ids, slot_cache,
-                       (const int32_t*)slot_valid, cache_in, cache_out, xin));
+                       (const int32_t*)slot_valid, cache_in, cache_out, xin, sr));
     FO_LAUNCHED();
     FO_CUDA(cudaGetLastError());
     return 0;
 }
-template int conv_stage<float>(const float*, const uint8_t*, int, int, int, int, int, const float*, const float*, const int32_t*, float*, int32_t*, const float*, float*, float*, cudaStream_t);
-template int conv_stage<__half>(const float*, const uint8_t*, int, int, int, int, int, const float*, const float*, const int32_t*, float*, int32_t*, const float*, float*, __half*, cudaStream_t);
+template int conv_stage<float>(const float*, const uint8_t*, int, int, int, int, int, const float*, const float*, const int32_t*, float*, int32_t*, const float*, float*, float*, cudaStream_t, const SessionRows&);
+template int conv_stage<__half>(const float*, const uint8_t*, int, int, int, int, int, const float*, const float*, const int32_t*, float*, int32_t*, const float*, float*, __half*, cudaStream_t, const SessionRows&);
+
+__global__ void session_blocks_kernel(const char* __restrict__ src, long long src_stride, char* __restrict__ dst, long long dst_stride,
+                                      long long bytes, int kmax, int j, int mode, const int32_t* __restrict__ cnt,
+                                      const int32_t* __restrict__ off) {
+    FO_PDL_TRIGGER();
+    FO_PDL_WAIT();
+    const int b = blockIdx.x, k = cnt[b];
+    long long si, di;
+    if (mode == BLOCKS_PACK) {
+        const int jj = blockIdx.y;
+        if (jj >= k) return;
+        si = (long long)b * kmax + jj; di = off[b] + jj;
+    } else if (mode == BLOCKS_GATHER) {
+        si = off[b] + min(j, k - 1); di = b;
+    } else {
+        if (k <= j) return;
+        si = b; di = off[b] + j;
+    }
+    const char* s = src + si * src_stride;
+    char* d = dst + di * dst_stride;
+    if (((bytes | src_stride | dst_stride | (long long)(size_t)src | (long long)(size_t)dst) & 15) == 0) {
+        for (long long i = threadIdx.x * 16LL; i < bytes; i += blockDim.x * 16LL)
+            *reinterpret_cast<uint4*>(d + i) = *reinterpret_cast<const uint4*>(s + i);
+    } else {
+        for (long long i = threadIdx.x * 2LL; i < bytes; i += blockDim.x * 2LL)     // rows of 16-bit or 32-bit elements
+            *reinterpret_cast<uint16_t*>(d + i) = *reinterpret_cast<const uint16_t*>(s + i);
+    }
+}
+int session_blocks(const void* src, long long src_stride, void* dst, long long dst_stride, long long bytes, int n, int kmax,
+                   int j, int mode, const int32_t* cnt, const int32_t* off, cudaStream_t st) {
+    if (n <= 0) return 0;
+    FO_CHECK(bytes % 2 == 0 && src_stride % 2 == 0 && dst_stride % 2 == 0, "session_blocks: blocks of 16-bit or 32-bit elements");
+    FO_CUDA(launch_pdl(session_blocks_kernel, dim3(n, mode == BLOCKS_PACK ? kmax : 1), dim3(256), 0, st, (const char*)src, src_stride,
+                       (char*)dst, dst_stride, bytes, kmax, j, mode, cnt, off));
+    FO_LAUNCHED();
+    FO_CUDA(cudaGetLastError());
+    return 0;
+}
 
 // stride-1 causal conv (kernel k) over xin[b * (k-1+T) + r][C]: tap tau of output row t reads row t + tau
 void conv1d_gather(int B, int T, int C, int k, AGather* ga, RowMap* rm) {
@@ -600,25 +660,28 @@ void conv1d_gather(int B, int T, int C, int k, AGather* ga, RowMap* rm) {
 
 template <typename TA>
 int depthwise_conv(const TA* x, int B, int T, int C, int k, const float* w, const float* bias, const int32_t* ids,
-                   float* slot_cache, long long slot_stride, TA* y, cudaStream_t st) {
+                   float* slot_cache, long long slot_stride, TA* y, cudaStream_t st, const int32_t* cnt, const int32_t* off, int t) {
     if (B <= 0 || T <= 0) return 0;
     FO_CHECK(k >= 2 && k <= DW_KMAX, "depthwise_conv: kernel size %d outside 2..%d", k, DW_KMAX);
-    if (ids && T > DW_TB) {
-        // streaming, several chunks per session (fo_encode_stream_chunks): the first rows read the carried context and the
-        // last ones replace it, so the row blocks run in order, one launch each
+    FO_CHECK(!cnt || (ids && off && t > 0), "depthwise_conv: per-session counts are a streaming layout");
+    if (ids && (T > DW_TB || cnt)) {
+        // streaming, several chunks per session (fo_encode_stream_chunks[_v]): the first rows read the carried context and the
+        // last ones replace it, so the row blocks run in order, one launch each (up to the largest session's rows)
         for (int r0 = 0; r0 < T; r0 += DW_TB) {
-            FO_CUDA(launch_pdl(depthwise_conv_kernel<TA>, dim3(1, B), dim3(256), 0, st, x, T, C, k, w, bias, ids, slot_cache, slot_stride, y, r0));
+            FO_CUDA(launch_pdl(depthwise_conv_kernel<TA>, dim3(1, B), dim3(256), 0, st, x, T, C, k, w, bias, ids, slot_cache, slot_stride, y, r0,
+                               cnt, off, t));
             FO_LAUNCHED();
         }
         return 0;
     }
     dim3 grid(cdiv(T, DW_TB), B);
-    FO_CUDA(launch_pdl(depthwise_conv_kernel<TA>, grid, dim3(256), 0, st, x, T, C, k, w, bias, ids, slot_cache, slot_stride, y, 0));
+    FO_CUDA(launch_pdl(depthwise_conv_kernel<TA>, grid, dim3(256), 0, st, x, T, C, k, w, bias, ids, slot_cache, slot_stride, y, 0,
+                       (const int32_t*)nullptr, (const int32_t*)nullptr, 0));
     FO_LAUNCHED();
     return 0;
 }
-template int depthwise_conv<float>(const float*, int, int, int, int, const float*, const float*, const int32_t*, float*, long long, float*, cudaStream_t);
-template int depthwise_conv<__half>(const __half*, int, int, int, int, const float*, const float*, const int32_t*, float*, long long, __half*, cudaStream_t);
+template int depthwise_conv<float>(const float*, int, int, int, int, const float*, const float*, const int32_t*, float*, long long, float*, cudaStream_t, const int32_t*, const int32_t*, int);
+template int depthwise_conv<__half>(const __half*, int, int, int, int, const float*, const float*, const int32_t*, float*, long long, __half*, cudaStream_t, const int32_t*, const int32_t*, int);
 
 // LLM hand-off bookkeeping (models/audioLLM.py:404-411): per session the attention-mask row over its block of the inputs_embeds
 // buffer, [prefix_mask | 1 x t_out | 0 ...] when the block opens an IPU (status 'ipu_sl': the chat prefix is part of the input) and

@@ -334,6 +334,28 @@ class Engine:
                                                     _ptr(adapter_out) if want_adapter else None, self._stream()))
         return enc_out, (adapter_out if want_adapter else None)
 
+    def encode_stream_chunks_v(self, ids, chunks, feats: ArrayLike, want_adapter: Optional[bool] = None,
+                               enc_out: Optional[torch.Tensor] = None, adapter_out: Optional[torch.Tensor] = None):
+        """Session ids[i] advances chunks[i] >= 1 consecutive chunks, all in one step, with the results of chunks[i]
+        single-chunk encode_stream calls.  feats (B, t_in, F), B = sum(chunks), blocks in (session, chunk) order: session i's
+        blocks start at chunks[0] + ... + chunks[i-1].  Returns enc (B, t, D) and adapter (B, t_out, E) in the same order."""
+        ids = _ids(ids)
+        n = len(ids)
+        cnt = _ids(chunks)
+        assert len(cnt) == n, "one chunk count per session"
+        assert feats is not None and feats.ndim == 3, "feats must be (sum(chunks), t_in, F)"
+        B, t_in = int(feats.shape[0]), int(feats.shape[1])
+        assert B == int(cnt.sum()) and tuple(feats.shape) == (B, t_in, self.cfg.feat_dim)
+        assert feats.dtype in (torch.float32, np.dtype(np.float32))
+        t, t_out = self.out_frames(t_in)
+        want_adapter = self.has_adapter if want_adapter is None else want_adapter
+        enc_out = self._out(enc_out, (B, t, self.cfg.d_model))
+        if want_adapter:
+            adapter_out = self._out(adapter_out, (B, t_out, self.cfg.llm_dim))
+        _lib.check(self.lib.fo_encode_stream_chunks_v(self._h, _i32p(ids), _i32p(cnt), n, _ptr(feats), t_in, _ptr(enc_out),
+                                                      _ptr(adapter_out) if want_adapter else None, self._stream()))
+        return enc_out, (adapter_out if want_adapter else None)
+
     def stream_step(self, ids, pcm: ArrayLike, scale: Optional[float] = None, enc_out: Optional[torch.Tensor] = None,
                     adapter_out: Optional[torch.Tensor] = None, want_enc: bool = True):
         """PCM in, encoder frames + LLM-space embeddings out, one library call."""

@@ -18,7 +18,8 @@ Per drain round the head block of every session with a non-empty queue forms one
 multiple of `bucket` with scratch sessions so that a handful of captured CUDA graphs serve every active-set size.
 With `max_chunks` > 1 a round takes up to that many queued blocks of a session at once (Engine.encode_stream_chunks, same
 results as one block per call): an onset tick then costs one call for the sessions with one block and one for those
-replaying their history, instead of 1 + onset_chunks calls.
+replaying their history, instead of 1 + onset_chunks calls.  With `mixed_calls` as well, a round is ONE call in which every
+session brings its own number of blocks (Engine.encode_stream_chunks_v), so an onset tick costs one encoder step.
 State (KV rings, adapter cache, sample carry, feature ring, history ring, queued blocks) never leaves the device, unless a
 session is moved: `detach` / `attach` carry it, history rows included, to another scheduler on any GPU.
 """
@@ -117,6 +118,33 @@ def plan_chunk_calls(queue_lens: Dict[Hashable, int], max_chunks: int, max_batch
             left[key] -= min(left[key], max_chunks)
 
 
+def plan_mixed_calls(queue_lens: Dict[Hashable, int], max_chunks: int, max_batch: int) -> List[List[Tuple[Hashable, int]]]:
+    """Drain order when one call may advance each of its sessions by its own number of queued blocks (up to `max_chunks`):
+    every round takes k = min(blocks left, max_chunks) blocks of each session that still has some, all in one call (split
+    only by `max_batch` sessions).  Within a call the sessions with k = 1 come first, in queue order, so that they form the
+    leading one-chunk run the encoder attends with its single-chunk kernel; the others follow in queue order.  Returns the
+    calls as [(session, k)].  Pure function of the queue lengths -> testable without a GPU."""
+    assert max_chunks >= 1
+    left = dict(queue_lens)
+    calls: List[List[Tuple[Hashable, int]]] = []
+    while True:
+        ready = [(key, min(n, max_chunks)) for key, n in left.items() if n > 0]
+        if not ready:
+            return calls
+        ordered = [r for r in ready if r[1] == 1] + [r for r in ready if r[1] > 1]
+        for i in range(0, len(ordered), max_batch):
+            calls.append(ordered[i:i + max_batch])
+        for key, k in ready:
+            left[key] -= k
+
+
+def mixed_padding(counts: List[int], bucket: int) -> int:
+    """Scratch sessions, one block each, that pad a call with these per-session block counts to a multiple of `bucket`
+    blocks (fewer than `bucket` of them).  They join the leading one-chunk run."""
+    blocks = sum(counts)
+    return bucket_size(blocks, bucket) - blocks
+
+
 def bucket_size(n: int, bucket: int) -> int:
     return (n + bucket - 1) // bucket * bucket
 
@@ -130,9 +158,11 @@ def chunk_bucket_size(n: int, k: int, bucket: int) -> int:
 
 class StreamScheduler:
     def __init__(self, engine, history_chunks: int = 10, onset_chunks: int = 6, bucket: int = 16,
-                 max_batch: Optional[int] = None, max_sessions: Optional[int] = None, max_chunks: int = 1):
+                 max_batch: Optional[int] = None, max_sessions: Optional[int] = None, max_chunks: int = 1,
+                 mixed_calls: bool = False):
         assert 0 <= onset_chunks <= history_chunks and max_chunks >= 1
         self.max_chunks = int(max_chunks)
+        self.mixed_calls = bool(mixed_calls)
         self.eng, self.cfg = engine, engine.cfg
         self.history_chunks, self.onset_chunks, self.bucket = history_chunks, onset_chunks, max(1, bucket)
         self.max_batch = max_batch or 1 << 30
@@ -246,6 +276,8 @@ class StreamScheduler:
                     self.block_log.extend((k, b, lab) for b, lab in labelled)
             self.pending.clear()
         cursor = 0
+        if self.mixed_calls:
+            return self._drain_mixed(out, handoff)
         if self.max_chunks > 1:
             return self._drain_chunks(out, handoff)
         for batch in plan_rounds({k: len(q) for k, q in self.queues.items()}, self.max_batch):
@@ -285,36 +317,88 @@ class StreamScheduler:
         """The drain of tick() with up to max_chunks blocks of a session per call (plan_chunk_calls)."""
         cursor = 0
         for k, batch in plan_chunk_calls({s: len(q) for s, q in self.queues.items()}, self.max_chunks, self.max_batch):
-            heads = [[self.queues[s].popleft() for _ in range(k)] for s in batch]
-            n = len(batch)
-            pad = chunk_bucket_size(n, k, self.bucket) - n
-            ids = np.concatenate([np.array([self.keys[s] for s in batch], np.int32), self.scratch[:pad]]).astype(np.int32)
-            x = torch.stack([h[0] for hs in heads + [heads[0]] * pad for h in hs])
-            x = x.view(n + pad, k, *x.shape[1:])                                                  # (n + pad, k, t_in, F)
+            cursor = self._chunk_call(k, batch, out, handoff, cursor)
+        return out
+
+    def _drain_mixed(self, out: Dict[Hashable, List[Block]], handoff: Optional[Handoff]) -> Dict[Hashable, List[Block]]:
+        """The drain of tick() with one call per round, each session bringing up to max_chunks blocks (plan_mixed_calls).
+        A round whose sessions all bring the same number of blocks keeps the uniform call."""
+        cursor = 0
+        for call in plan_mixed_calls({s: len(q) for s, q in self.queues.items()}, self.max_chunks, self.max_batch):
+            counts = [k for _, k in call]
+            batch = [s for s, _ in call]
+            if len(set(counts)) == 1:
+                cursor = self._chunk_call(counts[0], batch, out, handoff, cursor)
+                continue
+            heads = [[self.queues[s].popleft() for _ in range(k)] for s, k in call]
+            n1 = counts.index(next(k for k in counts if k > 1))           # the leading one-chunk run
+            pad = mixed_padding(counts, self.bucket)
+            order = list(range(n1)) + [-1] * pad + list(range(n1, len(call)))   # -1: a scratch session
+            ids = np.concatenate([np.array([self.keys[s] for s in batch[:n1]], np.int32), self.scratch[:pad],
+                                  np.array([self.keys[s] for s in batch[n1:]], np.int32)]).astype(np.int32)
+            chunks = np.array([counts[i] if i >= 0 else 1 for i in order], np.int32)
+            x = torch.stack([h[0] for i in order for h in (heads[i] if i >= 0 else heads[0][:1])])      # (sum(chunks), t_in, F)
+            first = np.concatenate([[0], np.cumsum(chunks)[:-1]])        # block of each session's first chunk
             self.stats["encode_calls"] += 1
-            self.stats["session_steps"] += n * k
-            self.stats["padded_steps"] += pad * k
+            self.stats["session_steps"] += sum(counts)
+            self.stats["padded_steps"] += pad
             if handoff is not None:
-                # block i*k + j of the armed call is chunk j of session i
-                n_blocks = (n + pad) * k
+                n_blocks = int(chunks.sum())
                 if cursor + n_blocks > handoff.embeds.shape[0]:
                     raise RuntimeError("Handoff capacity %d exceeded in one tick" % handoff.embeds.shape[0])
-                onset = [h[1] == IPU_START for hs in heads for h in hs] + [False] * (pad * k)
+                onset = [h[1] == IPU_START for i in order for h in (heads[i] if i >= 0 else [(None, None)])]
                 self.eng.handoff_arm(n_blocks, handoff.embeds[cursor:], handoff.prefix_len, onset, handoff.prefix_mask,
                                      handoff.attn_mask[cursor:], handoff.row_start[cursor:])
-                enc, _ = self._encode(ids, x, k, want_adapter=False)
-                for i, s in enumerate(batch):
-                    for j, h in enumerate(heads[i]):
-                        row = cursor + i * k + j
+                enc, _ = self.eng.encode_stream_chunks_v(ids, chunks, x, want_adapter=False)
+            else:
+                enc, emb = self.eng.encode_stream_chunks_v(ids, chunks, x)
+            for p, i in enumerate(order):
+                if i < 0:
+                    continue
+                for j, h in enumerate(heads[i]):
+                    b = int(first[p]) + j
+                    if handoff is not None:
                         st0 = 0 if h[1] == IPU_START else handoff.prefix_len
-                        out.setdefault(s, []).append(Block(enc[i, j], handoff.embeds[row, st0:], h[1], handoff.attn_mask[row, st0:]))
-                cursor += n_blocks
-                continue
-            enc, emb = self._encode(ids, x, k)
+                        out.setdefault(batch[i], []).append(Block(enc[b], handoff.embeds[cursor + b, st0:], h[1],
+                                                                  handoff.attn_mask[cursor + b, st0:]))
+                    else:
+                        out.setdefault(batch[i], []).append(Block(enc[b], emb[b] if emb is not None else None, h[1]))
+            if handoff is not None:
+                cursor += int(chunks.sum())
+        return out
+
+    def _chunk_call(self, k: int, batch: List[Hashable], out: Dict[Hashable, List[Block]], handoff: Optional[Handoff],
+                    cursor: int) -> int:
+        """One call advancing every session of `batch` by k queued blocks; returns the next free hand-off block."""
+        heads = [[self.queues[s].popleft() for _ in range(k)] for s in batch]
+        n = len(batch)
+        pad = chunk_bucket_size(n, k, self.bucket) - n
+        ids = np.concatenate([np.array([self.keys[s] for s in batch], np.int32), self.scratch[:pad]]).astype(np.int32)
+        x = torch.stack([h[0] for hs in heads + [heads[0]] * pad for h in hs])
+        x = x.view(n + pad, k, *x.shape[1:])                                                  # (n + pad, k, t_in, F)
+        self.stats["encode_calls"] += 1
+        self.stats["session_steps"] += n * k
+        self.stats["padded_steps"] += pad * k
+        if handoff is not None:
+            # block i*k + j of the armed call is chunk j of session i
+            n_blocks = (n + pad) * k
+            if cursor + n_blocks > handoff.embeds.shape[0]:
+                raise RuntimeError("Handoff capacity %d exceeded in one tick" % handoff.embeds.shape[0])
+            onset = [h[1] == IPU_START for hs in heads for h in hs] + [False] * (pad * k)
+            self.eng.handoff_arm(n_blocks, handoff.embeds[cursor:], handoff.prefix_len, onset, handoff.prefix_mask,
+                                 handoff.attn_mask[cursor:], handoff.row_start[cursor:])
+            enc, _ = self._encode(ids, x, k, want_adapter=False)
             for i, s in enumerate(batch):
                 for j, h in enumerate(heads[i]):
-                    out.setdefault(s, []).append(Block(enc[i, j], emb[i, j] if emb is not None else None, h[1]))
-        return out
+                    row = cursor + i * k + j
+                    st0 = 0 if h[1] == IPU_START else handoff.prefix_len
+                    out.setdefault(s, []).append(Block(enc[i, j], handoff.embeds[row, st0:], h[1], handoff.attn_mask[row, st0:]))
+            return cursor + n_blocks
+        enc, emb = self._encode(ids, x, k)
+        for i, s in enumerate(batch):
+            for j, h in enumerate(heads[i]):
+                out.setdefault(s, []).append(Block(enc[i, j], emb[i, j] if emb is not None else None, h[1]))
+        return cursor
 
     def _encode(self, ids, x, k, **kw):
         """(n, k, ...) results of one call: a single-chunk call keeps the engine's one-chunk entry point."""

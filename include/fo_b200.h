@@ -190,6 +190,15 @@ int fo_encode_stream(fo_ctx* ctx, const int32_t* ids, int n, const float* feats,
  * session i (onset flag, embedding rows, mask row and row_start per block).  Counts as one stream step and n*k session chunks. */
 int fo_encode_stream_chunks(fo_ctx* ctx, const int32_t* ids, int n, int k, const float* feats, int t_in,
                             float* enc_out, float* adapter_out, void* stream);
+/* fo_encode_stream_chunks with a chunk count per session: session ids[i] advances by chunks[i] >= 1 consecutive chunks.
+ * feats (B, t_in, feat_dim) with B = sum(chunks), blocks in (session, chunk) order: session i's blocks are
+ * [off_i, off_i + chunks[i]), off_i = chunks[0] + ... + chunks[i-1].  enc_out (B, t, d_model), adapter_out (B, t_out, llm_dim),
+ * same block order; either may be NULL.  Equal to chunks[i] successive single-chunk calls per session.
+ * An armed hand-off applies when armed for B blocks (block off_i + j is chunk j of session i).
+ * FO_ERR_ARG, with nothing enqueued, when a count is < 1 or window + chunks[i] * t exceeds the 128 keys of the streaming
+ * attention.  One stream step, sum(chunks) session chunks. */
+int fo_encode_stream_chunks_v(fo_ctx* ctx, const int32_t* ids, const int32_t* chunks, int n, const float* feats, int t_in,
+                              float* enc_out, float* adapter_out, void* stream);
 /* fbank + encode in one call (one captured graph): PCM in, embeddings out */
 int fo_stream_step(fo_ctx* ctx, const int32_t* ids, int n, const void* pcm, int pcm_dtype, float scale,
                    float* enc_out, float* adapter_out, void* stream);
