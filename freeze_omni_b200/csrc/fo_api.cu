@@ -187,6 +187,7 @@ struct fo_ctx {
     unsigned int* stack_bar = nullptr;        // grid-barrier words of the kernel
     unsigned long long* stack_trace = nullptr;
     long long stack_launches = 0;
+    int steps_pass_blocks = 0;                // option: blocks per pass of fo_stream_steps_v (0: from STEPS_PASS_BYTES)
     struct ProfRec { cudaEvent_t e0, e1; int M, N, K; };
     std::vector<ProfRec> prof_events;
     // captured step graphs, keyed by the shape of the call; invalidated when a workspace moves
@@ -217,7 +218,7 @@ struct fo_ctx {
 namespace {
 
 enum { WS_FEATS = 0, WS_C1, WS_C2, WS_XSUB, WS_EMB, WS_X, WS_H, WS_QKV, WS_ATT, WS_FFH, WS_ENC, WS_XIN, WS_ACONV, WS_AH,
-       WS_Y, WS_MASK2, WS_ILENS, WS_ILENS2, WS_AMASK, WS_PCM, WS_TMP0, WS_TMP1, WS_TMP2, WS_TMP3, WS_Q32, WS_HC, WS_PART, WS_PCM2, WS_ENC2, WS_Y2, WS_AC1, WS_XIN2, WS_TMP4, WS_TMP5, WS_HP, WS_FP, WS_ENCJ, WS_PACK, WS_ADJ, WS_COUNT };
+       WS_Y, WS_MASK2, WS_ILENS, WS_ILENS2, WS_AMASK, WS_PCM, WS_TMP0, WS_TMP1, WS_TMP2, WS_TMP3, WS_Q32, WS_HC, WS_PART, WS_PCM2, WS_ENC2, WS_Y2, WS_AC1, WS_XIN2, WS_TMP4, WS_TMP5, WS_HP, WS_FP, WS_ENCJ, WS_PACK, WS_ADJ, WS_SROWS, WS_COUNT };
 
 int dev_alloc(fo_ctx* c, void** p, size_t bytes) {
     *p = nullptr;
@@ -698,12 +699,14 @@ inline void chunk_rowmap(const AdOut& o, int t_out, RowMap* rm) {
 // cnt[b] chunks of `unit` frames from block off[b].  The convolutions run over B sessions x T = kmax * unit rows, padded at
 // the end of each session's run (the conv is causal, so the real rows' outputs are those of the sequential calls); the
 // real output rows are packed to (block, frame) order before the norm and the projection.  pass >= 0 (odd t, chunk pass
-// `pass`): B sessions x T rows as without mix, but sessions with cnt[b] <= pass keep their caches.
+// `pass`): B sessions x T rows as without mix, but sessions with cnt[b] <= pass keep their caches.  pick (odd t, passes of
+// fo_stream_steps_v): the grid as for even t, every conv at stride 1, then the rows of the stride-2 outputs picked per chunk.
 struct AdMix {
     const int32_t* cnt;
     const int32_t* off;
     int kmax, unit, blocks;
     int pass = -1;
+    bool pick = false;
 };
 template <typename TA>
 int adapter_program(fo_ctx* c, const float* enc, const uint8_t* mask, int B, int T, const int32_t* ids_dev,
@@ -715,26 +718,28 @@ int adapter_program(fo_ctx* c, const float* enc, const uint8_t* mask, int B, int
     const int M = grid ? mix->blocks * t_out : B * t_out;
     const bool run_gemm = !(c->debug_skip & 16);
     const float* x = enc;
+    const bool pick = grid && mix->pick;
     for (int i = 0; i < ns; ++i) {
         const fo_ctx::AdStage& s = c->ad_st[i];
-        const int Ti = ad_frames(c, T, i);
+        const int stride = pick ? 1 : s.stride;
+        const int Ti = pick ? T : ad_frames(c, T, i);
         AGather ga;
         RowMap rm;
-        if (s.stride == 1) conv1d_gather(B, Ti, s.cin, KA, &ga, &rm);
+        if (stride == 1) conv1d_gather(B, Ti, s.cin, KA, &ga, &rm);
         else adapter_gather(B, Ti, s.cin, KA, &ga, &rm);
         void *xin, *conv;
         FO_TRY(ws_ensure(c, i == 0 ? WS_XIN : WS_XIN2, (size_t)ga.planes * ga.rows * s.cin * sizeof(TA), &xin));
-        FO_TRY(ws_ensure(c, i + 1 == ns ? WS_ACONV : WS_AC1, (size_t)B * ad_frames(c, T, i + 1) * s.cout * sizeof(float), &conv));
+        FO_TRY(ws_ensure(c, i + 1 == ns ? WS_ACONV : WS_AC1, (size_t)B * (pick ? T : ad_frames(c, T, i + 1)) * s.cout * sizeof(float), &conv));
         SessionRows sr;
         if (mix) {
             sr.cnt = mix->cnt;
             sr.pass = mix->pass;
             if (grid) {
                 sr.off = i == 0 ? mix->off : nullptr;      // the first conv reads the packed encoder rows
-                sr.unit = ad_frames(c, mix->unit, i);
+                sr.unit = pick ? mix->unit : ad_frames(c, mix->unit, i);
             }
         }
-        FO_TRY(conv_stage<TA>(x, i == 0 ? mask : nullptr, B, Ti, s.cin, KA - 1, s.stride, s.in_scale, s.in_shift,
+        FO_TRY(conv_stage<TA>(x, i == 0 ? mask : nullptr, B, Ti, s.cin, KA - 1, stride, s.in_scale, s.in_shift,
                               c->ad_carry ? ids_dev : nullptr, s.cache, c->ad_valid, cache_in ? cache_in[i] : nullptr,
                               cache_out ? cache_out[i] : nullptr, reinterpret_cast<TA*>(xin), st, sr));
         Epilogue e;
@@ -749,7 +754,8 @@ int adapter_program(fo_ctx* c, const float* enc, const uint8_t* mask, int B, int
         void* pk;
         const long long blk = (long long)t_out * K * sizeof(float);
         FO_TRY(ws_ensure(c, WS_PACK, (size_t)M * K * sizeof(float), &pk));
-        FO_TRY(session_blocks(x, blk, pk, blk, blk, B, mix->kmax, 0, BLOCKS_PACK, mix->cnt, mix->off, st));
+        if (pick) FO_TRY(pick_chunk_rows(x, B, mix->kmax, mix->unit, t_out, K, mix->cnt, mix->off, reinterpret_cast<float*>(pk), st));
+        else FO_TRY(session_blocks(x, blk, pk, blk, blk, B, mix->kmax, 0, BLOCKS_PACK, mix->cnt, mix->off, st));
         x = reinterpret_cast<const float*>(pk);
     }
     const TA* a = reinterpret_cast<const TA*>(enc);
@@ -1074,6 +1080,7 @@ int stack_program(fo_ctx* c, int n, int t, float* x, void* qkv, float* q32, void
 struct Mix {
     int blocks = 0, kmax = 1, n1 = 0;
     const int32_t* off = nullptr;
+    int group = 0;               // > 0: a pass of fo_stream_steps_v (attention_steps, `group` chunks per CTA; counts uncapped)
     bool uniform(int n) const { return blocks == n * kmax; }
     int block(int i) const { return off ? off[i] : i * kmax; }
 };
@@ -1095,6 +1102,13 @@ int adapter_chunks(fo_ctx* c, const float* enc, int n, const Mix& m, int t, AdOu
         }
         // different counts: the same pass over a per-session grid of kmax*t rows, each session's padding at its end
         const AdMix mix{c->cnt_dev, c->off_dev, k, t, m.blocks};
+        return adapter_program<TA>(c, enc, nullptr, n, k * t, c->ids_dev, nullptr, nullptr, out, st, &mix);
+    }
+    if (m.group) {
+        // odd t in a pass of fo_stream_steps_v: in the session's continuous stream S = [cache | x_0 | x_1 ..], output m of
+        // chunk j is the conv at S position j * t + 2 m, so stride-1 convs over the grid and a row pick give every chunk at once
+        AdMix mix{c->cnt_dev, c->off_dev, k, t, m.blocks};
+        mix.pick = true;
         return adapter_program<TA>(c, enc, nullptr, n, k * t, c->ids_dev, nullptr, nullptr, out, st, &mix);
     }
     // odd t: the output phase of the stride-2 conv shifts between chunks (a joint pass yields other frames, and fewer), so
@@ -1161,7 +1175,7 @@ int stream_program(fo_ctx* c, int n, const Mix& m, const float* feats, int t_in,
     // two groups' kernels overlap each other's pipeline fill, epilogue and launch gaps.  Rows of one group are
     // contiguous, so the groups just take slices of the same workspaces.
     int stacked = 1;
-    if (sizeof(TA) == 2 && m.kmax == 1) {                   // the stack kernel's attention is single-chunk
+    if (sizeof(TA) == 2 && m.kmax == 1 && !m.group) {       // the stack kernel's attention is single-chunk
         stacked = stack_program(c, n, t, x, qkv, q32, att, ffh, enc_out_dev, st);
         if (stacked < 0) return stacked;
     }
@@ -1217,7 +1231,7 @@ int stream_program(fo_ctx* c, int n, const Mix& m, const float* feats, int t_in,
             }
             int qkv_splits = 0;
             // the multi-chunk attention reads finished QKV rows: no split-K reduction deferred to it
-            if (r == 0) r = layer_pre<TA>(c, w, Mg, hg, qkvg, q32g, pfq, sg, m.kmax == 1 ? &qkv_splits : nullptr);
+            if (r == 0) r = layer_pre<TA>(c, w, Mg, hg, qkvg, q32g, pfq, sg, m.kmax == 1 && !m.group ? &qkv_splits : nullptr);
             if (qkv_splits > 0) {
                 a.part = c->tc_cur->partial;
                 a.part_bias = w.bqkv;
@@ -1226,7 +1240,12 @@ int stream_program(fo_ctx* c, int n, const Mix& m, const float* feats, int t_in,
             }
             TA* ring_l = reinterpret_cast<TA*>(c->ring) + l * layer_stride;
             const int n1g = std::min(std::max(m.n1 - s0, 0), ng);  // the group's share of the leading one-chunk run
-            if (r == 0 && !(c->debug_skip & 1) && n1g < ng) {
+            if (r == 0 && !(c->debug_skip & 1) && m.group) {
+                AttnStream as = a;
+                as.chunks = m.group;
+                r = attention_steps<TA>(as, (m.kmax + m.group - 1) / m.group, qkvg, q32g, ring_l, reinterpret_cast<const TA*>(w.ptab_h),
+                                        w.pos_u, w.pos_v, attg, sg);
+            } else if (r == 0 && !(c->debug_skip & 1) && n1g < ng) {
                 // multi-chunk sessions (rows from the end of the one-chunk run): on a forked stream when both kernels run
                 AttnStream am = a;
                 am.ids += n1g; am.cnt += n1g; am.off += n1g; am.n = ng - n1g;
@@ -2408,6 +2427,118 @@ int fo_stream_step(fo_ctx* c, const int32_t* ids, int n, const void* pcm, int pc
                          adapter_out, (cudaStream_t)stream);
 }
 
+// ---- recorded audio: many chunks per session, exact-streaming ----------------------------------------
+// fo_stream_steps_v runs in passes of at most P blocks (option "steps_pass_blocks", else STEPS_PASS_BYTES over the workspace
+// bytes of one block): each pass gives every session that still has chunks its next min(remaining, q) chunks, q = the
+// longest remaining count spread evenly over the passes that max(1, P / sessions left) chunks per pass would take; it then
+// runs the fbank of those blocks (fbank_stream_blocks) and the streaming program with the pass attention (attention_steps).  Every workspace is sized by the pass, so the device memory a call adds does not grow with the recording.
+// Passes run eagerly: a captured graph per pass shape would multiply with recording lengths.
+constexpr long long STEPS_PASS_BYTES = 1LL << 30;
+
+// workspace bytes one block of a pass adds: PCM and sample rows, features, conv1 planes (the six-plane implicit-GEMM operand
+// of conv2) and conv2 rows, residual / LayerNorm / attention rows, QKV (+ fp32 Q), FFN hidden rows, encoder and adapter rows
+static long long steps_block_bytes(const fo_ctx* c, int t_in) {
+    const int t = ((t_in - 1) / 2 - 1) / 2, t_out = ad_frames(c, t);
+    const long long esz = (long long)c->esz, D = c->D;
+    long long b = (long long)(2 * c->chunk_samples + c->carry) * 4 + (long long)t_in * c->F * 4;
+    b += 6LL * t * (c->F2 + 1) * D * esz + (long long)t * c->F2 * D * esz;
+    b += (long long)t * D * (4 + 4 + 4 + 5 * esz) + (long long)t * 3 * D * (esz + 4) + (long long)t * c->FF * esz;
+    if (c->cfg.has_adapter) b += (long long)t * 4 * D * (esz + 4) + (long long)t_out * c->E * 4;
+    return b;
+}
+
+int fo_stream_steps_v(fo_ctx* c, const int32_t* ids, const int32_t* chunks, int n, const void* pcm, int pcm_dtype, float scale,
+                      float* enc_out, float* adapter_out, void* stream) {
+    FO_CHECK(c && c->finalized && c->cfg.has_encoder && c->fb_window, "fo_stream_steps_v: context has no finalized encoder + frontend");
+    FO_CHECK(pcm && (pcm_dtype == FO_F32 || pcm_dtype == FO_I16), "fo_stream_steps_v: pcm must be FO_F32 or FO_I16");
+    FO_CHECK(chunks, "fo_stream_steps_v: chunks must be a host array of n counts");
+    FO_CHECK(!c->armed.on, "fo_stream_steps_v: an LLM hand-off is armed (fo_handoff_arm); this call does not take it, and it stays "
+                           "armed for the next fo_stream_step / fo_encode_stream call");
+    FO_TRY(check_ids(c, ids, n));
+    const int t_in = c->cfg.context_frames + c->cfg.frames_per_chunk;
+    FO_TRY(stream_geometry(c, t_in));
+    FO_CHECK(!c->KM, "fo_stream_steps_v: MultiLayeredConv1d has no streaming form (models/encoder/attention.py:145-196); use fo_encode_offline");
+    if (adapter_out) FO_CHECK(c->cfg.has_adapter, "adapter_out requested but the context has no adapter");
+    std::vector<long long> off(n + 1, 0);
+    for (int i = 0; i < n; ++i) {
+        FO_CHECK(chunks[i] >= 1, "fo_stream_steps_v: session %d (id %d) has chunk count %d; counts must be >= 1", i, ids[i], chunks[i]);
+        off[i + 1] = off[i] + chunks[i];
+    }
+    FO_CUDA(cudaSetDevice(c->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    if (c->copy_stream && c->async_ticket > 0) {       // as in stream_common: pipelined steps still read the shared buffers
+        FO_CUDA(cudaStreamWaitEvent(st, c->ev_out[0], 0));
+        if (c->async_ticket > 1) FO_CUDA(cudaStreamWaitEvent(st, c->ev_out[1], 0));
+    }
+    const int T1 = (t_in - 1) / 2, t = (T1 - 1) / 2, t_out = ad_frames(c, t);
+    const int P = c->steps_pass_blocks > 0 ? c->steps_pass_blocks
+                                           : (int)std::max(1LL, std::min(1LL << 20, STEPS_PASS_BYTES / steps_block_bytes(c, t_in)));
+    const long long pcm_row = (long long)c->chunk_samples * (pcm_dtype == FO_I16 ? 2 : 4);
+    const long long enc_row = (long long)t * c->D, y_row = (long long)t_out * c->E;
+    const bool want_y = adapter_out != nullptr;
+    int sms = 148;
+    FO_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->device));
+    const int gmax = std::max(1, (STREAM_CHUNKS_MAX_KEYS - c->window) / t);
+    g_use_pdl = g_want_pdl;
+    std::vector<int32_t> done(n, 0), pids, pcnt, poff, psrc;
+    for (;;) {
+        pids.clear(); pcnt.clear(); psrc.clear();
+        for (int i = 0; i < n; ++i) if (done[i] < chunks[i]) psrc.push_back(i);
+        const int na = (int)psrc.size();
+        if (na == 0) break;
+        // at most P / na chunks per session, spread evenly over the passes the longest session still needs
+        int q = std::max(1, P / na), rmax = 0;
+        for (int i : psrc) rmax = std::max(rmax, chunks[i] - done[i]);
+        q = (rmax + (rmax + q - 1) / q - 1) / ((rmax + q - 1) / q);
+        poff.assign(1, 0);
+        Mix m;
+        for (int i : psrc) {
+            pids.push_back(ids[i]);
+            pcnt.push_back(std::min(q, chunks[i] - done[i]));
+            poff.push_back(poff.back() + pcnt.back());
+            m.kmax = std::max(m.kmax, (int)pcnt.back());
+        }
+        m.blocks = poff.back();
+        m.off = poff.data();
+        // chunks per attention CTA: enough (session, head, group) CTAs to fill the SMs, each staging at most 128 keys
+        const int want = std::max(1, (sms + na * c->H - 1) / (na * c->H));
+        m.group = std::min(gmax, std::max(1, (m.kmax + want - 1) / want));
+        FO_TRY(upload_ids(c, pids.data(), na, st, nullptr, 0, pcnt.data()));
+        c->pf_slot_lo = *std::min_element(pids.begin(), pids.end());
+        c->pf_slot_hi = *std::max_element(pids.begin(), pids.end());
+        void *dpcm, *drows, *dfeats, *denc, *dy = nullptr;
+        FO_TRY(ws_ensure(c, WS_PCM, (size_t)m.blocks * c->chunk_samples * 4, &dpcm));
+        FO_TRY(ws_ensure(c, WS_SROWS, (size_t)m.blocks * (c->carry + c->chunk_samples) * sizeof(float), &drows));
+        FO_TRY(ws_ensure(c, WS_FEATS, (size_t)m.blocks * t_in * c->F * sizeof(float), &dfeats));
+        FO_TRY(ws_ensure(c, WS_ENC, (size_t)m.blocks * enc_row * sizeof(float), &denc));
+        if (want_y) FO_TRY(ws_ensure(c, WS_Y, (size_t)m.blocks * y_row * sizeof(float), &dy));
+        for (int a = 0; a < na; ++a) {
+            const int i = psrc[a];
+            FO_CUDA(cudaMemcpyAsync((char*)dpcm + poff[a] * pcm_row, (const char*)pcm + (off[i] + done[i]) * pcm_row, pcnt[a] * pcm_row,
+                                    cudaMemcpyDefault, st));
+        }
+        FO_TRY(fbank_stream_blocks(fbank_params(c), c->ids_dev, c->cnt_dev, c->off_dev, na, m.kmax, m.blocks, dpcm, pcm_dtype == FO_I16,
+                                   scale, c->cfg.frames_per_chunk, c->cfg.context_frames, c->samples, c->feat_ring, (float*)drows,
+                                   (float*)dfeats, st));
+        FO_TRY(c->dtype == FO_BF16 ? stream_program<act16>(c, na, m, (const float*)dfeats, t_in, (float*)denc, (float*)dy, st)
+                                   : stream_program<float>(c, na, m, (const float*)dfeats, t_in, (float*)denc, (float*)dy, st));
+        for (int a = 0; a < na; ++a) {
+            const int i = psrc[a];
+            const long long b0 = off[i] + done[i];
+            if (enc_out) FO_CUDA(cudaMemcpyAsync(enc_out + b0 * enc_row, (float*)denc + poff[a] * enc_row, pcnt[a] * enc_row * sizeof(float),
+                                                 cudaMemcpyDefault, st));
+            if (want_y) FO_CUDA(cudaMemcpyAsync(adapter_out + b0 * y_row, (float*)dy + poff[a] * y_row, pcnt[a] * y_row * sizeof(float),
+                                                cudaMemcpyDefault, st));
+            done[i] += pcnt[a];
+        }
+    }
+    if (!c->ev_sync) FO_CUDA(cudaEventCreateWithFlags(&c->ev_sync, cudaEventDisableTiming));
+    FO_CUDA(cudaEventRecord(c->ev_sync, st));
+    c->stats.stream_steps += 1;
+    c->stats.session_chunks += off[n];
+    return 0;
+}
+
 // ---- full utterance -----------------------------------------------------------------------------------
 int fo_encode_offline(fo_ctx* c, const float* feats, const int32_t* ilens, int B, int T, int chunk, int left,
                       float* enc_out, uint8_t* mask_out, float* adapter_out, uint8_t* adapter_mask_out, void* stream) {
@@ -2553,6 +2684,10 @@ int fo_set_option(fo_ctx* c, const char* name, int64_t value) {
     }
     else if (!strcmp(name, "fuse_ln")) c->fuse_ln = value != 0;
     else if (!strcmp(name, "stack_rows")) c->stack_rows = (int)value;
+    else if (!strcmp(name, "steps_pass_blocks")) {
+        FO_CHECK(value >= 0 && value <= (1 << 20), "steps_pass_blocks must be 0 (byte budget) or 1..%d blocks", 1 << 20);
+        c->steps_pass_blocks = (int)value;
+    }
     else if (!strcmp(name, "defer_reduce")) c->defer_reduce = value != 0;
     else if (!strcmp(name, "tc_persist")) gemm_tc_set_persist(value != 0);
     else if (!strcmp(name, "l2_prefetch")) c->use_prefetch = (int)(value & 3);
@@ -2585,6 +2720,7 @@ int fo_get_option(fo_ctx* c, const char* name, int64_t* value) {
     else if (!strcmp(name, "session_groups")) *value = c->groups;
     else if (!strcmp(name, "fuse_ln")) *value = c->fuse_ln;
     else if (!strcmp(name, "stack_rows")) *value = c->stack_rows;
+    else if (!strcmp(name, "steps_pass_blocks")) *value = c->steps_pass_blocks;
     else if (!strcmp(name, "stack_launches")) *value = c->stack_launches;
     else if (!strcmp(name, "defer_reduce")) *value = c->defer_reduce;
     else if (!strcmp(name, "tc_persist_launches")) *value = gemm_tc_persist_launches();

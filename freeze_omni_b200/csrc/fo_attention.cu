@@ -474,8 +474,186 @@ attention_chunks_mma_kernel(AttnStream a, const __half* __restrict__ qkv, const 
         __syncthreads();                              // Ps / quh / ph / sc are restaged by the next chunk
     }
 }
+
 // ---------------------------------------------------------------------------------------------
-constexpr int KT = 96;          // key tile: the shipped band of a 32-query block (64 left + 32 own keys) in one pass
+// Passes of fo_stream_steps_v: a session brings any number of chunks.  CTA (b, h, z) takes chunks [j0, j1) = [z * G,
+// min(cnt[b], (z + 1) * G)) of session b, G = a.chunks, and stages the keys of all of them once: frames [first, nf + j1 * t)
+// with first = nf_j0 - min(nf_j0, window) -- those before the pass (frame < nf) from the ring, the rest from the pass's own
+// K|V rows (qkv row = frame - nf).  Chunk j is then attended as the multi-chunk kernels attend it (window + t keys at most);
+// its rel-pos start uses chunk_pe in closed form, (pe % wrap + j * chunk_size) % wrap, since j may run into the thousands.
+// The ring is only read here: steps_append_ring_kernel writes the new frames after the whole grid has read it.
+struct StepsGroup {
+    int j0, j1, nf, first, cr, kn;      // chunks; frames before the pass; first staged frame; staged rows from ring / from qkv
+};
+__device__ __forceinline__ bool steps_group(const AttnStream& a, int b, StepsGroup* g) {
+    g->j0 = blockIdx.z * a.chunks;
+    const int k = a.cnt[b];
+    if (g->j0 >= k) return false;
+    g->j1 = min(k, g->j0 + a.chunks);
+    g->nf = a.n_frames[a.ids[b]];
+    const int nf0 = g->nf + g->j0 * a.t;
+    g->first = nf0 - min(nf0, a.window);
+    g->cr = max(0, g->nf - g->first);
+    g->kn = g->nf + g->j1 * a.t - (g->first + g->cr);
+    return true;
+}
+__device__ __forceinline__ int steps_start(const AttnStream& a, int pe0, int j) {
+    return max(0, (int)(((long long)(pe0 % a.pe_wrap) + (long long)j * a.chunk_size) % a.pe_wrap) - a.full_chunk);
+}
+
+__global__ void __launch_bounds__(ATT_THREADS)
+attention_steps_kernel(AttnStream a, const float* __restrict__ qkv, const float* __restrict__ q32, const float* __restrict__ ring,
+                       const float* __restrict__ ptab_h, const float* __restrict__ pos_u, const float* __restrict__ pos_v,
+                       float* __restrict__ out) {
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    constexpr int EPC = 4, NCH = DK / EPC;
+    FO_PDL_TRIGGER();
+    FO_PDL_WAIT();
+    const int cap = a.ring_cap, t = a.t, D = a.H * DK;
+    const int rows = a.window + a.chunks * t, prow = a.window + t;
+    float* Ks = reinterpret_cast<float*>(smem_raw);
+    float* Vs = Ks + rows * DK;
+    float* Ps = Vs + rows * DK;
+    float* qu = Ps + prow * DK;
+    float* qv = qu + t * DK;
+    float* prob = qv + t * DK;                      // t x prow
+    __shared__ __align__(8) uint64_t bar;
+
+    const int b = blockIdx.x, h = blockIdx.y;
+    StepsGroup g;
+    if (!steps_group(a, b, &g)) return;
+    const int slot = a.ids[b];
+    const long long row0 = (long long)(a.off[b] - a.off[0]) * t;
+    qkv += row0 * 3 * D; q32 += row0 * 3 * D; out += row0 * D;
+    const float* ringK = ring + (long long)slot * a.ring_slot_stride + (long long)h * cap * DK;
+    const float* ringV = ringK + (long long)a.H * cap * DK;
+    const int tid = threadIdx.x;
+    if (tid == 0) {
+        mbar_init(&bar, 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        ring_window_copy<float>(ringK, ringV, cap, g.first, g.cr, Ks, Vs, nullptr, nullptr, 0, &bar);
+    }
+    const int fs = g.first + g.cr;
+    chunks_stage_new<float, NCH, false>(a, qkv + (long long)(fs - g.nf) * 3 * D, Ks, Vs, h, fs, g.cr, g.kn);
+    __syncthreads();
+    mbar_wait(&bar, 0);
+
+    const int pe0 = a.pe_index[slot];
+    for (int j = g.j0; j < g.j1; ++j) {
+        const int nfj = g.nf + j * t, clj = min(nfj, a.window);
+        const int o = nfj - clj - g.first;
+        const int nk = clj + t;
+        const int start = steps_start(a, pe0, j);
+        for (int i = tid; i < nk * NCH; i += ATT_THREADS) {
+            const int r = i / NCH, c = i % NCH, pos = min(start + r, a.pos_rows - 1);
+            *reinterpret_cast<uint4*>(Ps + r * DK + c * EPC) = *reinterpret_cast<const uint4*>(ptab_h + ((long long)h * a.pos_rows + pos) * DK + c * EPC);
+        }
+        for (int i = tid; i < t * DK; i += ATT_THREADS) {
+            const int r = i / DK, d = i % DK;
+            const float q = q32[(long long)(j * t + r) * 3 * D + h * DK + d];
+            qu[i] = q + pos_u[h * DK + d];
+            qv[i] = q + pos_v[h * DK + d];
+        }
+        __syncthreads();
+        attn_chunk_ffma(Ks + o * DK, Vs + o * DK, Ps, qu, qv, prob, prow, nk, t, out + (long long)(j * t) * D + h * DK, D);
+        __syncthreads();
+    }
+}
+
+__global__ void __launch_bounds__(ATT_THREADS)
+attention_steps_mma_kernel(AttnStream a, const __half* __restrict__ qkv, const float* __restrict__ q32, const __half* __restrict__ ring,
+                           const __half* __restrict__ ptab_h, const float* __restrict__ pos_u, const float* __restrict__ pos_v,
+                           __half* __restrict__ out) {
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    typedef __half TA;
+    constexpr int EPC = 8, NCH = 8;
+    FO_PDL_TRIGGER();
+    FO_PDL_WAIT();
+    const int cap = a.ring_cap, t = a.t, D = a.H * DK;
+    const int rows = a.window + a.chunks * t;
+    const int krows = ((rows + 15) & ~15) + 16;     // a chunk's last key tile may read up to 15 rows past the staged keys
+    const int vrows = (a.window + t + 15) & ~15;
+    TA* Ks = reinterpret_cast<TA*>(smem_raw);
+    TA* Vs = Ks + krows * DK;
+    TA* Ps = Vs + krows * DK;
+    TA* quh = Ps + vrows * DK;
+    TA* qvh = quh + t * DK;
+    TA* ph = qvh + t * DK;
+    float* sc = reinterpret_cast<float*>(ph + t * vrows);
+    __shared__ __align__(8) uint64_t bar;
+
+    const int b = blockIdx.x, h = blockIdx.y;
+    StepsGroup g;
+    if (!steps_group(a, b, &g)) return;
+    const int slot = a.ids[b];
+    const long long row0 = (long long)(a.off[b] - a.off[0]) * t;
+    qkv += row0 * 3 * D; q32 += row0 * 3 * D; out += row0 * D;
+    const int nk_all = g.cr + g.kn;
+    const TA* ringK = ring + (long long)slot * a.ring_slot_stride + (long long)h * cap * DK;
+    const TA* ringV = ringK + (long long)a.H * cap * DK;
+    const int tid = threadIdx.x;
+    if (tid == 0) {
+        mbar_init(&bar, 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        ring_window_copy<TA>(ringK, ringV, cap, g.first, g.cr, Ks, Vs, nullptr, nullptr, 0, &bar);
+    }
+    const int fs = g.first + g.cr;
+    chunks_stage_new<TA, NCH, true>(a, qkv + (long long)(fs - g.nf) * 3 * D, Ks, Vs, h, fs, g.cr, g.kn);
+    for (int i = tid; i < (krows - nk_all) * NCH; i += ATT_THREADS) {
+        *reinterpret_cast<uint4*>(Ks + (nk_all + i / NCH) * DK + (i % NCH) * EPC) = make_uint4(0, 0, 0, 0);
+        *reinterpret_cast<uint4*>(Vs + (nk_all + i / NCH) * DK + (i % NCH) * EPC) = make_uint4(0, 0, 0, 0);
+    }
+    __syncthreads();
+    mbar_wait(&bar, 0);
+
+    const int pe0 = a.pe_index[slot];
+    for (int j = g.j0; j < g.j1; ++j) {
+        const int nfj = g.nf + j * t, clj = min(nfj, a.window);
+        const int o = nfj - clj - g.first;
+        const int nk = clj + t;
+        const int start = steps_start(a, pe0, j);
+        for (int i = tid; i < nk * NCH; i += ATT_THREADS) {
+            const int r = i / NCH, cc = i % NCH, pos = min(start + r, a.pos_rows - 1);
+            *reinterpret_cast<uint4*>(Ps + r * DK + ((cc ^ ((start + r) & 7)) * EPC)) =
+                *reinterpret_cast<const uint4*>(ptab_h + ((long long)h * a.pos_rows + pos) * DK + ((cc ^ (pos & 7)) * EPC));
+        }
+        for (int i = tid; i < t * DK; i += ATT_THREADS) {
+            const int r = i / DK, d = i % DK;
+            const float q = q32[(long long)(j * t + r) * 3 * D + h * DK + d];
+            const int sw = r * DK + (((d >> 3) ^ (r & 7)) << 3) + (d & 7);
+            quh[sw] = from_f<TA>(q + pos_u[h * DK + d]);
+            qvh[sw] = from_f<TA>(q + pos_v[h * DK + d]);
+        }
+        __syncthreads();
+        attn_chunk_mma<ATT_THREADS / 32>(Ks + o * DK, Vs + o * DK, g.first + o, Ps, start, quh, qvh, ph, sc, vrows, nk, t,
+                                         out + (long long)(j * t) * D + h * DK, D);
+        __syncthreads();
+    }
+}
+
+// The ring after a pass: the last min(cnt[b] * t, cap) new K|V rows of session b at row frame % cap (fp16: chunk-swizzled by
+// frame), as the same frames appended by single steps leave it.  One CTA per (session, head).
+template <typename TA, bool SWZ>
+__global__ void __launch_bounds__(ATT_THREADS)
+steps_append_ring_kernel(AttnStream a, const TA* __restrict__ qkv, TA* __restrict__ ring) {
+    constexpr int EPC = 16 / sizeof(TA), NCH = DK / EPC;
+    FO_PDL_TRIGGER();
+    FO_PDL_WAIT();
+    const int b = blockIdx.x, h = blockIdx.y, D = a.H * DK;
+    const int kt = a.cnt[b] * a.t, r0 = max(0, kt - a.ring_cap), nr = kt - r0;
+    const int nf = a.n_frames[a.ids[b]];
+    qkv += (long long)(a.off[b] - a.off[0]) * a.t * 3 * D;
+    TA* ringK = ring + (long long)a.ids[b] * a.ring_slot_stride + (long long)h * a.ring_cap * DK;
+    TA* ringV = ringK + (long long)a.H * a.ring_cap * DK;
+    for (int i = threadIdx.x; i < nr * NCH * 2; i += ATT_THREADS) {
+        const int which = i / (nr * NCH), r = r0 + (i / NCH) % nr, c = i % NCH;
+        const int pc = SWZ ? (c ^ ((nf + r) & 7)) : c;
+        *reinterpret_cast<uint4*>((which ? ringV : ringK) + (long long)((nf + r) % a.ring_cap) * DK + pc * EPC) =
+            *reinterpret_cast<const uint4*>(qkv + (long long)r * 3 * D + (which + 1) * D + h * DK + c * EPC);
+    }
+}
+// ---------------------------------------------------------------------------------------------
+constexpr int KT = 96;         // key tile: the shipped band of a 32-query block (64 left + 32 own keys) in one pass
 constexpr int QB = 32;          // query rows per CTA
 constexpr int QPW = QB / (ATT_THREADS / 32);   // queries per warp
 
@@ -959,6 +1137,40 @@ int attention_stream(const AttnStream& a, const TA* qkv, const float* q32, TA* r
     return 0;
 }
 template int attention_stream<float>(const AttnStream&, const float*, const float*, float*, const float*, const float*, const float*, float*, cudaStream_t);
+
+template <typename TA>
+int attention_steps(const AttnStream& a, int groups, const TA* qkv, const float* q32, TA* ring, const TA* ptab_h,
+                    const float* pos_u, const float* pos_v, TA* out, cudaStream_t st) {
+    if (a.n <= 0) return 0;
+    const int t = a.t, rows = a.window + a.chunks * t, prow = a.window + t;
+    FO_CHECK(t <= STREAM_MAX_T && a.ring_cap >= prow && a.cnt && a.off && groups >= 1, "attention_steps: bad geometry");
+    FO_CHECK(rows <= STREAM_CHUNKS_MAX_KEYS, "attention_steps: window %d + %d chunks x %d frames exceeds %d keys", a.window,
+             a.chunks, t, STREAM_CHUNKS_MAX_KEYS);
+    size_t smem;
+    void (*kern)(AttnStream, const TA*, const float*, const TA*, const TA*, const float*, const float*, TA*);
+    if constexpr (sizeof(TA) == 2) {
+        kern = attention_steps_mma_kernel;
+        const int krows = ((rows + 15) & ~15) + 16, vrows = (prow + 15) & ~15;
+        smem = (size_t)(2 * krows + vrows) * DK * 2 + (size_t)2 * t * DK * 2 + (size_t)t * vrows * 2 + (size_t)t * std::max(vrows, DK) * 4;
+    } else {
+        kern = attention_steps_kernel;
+        smem = (size_t)(2 * rows + prow) * DK * 4 + (size_t)2 * t * DK * 4 + (size_t)t * prow * 4;
+    }
+    static bool opted_in = false;
+    if (!opted_in) {
+        FO_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
+        opted_in = true;
+    }
+    FO_CUDA(launch_pdl(kern, dim3(a.n, a.H, groups), dim3(ATT_THREADS), smem, st, a, qkv, q32, (const TA*)ring, ptab_h, pos_u, pos_v, out));
+    FO_LAUNCHED();
+    FO_CUDA(cudaGetLastError());
+    FO_CUDA(launch_pdl(steps_append_ring_kernel<TA, sizeof(TA) == 2>, dim3(a.n, a.H), dim3(ATT_THREADS), 0, st, a, qkv, ring));
+    FO_LAUNCHED();
+    FO_CUDA(cudaGetLastError());
+    return 0;
+}
+template int attention_steps<float>(const AttnStream&, int, const float*, const float*, float*, const float*, const float*, const float*, float*, cudaStream_t);
+template int attention_steps<__half>(const AttnStream&, int, const __half*, const float*, __half*, const __half*, const float*, const float*, __half*, cudaStream_t);
 // head-major copy of a rel-pos table in the activation type: out[h][pos][64] = (TA) in[pos][h*64 + d]
 template <typename TA>
 __global__ void ptab_head_major_kernel(const float* __restrict__ in, int pos_rows, int H, TA* __restrict__ out) {

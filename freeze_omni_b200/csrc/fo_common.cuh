@@ -300,6 +300,12 @@ struct FbankParams {
 int fbank_stream(const FbankParams& p, const int32_t* ids, int n, const void* pcm, int pcm_is_i16, float scale,
                  int frames_per_chunk, int ctx_frames, float* carry, float* ring, float* feats_out,
                  cudaStream_t st);
+// The same for cnt[b] consecutive chunks of session ids[b] (blocks (session, chunk) from off[b]; kmax the largest count):
+// pcm (blocks, chunk samples); feats_out (blocks, ctx+m, n_mel) gets every block as fbank_stream would return it after the
+// blocks before it, and each session ends holding its last block's carry and ring.  rows: (blocks, carry + chunk) fp32 scratch.
+int fbank_stream_blocks(const FbankParams& p, const int32_t* ids, const int32_t* cnt, const int32_t* off, int n, int kmax,
+                        int blocks, const void* pcm, int pcm_is_i16, float scale, int frames_per_chunk, int ctx_frames,
+                        float* carry, float* ring, float* rows, float* feats_out, cudaStream_t st);
 int fbank_offline(const FbankParams& p, const void* pcm, int pcm_is_i16, int B, long long n_samples, float scale,
                   float* out, cudaStream_t st);
 
@@ -351,6 +357,10 @@ int conv_stage(const float* in, const uint8_t* mask, int B, int T, int C, int km
 enum { BLOCKS_PACK = 0, BLOCKS_GATHER = 1, BLOCKS_SCATTER = 2 };
 int session_blocks(const void* src, long long src_stride, void* dst, long long dst_stride, long long bytes, int n, int kmax,
                    int j, int mode, const int32_t* cnt, const int32_t* off, cudaStream_t st);
+// The carried stride-2 adapter conv over chunks of odd t, run at stride 1 over each session's kmax * t grid rows: output m of
+// chunk j is grid row j * t + 2 m.  src (n, kmax * t, C) -> dst (blocks, t_out, C), session b's chunks j < cnt[b] from block off[b].
+int pick_chunk_rows(const float* src, int n, int kmax, int t, int t_out, int C, const int32_t* cnt, const int32_t* off, float* dst,
+                    cudaStream_t st);
 void conv1d_gather(int B, int T, int C, int k, AGather* ga, RowMap* rm);
 // (B, T, C) -> zero-padded (B, lead + T + trail, C) in the activation type
 template <typename TA>
@@ -403,6 +413,13 @@ constexpr int STREAM_MAX_T = 8;
 template <typename TA>
 int attention_stream(const AttnStream& a, const TA* qkv, const float* q32, TA* ring, const TA* ptab_h,
                      const float* pos_u, const float* pos_v, TA* out, cudaStream_t st);
+// One pass of fo_stream_steps_v: session b's cnt[b] chunks (any number) with the rows and tables of a multi-chunk call.
+// One CTA per (session, head, group of a.chunks chunks), grid z = `groups`; each chunk still sees window + t keys, staged
+// from the ring (frames before the pass) and from this pass's own K|V rows in qkv.  A second kernel then appends the last
+// min(cnt[b] * t, ring_cap) new frames to the ring, after every read of it.
+template <typename TA>
+int attention_steps(const AttnStream& a, int groups, const TA* qkv, const float* q32, TA* ring, const TA* ptab_h,
+                    const float* pos_u, const float* pos_v, TA* out, cudaStream_t st);
 // ptab_h: the same table as [H][pos_rows][64] in the activation type (rows of one head contiguous -> one bulk copy)
 template <typename TA>
 int ptab_head_major(const float* in, int pos_rows, int H, TA* out, cudaStream_t st);

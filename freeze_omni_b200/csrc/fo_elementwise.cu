@@ -639,6 +639,26 @@ __global__ void session_blocks_kernel(const char* __restrict__ src, long long sr
             *reinterpret_cast<uint16_t*>(d + i) = *reinterpret_cast<const uint16_t*>(s + i);
     }
 }
+// grid (kmax * t_out, n): row m of chunk j < cnt[b] of session b <- row j * t + 2 m of the session's T-row grid
+__global__ void pick_chunk_rows_kernel(const float* __restrict__ src, int T, int C, int t, int t_out, const int32_t* __restrict__ cnt,
+                                       const int32_t* __restrict__ off, float* __restrict__ dst) {
+    FO_PDL_TRIGGER();
+    FO_PDL_WAIT();
+    const int b = blockIdx.y, j = blockIdx.x / t_out, m = blockIdx.x % t_out;
+    if (j >= cnt[b]) return;
+    const float* s = src + ((long long)b * T + (long long)j * t + 2 * m) * C;
+    float* d = dst + ((long long)(off[b] + j) * t_out + m) * C;
+    for (int c = threadIdx.x; c < C; c += blockDim.x) d[c] = s[c];
+}
+int pick_chunk_rows(const float* src, int n, int kmax, int t, int t_out, int C, const int32_t* cnt, const int32_t* off, float* dst,
+                    cudaStream_t st) {
+    if (n <= 0) return 0;
+    FO_CUDA(launch_pdl(pick_chunk_rows_kernel, dim3(kmax * t_out, n), dim3(256), 0, st, src, kmax * t, C, t, t_out, cnt, off, dst));
+    FO_LAUNCHED();
+    FO_CUDA(cudaGetLastError());
+    return 0;
+}
+
 int session_blocks(const void* src, long long src_stride, void* dst, long long dst_stride, long long bytes, int n, int kmax,
                    int j, int mode, const int32_t* cnt, const int32_t* off, cudaStream_t st) {
     if (n <= 0) return 0;

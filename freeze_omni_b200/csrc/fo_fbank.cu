@@ -159,6 +159,47 @@ frontend_ingest_kernel(const int32_t* __restrict__ ids, const void* __restrict__
     }
 }
 
+// Several consecutive chunks per session (fbank_stream_blocks), block = (session b, chunk j), packed from off[b]: the sample row
+// of a block is [the carry samples before it | its chunk] -- block 0 takes them from the session's sample buffer, a later
+// block from the tail of the previous block's PCM.  Values are formed as frontend_ingest_kernel forms them.
+__global__ void __launch_bounds__(256)
+frontend_blocks_kernel(const int32_t* __restrict__ ids, const int32_t* __restrict__ cnt, const int32_t* __restrict__ off,
+                       const void* __restrict__ pcm, int is_i16, float scale, int carry, int chunk,
+                       const float* __restrict__ samples, float* __restrict__ rows) {
+    const int j = blockIdx.x, b = blockIdx.y;
+    if (j >= cnt[b]) return;
+    const long long blk = off[b] + j;
+    float* r = rows + blk * (carry + chunk);
+    const float* sm = samples + (long long)ids[b] * (carry + chunk) + chunk;
+    for (int i = threadIdx.x; i < carry + chunk; i += blockDim.x) {
+        if (i < carry && j == 0) { r[i] = sm[i]; continue; }
+        const long long o = blk * chunk + i - carry;            // i < carry: the previous block's tail
+        r[i] = is_i16 ? (float)reinterpret_cast<const int16_t*>(pcm)[o] * scale : reinterpret_cast<const float*>(pcm)[o] * scale;
+    }
+}
+
+// One CTA per session, after the per-frame kernel: the context rows of every block (block 0: the last ctx frames of the
+// session's feature ring; block j: the last ctx new frames of block j - 1, which frames_per_chunk >= ctx puts among that
+// block's computed rows), then the session keeps its last block's sample row and features, as fo_fbank_stream leaves them.
+__global__ void __launch_bounds__(256)
+frontend_blocks_finish_kernel(const int32_t* __restrict__ ids, const int32_t* __restrict__ cnt, const int32_t* __restrict__ off,
+                              int carry, int chunk, int ctx, int m, int n_mel, const float* __restrict__ rows,
+                              float* __restrict__ feats, float* __restrict__ samples, float* __restrict__ ring) {
+    const int b = blockIdx.x, s = ids[b], k = cnt[b];
+    const long long blk_feats = (long long)(ctx + m) * n_mel;
+    float* f0 = feats + off[b] * blk_feats;
+    float* rg = ring + (long long)s * blk_feats;
+    for (long long i = threadIdx.x; i < (long long)k * ctx * n_mel; i += blockDim.x) {
+        const int j = (int)(i / (ctx * n_mel)), e = (int)(i % (ctx * n_mel));
+        f0[j * blk_feats + e] = j == 0 ? rg[m * n_mel + e] : f0[(j - 1) * blk_feats + m * n_mel + e];
+    }
+    __syncthreads();
+    const float* last = f0 + (k - 1) * blk_feats;
+    for (int i = threadIdx.x; i < blk_feats; i += blockDim.x) rg[i] = last[i];
+    const float* lr = rows + (off[b] + k - 1) * (long long)(carry + chunk);
+    for (int i = threadIdx.x; i < carry + chunk; i += blockDim.x) samples[(long long)s * (carry + chunk) + i] = lr[i];
+}
+
 int upload_twiddles(int P) {
     if (g_twiddle_fft == P) return 0;
     FO_CHECK(P >= 64 && P <= MAX_FFT && (P & (P - 1)) == 0, "fbank: FFT size %d unsupported", P);
@@ -196,6 +237,30 @@ int fbank_stream(const FbankParams& p, const int32_t* ids, int n, const void* pc
     fbank_kernel<<<grid, FB_WARPS * 32, fbank_smem(p.fft_size), st>>>(
         p, src, n, frames_per_chunk, ring, ids, (long long)(ctx_frames + frames_per_chunk) * p.n_mel, ctx_frames,
         feats_out, ctx_frames + frames_per_chunk, ctx_frames);
+    FO_LAUNCHED();
+    FO_CUDA(cudaGetLastError());
+    return 0;
+}
+
+int fbank_stream_blocks(const FbankParams& p, const int32_t* ids, const int32_t* cnt, const int32_t* off, int n, int kmax,
+                        int blocks, const void* pcm, int pcm_is_i16, float scale, int frames_per_chunk, int ctx_frames,
+                        float* carry, float* ring, float* rows, float* feats_out, cudaStream_t st) {
+    if (n <= 0) return 0;
+    FO_TRY(upload_twiddles(p.fft_size));
+    const int carry_n = p.frame_len - p.frame_shift, chunk = p.frame_shift * frames_per_chunk;
+    FO_CHECK(frames_per_chunk >= ctx_frames && chunk >= carry_n, "fbank_stream_blocks: chunk shorter than its carry/context");
+    frontend_blocks_kernel<<<dim3(kmax, n), 256, 0, st>>>(ids, cnt, off, pcm, pcm_is_i16, scale, carry_n, chunk, carry, rows);
+    FO_LAUNCHED();
+    FO_CUDA(cudaGetLastError());
+    SampleSrc src{rows, 0, 1.0f, (long long)(carry_n + chunk), nullptr};
+    const long long frames = (long long)blocks * frames_per_chunk;
+    fbank_kernel<<<(int)((frames + FB_WARPS - 1) / FB_WARPS), FB_WARPS * 32, fbank_smem(p.fft_size), st>>>(
+        p, src, blocks, frames_per_chunk, feats_out, nullptr, (long long)(ctx_frames + frames_per_chunk) * p.n_mel, ctx_frames,
+        nullptr, 0, 0);
+    FO_LAUNCHED();
+    FO_CUDA(cudaGetLastError());
+    frontend_blocks_finish_kernel<<<n, 256, 0, st>>>(ids, cnt, off, carry_n, chunk, ctx_frames, frames_per_chunk, p.n_mel, rows,
+                                                     feats_out, carry, ring);
     FO_LAUNCHED();
     FO_CUDA(cudaGetLastError());
     return 0;

@@ -373,6 +373,27 @@ class Engine:
                                            _ptr(adapter_out) if self.has_adapter else None, self._stream()))
         return (enc_out if want_enc else None), (adapter_out if self.has_adapter else None)
 
+    def stream_steps_v(self, ids, chunks, pcm: ArrayLike, scale: Optional[float] = None, want_adapter: Optional[bool] = None,
+                       enc_out: Optional[torch.Tensor] = None, adapter_out: Optional[torch.Tensor] = None):
+        """Recorded audio of any length: session ids[i] takes chunks[i] >= 1 consecutive chunks of PCM in one call, with the
+        results and the session state of chunks[i] stream_step calls.  pcm (B, samples_per_chunk), B = sum(chunks), blocks in
+        (session, chunk) order as in encode_stream_chunks_v.  Returns enc (B, t, D) and adapter (B, t_out, E) in that order."""
+        ids = _ids(ids)
+        n = len(ids)
+        cnt = _ids(chunks)
+        assert len(cnt) == n, "one chunk count per session"
+        B = int(cnt.sum())
+        assert tuple(pcm.shape) == (B, self.cfg.samples_per_chunk), "pcm must be (sum(chunks), samples_per_chunk)"
+        t, t_out = self.out_frames(self.cfg.chunk_feat_frames)
+        want_adapter = self.has_adapter if want_adapter is None else want_adapter
+        enc_out = self._out(enc_out, (B, t, self.cfg.d_model))
+        if want_adapter:
+            adapter_out = self._out(adapter_out, (B, t_out, self.cfg.llm_dim))
+        _lib.check(self.lib.fo_stream_steps_v(self._h, _i32p(ids), _i32p(cnt), n, _ptr(pcm), self._pcm_dtype(pcm),
+                                              self._scale(pcm, scale), _ptr(enc_out),
+                                              _ptr(adapter_out) if want_adapter else None, self._stream()))
+        return enc_out, (adapter_out if want_adapter else None)
+
     def stream_step_async(self, ids, pcm: ArrayLike, adapter_out: torch.Tensor, scale: Optional[float] = None,
                           enc_out: Optional[torch.Tensor] = None) -> int:
         """Pipelined stream_step for pinned HOST buffers: returns a ticket; `adapter_out` (and `enc_out`) are valid after

@@ -89,7 +89,7 @@ typedef struct fo_config {
 } fo_config;
 
 typedef struct fo_stats_t {
-    int64_t stream_steps;      /* fo_encode_stream / fo_encode_stream_chunks / fo_stream_step calls */
+    int64_t stream_steps;      /* fo_encode_stream / fo_encode_stream_chunks[_v] / fo_stream_step[s_v] calls */
     int64_t session_chunks;    /* sum over steps of sessions x chunks advanced */
     int64_t offline_calls;
     int64_t offline_frames;    /* encoder frames produced offline */
@@ -202,6 +202,17 @@ int fo_encode_stream_chunks_v(fo_ctx* ctx, const int32_t* ids, const int32_t* ch
 /* fbank + encode in one call (one captured graph): PCM in, embeddings out */
 int fo_stream_step(fo_ctx* ctx, const int32_t* ids, int n, const void* pcm, int pcm_dtype, float scale,
                    float* enc_out, float* adapter_out, void* stream);
+/* recorded audio of any length: session ids[i] takes chunks[i] >= 1 consecutive chunks of PCM, with the results and the session
+ * state afterwards (KV ring, n_frames, pe_index, adapter caches, Conv1dLinear context, fbank sample carry, feature ring) of
+ * chunks[i] successive fo_stream_step calls.  pcm (B, frame_shift * frames_per_chunk) samples, B = sum(chunks), blocks in
+ * (session, chunk) order as in fo_encode_stream_chunks_v; FO_F32 or FO_I16, value used = sample * scale.  enc_out (B, t, d_model),
+ * adapter_out (B, t_out, llm_dim), same block order; either may be NULL.  No cap on the counts: the call runs in passes of a
+ * bounded number of blocks (option "steps_pass_blocks"), so the device memory it adds does not grow with the recording.
+ * FO_ERR_ARG, with nothing enqueued and no session touched: the geometry rules of every streaming entry, a count < 1, a
+ * duplicate or unallocated id, a MultiLayeredConv1d context, and a call while a hand-off is armed (fo_handoff_arm; the arm
+ * stays for the next step).  Ordered after outstanding fo_stream_step_async steps.  One stream step, sum(chunks) session chunks. */
+int fo_stream_steps_v(fo_ctx* ctx, const int32_t* ids, const int32_t* chunks, int n, const void* pcm, int pcm_dtype,
+                      float scale, float* enc_out, float* adapter_out, void* stream);
 /* pipelined form for HOST buffers (a server loop that already holds the next chunk; the reference runs this loop one chunk
  * and one session at a time, bin/dialog_state_pred.py:793-814 -> models/audioLLM.py:380-387): returns once the step is enqueued.
  * The PCM upload and the read-back of enc_out / adapter_out run on two internal copy streams with double-buffered staging,
@@ -264,6 +275,8 @@ int fo_stats(fo_ctx* ctx, fo_stats_t* out);
  *       transformer layers in ONE cooperative launch (csrc/fo_stack.cu; bf16 contexts, pre-norm linear-FFN layers) instead of
  *       the per-kernel chain; the first such step builds the kernel's row-padded copy of the layer matrices (+ 2 x 12 D^2 bytes
  *       per layer, 604 MB for the shipped model).  0 = always the chain.
+ *   "steps_pass_blocks" 0: blocks (session chunks) per pass of fo_stream_steps_v; 0 = as many as 1 GiB of workspace holds
+ *       (720 blocks of the shipped model in bf16)
  *   "profile_gemm" 0/1, "debug_skip" (timing attribution), "tc_swap"/"tc_bn"/"tc_split" (-1 = cost model): development
  * get-only: "tc_launches", "tc_persist_launches", "stack_launches", "ring_cap", "max_t", "profile_gemm_us", "profile_gemm_count".
  * Development environment variables read once per process: FO_TC_OCC, FO_TC_KB, FO_TC_KBD, FO_TC_SMAX, FO_TC_CAP, FO_TC_SKINNY (tile
