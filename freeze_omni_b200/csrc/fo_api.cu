@@ -218,7 +218,7 @@ struct fo_ctx {
 namespace {
 
 enum { WS_FEATS = 0, WS_C1, WS_C2, WS_XSUB, WS_EMB, WS_X, WS_H, WS_QKV, WS_ATT, WS_FFH, WS_ENC, WS_XIN, WS_ACONV, WS_AH,
-       WS_Y, WS_MASK2, WS_ILENS, WS_ILENS2, WS_AMASK, WS_PCM, WS_TMP0, WS_TMP1, WS_TMP2, WS_TMP3, WS_Q32, WS_HC, WS_PART, WS_PCM2, WS_ENC2, WS_Y2, WS_AC1, WS_XIN2, WS_TMP4, WS_TMP5, WS_HP, WS_FP, WS_ENCJ, WS_PACK, WS_ADJ, WS_SROWS, WS_COUNT };
+       WS_Y, WS_MASK2, WS_ILENS, WS_ILENS2, WS_AMASK, WS_PCM, WS_TMP0, WS_TMP1, WS_TMP2, WS_TMP3, WS_Q32, WS_HC, WS_PART, WS_PCM2, WS_ENC2, WS_Y2, WS_AC1, WS_XIN2, WS_TMP4, WS_TMP5, WS_HP, WS_FP, WS_PACK, WS_SROWS, WS_COUNT };
 
 int dev_alloc(fo_ctx* c, void** p, size_t bytes) {
     *p = nullptr;
@@ -675,18 +675,18 @@ inline int ad_frames(const fo_ctx* c, int T, int n = -1) {
 }
 
 // Where the adapter's projection writes: fp32 rows of y, or fp16 rows of an LLM hand-off buffer (audioLLM.py:404-411), base
-// past the prefix.  The rows of a pass are (session, kk chunks, t_out frames); row r of chunk jj of session b goes to row r of
-// output block b * k + jj, blocks `pitch` rows apart.  A pass into y with kk == k is plain row-major.
+// past the prefix.  The rows are (session, k chunks, t_out frames); row r of chunk j of session b goes to row r of output
+// block b * k + j, blocks `pitch` rows apart.  Into y they are plain row-major.
 struct AdOut {
     float* y = nullptr;
     void* h16 = nullptr;      // instead of y
     long long pitch = 0;      // rows per output block
-    int k = 1, kk = 1;
+    int k = 1;
 };
 
 // RowMap of the projection onto o's blocks, t_out rows per chunk
 inline void chunk_rowmap(const AdOut& o, int t_out, RowMap* rm) {
-    rm->p1 = o.kk * t_out; rm->p0 = t_out; rm->v1 = o.kk; rm->v0 = t_out; rm->q1 = (int)(o.k * o.pitch); rm->q0 = (int)o.pitch;
+    rm->p1 = o.k * t_out; rm->p0 = t_out; rm->v1 = o.k; rm->v0 = t_out; rm->q1 = (int)(o.k * o.pitch); rm->q0 = (int)o.pitch;
 }
 
 // ---- adapter program on device buffers -----------------------------------------------------------
@@ -695,25 +695,23 @@ inline void chunk_rowmap(const AdOut& o, int t_out, RowMap* rm) {
 // GEMM into fp32; the last conv's rows are normalised and projected.  LinearAdapter projects the encoder rows as they are
 // (the reference does not even apply the pad mask).  Left context: the slot caches of ids_dev when the adapter carries them,
 // else per stage cache_in[i] (reference layout (B, C, k-1); null = zeros), the new one to cache_out[i] if given.
-// mix (carried caches, sessions with different chunk counts, even t): enc holds the call's blocks packed, session b's
+// mix (carried caches, chunks of sessions with different counts or odd t): enc holds the call's blocks packed, session b's
 // cnt[b] chunks of `unit` frames from block off[b].  The convolutions run over B sessions x T = kmax * unit rows, padded at
 // the end of each session's run (the conv is causal, so the real rows' outputs are those of the sequential calls); the
-// real output rows are packed to (block, frame) order before the norm and the projection.  pass >= 0 (odd t, chunk pass
-// `pass`): B sessions x T rows as without mix, but sessions with cnt[b] <= pass keep their caches.  pick (odd t, passes of
-// fo_stream_steps_v): the grid as for even t, every conv at stride 1, then the rows of the stride-2 outputs picked per chunk.
+// real output rows are packed to (block, frame) order before the norm and the projection.  pick (odd t): every conv at
+// stride 1, then the rows of the stride-2 outputs picked per chunk.
 struct AdMix {
     const int32_t* cnt;
     const int32_t* off;
     int kmax, unit, blocks;
-    int pass = -1;
-    bool pick = false;
+    bool pick;
 };
 template <typename TA>
 int adapter_program(fo_ctx* c, const float* enc, const uint8_t* mask, int B, int T, const int32_t* ids_dev,
                     const float* const* cache_in, float* const* cache_out, const AdOut& out, cudaStream_t st,
                     const AdMix* mix = nullptr) {
     const int D = c->D, E = c->E, KA = c->KA, ns = c->ad_nst;
-    const bool grid = mix && mix->pass < 0;                                    // per-session padded grid
+    const bool grid = mix != nullptr;                                          // per-session padded grid
     const int t_out = grid ? ad_frames(c, mix->unit) : ad_frames(c, T);       // grid: frames out of one chunk
     const int M = grid ? mix->blocks * t_out : B * t_out;
     const bool run_gemm = !(c->debug_skip & 16);
@@ -731,13 +729,10 @@ int adapter_program(fo_ctx* c, const float* enc, const uint8_t* mask, int B, int
         FO_TRY(ws_ensure(c, i == 0 ? WS_XIN : WS_XIN2, (size_t)ga.planes * ga.rows * s.cin * sizeof(TA), &xin));
         FO_TRY(ws_ensure(c, i + 1 == ns ? WS_ACONV : WS_AC1, (size_t)B * (pick ? T : ad_frames(c, T, i + 1)) * s.cout * sizeof(float), &conv));
         SessionRows sr;
-        if (mix) {
+        if (grid) {
             sr.cnt = mix->cnt;
-            sr.pass = mix->pass;
-            if (grid) {
-                sr.off = i == 0 ? mix->off : nullptr;      // the first conv reads the packed encoder rows
-                sr.unit = pick ? mix->unit : ad_frames(c, mix->unit, i);
-            }
+            sr.off = i == 0 ? mix->off : nullptr;          // the first conv reads the packed encoder rows
+            sr.unit = pick ? mix->unit : ad_frames(c, mix->unit, i);
         }
         FO_TRY(conv_stage<TA>(x, i == 0 ? mask : nullptr, B, Ti, s.cin, KA - 1, stride, s.in_scale, s.in_shift,
                               c->ad_carry ? ids_dev : nullptr, s.cache, c->ad_valid, cache_in ? cache_in[i] : nullptr,
@@ -752,10 +747,10 @@ int adapter_program(fo_ctx* c, const float* enc, const uint8_t* mask, int B, int
     const int K = ns > 0 ? c->ad_st[ns - 1].cout : D;
     if (grid && ns > 0) {
         void* pk;
-        const long long blk = (long long)t_out * K * sizeof(float);
         FO_TRY(ws_ensure(c, WS_PACK, (size_t)M * K * sizeof(float), &pk));
         if (pick) FO_TRY(pick_chunk_rows(x, B, mix->kmax, mix->unit, t_out, K, mix->cnt, mix->off, reinterpret_cast<float*>(pk), st));
-        else FO_TRY(session_blocks(x, blk, pk, blk, blk, B, mix->kmax, 0, BLOCKS_PACK, mix->cnt, mix->off, st));
+        else FO_TRY(pack_session_blocks(x, reinterpret_cast<float*>(pk), (long long)t_out * K * sizeof(float), B, mix->kmax, mix->cnt,
+                                        mix->off, st));
         x = reinterpret_cast<const float*>(pk);
     }
     const TA* a = reinterpret_cast<const TA*>(enc);
@@ -770,7 +765,7 @@ int adapter_program(fo_ctx* c, const float* enc, const uint8_t* mask, int B, int
     e.bias = c->ad_proj_b;
     e.ldc = E;
     RowMap rm;
-    if (out.h16 || out.kk != out.k) chunk_rowmap(out, grid ? t_out : t_out / out.kk, &rm);
+    if (out.h16) chunk_rowmap(out, grid ? t_out : t_out / out.k, &rm);
     if (out.h16) e.c_act = reinterpret_cast<TA*>(out.h16);     // straight from the epilogue: no fp32 copy, no .half()
     else e.c_f32 = out.y;
     if (run_gemm) FO_TRY(gemm<TA>(c, a, plain_rows(K, M), c->ad_proj_w, M, E, K, e, rm, st));
@@ -1080,7 +1075,7 @@ int stack_program(fo_ctx* c, int n, int t, float* x, void* qkv, float* q32, void
 struct Mix {
     int blocks = 0, kmax = 1, n1 = 0;
     const int32_t* off = nullptr;
-    int group = 0;               // > 0: a pass of fo_stream_steps_v (attention_steps, `group` chunks per CTA; counts uncapped)
+    int group = 0;               // > 0: a pass of fo_stream_steps_v (`group` chunks per attention CTA; counts uncapped)
     bool uniform(int n) const { return blocks == n * kmax; }
     int block(int i) const { return off ? off[i] : i * kmax; }
 };
@@ -1093,48 +1088,18 @@ int adapter_chunks(fo_ctx* c, const float* enc, int n, const Mix& m, int t, AdOu
     // independent blocks of t frames
     if (!c->ad_carry) return adapter_program<TA>(c, enc, nullptr, m.blocks, t, c->ids_dev, nullptr, nullptr, out, st);
     const int k = m.kmax;
-    if (t % 2 == 0) {
+    if (t % 2 == 0 && m.uniform(n)) {
         // CNNSubsampling with even t: every chunk brings an even number of frames to the stride-2 conv, so one pass over a
         // session's k*t frames with the carried cache gives the k sequential outputs and leaves the same cache
-        if (m.uniform(n)) {
-            out.k = out.kk = k;
-            return adapter_program<TA>(c, enc, nullptr, n, k * t, c->ids_dev, nullptr, nullptr, out, st);
-        }
-        // different counts: the same pass over a per-session grid of kmax*t rows, each session's padding at its end
-        const AdMix mix{c->cnt_dev, c->off_dev, k, t, m.blocks};
-        return adapter_program<TA>(c, enc, nullptr, n, k * t, c->ids_dev, nullptr, nullptr, out, st, &mix);
+        out.k = k;
+        return adapter_program<TA>(c, enc, nullptr, n, k * t, c->ids_dev, nullptr, nullptr, out, st);
     }
-    if (m.group) {
-        // odd t in a pass of fo_stream_steps_v: in the session's continuous stream S = [cache | x_0 | x_1 ..], output m of
-        // chunk j is the conv at S position j * t + 2 m, so stride-1 convs over the grid and a row pick give every chunk at once
-        AdMix mix{c->cnt_dev, c->off_dev, k, t, m.blocks};
-        mix.pick = true;
-        return adapter_program<TA>(c, enc, nullptr, n, k * t, c->ids_dev, nullptr, nullptr, out, st, &mix);
-    }
-    // odd t: the output phase of the stride-2 conv shifts between chunks (a joint pass yields other frames, and fewer), so
-    // the chunks run one by one, flipping the live half of the double-buffered cache in between as a session advance does.
-    // Pass j covers the sessions with more than j chunks (the others keep their cache and its flag); its rows are gathered
-    // from blocks off[b] + j and its output rows scattered back to them.
-    const int t_out = ad_frames(c, t);
-    const size_t row = (size_t)t * c->D * sizeof(float);
-    const size_t esz = out.h16 ? sizeof(TA) : sizeof(float);
-    const long long blk = (long long)t_out * c->E * esz;
-    void *ej, *yj;
-    FO_TRY(ws_ensure(c, WS_ENCJ, (size_t)n * row, &ej));
-    FO_TRY(ws_ensure(c, WS_ADJ, (size_t)n * blk, &yj));
-    AdOut oj;
-    oj.pitch = t_out;
-    if (out.h16) oj.h16 = yj;
-    else oj.y = reinterpret_cast<float*>(yj);
-    void* dst = out.h16 ? out.h16 : (void*)out.y;
-    for (int j = 0; j < k; ++j) {
-        FO_TRY(session_blocks(enc, (long long)row, ej, (long long)row, (long long)row, n, k, j, BLOCKS_GATHER, c->cnt_dev, c->off_dev, st));
-        const AdMix pass{c->cnt_dev, nullptr, k, t, 0, j};
-        FO_TRY(adapter_program<TA>(c, reinterpret_cast<const float*>(ej), nullptr, n, t, c->ids_dev, nullptr, nullptr, oj, st, &pass));
-        FO_TRY(session_blocks(yj, blk, dst, out.pitch * c->E * (long long)esz, blk, n, k, j, BLOCKS_SCATTER, c->cnt_dev, c->off_dev, st));
-        if (j + 1 < k) FO_TRY(advance_sessions(c->ids_dev, n, 0, 0, 1, nullptr, nullptr, c->ad_valid, st, 1, c->cnt_dev, j + 2));
-    }
-    return 0;
+    // The same pass over a per-session grid of kmax*t rows, each session's padding at its end.  With odd t the output phase of
+    // the stride-2 conv shifts between chunks (a joint stride-2 pass yields other frames, and fewer), but in the session's
+    // continuous stream S = [cache | x_0 | x_1 ..] output m of chunk j is the conv at S position j * t + 2 m: stride-1 convs over
+    // the grid and a row pick give every chunk at once.
+    const AdMix mix{c->cnt_dev, c->off_dev, k, t, m.blocks, t % 2 != 0};
+    return adapter_program<TA>(c, enc, nullptr, n, k * t, c->ids_dev, nullptr, nullptr, out, st, &mix);
 }
 
 // Session groups of a streaming step of n sessions (see stream_program)
@@ -1205,7 +1170,6 @@ int stream_program(fo_ctx* c, int n, const Mix& m, const float* feats, int t_in,
             a.n = ng; a.t = t; a.H = H; a.ring_cap = c->ring_cap; a.window = c->window; a.full_chunk = c->full_chunk;
             a.pe_wrap = c->pe_wrap; a.pos_rows = c->pos_rows;
             a.ring_slot_stride = 2LL * H * c->ring_cap * 64;
-            a.chunks = m.kmax;
             a.chunk_size = c->cfg.chunk_size;
             a.cnt = c->cnt_dev + s0;
             a.off = c->off_dev + s0;
@@ -1240,15 +1204,12 @@ int stream_program(fo_ctx* c, int n, const Mix& m, const float* feats, int t_in,
             }
             TA* ring_l = reinterpret_cast<TA*>(c->ring) + l * layer_stride;
             const int n1g = std::min(std::max(m.n1 - s0, 0), ng);  // the group's share of the leading one-chunk run
-            if (r == 0 && !(c->debug_skip & 1) && m.group) {
-                AttnStream as = a;
-                as.chunks = m.group;
-                r = attention_steps<TA>(as, (m.kmax + m.group - 1) / m.group, qkvg, q32g, ring_l, reinterpret_cast<const TA*>(w.ptab_h),
-                                        w.pos_u, w.pos_v, attg, sg);
-            } else if (r == 0 && !(c->debug_skip & 1) && n1g < ng) {
-                // multi-chunk sessions (rows from the end of the one-chunk run): on a forked stream when both kernels run
+            if (r == 0 && !(c->debug_skip & 1) && n1g < ng) {
+                // multi-chunk sessions (rows from the end of the one-chunk run): on a forked stream when both kernels run.  A pass
+                // of fo_stream_steps_v (n1 = 0, never forked) spreads a session's chunks over groups of m.group per CTA.
                 AttnStream am = a;
                 am.ids += n1g; am.cnt += n1g; am.off += n1g; am.n = ng - n1g;
+                am.chunks = m.group ? m.group : m.kmax;
                 const long long ro = (long long)n1g * t;
                 const bool fork = n1g > 0;
                 cudaStream_t sm = fork ? c->mix_stream[g] : sg;
@@ -1256,21 +1217,19 @@ int stream_program(fo_ctx* c, int n, const Mix& m, const float* feats, int t_in,
                     FO_CUDA(cudaEventRecord(c->ev_mix_fork[g], sg));
                     FO_CUDA(cudaStreamWaitEvent(sm, c->ev_mix_fork[g], 0));
                 }
-                r = attention_stream<TA>(am, qkvg + ro * 3 * D, q32g + ro * 3 * D, ring_l, reinterpret_cast<const TA*>(w.ptab_h),
-                                         w.pos_u, w.pos_v, attg + ro * D, sm);
+                r = attention_chunks<TA>(am, cdiv(m.kmax, am.chunks), qkvg + ro * 3 * D, q32g + ro * 3 * D, ring_l,
+                                         reinterpret_cast<const TA*>(w.ptab_h), w.pos_u, w.pos_v, attg + ro * D, sm);
                 if (r == 0 && n1g > 0) {
                     AttnStream a1 = a;
-                    a1.n = n1g; a1.chunks = 1;
+                    a1.n = n1g;
                     r = attention_stream<TA>(a1, qkvg, q32g, ring_l, reinterpret_cast<const TA*>(w.ptab_h), w.pos_u, w.pos_v, attg, sg);
                 }
                 if (fork) {
                     FO_CUDA(cudaEventRecord(c->ev_mix_join[g], sm));
                     FO_CUDA(cudaStreamWaitEvent(sg, c->ev_mix_join[g], 0));
                 }
-            } else if (r == 0 && !(c->debug_skip & 1)) {
-                AttnStream a1 = a;
-                a1.chunks = 1;                                  // every session of the group brings one chunk
-                r = attention_stream<TA>(a1, qkvg, q32g, ring_l, reinterpret_cast<const TA*>(w.ptab_h), w.pos_u, w.pos_v, attg, sg);
+            } else if (r == 0 && !(c->debug_skip & 1)) {        // every session of the group brings one chunk
+                r = attention_stream<TA>(a, qkvg, q32g, ring_l, reinterpret_cast<const TA*>(w.ptab_h), w.pos_u, w.pos_v, attg, sg);
             }
             NextNorm nn{last ? c->after_g : c->layers[l + 1].ln1g, last ? c->after_b : c->layers[l + 1].ln1b,
                         last ? enc_out_dev + r0 * D : nullptr};
@@ -2431,7 +2390,7 @@ int fo_stream_step(fo_ctx* c, const int32_t* ids, int n, const void* pcm, int pc
 // fo_stream_steps_v runs in passes of at most P blocks (option "steps_pass_blocks", else STEPS_PASS_BYTES over the workspace
 // bytes of one block): each pass gives every session that still has chunks its next min(remaining, q) chunks, q = the
 // longest remaining count spread evenly over the passes that max(1, P / sessions left) chunks per pass would take; it then
-// runs the fbank of those blocks (fbank_stream_blocks) and the streaming program with the pass attention (attention_steps).  Every workspace is sized by the pass, so the device memory a call adds does not grow with the recording.
+// runs the fbank of those blocks (fbank_stream_blocks) and the streaming program, whose attention spreads a session's chunks over groups of CTAs (Mix::group).  Every workspace is sized by the pass, so the device memory a call adds does not grow with the recording.
 // Passes run eagerly: a captured graph per pass shape would multiply with recording lengths.
 constexpr long long STEPS_PASS_BYTES = 1LL << 30;
 

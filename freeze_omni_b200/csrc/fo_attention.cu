@@ -1,7 +1,7 @@
 // Chunk attention with key-position rel-pos bias (reference: MultiHeadedAttention.infer / .forward,
 // models/encoder/attention.py:407-459 / 350-405; no rel_shift, SURVEY 2.4-3):
 //     score[i][j] = ((q_i + u) . K_j + (q_i + v) . P[pos_j]) / sqrt(d_k),   softmax over j,   out = sum_j p_ij V_j
-// d_k is 64.  Streaming: one CTA per (session, head); the cached K/V rows come from the session's ring in
+// d_k is 64.  Streaming: one CTA per (session, head[, group of chunks]); the cached K/V rows come from the session's ring in
 // HBM with cp.async.bulk (TMA bulk copy, mbarrier completion) while the chunk's own rows arrive from the
 // fused QKV GEMM output and are appended to the ring.  The four streaming kernels (one chunk or several, fp16 or fp32)
 // differ in how they stage the rows; the per-chunk math is attn_chunk_mma / attn_chunk_ffma (fo_attn_core.cuh).
@@ -296,24 +296,37 @@ attention_stream_mma_kernel(AttnStream a, const __half* __restrict__ qkv, const 
 }
 
 // ---------------------------------------------------------------------------------------------
-// Several consecutive chunks of every session in one call (fo_encode_stream_chunks[_v]): session b brings k = cnt[b] chunks
-// from row row0 = (off[b] - off[0]) * t.  One CTA per (session, head) stages the keys once -- the ring window of frames
-// [first, nf) (first = nf - min(nf, window)) by bulk copy, then the session's own k*t rows -- and walks the k query chunks
-// in order.  Shared memory is sized by the largest count of the call (AttnStream::chunks).  Chunk j sees exactly what the j-th
+// Several consecutive chunks of every session in one call (fo_encode_stream_chunks[_v], passes of fo_stream_steps_v): session b
+// brings k = cnt[b] chunks from row row0 = (off[b] - off[0]) * t.  CTA (b, h, z) takes chunks [j0, j1) = [z * G, min(k, (z + 1)
+// * G)), G = a.chunks, and stages the keys of all of them once: frames [first, nf + j1 * t) with first = nf_j0 - min(nf_j0,
+// window) -- those before the call (frame < nf) from the ring by bulk copy, the rest from the call's own K|V rows (qkv row =
+// frame - nf) -- then walks its query chunks in order.  Shared memory is sized by G.  Chunk j sees exactly what the j-th
 // sequential single-chunk call would see:
 //     nf_j = nf + j*t,  keys = frames [nf_j - min(nf_j, window), nf_j + t)   (a contiguous run of the staged rows)
-//     pe_j = pe_index stepped j times by pe = pe % wrap + chunk_size,  rel-pos rows P[max(0, pe_j % wrap - full_chunk) + m]
+//     pe_j = pe_after(pe_index, j),  rel-pos rows P[max(0, pe_j % wrap - full_chunk) + m]
 // The rel-pos window moves (and may wrap) with pe_j, so it is re-staged per chunk.  The new rows go to the ring only after
-// the staged copy of the old window has landed: the ring holds window + max_t rows, fewer than the call's keys, so a later
-// chunk's rows would overwrite frames an earlier chunk still needs.  Layouts (fp16 chunk swizzle of K/V by frame and of P
-// by position, q swizzled by query row) are those of the single-chunk kernels.
-__device__ __forceinline__ int chunk_pe(int pe, int j, const AttnStream& a) {
-    for (int i = 0; i < j; ++i) pe = pe % a.pe_wrap + a.chunk_size;
-    return pe % a.pe_wrap;
+// every read of the old window: the ring holds window + max_t rows, fewer than the call's keys, so a later chunk's rows would
+// overwrite frames an earlier chunk still needs.  With one group per session (gridDim.z == 1) the CTA is the only reader of
+// its (slot, head) ring and appends them itself once its window copy has landed; with several, chunks_append_ring_kernel
+// appends them after the grid.  Layouts (fp16 chunk swizzle of K/V by frame and of P by position, q swizzled by query row)
+// are those of the single-chunk kernels.
+struct StepsGroup {
+    int j0, j1, nf, first, cr, kn;      // chunks; frames before the call; first staged frame; staged rows from ring / from qkv
+};
+__device__ __forceinline__ bool steps_group(const AttnStream& a, int b, StepsGroup* g) {
+    g->j0 = blockIdx.z * a.chunks;
+    const int k = a.cnt[b];
+    if (g->j0 >= k) return false;
+    g->j1 = min(k, g->j0 + a.chunks);
+    g->nf = a.n_frames[a.ids[b]];
+    const int nf0 = g->nf + g->j0 * a.t;
+    g->first = nf0 - min(nf0, a.window);
+    g->cr = max(0, g->nf - g->first);
+    g->kn = g->nf + g->j1 * a.t - (g->first + g->cr);
+    return true;
 }
 
-// stage the session's new K/V rows (qkv row r -> smem row cl + r, frame nf + r) and, once the ring window has landed, append them to the
-// ring (only the last `cap` of them when the call brings more frames than the ring holds)
+// stage the new K/V rows (qkv row r -> smem row cl + r, frame nf + r)
 template <typename TA, int NCH, bool SWZ>
 __device__ __forceinline__ void chunks_stage_new(const AttnStream& a, const TA* qkv, TA* Ks, TA* Vs, int h, int nf, int cl,
                                                  int kt) {
@@ -326,6 +339,8 @@ __device__ __forceinline__ void chunks_stage_new(const AttnStream& a, const TA* 
             *reinterpret_cast<const uint4*>(qkv + (long long)r * 3 * D + (which + 1) * D + h * DK + c * EPC);
     }
 }
+// append the staged new rows (smem row cl + r = frame nf + r) to the ring: only the last `cap` of them when the call brings
+// more frames than the ring holds
 template <typename TA, int NCH>
 __device__ __forceinline__ void chunks_append_ring(const AttnStream& a, const TA* Ks, const TA* Vs, TA* ringK, TA* ringV, int nf,
                                                    int cl, int kt) {
@@ -338,8 +353,8 @@ __device__ __forceinline__ void chunks_append_ring(const AttnStream& a, const TA
     }
 }
 
-// Multi-chunk streaming attention of fp32 contexts.  Staging: the ring window and the call's k*t new rows once, the ring
-// append after the window has landed, the rel-pos rows and Q of every chunk re-staged before its core (attn_chunk_ffma).
+// Multi-chunk streaming attention of fp32 contexts.  The rel-pos rows and Q of every chunk are re-staged before its core
+// (attn_chunk_ffma).
 __global__ void __launch_bounds__(ATT_THREADS)
 attention_chunks_kernel(AttnStream a, const float* __restrict__ qkv, const float* __restrict__ q32, float* __restrict__ ring,
                         const float* __restrict__ ptab_h, const float* __restrict__ pos_u, const float* __restrict__ pos_v,
@@ -359,31 +374,31 @@ attention_chunks_kernel(AttnStream a, const float* __restrict__ qkv, const float
     __shared__ __align__(8) uint64_t bar;
 
     const int b = blockIdx.x, h = blockIdx.y;
+    StepsGroup g;
+    if (!steps_group(a, b, &g)) return;
     const int slot = a.ids[b];
-    const int k = a.cnt[b], kt = k * t;
     const long long row0 = (long long)(a.off[b] - a.off[0]) * t;     // the session's rows: the pointers start there
     qkv += row0 * 3 * D; q32 += row0 * 3 * D; out += row0 * D;
-    const int nf = a.n_frames[slot];
-    const int cl = min(nf, a.window), first = nf - cl;
     float* ringK = ring + (long long)slot * a.ring_slot_stride + (long long)h * cap * DK;
     float* ringV = ringK + (long long)a.H * cap * DK;
     const int tid = threadIdx.x;
     if (tid == 0) {
         mbar_init(&bar, 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        ring_window_copy<float>(ringK, ringV, cap, first, cl, Ks, Vs, nullptr, nullptr, 0, &bar);
+        ring_window_copy<float>(ringK, ringV, cap, g.first, g.cr, Ks, Vs, nullptr, nullptr, 0, &bar);
     }
-    chunks_stage_new<float, NCH, false>(a, qkv, Ks, Vs, h, nf, cl, kt);
+    const int fs = g.first + g.cr;
+    chunks_stage_new<float, NCH, false>(a, qkv + (long long)(fs - g.nf) * 3 * D, Ks, Vs, h, fs, g.cr, g.kn);
     __syncthreads();
     mbar_wait(&bar, 0);
-    chunks_append_ring<float, NCH>(a, Ks, Vs, ringK, ringV, nf, cl, kt);
+    if (gridDim.z == 1) chunks_append_ring<float, NCH>(a, Ks, Vs, ringK, ringV, g.nf, g.cr, g.kn);
 
     const int pe0 = a.pe_index[slot];
-    for (int j = 0; j < k; ++j) {
-        const int nfj = nf + j * t, clj = min(nfj, a.window);
-        const int o = nfj - clj - first;            // staged row of this chunk's first key
+    for (int j = g.j0; j < g.j1; ++j) {
+        const int nfj = g.nf + j * t, clj = min(nfj, a.window);
+        const int o = nfj - clj - g.first;          // staged row of this chunk's first key
         const int nk = clj + t;
-        const int start = max(0, chunk_pe(pe0, j, a) - a.full_chunk);
+        const int start = max(0, pe_after(pe0, j, a.chunk_size, a.pe_wrap) % a.pe_wrap - a.full_chunk);
         for (int i = tid; i < nk * NCH; i += ATT_THREADS) {        // the min() keeps reads in bounds; pos_rows covers every reachable position
             const int r = i / NCH, c = i % NCH, pos = min(start + r, a.pos_rows - 1);
             *reinterpret_cast<uint4*>(Ps + r * DK + c * EPC) = *reinterpret_cast<const uint4*>(ptab_h + ((long long)h * a.pos_rows + pos) * DK + c * EPC);
@@ -425,172 +440,14 @@ attention_chunks_mma_kernel(AttnStream a, const __half* __restrict__ qkv, const 
     __shared__ __align__(8) uint64_t bar;
 
     const int b = blockIdx.x, h = blockIdx.y;
+    StepsGroup g;
+    if (!steps_group(a, b, &g)) return;
     const int slot = a.ids[b];
-    const int k = a.cnt[b], kt = k * t;
     const long long row0 = (long long)(a.off[b] - a.off[0]) * t;     // the session's rows: the pointers start there
     qkv += row0 * 3 * D; q32 += row0 * 3 * D; out += row0 * D;
-    const int nf = a.n_frames[slot];
-    const int cl = min(nf, a.window), first = nf - cl;
-    const int nk_all = cl + kt;
+    const int nk_all = g.cr + g.kn;
     TA* ringK = ring + (long long)slot * a.ring_slot_stride + (long long)h * cap * DK;
     TA* ringV = ringK + (long long)a.H * cap * DK;
-    const int tid = threadIdx.x;
-    if (tid == 0) {
-        mbar_init(&bar, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        ring_window_copy<TA>(ringK, ringV, cap, first, cl, Ks, Vs, nullptr, nullptr, 0, &bar);
-    }
-    chunks_stage_new<TA, NCH, true>(a, qkv, Ks, Vs, h, nf, cl, kt);
-    // rows behind the last key: K is masked there, V enters the PV MMAs with probability 0 and must be finite
-    for (int i = tid; i < (krows - nk_all) * NCH; i += ATT_THREADS) {
-        *reinterpret_cast<uint4*>(Ks + (nk_all + i / NCH) * DK + (i % NCH) * EPC) = make_uint4(0, 0, 0, 0);
-        *reinterpret_cast<uint4*>(Vs + (nk_all + i / NCH) * DK + (i % NCH) * EPC) = make_uint4(0, 0, 0, 0);
-    }
-    __syncthreads();
-    mbar_wait(&bar, 0);
-    chunks_append_ring<TA, NCH>(a, Ks, Vs, ringK, ringV, nf, cl, kt);
-
-    const int pe0 = a.pe_index[slot];
-    for (int j = 0; j < k; ++j) {
-        const int nfj = nf + j * t, clj = min(nfj, a.window);
-        const int o = nfj - clj - first;            // staged row of this chunk's first key
-        const int nk = clj + t;
-        const int start = max(0, chunk_pe(pe0, j, a) - a.full_chunk);
-        for (int i = tid; i < nk * NCH; i += ATT_THREADS) {        // row r = position start + r, swizzled by that position
-            const int r = i / NCH, cc = i % NCH, pos = min(start + r, a.pos_rows - 1);
-            *reinterpret_cast<uint4*>(Ps + r * DK + ((cc ^ ((start + r) & 7)) * EPC)) =
-                *reinterpret_cast<const uint4*>(ptab_h + ((long long)h * a.pos_rows + pos) * DK + ((cc ^ (pos & 7)) * EPC));
-        }
-        for (int i = tid; i < t * DK; i += ATT_THREADS) {
-            const int r = i / DK, d = i % DK;
-            const float q = q32[(long long)(j * t + r) * 3 * D + h * DK + d];
-            const int sw = r * DK + (((d >> 3) ^ (r & 7)) << 3) + (d & 7);
-            quh[sw] = from_f<TA>(q + pos_u[h * DK + d]);
-            qvh[sw] = from_f<TA>(q + pos_v[h * DK + d]);
-        }
-        __syncthreads();
-        attn_chunk_mma<ATT_THREADS / 32>(Ks + o * DK, Vs + o * DK, first + o, Ps, start, quh, qvh, ph, sc, vrows, nk, t,
-                                         out + (long long)(j * t) * D + h * DK, D);
-        __syncthreads();                              // Ps / quh / ph / sc are restaged by the next chunk
-    }
-}
-
-// ---------------------------------------------------------------------------------------------
-// Passes of fo_stream_steps_v: a session brings any number of chunks.  CTA (b, h, z) takes chunks [j0, j1) = [z * G,
-// min(cnt[b], (z + 1) * G)) of session b, G = a.chunks, and stages the keys of all of them once: frames [first, nf + j1 * t)
-// with first = nf_j0 - min(nf_j0, window) -- those before the pass (frame < nf) from the ring, the rest from the pass's own
-// K|V rows (qkv row = frame - nf).  Chunk j is then attended as the multi-chunk kernels attend it (window + t keys at most);
-// its rel-pos start uses chunk_pe in closed form, (pe % wrap + j * chunk_size) % wrap, since j may run into the thousands.
-// The ring is only read here: steps_append_ring_kernel writes the new frames after the whole grid has read it.
-struct StepsGroup {
-    int j0, j1, nf, first, cr, kn;      // chunks; frames before the pass; first staged frame; staged rows from ring / from qkv
-};
-__device__ __forceinline__ bool steps_group(const AttnStream& a, int b, StepsGroup* g) {
-    g->j0 = blockIdx.z * a.chunks;
-    const int k = a.cnt[b];
-    if (g->j0 >= k) return false;
-    g->j1 = min(k, g->j0 + a.chunks);
-    g->nf = a.n_frames[a.ids[b]];
-    const int nf0 = g->nf + g->j0 * a.t;
-    g->first = nf0 - min(nf0, a.window);
-    g->cr = max(0, g->nf - g->first);
-    g->kn = g->nf + g->j1 * a.t - (g->first + g->cr);
-    return true;
-}
-__device__ __forceinline__ int steps_start(const AttnStream& a, int pe0, int j) {
-    return max(0, (int)(((long long)(pe0 % a.pe_wrap) + (long long)j * a.chunk_size) % a.pe_wrap) - a.full_chunk);
-}
-
-__global__ void __launch_bounds__(ATT_THREADS)
-attention_steps_kernel(AttnStream a, const float* __restrict__ qkv, const float* __restrict__ q32, const float* __restrict__ ring,
-                       const float* __restrict__ ptab_h, const float* __restrict__ pos_u, const float* __restrict__ pos_v,
-                       float* __restrict__ out) {
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    constexpr int EPC = 4, NCH = DK / EPC;
-    FO_PDL_TRIGGER();
-    FO_PDL_WAIT();
-    const int cap = a.ring_cap, t = a.t, D = a.H * DK;
-    const int rows = a.window + a.chunks * t, prow = a.window + t;
-    float* Ks = reinterpret_cast<float*>(smem_raw);
-    float* Vs = Ks + rows * DK;
-    float* Ps = Vs + rows * DK;
-    float* qu = Ps + prow * DK;
-    float* qv = qu + t * DK;
-    float* prob = qv + t * DK;                      // t x prow
-    __shared__ __align__(8) uint64_t bar;
-
-    const int b = blockIdx.x, h = blockIdx.y;
-    StepsGroup g;
-    if (!steps_group(a, b, &g)) return;
-    const int slot = a.ids[b];
-    const long long row0 = (long long)(a.off[b] - a.off[0]) * t;
-    qkv += row0 * 3 * D; q32 += row0 * 3 * D; out += row0 * D;
-    const float* ringK = ring + (long long)slot * a.ring_slot_stride + (long long)h * cap * DK;
-    const float* ringV = ringK + (long long)a.H * cap * DK;
-    const int tid = threadIdx.x;
-    if (tid == 0) {
-        mbar_init(&bar, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        ring_window_copy<float>(ringK, ringV, cap, g.first, g.cr, Ks, Vs, nullptr, nullptr, 0, &bar);
-    }
-    const int fs = g.first + g.cr;
-    chunks_stage_new<float, NCH, false>(a, qkv + (long long)(fs - g.nf) * 3 * D, Ks, Vs, h, fs, g.cr, g.kn);
-    __syncthreads();
-    mbar_wait(&bar, 0);
-
-    const int pe0 = a.pe_index[slot];
-    for (int j = g.j0; j < g.j1; ++j) {
-        const int nfj = g.nf + j * t, clj = min(nfj, a.window);
-        const int o = nfj - clj - g.first;
-        const int nk = clj + t;
-        const int start = steps_start(a, pe0, j);
-        for (int i = tid; i < nk * NCH; i += ATT_THREADS) {
-            const int r = i / NCH, c = i % NCH, pos = min(start + r, a.pos_rows - 1);
-            *reinterpret_cast<uint4*>(Ps + r * DK + c * EPC) = *reinterpret_cast<const uint4*>(ptab_h + ((long long)h * a.pos_rows + pos) * DK + c * EPC);
-        }
-        for (int i = tid; i < t * DK; i += ATT_THREADS) {
-            const int r = i / DK, d = i % DK;
-            const float q = q32[(long long)(j * t + r) * 3 * D + h * DK + d];
-            qu[i] = q + pos_u[h * DK + d];
-            qv[i] = q + pos_v[h * DK + d];
-        }
-        __syncthreads();
-        attn_chunk_ffma(Ks + o * DK, Vs + o * DK, Ps, qu, qv, prob, prow, nk, t, out + (long long)(j * t) * D + h * DK, D);
-        __syncthreads();
-    }
-}
-
-__global__ void __launch_bounds__(ATT_THREADS)
-attention_steps_mma_kernel(AttnStream a, const __half* __restrict__ qkv, const float* __restrict__ q32, const __half* __restrict__ ring,
-                           const __half* __restrict__ ptab_h, const float* __restrict__ pos_u, const float* __restrict__ pos_v,
-                           __half* __restrict__ out) {
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    typedef __half TA;
-    constexpr int EPC = 8, NCH = 8;
-    FO_PDL_TRIGGER();
-    FO_PDL_WAIT();
-    const int cap = a.ring_cap, t = a.t, D = a.H * DK;
-    const int rows = a.window + a.chunks * t;
-    const int krows = ((rows + 15) & ~15) + 16;     // a chunk's last key tile may read up to 15 rows past the staged keys
-    const int vrows = (a.window + t + 15) & ~15;
-    TA* Ks = reinterpret_cast<TA*>(smem_raw);
-    TA* Vs = Ks + krows * DK;
-    TA* Ps = Vs + krows * DK;
-    TA* quh = Ps + vrows * DK;
-    TA* qvh = quh + t * DK;
-    TA* ph = qvh + t * DK;
-    float* sc = reinterpret_cast<float*>(ph + t * vrows);
-    __shared__ __align__(8) uint64_t bar;
-
-    const int b = blockIdx.x, h = blockIdx.y;
-    StepsGroup g;
-    if (!steps_group(a, b, &g)) return;
-    const int slot = a.ids[b];
-    const long long row0 = (long long)(a.off[b] - a.off[0]) * t;
-    qkv += row0 * 3 * D; q32 += row0 * 3 * D; out += row0 * D;
-    const int nk_all = g.cr + g.kn;
-    const TA* ringK = ring + (long long)slot * a.ring_slot_stride + (long long)h * cap * DK;
-    const TA* ringV = ringK + (long long)a.H * cap * DK;
     const int tid = threadIdx.x;
     if (tid == 0) {
         mbar_init(&bar, 1);
@@ -599,20 +456,22 @@ attention_steps_mma_kernel(AttnStream a, const __half* __restrict__ qkv, const f
     }
     const int fs = g.first + g.cr;
     chunks_stage_new<TA, NCH, true>(a, qkv + (long long)(fs - g.nf) * 3 * D, Ks, Vs, h, fs, g.cr, g.kn);
+    // rows behind the last key: K is masked there, V enters the PV MMAs with probability 0 and must be finite
     for (int i = tid; i < (krows - nk_all) * NCH; i += ATT_THREADS) {
         *reinterpret_cast<uint4*>(Ks + (nk_all + i / NCH) * DK + (i % NCH) * EPC) = make_uint4(0, 0, 0, 0);
         *reinterpret_cast<uint4*>(Vs + (nk_all + i / NCH) * DK + (i % NCH) * EPC) = make_uint4(0, 0, 0, 0);
     }
     __syncthreads();
     mbar_wait(&bar, 0);
+    if (gridDim.z == 1) chunks_append_ring<TA, NCH>(a, Ks, Vs, ringK, ringV, g.nf, g.cr, g.kn);
 
     const int pe0 = a.pe_index[slot];
     for (int j = g.j0; j < g.j1; ++j) {
         const int nfj = g.nf + j * t, clj = min(nfj, a.window);
-        const int o = nfj - clj - g.first;
+        const int o = nfj - clj - g.first;          // staged row of this chunk's first key
         const int nk = clj + t;
-        const int start = steps_start(a, pe0, j);
-        for (int i = tid; i < nk * NCH; i += ATT_THREADS) {
+        const int start = max(0, pe_after(pe0, j, a.chunk_size, a.pe_wrap) % a.pe_wrap - a.full_chunk);
+        for (int i = tid; i < nk * NCH; i += ATT_THREADS) {        // row r = position start + r, swizzled by that position
             const int r = i / NCH, cc = i % NCH, pos = min(start + r, a.pos_rows - 1);
             *reinterpret_cast<uint4*>(Ps + r * DK + ((cc ^ ((start + r) & 7)) * EPC)) =
                 *reinterpret_cast<const uint4*>(ptab_h + ((long long)h * a.pos_rows + pos) * DK + ((cc ^ (pos & 7)) * EPC));
@@ -627,15 +486,16 @@ attention_steps_mma_kernel(AttnStream a, const __half* __restrict__ qkv, const f
         __syncthreads();
         attn_chunk_mma<ATT_THREADS / 32>(Ks + o * DK, Vs + o * DK, g.first + o, Ps, start, quh, qvh, ph, sc, vrows, nk, t,
                                          out + (long long)(j * t) * D + h * DK, D);
-        __syncthreads();
+        __syncthreads();                              // Ps / quh / ph / sc are restaged by the next chunk
     }
 }
 
-// The ring after a pass: the last min(cnt[b] * t, cap) new K|V rows of session b at row frame % cap (fp16: chunk-swizzled by
-// frame), as the same frames appended by single steps leave it.  One CTA per (session, head).
+// The ring after a multi-chunk call of several groups per session: the last min(cnt[b] * t, cap) new K|V rows of session b at
+// row frame % cap (fp16: chunk-swizzled by frame), as the same frames appended by single steps leave it.  One CTA per
+// (session, head).
 template <typename TA, bool SWZ>
 __global__ void __launch_bounds__(ATT_THREADS)
-steps_append_ring_kernel(AttnStream a, const TA* __restrict__ qkv, TA* __restrict__ ring) {
+chunks_append_ring_kernel(AttnStream a, const TA* __restrict__ qkv, TA* __restrict__ ring) {
     constexpr int EPC = 16 / sizeof(TA), NCH = DK / EPC;
     FO_PDL_TRIGGER();
     FO_PDL_WAIT();
@@ -1070,21 +930,16 @@ attention_offline_fa_kernel(const __half* __restrict__ qkv, const float* __restr
 
 __global__ void advance_sessions_kernel(const int32_t* __restrict__ ids, int n, int t, int chunk_size, int pe_wrap,
                                         int32_t* n_frames, int32_t* pe_index, int32_t* adapter_valid, int chunks,
-                                        const int32_t* __restrict__ cnt, int min_cnt) {
+                                        const int32_t* __restrict__ cnt) {
     FO_PDL_TRIGGER();
     FO_PDL_WAIT();
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= n) return;
-    if (cnt) {
-        chunks = cnt[b];
-        if (chunks < min_cnt) return;
-    }
+    if (cnt) chunks = cnt[b];
     const int s = ids[b];
     if (n_frames) {
         n_frames[s] += chunks * t;
-        int pe = pe_index[s];
-        for (int j = 0; j < chunks; ++j) pe = pe % pe_wrap + chunk_size;   // attention.py:107,120 (+chunk_size, not +t)
-        pe_index[s] = pe;
+        pe_index[s] = pe_after(pe_index[s], chunks, chunk_size, pe_wrap);   // attention.py:107,120 (+chunk_size, not +t)
     }
     if (adapter_valid) adapter_valid[s] = adapter_valid[s] == 1 ? 2 : 1;
 }
@@ -1095,24 +950,19 @@ template <typename TA>
 int attention_stream(const AttnStream& a, const TA* qkv, const float* q32, TA* ring, const TA* ptab_h,
                      const float* pos_u, const float* pos_v, TA* out, cudaStream_t st) {
     if (a.n <= 0) return 0;
-    const int t = a.t, rows = a.window + a.chunks * t, prow = a.window + t;     // staged keys, keys of one chunk
+    const int t = a.t, prow = a.window + t;
     FO_CHECK(t <= STREAM_MAX_T, "attention_stream: %d frames per chunk exceeds %d", t, STREAM_MAX_T);
     FO_CHECK(a.ring_cap >= prow, "attention_stream: ring capacity %d < window %d + %d", a.ring_cap, a.window, t);
-    FO_CHECK(rows <= STREAM_CHUNKS_MAX_KEYS, "attention_stream: window %d + %d chunks x %d frames exceeds %d keys", a.window,
-             a.chunks, t, STREAM_CHUNKS_MAX_KEYS);
     using Kernel = void (*)(AttnStream, const TA*, const float*, TA*, const TA*, const float*, const float*, TA*);
-    // [0] one chunk, [1] one chunk summed from the QKV GEMM's split-K partials (fp16 only), [2] several chunks
-    std::array<Kernel, 3> kernels;
+    // [0] one chunk, [1] one chunk summed from the QKV GEMM's split-K partials (fp16 only)
+    std::array<Kernel, 2> kernels;
     size_t smem;
     if constexpr (sizeof(TA) == 2) {
-        kernels = {attention_stream_mma_kernel<false>, attention_stream_mma_kernel<true>, attention_chunks_mma_kernel};
-        const int krows = ((rows + 15) & ~15) + 16, vrows = (prow + 15) & ~15;
-        smem = a.chunks > 1 ? (size_t)(2 * krows + vrows) * DK * 2 + (size_t)2 * t * DK * 2 + (size_t)t * vrows * 2 +
-                                  (size_t)t * std::max(vrows, DK) * 4
-                            : (size_t)mma_unit_layout(a.window, t).bytes;
+        kernels = {attention_stream_mma_kernel<false>, attention_stream_mma_kernel<true>};
+        smem = (size_t)mma_unit_layout(a.window, t).bytes;
     } else {
-        kernels = {attention_stream_kernel, attention_stream_kernel, attention_chunks_kernel};
-        smem = (size_t)(2 * rows + prow) * DK * 4 + (size_t)2 * t * DK * 4 + (size_t)t * prow * 4;
+        kernels = {attention_stream_kernel, attention_stream_kernel};
+        smem = (size_t)3 * prow * DK * 4 + (size_t)2 * t * DK * 4 + (size_t)t * prow * 4;
     }
     FO_CHECK(smem <= 160 * 1024, "attention_stream: window too large for shared memory");
     static bool opted_in = false;      // past 48 KB (window + t > ~115 keys, e.g. left_chunks 31) a launch needs the opt-in
@@ -1120,11 +970,11 @@ int attention_stream(const AttnStream& a, const TA* qkv, const float* q32, TA* r
         for (Kernel k : kernels) FO_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
         opted_in = true;
     }
-    const Kernel kern = kernels[a.chunks > 1 ? 2 : a.nsplit > 0 ? 1 : 0];
+    const Kernel kern = kernels[a.nsplit > 0 ? 1 : 0];
     FO_CUDA(launch_pdl(kern, dim3(a.n, a.H), dim3(ATT_THREADS), smem, st, a, qkv, q32, ring, ptab_h, pos_u, pos_v, out));
     FO_LAUNCHED();
 #ifdef FO_TC_TRACE_BUILD
-    if (sizeof(TA) == 2 && a.chunks == 1 && getenv("FO_TC_TRACE") && st == nullptr) {
+    if (sizeof(TA) == 2 && getenv("FO_TC_TRACE") && st == nullptr) {
         cudaStreamSynchronize(st);
         unsigned long long hb[16];
         cudaMemcpyFromSymbol(hb, g_attn_trace, sizeof(hb));
@@ -1139,38 +989,40 @@ int attention_stream(const AttnStream& a, const TA* qkv, const float* q32, TA* r
 template int attention_stream<float>(const AttnStream&, const float*, const float*, float*, const float*, const float*, const float*, float*, cudaStream_t);
 
 template <typename TA>
-int attention_steps(const AttnStream& a, int groups, const TA* qkv, const float* q32, TA* ring, const TA* ptab_h,
-                    const float* pos_u, const float* pos_v, TA* out, cudaStream_t st) {
+int attention_chunks(const AttnStream& a, int groups, const TA* qkv, const float* q32, TA* ring, const TA* ptab_h,
+                     const float* pos_u, const float* pos_v, TA* out, cudaStream_t st) {
     if (a.n <= 0) return 0;
-    const int t = a.t, rows = a.window + a.chunks * t, prow = a.window + t;
-    FO_CHECK(t <= STREAM_MAX_T && a.ring_cap >= prow && a.cnt && a.off && groups >= 1, "attention_steps: bad geometry");
-    FO_CHECK(rows <= STREAM_CHUNKS_MAX_KEYS, "attention_steps: window %d + %d chunks x %d frames exceeds %d keys", a.window,
+    const int t = a.t, rows = a.window + a.chunks * t, prow = a.window + t;     // staged keys, keys of one chunk
+    FO_CHECK(t <= STREAM_MAX_T && a.ring_cap >= prow && a.cnt && a.off && groups >= 1, "attention_chunks: bad geometry");
+    FO_CHECK(rows <= STREAM_CHUNKS_MAX_KEYS, "attention_chunks: window %d + %d chunks x %d frames exceeds %d keys", a.window,
              a.chunks, t, STREAM_CHUNKS_MAX_KEYS);
     size_t smem;
-    void (*kern)(AttnStream, const TA*, const float*, const TA*, const TA*, const float*, const float*, TA*);
+    void (*kern)(AttnStream, const TA*, const float*, TA*, const TA*, const float*, const float*, TA*);
     if constexpr (sizeof(TA) == 2) {
-        kern = attention_steps_mma_kernel;
+        kern = attention_chunks_mma_kernel;
         const int krows = ((rows + 15) & ~15) + 16, vrows = (prow + 15) & ~15;
         smem = (size_t)(2 * krows + vrows) * DK * 2 + (size_t)2 * t * DK * 2 + (size_t)t * vrows * 2 + (size_t)t * std::max(vrows, DK) * 4;
     } else {
-        kern = attention_steps_kernel;
+        kern = attention_chunks_kernel;
         smem = (size_t)(2 * rows + prow) * DK * 4 + (size_t)2 * t * DK * 4 + (size_t)t * prow * 4;
     }
-    static bool opted_in = false;
+    static bool opted_in = false;      // past 48 KB a launch needs the opt-in
     if (!opted_in) {
         FO_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
         opted_in = true;
     }
-    FO_CUDA(launch_pdl(kern, dim3(a.n, a.H, groups), dim3(ATT_THREADS), smem, st, a, qkv, q32, (const TA*)ring, ptab_h, pos_u, pos_v, out));
+    FO_CUDA(launch_pdl(kern, dim3(a.n, a.H, groups), dim3(ATT_THREADS), smem, st, a, qkv, q32, ring, ptab_h, pos_u, pos_v, out));
     FO_LAUNCHED();
     FO_CUDA(cudaGetLastError());
-    FO_CUDA(launch_pdl(steps_append_ring_kernel<TA, sizeof(TA) == 2>, dim3(a.n, a.H), dim3(ATT_THREADS), 0, st, a, qkv, ring));
-    FO_LAUNCHED();
-    FO_CUDA(cudaGetLastError());
+    if (groups > 1) {                  // several CTAs read a session's ring: the append waits for the whole grid
+        FO_CUDA(launch_pdl(chunks_append_ring_kernel<TA, sizeof(TA) == 2>, dim3(a.n, a.H), dim3(ATT_THREADS), 0, st, a, qkv, ring));
+        FO_LAUNCHED();
+        FO_CUDA(cudaGetLastError());
+    }
     return 0;
 }
-template int attention_steps<float>(const AttnStream&, int, const float*, const float*, float*, const float*, const float*, const float*, float*, cudaStream_t);
-template int attention_steps<__half>(const AttnStream&, int, const __half*, const float*, __half*, const __half*, const float*, const float*, __half*, cudaStream_t);
+template int attention_chunks<float>(const AttnStream&, int, const float*, const float*, float*, const float*, const float*, const float*, float*, cudaStream_t);
+template int attention_chunks<__half>(const AttnStream&, int, const __half*, const float*, __half*, const __half*, const float*, const float*, __half*, cudaStream_t);
 // head-major copy of a rel-pos table in the activation type: out[h][pos][64] = (TA) in[pos][h*64 + d]
 template <typename TA>
 __global__ void ptab_head_major_kernel(const float* __restrict__ in, int pos_rows, int H, TA* __restrict__ out) {
@@ -1228,10 +1080,10 @@ template int attention_offline<float>(const float*, const float*, int, int, int,
 template int attention_offline<__half>(const __half*, const float*, int, int, int, const int32_t*, int, int, const float*, const __half*, int, const float*, const float*, __half*, cudaStream_t);
 
 int advance_sessions(const int32_t* ids, int n, int t, int chunk_size, int pe_wrap, int32_t* n_frames,
-                      int32_t* pe_index, int32_t* adapter_valid, cudaStream_t st, int chunks, const int32_t* cnt, int min_cnt) {
+                      int32_t* pe_index, int32_t* adapter_valid, cudaStream_t st, int chunks, const int32_t* cnt) {
     if (n <= 0) return 0;
     FO_CUDA(launch_pdl(advance_sessions_kernel, dim3(cdiv(n, 128)), dim3(128), 0, st, ids, n, t, chunk_size, pe_wrap, n_frames, pe_index, adapter_valid,
-                       chunks, cnt, min_cnt));
+                       chunks, cnt));
     FO_LAUNCHED();
     FO_CUDA(cudaGetLastError());
     return 0;

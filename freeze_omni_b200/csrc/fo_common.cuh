@@ -40,6 +40,12 @@ extern long long g_launches;      // kernels enqueued by this library (fo_stats.
 #define FO_LAUNCHED() (++fo::g_launches)
 
 __host__ __device__ inline int cdiv(int a, int b) { return (a + b - 1) / b; }
+// pe_index after j streaming steps of pe = pe % wrap + chunk_size (attention.py:107,120), in closed form since j may run into
+// the thousands: pe itself for j = 0, else (pe % wrap + (j - 1) * chunk_size) % wrap + chunk_size.  Equal to the loop for every
+// int pe, negative ones included; its value mod wrap is (pe % wrap + j * chunk_size) % wrap.
+__host__ __device__ inline int pe_after(int pe, int j, int chunk_size, int wrap) {
+    return j == 0 ? pe : (int)(((long long)(pe % wrap) + (long long)(j - 1) * chunk_size) % wrap) + chunk_size;
+}
 
 // ---- programmatic dependent launch ------------------------------------------------------------------
 // The kernels of the streaming chain are launched with programmaticStreamSerialization: a kernel may start (launch
@@ -335,28 +341,21 @@ int scale_rows(const float* x, float* y, long long n, float s, cudaStream_t st);
 // (conv1d_gather layout) or 2 (adapter_gather layout); new cache = last k-1 rows (fp32), slot-resident (ids != null,
 // (slot, 2, k-1, C) time-major) or explicit (B, C, k-1)
 // Per-session rows of a call whose sessions bring different chunk counts (fo_encode_stream_chunks_v); cnt == null: every
-// session has the T rows of the uniform layout.
-//   pass < 0 (even t): session b's real input is its first cnt[b] * unit of T padded rows; with `off` non-null, `in` is
-//            packed instead, session b's rows starting at row off[b] * unit.  The new cache comes from the real rows.
-//   pass >= 0 (odd t, chunk pass `pass`): sessions with cnt[b] <= pass have no chunk in this pass and keep their cache.
+// session has the T rows of the uniform layout.  Session b's real input is its first cnt[b] * unit of T padded rows; with
+// `off` non-null, `in` is packed instead, session b's rows starting at row off[b] * unit.  The new cache comes from the real rows.
 struct SessionRows {
     const int32_t* cnt = nullptr;
     const int32_t* off = nullptr;
     int unit = 0;
-    int pass = -1;
 };
 template <typename TA>
 int conv_stage(const float* in, const uint8_t* mask, int B, int T, int C, int km1, int stride, const float* scale,
                const float* shift, const int32_t* ids, float* slot_cache, int32_t* slot_valid, const float* cache_in,
                float* cache_out, TA* xin, cudaStream_t st, const SessionRows& sr = SessionRows());
-// Moves blocks of `bytes` between per-session and packed (block) layouts, session b owning blocks [off[b], off[b] + cnt[b]):
-//   PACK:    grid (n, kmax), src block b * kmax + j (j < cnt[b]) -> dst block off[b] + j
-//   GATHER:  src block off[b] + min(j, cnt[b] - 1) -> dst block b
-//   SCATTER: src block b -> dst block off[b] + j, only where cnt[b] > j
-// Block i of src / dst starts at byte i * src_stride / i * dst_stride.
-enum { BLOCKS_PACK = 0, BLOCKS_GATHER = 1, BLOCKS_SCATTER = 2 };
-int session_blocks(const void* src, long long src_stride, void* dst, long long dst_stride, long long bytes, int n, int kmax,
-                   int j, int mode, const int32_t* cnt, const int32_t* off, cudaStream_t st);
+// Packs fp32 blocks of `bytes` from a per-session grid of kmax blocks to block order: src block b * kmax + j (j < cnt[b]) ->
+// dst block off[b] + j.
+int pack_session_blocks(const float* src, float* dst, long long bytes, int n, int kmax, const int32_t* cnt, const int32_t* off,
+                        cudaStream_t st);
 // The carried stride-2 adapter conv over chunks of odd t, run at stride 1 over each session's kmax * t grid rows: output m of
 // chunk j is grid row j * t + 2 m.  src (n, kmax * t, C) -> dst (blocks, t_out, C), session b's chunks j < cnt[b] from block off[b].
 int pick_chunk_rows(const float* src, int n, int kmax, int t, int t_out, int C, const int32_t* cnt, const int32_t* off, float* dst,
@@ -394,10 +393,10 @@ struct AttnStream {
     const float* part_bias = nullptr;
     int nsplit = 0;
     long long part_stride = 0;
-    // consecutive chunks per session in this call (fo_encode_stream_chunks[_v]): rows are (session, chunk, frame); session b
-    // brings cnt[b] chunks and its rows start at row (off[b] - off[0]) * t; chunk j of a session is attended exactly as the
-    // j-th of cnt[b] sequential calls (chunk_size: pe_index step).  `chunks` is the largest count (it sizes shared memory);
-    // chunks == 1 is the single-chunk kernel, which reads rows b * t and no table.
+    // consecutive chunks per session (attention_chunks: fo_encode_stream_chunks[_v], passes of fo_stream_steps_v): rows are
+    // (session, chunk, frame); session b brings cnt[b] chunks and its rows start at row (off[b] - off[0]) * t; chunk j of a
+    // session is attended exactly as the j-th of cnt[b] sequential calls (chunk_size: pe_index step).  `chunks` is the number
+    // of chunks one CTA attends (it sizes shared memory).  attention_stream reads rows b * t and no table.
     int chunks = 1;
     int chunk_size = 0;
     const int32_t* cnt = nullptr;
@@ -409,17 +408,18 @@ constexpr int STREAM_CHUNKS_MAX_KEYS = 128;
 constexpr int STREAM_MAX_T = 8;
 // qkv (n*t, 3*D) activation type (K and V columns are read from it); q32 (n*t, 3*D) fp32 whose first D
 // columns hold Q (the QKV GEMM keeps Q in fp32, Epilogue::split_col); ring = this layer's
-// (slot, 2, H, ring_cap, 64); ptab (pos_rows, D) fp32; out (n*t, D).  Appends the new K/V rows to the ring.
+// (slot, 2, H, ring_cap, 64); ptab (pos_rows, D) fp32; out (n*t, D).  One chunk per session; appends the new K/V rows to
+// the ring.
 template <typename TA>
 int attention_stream(const AttnStream& a, const TA* qkv, const float* q32, TA* ring, const TA* ptab_h,
                      const float* pos_u, const float* pos_v, TA* out, cudaStream_t st);
-// One pass of fo_stream_steps_v: session b's cnt[b] chunks (any number) with the rows and tables of a multi-chunk call.
-// One CTA per (session, head, group of a.chunks chunks), grid z = `groups`; each chunk still sees window + t keys, staged
-// from the ring (frames before the pass) and from this pass's own K|V rows in qkv.  A second kernel then appends the last
-// min(cnt[b] * t, ring_cap) new frames to the ring, after every read of it.
+// Session b's cnt[b] consecutive chunks (cnt[b] <= groups * a.chunks), with the same tensors.  One CTA per (session, head,
+// group of a.chunks chunks), grid z = `groups`; each chunk sees window + t keys, staged from the ring (frames before the
+// call) and from the call's own K|V rows in qkv.  The last min(cnt[b] * t, ring_cap) new frames go to the ring after every
+// read of it: appended by the CTA itself when groups == 1 (the only reader of its ring), else by a second kernel.
 template <typename TA>
-int attention_steps(const AttnStream& a, int groups, const TA* qkv, const float* q32, TA* ring, const TA* ptab_h,
-                    const float* pos_u, const float* pos_v, TA* out, cudaStream_t st);
+int attention_chunks(const AttnStream& a, int groups, const TA* qkv, const float* q32, TA* ring, const TA* ptab_h,
+                     const float* pos_u, const float* pos_v, TA* out, cudaStream_t st);
 // ptab_h: the same table as [H][pos_rows][64] in the activation type (rows of one head contiguous -> one bulk copy)
 template <typename TA>
 int ptab_head_major(const float* in, int pos_rows, int H, TA* out, cudaStream_t st);
@@ -431,10 +431,10 @@ int attention_offline(const TA* qkv, const float* q32, int B, int T, int H, cons
 // end of a streaming step: n_frames += t, pe_index = pe_index % wrap + chunk_size (attention.py:107,120),
 // and flip the live half of the double-buffered adapter cache.  Either group may be null.  chunks > 1: the session
 // advanced by that many chunks of t frames (pe_index stepped `chunks` times; the adapter cache still flips once).  cnt
-// non-null: session b's own count cnt[b] replaces `chunks`, and sessions with cnt[b] < min_cnt are left as they are.
+// non-null: session b's own count cnt[b] replaces `chunks`.
 int advance_sessions(const int32_t* ids, int n, int t, int chunk_size, int pe_wrap, int32_t* n_frames,
                      int32_t* pe_index, int32_t* adapter_valid, cudaStream_t st, int chunks = 1,
-                     const int32_t* cnt = nullptr, int min_cnt = 0);
+                     const int32_t* cnt = nullptr);
 
 // ---- weight-streaming layer stack for a handful of sessions (fo_stack.cu) ---------------------------
 // All transformer layers of a streaming step in ONE cooperative launch when the step has at most 16 token rows (1-4

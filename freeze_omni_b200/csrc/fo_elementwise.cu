@@ -274,8 +274,7 @@ __global__ void scale_rows_kernel(const float* __restrict__ x, float* __restrict
 // The new cache = the last km1 virtual rows, fp32: explicit caches in the reference layout (B, C, km1); slot-resident caches
 // time-major and double-buffered per slot: slot_valid = 0 (None), 1 (half 0 live), 2 (half 1 live); the new rows go to the
 // other half and advance_sessions() flips the flag after every block has read it.  SessionRows: rows of a session past its
-// real length Tb are padding (0, no cache), and the cache comes from its last real rows; a session without a chunk in an odd-t
-// pass writes no cache.
+// real length Tb are padding (0, no cache), and the cache comes from its last real rows.
 template <typename TA>
 __global__ void conv_stage_kernel(const float* __restrict__ in, const uint8_t* __restrict__ mask, int T, int C, int km1, int stride,
                                   const float* __restrict__ scale, const float* __restrict__ shift,
@@ -286,14 +285,9 @@ __global__ void conv_stage_kernel(const float* __restrict__ in, const uint8_t* _
     const int b = blockIdx.x, r = blockIdx.y;          // r in [0, km1 + T)
     int Tb = T;
     long long in0 = (long long)b * T;                  // input row of the session's first frame
-    bool keep_cache = false;
     if (sr.cnt) {
-        if (sr.pass >= 0) {
-            keep_cache = sr.cnt[b] <= sr.pass;
-        } else {
-            Tb = sr.cnt[b] * sr.unit;
-            if (sr.off) in0 = (long long)sr.off[b] * sr.unit;
-        }
+        Tb = sr.cnt[b] * sr.unit;
+        if (sr.off) in0 = (long long)sr.off[b] * sr.unit;
     }
     const int slot = ids ? ids[b] : -1;
     const int live = ids ? slot_valid[slot] : 0;
@@ -318,7 +312,7 @@ __global__ void conv_stage_kernel(const float* __restrict__ in, const uint8_t* _
         if (stride == 1) xin[((long long)b * R1 + r) * C + c] = from_f<TA>(v);
         else xin[(((long long)(r & 1) * gridDim.x + b) * RP + (r >> 1)) * C + c] = from_f<TA>(v);
         const int cr = r - Tb;                           // row of the new cache this element becomes
-        if (cr >= 0 && cr < km1 && !keep_cache) {
+        if (cr >= 0 && cr < km1) {
             if (ids) new_half[(long long)cr * C + c] = v;
             else if (cache_out) cache_out[((long long)b * C + c) * km1 + cr] = v;
         }
@@ -612,31 +606,21 @@ int conv_stage(const float* in, const uint8_t* mask, int B, int T, int C, int km
 template int conv_stage<float>(const float*, const uint8_t*, int, int, int, int, int, const float*, const float*, const int32_t*, float*, int32_t*, const float*, float*, float*, cudaStream_t, const SessionRows&);
 template int conv_stage<__half>(const float*, const uint8_t*, int, int, int, int, int, const float*, const float*, const int32_t*, float*, int32_t*, const float*, float*, __half*, cudaStream_t, const SessionRows&);
 
-__global__ void session_blocks_kernel(const char* __restrict__ src, long long src_stride, char* __restrict__ dst, long long dst_stride,
-                                      long long bytes, int kmax, int j, int mode, const int32_t* __restrict__ cnt,
-                                      const int32_t* __restrict__ off) {
+// grid (n, kmax): block j < cnt[b] of session b
+__global__ void pack_session_blocks_kernel(const char* __restrict__ src, char* __restrict__ dst, long long bytes, int kmax,
+                                           const int32_t* __restrict__ cnt, const int32_t* __restrict__ off) {
     FO_PDL_TRIGGER();
     FO_PDL_WAIT();
-    const int b = blockIdx.x, k = cnt[b];
-    long long si, di;
-    if (mode == BLOCKS_PACK) {
-        const int jj = blockIdx.y;
-        if (jj >= k) return;
-        si = (long long)b * kmax + jj; di = off[b] + jj;
-    } else if (mode == BLOCKS_GATHER) {
-        si = off[b] + min(j, k - 1); di = b;
-    } else {
-        if (k <= j) return;
-        si = b; di = off[b] + j;
-    }
-    const char* s = src + si * src_stride;
-    char* d = dst + di * dst_stride;
-    if (((bytes | src_stride | dst_stride | (long long)(size_t)src | (long long)(size_t)dst) & 15) == 0) {
+    const int b = blockIdx.x, j = blockIdx.y;
+    if (j >= cnt[b]) return;
+    const char* s = src + ((long long)b * kmax + j) * bytes;
+    char* d = dst + ((long long)off[b] + j) * bytes;
+    if (((bytes | (long long)(size_t)src | (long long)(size_t)dst) & 15) == 0) {
         for (long long i = threadIdx.x * 16LL; i < bytes; i += blockDim.x * 16LL)
             *reinterpret_cast<uint4*>(d + i) = *reinterpret_cast<const uint4*>(s + i);
     } else {
-        for (long long i = threadIdx.x * 2LL; i < bytes; i += blockDim.x * 2LL)     // rows of 16-bit or 32-bit elements
-            *reinterpret_cast<uint16_t*>(d + i) = *reinterpret_cast<const uint16_t*>(s + i);
+        for (long long i = threadIdx.x * 4LL; i < bytes; i += blockDim.x * 4LL)
+            *reinterpret_cast<float*>(d + i) = *reinterpret_cast<const float*>(s + i);
     }
 }
 // grid (kmax * t_out, n): row m of chunk j < cnt[b] of session b <- row j * t + 2 m of the session's T-row grid
@@ -659,12 +643,11 @@ int pick_chunk_rows(const float* src, int n, int kmax, int t, int t_out, int C, 
     return 0;
 }
 
-int session_blocks(const void* src, long long src_stride, void* dst, long long dst_stride, long long bytes, int n, int kmax,
-                   int j, int mode, const int32_t* cnt, const int32_t* off, cudaStream_t st) {
+int pack_session_blocks(const float* src, float* dst, long long bytes, int n, int kmax, const int32_t* cnt, const int32_t* off,
+                        cudaStream_t st) {
     if (n <= 0) return 0;
-    FO_CHECK(bytes % 2 == 0 && src_stride % 2 == 0 && dst_stride % 2 == 0, "session_blocks: blocks of 16-bit or 32-bit elements");
-    FO_CUDA(launch_pdl(session_blocks_kernel, dim3(n, mode == BLOCKS_PACK ? kmax : 1), dim3(256), 0, st, (const char*)src, src_stride,
-                       (char*)dst, dst_stride, bytes, kmax, j, mode, cnt, off));
+    FO_CHECK(bytes % 4 == 0, "pack_session_blocks: blocks of fp32 elements");
+    FO_CUDA(launch_pdl(pack_session_blocks_kernel, dim3(n, kmax), dim3(256), 0, st, (const char*)src, (char*)dst, bytes, kmax, cnt, off));
     FO_LAUNCHED();
     FO_CUDA(cudaGetLastError());
     return 0;

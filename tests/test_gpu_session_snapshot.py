@@ -157,7 +157,7 @@ def test_across_ring_capacities(dtype):
 @pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16])
 @pytest.mark.parametrize("name", ["tiny_linear", "cnn", "two", "tiny_bn", "fork_t7", "tiny_conv1d"])
 def test_adapter_and_layer_variants(name, dtype):
-    """Every adapter variant (LinearAdapter, CNNAdapter, two-conv CNNSubsampling, BatchNorm, t = 7 chunk by chunk) and the
+    """Every adapter variant (LinearAdapter, CNNAdapter, two-conv CNNSubsampling, BatchNorm, t = 7 through the stride-1 grid and row pick) and the
     Conv1dLinear layers, whose left context the record carries."""
     cfg = variant(name)
     t_in = 32 if name == "fork_t7" else cfg.chunk_feat_frames

@@ -8,7 +8,7 @@ default), with sessions at different fill levels and pe_index phases sharing cal
   C   L   t_in  window  keys/call  largest k  reaches
   4   16  19    64      68         16         control (shipped geometry)
   4   2   19    8       12         30         k*t = 120 > ring_cap 16: the ring append keeps only the last ring_cap rows
-  3   1   15    3       6          41         odd t (adapter chunk by chunk)
+  3   1   15    3       6          41         odd t (adapter: stride-1 grid + row pick)
   3   5   15    15      18         37         window not a multiple of 8
   2   8   11    16      18         56
   1   16  7     16      17         112        t = 1

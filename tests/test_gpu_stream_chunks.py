@@ -126,7 +126,8 @@ def _variant(name):
 @pytest.mark.parametrize("name", ["tiny_linear", "cnn", "two", "tiny_bn", "tiny_conv1d", "tiny_postnorm_concat", "fork_t7"])
 def test_variants_vs_sequential_single_chunk_calls(name):
     """Every adapter / layer variant, k = 3 then 7, against single-chunk calls of twin sessions on the same engine.
-    fork_t7: 32 feature frames per chunk -> t = 7, odd, so the CNNSubsampling adapter runs chunk by chunk inside the step."""
+    fork_t7: 32 feature frames per chunk -> t = 7, odd, so the CNNSubsampling adapter runs its convolutions at stride 1 over
+    each session's frames and picks every chunk's output rows."""
     cfg = _variant(name)
     t_in = 32 if name == "fork_t7" else cfg.chunk_feat_frames
     eng = engine(cfg, adapter_seed=5 if name in ("cnn", "two") else 3, max_sessions=6)
@@ -155,7 +156,7 @@ def test_handoff_through_every_adapter_variant(name):
     """The fp16 LLM hand-off of every adapter variant on a bf16 engine, k = 1 then 3: an armed call writes, behind the prefix of
     each (session, chunk) block, the adapter rows that twin sessions get as fp32, rounded to fp16 bit for bit; the prefix and
     trailing rows keep what they held; both sets of sessions end in the same state.  fork_t7 (t = 7): the CNNSubsampling adapter
-    runs chunk by chunk, so its later chunks land in blocks j0 > 0 of a session."""
+    picks every chunk's rows from a stride-1 pass, and its later chunks land in blocks j0 > 0 of a session."""
     cfg = _variant(name)
     t_in = 32 if name == "fork_t7" else cfg.chunk_feat_frames
     eng = engine(cfg, adapter_seed=5 if name in ("cnn", "two") else 3, dtype=torch.bfloat16, max_sessions=4)

@@ -7,7 +7,8 @@ calls per 30 s) and fo_encode_offline of the same audio (the ceiling; its rel-po
     one process after one warm-up round each (best and median ms, audio-s per s).  stream_steps_v includes the fbank; the
     k = 16 loop and offline start from features computed beforehand.
   * --profile: a separate run with torch.profiler around one stream_steps_v call per session count, programmatic dependent
-    launch off: device time per kernel name, and the share of the pass attention (attention_steps*) and its ring append.
+    launch off: device time per kernel name, and the share of the pass attention (attention_chunks*) and its separate ring append
+    (chunks_append_ring*, launched when a session spreads over several CTAs of a head).
 
 Writes one JSON file (--out) that names the GPU, its power limit and its clocks."""
 import argparse
@@ -106,8 +107,8 @@ def profile(eng, cfg, n):
         if e.device_type == torch.autograd.DeviceType.CUDA and e.device_time_total > 0:
             per[e.name] = per.get(e.name, 0.0) + e.device_time_total
     total = sum(per.values())
-    attn = sum(v for k, v in per.items() if "attention_steps" in k)
-    append = sum(v for k, v in per.items() if "steps_append_ring" in k)
+    attn = sum(v for k, v in per.items() if "attention_chunks" in k)
+    append = sum(v for k, v in per.items() if "chunks_append_ring" in k)
     top = sorted(per.items(), key=lambda kv: -kv[1])[:15]
     eng.set_option("pdl", 1)
     eng.free(ids)
