@@ -69,6 +69,7 @@ SYMBOLS = {
     "fo_stream_step_embeds": (C.c_int, [_P, _I32P, C.c_int, _P, C.c_int, C.c_float, _P, _P, C.c_int64, C.c_int64, _P]),
     "fo_handoff_arm": (C.c_int, [_P, C.c_int, _P, C.c_int64, C.c_int64, _P, _P, _P, _P]),
     "fo_encode_offline": (C.c_int, [_P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, _P, _P, _P]),
+    "fo_encode_offline_packed": (C.c_int, [_P, _P, _P, C.c_int, C.c_int, C.c_int, _P, _P, _P]),
     "fo_adapter_forward": (C.c_int, [_P, _P, _P, C.c_int, C.c_int, _P, _P, _P, _P]),
     "fo_adapter_forward2": (C.c_int, [_P, _P, _P, C.c_int, C.c_int, _P, _P, _P, _P, _P, _P]),
     "fo_stats": (C.c_int, [_P, C.POINTER(FoStats)]),

@@ -120,6 +120,22 @@ class PathConfig:
         """Frames after Conv2dSubsampling4: ((T-1)//2 - 1)//2 (subsampling.py:28-34)."""
         return ((t - 1) // 2 - 1) // 2
 
+    def adapter_len(self, t: int) -> int:
+        """Adapter frames for t encoder frames: CNNSubsampling's stride-2 conv over k-1 left frames gives (t-1)//2 + 1
+        (adapter.py:137-144); LinearAdapter and CNNAdapter keep the rate."""
+        return t if self.adapter_type in ("linear", "cnn") else (t - 1) // 2 + 1
+
+    def packed_offsets(self, lens):
+        """Row offsets of a packed offline call (fo_encode_offline_packed) for feature lengths ``lens``: (enc_offsets,
+        adapter_offsets), int64 arrays of B + 1 prefix sums of the per-utterance encoder / adapter rows."""
+        import numpy as np
+        t = np.asarray(lens, dtype=np.int64).reshape(-1)
+        if t.size == 0 or (t < 7).any():
+            raise ValueError("every utterance needs >= 7 feature frames")
+        t2 = ((t - 1) // 2 - 1) // 2
+        t3 = t2 if self.adapter_type in ("linear", "cnn") else (t2 - 1) // 2 + 1
+        return np.concatenate([[0], np.cumsum(t2)]), np.concatenate([[0], np.cumsum(t3)])
+
     def validate(self) -> None:
         """The reference exits on an inconsistent config (encoder.py:74-75,86-87,94); here a
         ValueError.  Variants whose streaming path is broken upstream are refused loudly

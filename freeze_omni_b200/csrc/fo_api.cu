@@ -126,7 +126,7 @@ struct fo_ctx {
     int32_t* ids_dev = nullptr;               // [3][max_sessions]: session ids, then cnt_dev and off_dev
     int32_t* cnt_dev = nullptr;               // chunks per session of a multi-chunk call (fo_encode_stream_chunks[_v])
     int32_t* off_dev = nullptr;               // first block of each session in that call (prefix sums of cnt)
-    DevBuf ws[40];                            // named workspaces, see enum below
+    DevBuf ws[48];                            // named workspaces, see enum below
     // options
     int gemm_backend = 0, use_graph = 0, split_k = 1;
     int tc_npa = 0, tc_npb = 0;
@@ -218,7 +218,9 @@ struct fo_ctx {
 namespace {
 
 enum { WS_FEATS = 0, WS_C1, WS_C2, WS_XSUB, WS_EMB, WS_X, WS_H, WS_QKV, WS_ATT, WS_FFH, WS_ENC, WS_XIN, WS_ACONV, WS_AH,
-       WS_Y, WS_MASK2, WS_ILENS, WS_ILENS2, WS_AMASK, WS_PCM, WS_TMP0, WS_TMP1, WS_TMP2, WS_TMP3, WS_Q32, WS_HC, WS_PART, WS_PCM2, WS_ENC2, WS_Y2, WS_AC1, WS_XIN2, WS_TMP4, WS_TMP5, WS_HP, WS_FP, WS_PACK, WS_SROWS, WS_COUNT };
+       WS_Y, WS_MASK2, WS_ILENS, WS_ILENS2, WS_AMASK, WS_PCM, WS_TMP0, WS_TMP1, WS_TMP2, WS_TMP3, WS_Q32, WS_HC, WS_PART, WS_PCM2, WS_ENC2, WS_Y2, WS_AC1, WS_XIN2, WS_TMP4, WS_TMP5, WS_HP, WS_FP, WS_PACK, WS_SROWS,
+       WS_PKTAB, WS_FGRID, WS_XP, WS_COUNT };
+static_assert(WS_COUNT <= (int)(sizeof(fo_ctx::ws) / sizeof(DevBuf)), "fo_ctx::ws holds every named workspace");
 
 int dev_alloc(fo_ctx* c, void** p, size_t bytes) {
     *p = nullptr;
@@ -706,14 +708,24 @@ struct AdMix {
     int kmax, unit, blocks;
     bool pick;
 };
+// pack (fo_encode_offline_packed): enc holds B utterances packed end to end, utterance b's rows from enc_off[b]; cnt[i * B + b]
+// = its rows into conv i, cnt[ns * B + b] its output rows, which go to out.y packed from off[b] (`rows` in all).  The convs run
+// over a grid of B x T rows (T = the longest utterance): each utterance from the first row of its run, with zero left context
+// (so the stride-2 phase starts at its first frame) and zeros behind it.
+struct AdPack {
+    const int32_t* cnt;
+    const int32_t* enc_off;
+    const int32_t* off;
+    int rows;
+};
 template <typename TA>
 int adapter_program(fo_ctx* c, const float* enc, const uint8_t* mask, int B, int T, const int32_t* ids_dev,
                     const float* const* cache_in, float* const* cache_out, const AdOut& out, cudaStream_t st,
-                    const AdMix* mix = nullptr) {
+                    const AdMix* mix = nullptr, const AdPack* pack = nullptr) {
     const int D = c->D, E = c->E, KA = c->KA, ns = c->ad_nst;
     const bool grid = mix != nullptr;                                          // per-session padded grid
     const int t_out = grid ? ad_frames(c, mix->unit) : ad_frames(c, T);       // grid: frames out of one chunk
-    const int M = grid ? mix->blocks * t_out : B * t_out;
+    const int M = pack ? pack->rows : grid ? mix->blocks * t_out : B * t_out;
     const bool run_gemm = !(c->debug_skip & 16);
     const float* x = enc;
     const bool pick = grid && mix->pick;
@@ -733,6 +745,10 @@ int adapter_program(fo_ctx* c, const float* enc, const uint8_t* mask, int B, int
             sr.cnt = mix->cnt;
             sr.off = i == 0 ? mix->off : nullptr;          // the first conv reads the packed encoder rows
             sr.unit = pick ? mix->unit : ad_frames(c, mix->unit, i);
+        } else if (pack) {
+            sr.cnt = pack->cnt + (long long)i * B;
+            sr.off = i == 0 ? pack->enc_off : nullptr;
+            sr.unit = 1;
         }
         FO_TRY(conv_stage<TA>(x, i == 0 ? mask : nullptr, B, Ti, s.cin, KA - 1, stride, s.in_scale, s.in_shift,
                               c->ad_carry ? ids_dev : nullptr, s.cache, c->ad_valid, cache_in ? cache_in[i] : nullptr,
@@ -751,6 +767,12 @@ int adapter_program(fo_ctx* c, const float* enc, const uint8_t* mask, int B, int
         if (pick) FO_TRY(pick_chunk_rows(x, B, mix->kmax, mix->unit, t_out, K, mix->cnt, mix->off, reinterpret_cast<float*>(pk), st));
         else FO_TRY(pack_session_blocks(x, reinterpret_cast<float*>(pk), (long long)t_out * K * sizeof(float), B, mix->kmax, mix->cnt,
                                         mix->off, st));
+        x = reinterpret_cast<const float*>(pk);
+    } else if (pack && ns > 0) {
+        void* pk;
+        FO_TRY(ws_ensure(c, WS_PACK, (size_t)M * K * sizeof(float), &pk));
+        FO_TRY(pack_session_blocks(x, reinterpret_cast<float*>(pk), (long long)K * sizeof(float), B, ad_frames(c, T),
+                                   pack->cnt + (long long)ns * B, pack->off, st));
         x = reinterpret_cast<const float*>(pk);
     }
     const TA* a = reinterpret_cast<const TA*>(enc);
@@ -872,6 +894,10 @@ struct FfnConv {                  // Conv1dLinear only: where the rows come from
     void* hc = nullptr;           // depthwise output buffer (M, D), activation type
     void* hp = nullptr;           // MultiLayeredConv1d: zero-padded layer input (B, T + k - 1, D) and hidden rows (B, T + k - 1, FF)
     void* fp = nullptr;
+    // MultiLayeredConv1d over packed utterances (B = 1, T = all rows): k - 1 rows between two utterances, from row gap_at[i],
+    // are zeroed in both padded buffers, so each utterance sees (k-1)/2 zero rows on either side
+    const int32_t* gap_at = nullptr;
+    int n_gaps = 0;
 };
 template <typename TA>
 int layer_post(fo_ctx* c, const LayerW& w, float* x, int M, TA* att, TA* h, TA* ffh, const NextNorm& nn,
@@ -934,12 +960,14 @@ int layer_post(fo_ctx* c, const LayerW& w, float* x, int M, TA* att, TA* h, TA* 
         TA* hp = reinterpret_cast<TA*>(fc.hp);
         TA* fp = reinterpret_cast<TA*>(fc.fp);
         FO_TRY(pad_rows<TA>(h, fc.B, fc.T, D, lead, k - 1 - lead, hp, st));
+        FO_TRY(zero_row_runs<TA>(hp + (long long)lead * D, fc.gap_at, fc.n_gaps, k - 1, D, st));
         AGather ga1;
         RowMap rm1;
         conv1d_gather(fc.B, fc.T, D, k, &ga1, &rm1);
         rm1.q1 = R1;                                           // output rows stay on the padded grid ...
         e1.c_act = fp + (long long)lead * FF;                  // ... shifted past the leading zero rows
         FO_TRY(gemm<TA>(c, hp, ga1, w.w1, (int)ga1.rows, FF, k * D, e1, rm1, st));
+        FO_TRY(zero_row_runs<TA>(fp + (long long)lead * FF, fc.gap_at, fc.n_gaps, k - 1, FF, st));
         conv1d_gather(fc.B, fc.T, FF, k, &ga2, &rm2);
         ffn2_in = fp;
         M2 = (int)ga2.rows;
@@ -1310,6 +1338,85 @@ int offline_program(fo_ctx* c, const float* feats, const int32_t* ilens_dev, int
         AdOut out;
         out.y = y_dev;
         FO_TRY(adapter_program<TA>(c, enc_out_dev, mask2, B, T2, nullptr, nullptr, nullptr, out, st));
+    }
+    return 0;
+}
+
+// Device tables of a packed call (fo_encode_offline_packed), one int32 upload; each field is an offset into it.
+struct PackTab {
+    int B = 0, tmax = 0, fmax = 0;    // utterances, longest in encoder rows, longest in feature frames
+    int rows = 0, trunk = 0, ad_rows = 0, gap = 0, tiles = 0, grid_frames = 0;
+    int o_tiles = 0, o_lens = 0, o_eoff = 0, o_xrow = 0, o_grow = 0, o_flen = 0, o_foff = 0, o_frow = 0, o_gaps = 0, o_adcnt = 0,
+        o_aoff = 0;
+    std::vector<int32_t> h;
+};
+// Packed twin of offline_program: B utterances back to back, every kernel on their rows only.
+//  - front: the features go onto one grid where every utterance starts at a multiple of 4 frames (the subsampling's stride),
+//    so each conv2 output row sees the frames of one utterance; its rows (at most 2 extra per utterance) are gathered out.
+//  - layers: row-generic GEMMs / LayerNorms over all rows; attention per (utterance, query tile) from a tile table; the
+//    depthwise conv restarts at each utterance.  MultiLayeredConv1d (two-sided conv) keeps k - 1 zeroed rows between
+//    utterances in the residual stream (`gap`), and the encoder rows are gathered out of it at the end.
+//  - adapter: adapter_program's packed mode.
+template <typename TA>
+int offline_packed_program(fo_ctx* c, const float* feats, const PackTab& p, const int32_t* tab, int chunk, int left,
+                           float* enc_out_dev, float* y_dev, cudaStream_t st) {
+    const int D = c->D, FF = c->FF, H = c->H, F = c->F, B = p.B, M = p.trunk;
+    void *fg, *xp;
+    FO_TRY(ws_ensure(c, WS_FGRID, (size_t)p.grid_frames * F * sizeof(float), &fg));
+    FO_CUDA(cudaMemsetAsync(fg, 0, (size_t)p.grid_frames * F * sizeof(float), st));
+    FO_TRY(copy_utt_rows(feats, tab + p.o_foff, reinterpret_cast<float*>(fg), tab + p.o_frow, tab + p.o_flen, B, p.fmax, F, st));
+    float* xg;
+    FO_TRY(subsample_program<TA>(c, reinterpret_cast<const float*>(fg), 1, p.grid_frames, &xg, st));
+    FO_TRY(ws_ensure(c, WS_XP, (size_t)M * D * sizeof(float), &xp));
+    float* x = reinterpret_cast<float*>(xp);
+    if (p.gap) FO_CUDA(cudaMemsetAsync(x, 0, (size_t)M * D * sizeof(float), st));
+    FO_TRY(copy_utt_rows(xg, tab + p.o_grow, x, tab + p.o_xrow, tab + p.o_lens, B, p.tmax, D, st));
+    void *h, *qkv, *att, *ffh;
+    FO_TRY(ws_ensure(c, WS_H, (size_t)(c->cfg.concat_after ? 2 : 1) * M * D * sizeof(TA), &h));
+    FO_TRY(ws_ensure(c, WS_QKV, (size_t)M * 3 * D * sizeof(TA), &qkv));
+    FO_TRY(ws_ensure(c, WS_ATT, (size_t)M * D * sizeof(TA), &att));
+    FO_TRY(ws_ensure(c, WS_FFH, (size_t)M * FF * sizeof(TA), &ffh));
+    float* q32 = reinterpret_cast<float*>(qkv);
+    if (sizeof(TA) == 2) { void* q; FO_TRY(ws_ensure(c, WS_Q32, (size_t)M * 3 * D * sizeof(float), &q)); q32 = reinterpret_cast<float*>(q); }
+    void* hc = nullptr;
+    if (c->KF >= 2) FO_TRY(ws_ensure(c, WS_HC, (size_t)M * D * sizeof(TA), &hc));
+    void *hp = nullptr, *fp = nullptr;
+    if (c->KM) {
+        const size_t rows = (size_t)M + c->KM - 1;
+        FO_TRY(ws_ensure(c, WS_HP, rows * D * sizeof(TA), &hp));
+        FO_TRY(ws_ensure(c, WS_FP, rows * FF * sizeof(TA), &fp));
+        FO_CUDA(cudaMemsetAsync(fp, 0, rows * FF * sizeof(TA), st));
+    }
+    float* enc_rows = enc_out_dev;                  // the last layer's output rows: straight to enc_out unless there are gaps
+    if (p.gap) { void* e; FO_TRY(ws_ensure(c, WS_ENC2, (size_t)M * D * sizeof(float), &e)); enc_rows = reinterpret_cast<float*>(e); }
+    AttnVarlen vl;
+    vl.tiles = reinterpret_cast<const int2*>(tab + p.o_tiles);
+    vl.lens = tab + p.o_lens;
+    vl.rows = tab + p.o_xrow;
+    vl.n = p.tiles;
+    if (c->cfg.post_norm) FO_TRY(to_act<TA>(x, reinterpret_cast<TA*>(h), (long long)M * D, st));
+    else FO_TRY(layer_norm<TA>(x, M, D, c->layers[0].ln1g, c->layers[0].ln1b, 1e-5f, 0, 1.0f, reinterpret_cast<TA*>(h), nullptr, st));
+    for (int l = 0; l < c->L; ++l) {
+        const LayerW& w = c->layers[l];
+        const bool last = l + 1 == c->L;
+        FO_TRY(layer_pre<TA>(c, w, M, reinterpret_cast<TA*>(h), reinterpret_cast<TA*>(qkv), q32, L2Prefetch(), st));
+        if (!(c->debug_skip & 1))
+        FO_TRY(attention_offline_packed<TA>(reinterpret_cast<const TA*>(qkv), q32, vl, B, p.tmax, H, chunk, left, w.ptab,
+                                            reinterpret_cast<const TA*>(w.ptab_h), c->pos_rows, w.pos_u, w.pos_v,
+                                            reinterpret_cast<TA*>(att), st));
+        NextNorm nn{last ? c->after_g : c->layers[l + 1].ln1g, last ? c->after_b : c->layers[l + 1].ln1b, last ? enc_rows : nullptr};
+        FfnConv fc;
+        fc.ids = nullptr; fc.layer = l; fc.hc = hc; fc.hp = hp; fc.fp = fp;
+        if (c->KM) { fc.B = 1; fc.T = M; fc.gap_at = tab + p.o_gaps; fc.n_gaps = B - 1; }
+        else { fc.B = B; fc.T = p.tmax; fc.cnt = tab + p.o_lens; fc.off = tab + p.o_eoff; fc.t = 1; }
+        FO_TRY(layer_post<TA>(c, w, x, M, reinterpret_cast<TA*>(att), reinterpret_cast<TA*>(h), reinterpret_cast<TA*>(ffh), nn, nullptr, fc, st));
+    }
+    if (p.gap) FO_TRY(copy_utt_rows(enc_rows, tab + p.o_xrow, enc_out_dev, tab + p.o_eoff, tab + p.o_lens, B, p.tmax, D, st));
+    if (c->cfg.has_adapter && y_dev) {
+        AdOut out;
+        out.y = y_dev;
+        const AdPack pk{tab + p.o_adcnt, tab + p.o_eoff, tab + p.o_aoff, p.ad_rows};
+        FO_TRY(adapter_program<TA>(c, enc_out_dev, nullptr, B, p.tmax, nullptr, nullptr, nullptr, out, st, nullptr, &pk));
     }
     return 0;
 }
@@ -2535,6 +2642,82 @@ int fo_encode_offline(fo_ctx* c, const float* feats, const int32_t* ilens, int B
     if (adapter_out) FO_TRY(out_done(adapter_out, dy, y_bytes, st));
     c->stats.offline_calls += 1;
     c->stats.offline_frames += (long long)B * T2;
+    return 0;
+}
+
+// ---- full utterances packed end to end ---------------------------------------------------------------------
+int fo_encode_offline_packed(fo_ctx* c, const float* feats, const int32_t* lens, int B, int chunk, int left, float* enc_out,
+                             float* adapter_out, void* stream) {
+    FO_CHECK(c && c->finalized && c->cfg.has_encoder, "fo_encode_offline_packed: context has no finalized encoder");
+    FO_CHECK(feats && lens && B > 0 && B <= 65535, "fo_encode_offline_packed: need feats, lens and 1 <= B <= 65535");
+    if (adapter_out) FO_CHECK(c->cfg.has_adapter, "adapter_out requested but the context has no adapter");
+    FO_CUDA(cudaSetDevice(c->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    PackTab p;
+    p.B = B;
+    std::vector<int32_t> T(B);
+    if (is_device_ptr(lens)) {
+        FO_CUDA(cudaMemcpyAsync(T.data(), lens, (size_t)B * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+        FO_CUDA(cudaStreamSynchronize(st));
+    } else {
+        std::copy(lens, lens + B, T.begin());
+    }
+    const int ns = c->cfg.has_adapter ? c->ad_nst : 0, tq = attention_offline_tile_rows(c->dtype == FO_BF16);
+    p.gap = c->KM ? c->KM - 1 : 0;
+    long long frames = 0, rows = 0, ad_rows = 0, grid = 0, tiles = 0;
+    for (int b = 0; b < B; ++b) {
+        FO_CHECK(T[b] >= 7, "fo_encode_offline_packed: utterance %d has %d feature frames; each needs >= 7", b, T[b]);
+        const int t2 = ((T[b] - 1) / 2 - 1) / 2;
+        FO_CHECK(t2 <= c->cfg.pos_max_len, "fo_encode_offline_packed: utterance %d has %d encoder frames, past the positional table (%d)",
+                 b, t2, c->cfg.pos_max_len);
+        frames += T[b];
+        rows += t2;
+        ad_rows += ad_frames(c, t2);
+        grid += b + 1 < B ? (T[b] + 3) / 4 * 4 : T[b];
+        tiles += cdiv(t2, tq);
+        p.tmax = std::max(p.tmax, t2);
+        p.fmax = std::max(p.fmax, T[b]);
+    }
+    FO_CHECK(grid < (1LL << 28), "fo_encode_offline_packed: %lld feature frames in one call; pass fewer utterances", frames);
+    p.rows = (int)rows; p.ad_rows = (int)ad_rows; p.grid_frames = (int)grid; p.tiles = (int)tiles;
+    p.trunk = (int)(rows + (long long)(B - 1) * p.gap);
+    // table: tiles {b, q} | lens | eoff | xrow | grow | flen | foff | frow | gaps | adcnt | aoff
+    p.o_tiles = 0; p.o_lens = 2 * p.tiles; p.o_eoff = p.o_lens + B; p.o_xrow = p.o_eoff + B + 1; p.o_grow = p.o_xrow + B;
+    p.o_flen = p.o_grow + B; p.o_foff = p.o_flen + B; p.o_frow = p.o_foff + B + 1; p.o_gaps = p.o_frow + B;
+    p.o_adcnt = p.o_gaps + B; p.o_aoff = p.o_adcnt + (ns + 1) * B;
+    std::vector<int32_t>& h = p.h;
+    h.assign(p.o_aoff + B + 1, 0);
+    int32_t* tl = h.data();
+    for (int b = 0, g = 0; b < B; ++b) {
+        const int t2 = ((T[b] - 1) / 2 - 1) / 2;
+        h[p.o_lens + b] = t2;
+        h[p.o_eoff + b + 1] = h[p.o_eoff + b] + t2;
+        h[p.o_xrow + b] = h[p.o_eoff + b] + b * p.gap;
+        h[p.o_gaps + b] = h[p.o_xrow + b] + t2;
+        h[p.o_frow + b] = g;
+        h[p.o_grow + b] = g / 4;                           // encoder row of frame g on the grid: rows 4 r .. 4 r + 6 feed row r
+        h[p.o_flen + b] = T[b];
+        h[p.o_foff + b + 1] = h[p.o_foff + b] + T[b];
+        g += (T[b] + 3) / 4 * 4;
+        for (int i = 0; i <= ns; ++i) h[p.o_adcnt + i * B + b] = ad_frames(c, t2, i);
+        h[p.o_aoff + b + 1] = h[p.o_aoff + b] + ad_frames(c, t2);
+        for (int q = 0; q < cdiv(t2, tq); ++q) { *tl++ = b; *tl++ = q; }
+    }
+    void *dtab, *dfeats, *denc, *dy = nullptr;
+    FO_TRY(ws_ensure(c, WS_PKTAB, h.size() * sizeof(int32_t), &dtab));
+    FO_CUDA(cudaMemcpyAsync(dtab, h.data(), h.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    FO_TRY(in_dev(c, feats, (size_t)frames * c->F * sizeof(float), WS_FEATS, st, (const void**)&dfeats));
+    const size_t enc_bytes = (size_t)rows * c->D * sizeof(float), y_bytes = (size_t)ad_rows * c->E * sizeof(float);
+    FO_TRY(out_dev(c, enc_out, enc_bytes, WS_ENC, &denc));
+    if (adapter_out) FO_TRY(out_dev(c, adapter_out, y_bytes, WS_Y, &dy));
+    const int32_t* tab = reinterpret_cast<const int32_t*>(dtab);
+    FO_TRY(c->dtype == FO_BF16
+               ? offline_packed_program<act16>(c, (const float*)dfeats, p, tab, chunk, left, (float*)denc, (float*)dy, st)
+               : offline_packed_program<float>(c, (const float*)dfeats, p, tab, chunk, left, (float*)denc, (float*)dy, st));
+    if (enc_out) FO_TRY(out_done(enc_out, denc, enc_bytes, st));
+    if (adapter_out) FO_TRY(out_done(adapter_out, dy, y_bytes, st));
+    c->stats.offline_calls += 1;
+    c->stats.offline_frames += rows;
     return 0;
 }
 

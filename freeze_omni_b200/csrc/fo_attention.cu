@@ -517,6 +517,27 @@ constexpr int KT = 96;         // key tile: the shipped band of a 32-query block
 constexpr int QB = 32;          // query rows per CTA
 constexpr int QPW = QB / (ATT_THREADS / 32);   // queries per warp
 
+// Which query tile of which utterance a CTA of the offline kernels takes, and where that utterance's rows are.  Padded
+// (VL = false): tile blockIdx.x of utterance blockIdx.z, rows b * T.., keys cut by the pad mask ilens.  Packed (VL = true,
+// attention_offline_packed): entry blockIdx.x of the tile table; T becomes the utterance's own length, every key of it valid.
+template <bool VL>
+__device__ __forceinline__ void utterance_tile(const AttnVarlen& vl, const int32_t* ilens, int& T, int& qb, int& b, int& klen,
+                                               long long& row0) {
+    if constexpr (VL) {
+        const int2 tl = vl.tiles[blockIdx.x];
+        b = tl.x;
+        qb = tl.y;
+        T = vl.lens[b];
+        klen = T;
+        row0 = vl.rows[b];
+    } else {
+        qb = blockIdx.x;
+        b = blockIdx.z;
+        klen = ilens ? min(ilens[b], T) : T;               // pad mask on keys (masks.py:110-120)
+        row0 = (long long)b * T;
+    }
+}
+
 // Full-utterance attention.  CTA = (32-query block, head, utterance), 4 warps x 8 queries.  The union of the block's
 // key windows is walked in tiles of 96 keys (K, V and the rel-pos rows staged once per tile and shared by the 32
 // queries; rows padded by 16 B so that lanes reading different rows hit different banks).  Scores are register
@@ -525,10 +546,12 @@ constexpr int QPW = QB / (ATT_THREADS / 32);   // queries per warp
 // masks.py:50-56 and the pad mask (masks.py:110-120) are applied arithmetically; online softmax across tiles
 // (unbounded left context works); PV with lane = output dims.  A row whose whole window is masked yields zeros
 // (attention.py:396-397).  fp32 contexts; fp16 contexts run attention_offline_fa_kernel below.
+template <bool VL>
 __global__ void __launch_bounds__(ATT_THREADS)
 attention_offline_kernel(const float* __restrict__ qkv, const float* __restrict__ q32, int T, int H,
                          const int32_t* __restrict__ ilens, int chunk, int left, const float* __restrict__ ptab,
-                         const float* __restrict__ pos_u, const float* __restrict__ pos_v, float* __restrict__ out) {
+                         const float* __restrict__ pos_u, const float* __restrict__ pos_v, float* __restrict__ out,
+                         AttnVarlen vl) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     constexpr int EPC = 4, NCH = DK / EPC;
     constexpr int DKP = DK + EPC;                          // padded row (16 B): conflict-free 16-byte row reads
@@ -541,11 +564,13 @@ attention_offline_kernel(const float* __restrict__ qkv, const float* __restrict_
     float* prob = qv + QB * DK;                            // warps x KT
     __shared__ int win[QB][2];
 
-    const int qb = blockIdx.x, h = blockIdx.y, b = blockIdx.z;
+    const int h = blockIdx.y;
+    int qb, b, klen;
+    long long row0;
+    utterance_tile<VL>(vl, ilens, T, qb, b, klen, row0);
     const int D = H * DK;
     const int q0 = qb * QB;
     const int nq = min(QB, T - q0);
-    const int klen = ilens ? min(ilens[b], T) : T;        // pad mask on keys (masks.py:110-120)
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
 
     if (tid < QB) {
@@ -565,7 +590,7 @@ attention_offline_kernel(const float* __restrict__ qkv, const float* __restrict_
     for (int i = tid; i < QB * (DK / 4); i += ATT_THREADS) {
         const int r = i / (DK / 4), c = (i % (DK / 4)) * 4;
         float4 q = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (r < nq) q = *reinterpret_cast<const float4*>(q32 + ((long long)b * T + q0 + r) * 3 * D + h * DK + c);
+        if (r < nq) q = *reinterpret_cast<const float4*>(q32 + (row0 + q0 + r) * 3 * D + h * DK + c);
         const float4 u = *reinterpret_cast<const float4*>(pos_u + h * DK + c);
         const float4 v = *reinterpret_cast<const float4*>(pos_v + h * DK + c);
         *reinterpret_cast<float4*>(qu + r * DK + c) = make_float4(q.x + u.x, q.y + u.y, q.z + u.z, q.w + u.w);
@@ -587,7 +612,7 @@ attention_offline_kernel(const float* __restrict__ qkv, const float* __restrict_
         for (int i = tid; i < nk * NCH * 2; i += ATT_THREADS) {
             const int which = i / (nk * NCH);              // 0 K, 1 V
             const int j = (i / NCH) % nk, c = i % NCH;
-            const float* src = qkv + ((long long)b * T + kt + j) * 3 * D + (which + 1) * D + h * DK + c * EPC;
+            const float* src = qkv + (row0 + kt + j) * 3 * D + (which + 1) * D + h * DK + c * EPC;
             float* dst = (which == 0 ? Ks : Vs) + j * DKP + c * EPC;
             *reinterpret_cast<uint4*>(dst) = *reinterpret_cast<const uint4*>(src);
         }
@@ -685,7 +710,7 @@ attention_offline_kernel(const float* __restrict__ qkv, const float* __restrict_
         const int r = warp * QPW + qi;
         if (r < nq) {
             const float inv = l_run[qi] > 0.f ? 1.f / l_run[qi] : 0.f;
-            float* o = out + ((long long)b * T + q0 + r) * D + h * DK + 2 * lane;
+            float* o = out + (row0 + q0 + r) * D + h * DK + 2 * lane;
             o[0] = o0[qi] * inv;
             o[1] = o1[qi] * inv;
         }
@@ -733,19 +758,22 @@ __device__ __forceinline__ uint32_t pack2_nosat(float a, float b) {      // valu
     __half2 h = __floats2half2_rn(a, b);
     return *reinterpret_cast<uint32_t*>(&h);
 }
+template <bool VL>
 __global__ void __launch_bounds__(ATT_THREADS, 4)
 attention_offline_fa_kernel(const __half* __restrict__ qkv, const float* __restrict__ q32, int T, int H,
                             const int32_t* __restrict__ ilens, int chunk, int left, const __half* __restrict__ ptab_h,
                             int pos_rows, const float* __restrict__ pos_u, const float* __restrict__ pos_v,
-                            __half* __restrict__ out) {
+                            __half* __restrict__ out, AttnVarlen vl) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     typedef __half TA;
     constexpr int NCH = 8;                                   // 16-byte chunks per 64-element row
     TA* tiles = reinterpret_cast<TA*>(smem_raw);             // [2 stages][K | P | V][FK][64]
-    const int qb = blockIdx.x, h = blockIdx.y, b = blockIdx.z;
+    const int h = blockIdx.y;
+    int qb, b, klen;
+    long long row0;
+    utterance_tile<VL>(vl, ilens, T, qb, b, klen, row0);
     const int D = H * DK;
     const int q0 = qb * FQ;
-    const int klen = ilens ? min(ilens[b], T) : T;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int g = lane >> 2, c = lane & 3;
 
@@ -777,7 +805,7 @@ attention_offline_fa_kernel(const __half* __restrict__ qkv, const float* __restr
                 else *reinterpret_cast<uint4*>(dst + (cc << 3)) = make_uint4(0, 0, 0, 0);
             } else {
                 TA* d2 = dst + ((cc ^ (j & 7)) << 3);
-                if (key < k_hi) cp_async16(d2, qkv + ((long long)b * T + key) * 3 * D + (which == 0 ? 1 : 2) * D + h * DK + cc * 8);
+                if (key < k_hi) cp_async16(d2, qkv + (row0 + key) * 3 * D + (which == 0 ? 1 : 2) * D + h * DK + cc * 8);
                 else *reinterpret_cast<uint4*>(d2) = make_uint4(0, 0, 0, 0);     // finite operands for the masked columns
             }
         }
@@ -788,8 +816,8 @@ attention_offline_fa_kernel(const __half* __restrict__ qkv, const float* __restr
     // (q+u), (q+v) A fragments of this warp's 16 queries: a0 (row g, k 2c..), a1 (row g+8), a2 (row g, k 2c+8..), a3 (row g+8)
     uint32_t qu[4][4], qv[4][4];
     {
-        const float* qr0 = q32 + ((long long)b * T + min(r0, T - 1)) * 3 * D + h * DK;
-        const float* qr1 = q32 + ((long long)b * T + min(r1, T - 1)) * 3 * D + h * DK;
+        const float* qr0 = q32 + (row0 + min(r0, T - 1)) * 3 * D + h * DK;
+        const float* qr1 = q32 + (row0 + min(r1, T - 1)) * 3 * D + h * DK;
 #pragma unroll
         for (int ks = 0; ks < 4; ++ks) {
 #pragma unroll
@@ -924,7 +952,7 @@ attention_offline_fa_kernel(const __half* __restrict__ qkv, const float* __restr
     for (int i = lane; i < 16 * NCH; i += 32) {
         const int r = i >> 3, cc = i & 7, row = q0 + warp * 16 + r;
         if (row < T)
-            *reinterpret_cast<uint4*>(out + ((long long)b * T + row) * D + h * DK + cc * 8) = *reinterpret_cast<const uint4*>(ot + r * DK + cc * 8);
+            *reinterpret_cast<uint4*>(out + (row0 + row) * D + h * DK + cc * 8) = *reinterpret_cast<const uint4*>(ot + r * DK + cc * 8);
     }
 }
 
@@ -1047,37 +1075,65 @@ template int ptab_head_major<float>(const float*, int, int, float*, cudaStream_t
 template int ptab_head_major<__half>(const float*, int, int, __half*, cudaStream_t);
 template int attention_stream<__half>(const AttnStream&, const __half*, const float*, __half*, const __half*, const float*, const float*, __half*, cudaStream_t);
 
+// One launcher for both forms: vl == null is the padded batch (grid x = query tiles, z = utterances), else the packed one
+// (grid x = vl->n tile table entries).
 template <typename TA>
-int attention_offline(const TA* qkv, const float* q32, int B, int T, int H, const int32_t* ilens, int chunk, int left,
-                      const float* ptab, const TA* ptab_h, int pos_rows, const float* pos_u, const float* pos_v, TA* out,
-                      cudaStream_t st) {
-    if (B <= 0 || T <= 0) return 0;
+int attention_offline_any(const TA* qkv, const float* q32, int B, int T, int H, const int32_t* ilens, int chunk, int left,
+                          const float* ptab, const TA* ptab_h, int pos_rows, const float* pos_u, const float* pos_v, TA* out,
+                          const AttnVarlen* vl, cudaStream_t st) {
+    if (B <= 0 || T <= 0 || (vl && vl->n <= 0)) return 0;
+    const AttnVarlen v = vl ? *vl : AttnVarlen();
     if constexpr (sizeof(TA) == 2) {
         if (!ptab_h || T > pos_rows) return 1;
         const size_t smem = (size_t)2 * 3 * FK * DK * 2;      // 48 KB: double-buffered K | P | V tiles
         static bool attr_set = false;
         if (!attr_set) {
-            FO_CUDA(cudaFuncSetAttribute(attention_offline_fa_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
+            FO_CUDA(cudaFuncSetAttribute(attention_offline_fa_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
+            FO_CUDA(cudaFuncSetAttribute(attention_offline_fa_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
             attr_set = true;
         }
-        attention_offline_fa_kernel<<<dim3(cdiv(T, FQ), H, B), ATT_THREADS, smem, st>>>(qkv, q32, T, H, ilens, chunk, left, ptab_h,
-                                                                                         pos_rows, pos_u, pos_v, out);
+        if (vl)
+            attention_offline_fa_kernel<true><<<dim3(v.n, H, 1), ATT_THREADS, smem, st>>>(qkv, q32, T, H, ilens, chunk, left, ptab_h,
+                                                                                         pos_rows, pos_u, pos_v, out, v);
+        else
+            attention_offline_fa_kernel<false><<<dim3(cdiv(T, FQ), H, B), ATT_THREADS, smem, st>>>(qkv, q32, T, H, ilens, chunk, left,
+                                                                                                  ptab_h, pos_rows, pos_u, pos_v, out, v);
     } else {
         const size_t smem = (size_t)3 * KT * (DK + 4) * 4 + (size_t)2 * QB * DK * 4 + (size_t)(ATT_THREADS / 32) * KT * 4;
         static bool attr_set = false;
         if (!attr_set) {
-            FO_CUDA(cudaFuncSetAttribute(attention_offline_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
+            FO_CUDA(cudaFuncSetAttribute(attention_offline_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
+            FO_CUDA(cudaFuncSetAttribute(attention_offline_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
             attr_set = true;
         }
-        attention_offline_kernel<<<dim3(cdiv(T, QB), H, B), ATT_THREADS, smem, st>>>(qkv, q32, T, H, ilens, chunk, left, ptab, pos_u,
-                                                                                    pos_v, out);
+        if (vl)
+            attention_offline_kernel<true><<<dim3(v.n, H, 1), ATT_THREADS, smem, st>>>(qkv, q32, T, H, ilens, chunk, left, ptab, pos_u,
+                                                                                      pos_v, out, v);
+        else
+            attention_offline_kernel<false><<<dim3(cdiv(T, QB), H, B), ATT_THREADS, smem, st>>>(qkv, q32, T, H, ilens, chunk, left, ptab,
+                                                                                               pos_u, pos_v, out, v);
     }
     FO_LAUNCHED();
     FO_CUDA(cudaGetLastError());
     return 0;
 }
+template <typename TA>
+int attention_offline(const TA* qkv, const float* q32, int B, int T, int H, const int32_t* ilens, int chunk, int left,
+                      const float* ptab, const TA* ptab_h, int pos_rows, const float* pos_u, const float* pos_v, TA* out,
+                      cudaStream_t st) {
+    return attention_offline_any<TA>(qkv, q32, B, T, H, ilens, chunk, left, ptab, ptab_h, pos_rows, pos_u, pos_v, out, nullptr, st);
+}
+template <typename TA>
+int attention_offline_packed(const TA* qkv, const float* q32, const AttnVarlen& vl, int B, int tmax, int H, int chunk, int left,
+                             const float* ptab, const TA* ptab_h, int pos_rows, const float* pos_u, const float* pos_v, TA* out,
+                             cudaStream_t st) {
+    return attention_offline_any<TA>(qkv, q32, B, tmax, H, nullptr, chunk, left, ptab, ptab_h, pos_rows, pos_u, pos_v, out, &vl, st);
+}
+int attention_offline_tile_rows(int is16) { return is16 ? FQ : QB; }
 template int attention_offline<float>(const float*, const float*, int, int, int, const int32_t*, int, int, const float*, const float*, int, const float*, const float*, float*, cudaStream_t);
 template int attention_offline<__half>(const __half*, const float*, int, int, int, const int32_t*, int, int, const float*, const __half*, int, const float*, const float*, __half*, cudaStream_t);
+template int attention_offline_packed<float>(const float*, const float*, const AttnVarlen&, int, int, int, int, int, const float*, const float*, int, const float*, const float*, float*, cudaStream_t);
+template int attention_offline_packed<__half>(const __half*, const float*, const AttnVarlen&, int, int, int, int, int, const float*, const __half*, int, const float*, const float*, __half*, cudaStream_t);
 
 int advance_sessions(const int32_t* ids, int n, int t, int chunk_size, int pe_wrap, int32_t* n_frames,
                       int32_t* pe_index, int32_t* adapter_valid, cudaStream_t st, int chunks, const int32_t* cnt) {

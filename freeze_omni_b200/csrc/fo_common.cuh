@@ -364,11 +364,19 @@ void conv1d_gather(int B, int T, int C, int k, AGather* ga, RowMap* rm);
 // (B, T, C) -> zero-padded (B, lead + T + trail, C) in the activation type
 template <typename TA>
 int pad_rows(const TA* in, int B, int T, int C, int lead, int trail, TA* out, cudaStream_t st);
+// runs of `gap` rows starting at rows at[0..n) of buf (device table) set to zero
+template <typename TA>
+int zero_row_runs(TA* buf, const int32_t* at, int n, int gap, int C, cudaStream_t st);
+// fp32 rows of n utterances moved between layouts: utterance b's lens[b] (<= rows_max) rows from src row srow[b] to dst
+// row drow[b] (device tables)
+int copy_utt_rows(const float* src, const int32_t* srow, float* dst, const int32_t* drow, const int32_t* lens, int n, int rows_max,
+                  int C, cudaStream_t st);
 // Conv1dLinear's causal depthwise Conv1d over time (attention.py:217-224,251): y[r][c] = b[c] + sum_tau w[c][tau] *
 // xin[r + tau][c], xin = [left context (k-1 rows) | x].  Streaming (ids != null): x is (n, t, C), the left context of
 // session ids[b] lives in slot_cache (fp32, (k-1, C) per slot, stride slot_stride) and is replaced by the last k-1 rows
 // of xin.  Offline (ids == null): x is (B, T, C) with zero left padding per utterance.  cnt / off (streaming, per-session
 // chunk counts): session b's rows are the cnt[b] * t rows from row (off[b] - off[0]) * t; T is then the largest of them.
+// With ids == null the same tables describe utterances packed end to end (t = 1), each with zero left context.
 template <typename TA>
 int depthwise_conv(const TA* x, int B, int T, int C, int k, const float* w, const float* bias, const int32_t* ids,
                    float* slot_cache, long long slot_stride, TA* y, cudaStream_t st, const int32_t* cnt = nullptr,
@@ -428,6 +436,21 @@ template <typename TA>
 int attention_offline(const TA* qkv, const float* q32, int B, int T, int H, const int32_t* ilens, int chunk, int left,
                       const float* ptab, const TA* ptab_h, int pos_rows, const float* pos_u, const float* pos_v, TA* out,
                       cudaStream_t st);
+// offline, utterances of different lengths packed end to end (fo_encode_offline_packed): utterance b has lens[b] rows from
+// row rows[b] of qkv / q32 / out, all valid, positions 0..lens[b]-1.  One CTA per tile table entry {b, query tile} and head;
+// the host lists ceil(lens[b] / attention_offline_tile_rows()) tiles per utterance.  Device pointers.
+struct AttnVarlen {
+    const int2* tiles = nullptr;
+    const int32_t* lens = nullptr;
+    const int32_t* rows = nullptr;
+    int n = 0;                    // tile table entries
+};
+int attention_offline_tile_rows(int is16);
+// tmax: the longest utterance (bounds pos_rows as T does for the padded form)
+template <typename TA>
+int attention_offline_packed(const TA* qkv, const float* q32, const AttnVarlen& vl, int B, int tmax, int H, int chunk, int left,
+                             const float* ptab, const TA* ptab_h, int pos_rows, const float* pos_u, const float* pos_v, TA* out,
+                             cudaStream_t st);
 // end of a streaming step: n_frames += t, pe_index = pe_index % wrap + chunk_size (attention.py:107,120),
 // and flip the live half of the double-buffered adapter cache.  Either group may be null.  chunks > 1: the session
 // advanced by that many chunks of t frames (pe_index stepped `chunks` times; the adapter cache still flips once).  cnt

@@ -590,6 +590,45 @@ int pad_rows(const TA* in, int B, int T, int C, int lead, int trail, TA* out, cu
 template int pad_rows<float>(const float*, int, int, int, int, int, float*, cudaStream_t);
 template int pad_rows<__half>(const __half*, int, int, int, int, int, __half*, cudaStream_t);
 
+// grid (gap, n): rows at[i] .. at[i] + gap - 1 of buf set to zero
+template <typename TA>
+__global__ void zero_row_runs_kernel(TA* __restrict__ buf, const int32_t* __restrict__ at, int C) {
+    FO_PDL_TRIGGER();
+    FO_PDL_WAIT();
+    TA* d = buf + ((long long)at[blockIdx.y] + blockIdx.x) * C;
+    for (int c = threadIdx.x; c < C; c += blockDim.x) d[c] = from_f<TA>(0.f);
+}
+template <typename TA>
+int zero_row_runs(TA* buf, const int32_t* at, int n, int gap, int C, cudaStream_t st) {
+    if (n <= 0 || gap <= 0) return 0;
+    FO_CUDA(launch_pdl(zero_row_runs_kernel<TA>, dim3(gap, n), dim3(128), 0, st, buf, at, C));
+    FO_LAUNCHED();
+    FO_CUDA(cudaGetLastError());
+    return 0;
+}
+template int zero_row_runs<float>(float*, const int32_t*, int, int, int, cudaStream_t);
+template int zero_row_runs<__half>(__half*, const int32_t*, int, int, int, cudaStream_t);
+
+// grid (rows_max, n): row r < lens[b] of utterance b, src row srow[b] + r -> dst row drow[b] + r
+__global__ void copy_utt_rows_kernel(const float* __restrict__ src, const int32_t* __restrict__ srow, float* __restrict__ dst,
+                                     const int32_t* __restrict__ drow, const int32_t* __restrict__ lens, int C) {
+    FO_PDL_TRIGGER();
+    FO_PDL_WAIT();
+    const int b = blockIdx.y, r = blockIdx.x;
+    if (r >= lens[b]) return;
+    const float* s = src + ((long long)srow[b] + r) * C;
+    float* d = dst + ((long long)drow[b] + r) * C;
+    for (int c = threadIdx.x; c < C; c += blockDim.x) d[c] = s[c];
+}
+int copy_utt_rows(const float* src, const int32_t* srow, float* dst, const int32_t* drow, const int32_t* lens, int n, int rows_max,
+                  int C, cudaStream_t st) {
+    if (n <= 0 || rows_max <= 0) return 0;
+    FO_CUDA(launch_pdl(copy_utt_rows_kernel, dim3(rows_max, n), dim3(C >= 256 ? 256 : 128), 0, st, src, srow, dst, drow, lens, C));
+    FO_LAUNCHED();
+    FO_CUDA(cudaGetLastError());
+    return 0;
+}
+
 template <typename TA>
 int conv_stage(const float* in, const uint8_t* mask, int B, int T, int C, int km1, int stride, const float* scale,
                const float* shift, const int32_t* ids, float* slot_cache, int32_t* slot_valid, const float* cache_in,
@@ -666,7 +705,7 @@ int depthwise_conv(const TA* x, int B, int T, int C, int k, const float* w, cons
                    float* slot_cache, long long slot_stride, TA* y, cudaStream_t st, const int32_t* cnt, const int32_t* off, int t) {
     if (B <= 0 || T <= 0) return 0;
     FO_CHECK(k >= 2 && k <= DW_KMAX, "depthwise_conv: kernel size %d outside 2..%d", k, DW_KMAX);
-    FO_CHECK(!cnt || (ids && off && t > 0), "depthwise_conv: per-session counts are a streaming layout");
+    FO_CHECK(!cnt || (off && t > 0), "depthwise_conv: per-session counts need their row offsets");
     if (ids && (T > DW_TB || cnt)) {
         // streaming, several chunks per session (fo_encode_stream_chunks[_v]): the first rows read the carried context and the
         // last ones replace it, so the row blocks run in order, one launch each (up to the largest session's rows)
@@ -677,9 +716,11 @@ int depthwise_conv(const TA* x, int B, int T, int C, int k, const float* w, cons
         }
         return 0;
     }
+    // one launch: per-utterance rows with zero left context (offline; cnt / off: utterances packed end to end, T the longest),
+    // or a streaming call whose sessions' rows fit one row block
     dim3 grid(cdiv(T, DW_TB), B);
     FO_CUDA(launch_pdl(depthwise_conv_kernel<TA>, grid, dim3(256), 0, st, x, T, C, k, w, bias, ids, slot_cache, slot_stride, y, 0,
-                       (const int32_t*)nullptr, (const int32_t*)nullptr, 0));
+                       cnt, off, t));
     FO_LAUNCHED();
     return 0;
 }

@@ -470,6 +470,26 @@ class Engine:
                                               _ptr(mask), _ptr(y), _ptr(ymask), self._stream()))
         return enc, mask.bool().unsqueeze(1), y, (ymask.bool().unsqueeze(1) if want_adapter else None)
 
+    def encode_offline_packed(self, feats: ArrayLike, lens, chunk: Optional[int] = None, left: Optional[int] = None,
+                              want_adapter: Optional[bool] = None):
+        """Utterances of different lengths packed end to end, no padding rows.  feats (sum T_i, F), lens (B) the T_i.
+        Returns (enc (sum T'_i, D), adapter rows (sum T''_i, E) or None, enc_offsets, adapter_offsets); the offsets are
+        int64 (B + 1) prefix sums, utterance i's rows being [off[i], off[i+1]).  Each utterance's rows equal the padded
+        forward of it alone."""
+        N, F = feats.shape
+        assert F == self.cfg.feat_dim
+        ln = np.ascontiguousarray(np.asarray(lens.cpu() if isinstance(lens, torch.Tensor) else lens, dtype=np.int32).reshape(-1))
+        assert int(ln.sum()) == N, "lens must sum to the feature rows"
+        chunk = self.cfg.chunk_size if chunk is None else int(chunk)
+        left = self.cfg.left_chunks if left is None else int(left)
+        eoff, aoff = self.cfg.packed_offsets(ln)
+        want_adapter = self.has_adapter if want_adapter is None else want_adapter
+        enc = torch.empty(int(eoff[-1]), self.cfg.d_model, device=self.torch_device)
+        y = torch.empty(int(aoff[-1]), self.cfg.llm_dim, device=self.torch_device) if want_adapter else None
+        _lib.check(self.lib.fo_encode_offline_packed(self._h, _ptr(feats), ln.ctypes.data, len(ln), chunk, left, _ptr(enc), _ptr(y),
+                                                     self._stream()))
+        return enc, y, eoff, aoff
+
     def adapter_forward(self, x: torch.Tensor, mask: Optional[torch.Tensor], cache):
         """Stateless adapter: x (B,T,D), mask (B,1,T)|(B,T) bool or None.  `cache`: None, a tensor (B,D,k-1) (single-conv
         CNNSubsampling), or the reference's list [c0 (B,2D,k-1), c1 (B,D,k-1)] for the two-conv branch (entries may be None

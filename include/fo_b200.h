@@ -251,6 +251,15 @@ int fo_encode_offline(fo_ctx* ctx, const float* feats, const int32_t* ilens, int
                       float* enc_out, uint8_t* mask_out, float* adapter_out, uint8_t* adapter_mask_out,
                       void* stream);
 
+/* ---- full utterances of different lengths packed end to end, no padding rows: utterance i (T_i >= 7 feature frames) gets
+ * exactly the rows speechEncoder.forward + CNNSubsampling.forward(cache=None) (or the configured adapter) return for it alone.
+ * feats (sum T_i, feat_dim), lens (B) int32 T_i; enc_out (sum T'_i, d_model) with T'_i = ((T_i - 1)/2 - 1)/2, adapter_out
+ * (sum T''_i, llm_dim) with T''_i = (T'_i - 1)/2 + 1 for CNNSubsampling and T'_i for CNNAdapter / LinearAdapter, both in
+ * utterance order, every row valid; either may be NULL.  chunk / left as for fo_encode_offline.  FO_ERR_ARG, with nothing
+ * enqueued, for B <= 0, a T_i < 7 or a T'_i past pos_max_len. */
+int fo_encode_offline_packed(fo_ctx* ctx, const float* feats, const int32_t* lens, int B, int chunk, int left,
+                             float* enc_out, float* adapter_out, void* stream);
+
 /* ---- stateless adapter: replaces CNNSubsampling.forward (models/adapter.py:112-157) when the
  * caller owns the cache tensor.  x (B, T, d_model); mask (B, T) uint8 or NULL (all valid);
  * cache_in (B, d_model, kernel-1) or NULL (left zero pad); cache_out same shape or NULL;
