@@ -78,7 +78,11 @@ SYMBOLS = {
     "fo_profile_dump": (C.c_int, [_P, C.c_char_p, C.c_int]),
     "fo_debug_gemm": (C.c_int, [_P, _P, _P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                 C.POINTER(C.c_float), _P]),
+    "fo_debug_attention": (C.c_int, [_P, C.c_int, C.c_int, _I32P, _I32P, _I32P] + [C.c_int] * 7 + [_P, _P, C.c_int, _P, _P, C.c_int,
+                                                                                           _P, _P, _P, _P]),
 }
+
+FO_ATT_OFFLINE, FO_ATT_PACKED, FO_ATT_STREAM, FO_ATT_CHUNKS = 0, 1, 2, 3
 
 _lib: Optional[C.CDLL] = None
 

@@ -1421,6 +1421,82 @@ int offline_packed_program(fo_ctx* c, const float* feats, const PackTab& p, cons
     return 0;
 }
 
+// Arguments of fo_debug_attention once checked: the device tables (`tab`, uploaded to the entry's own scratch), the rows of
+// qkv / out, and the launch geometry of the mode.
+struct DebugAttn {
+    int mode = 0, n = 0, T = 0, chunk = 0, left = 0, t = 0, layer = 0, group = 1, groups = 1, tmax = 0, ntiles = 0, nsplit = 0;
+    long long rows = 0;
+    std::vector<int32_t> tab;          // offline: ilens | packed: tiles {b, q}, lens, rows | streaming: ids, cnt, off
+    const float *qkv = nullptr, *part = nullptr, *part_bias = nullptr, *ptab = nullptr, *pos_u = nullptr, *pos_v = nullptr;
+    float* out = nullptr;
+};
+
+// fo_debug_attention in the context's element type: K|V and the rel-pos table converted as the step programs hold them, one
+// launcher call, the output converted back to fp32.  Nothing here advances a session or touches the step's id tables.
+template <typename TA>
+int debug_attention_run(fo_ctx* c, const DebugAttn& d, cudaStream_t st) {
+    const int D = c->D, H = c->H;
+    constexpr bool F16 = sizeof(TA) == 2;
+    const bool need_qkv = F16 && d.nsplit == 0;
+    const size_t tab_b = (d.tab.size() * sizeof(int32_t) + 255) & ~(size_t)255;
+    const size_t qkv_b = need_qkv ? (((size_t)d.rows * 3 * D * sizeof(TA) + 255) & ~(size_t)255) : 0;
+    const size_t ptab_b = ((size_t)H * c->pos_rows * 64 * sizeof(TA) + 255) & ~(size_t)255;
+    const size_t out_b = F16 ? (size_t)d.rows * D * sizeof(TA) : 0;
+    char* scratch = nullptr;
+    FO_CUDA(cudaMalloc(&scratch, tab_b + qkv_b + ptab_b + out_b));
+    int32_t* tab = reinterpret_cast<int32_t*>(scratch);
+    TA* qkv = need_qkv ? reinterpret_cast<TA*>(scratch + tab_b) : F16 ? nullptr : reinterpret_cast<TA*>(const_cast<float*>(d.qkv));
+    TA* ptab_h = reinterpret_cast<TA*>(scratch + tab_b + qkv_b);
+    TA* out = F16 ? reinterpret_cast<TA*>(scratch + tab_b + qkv_b + ptab_b) : reinterpret_cast<TA*>(d.out);
+    int r = 0;
+    auto run = [&]() -> int {
+        FO_CUDA(cudaMemcpyAsync(tab, d.tab.data(), d.tab.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+        if (need_qkv) FO_TRY(f32_to_act16(d.qkv, reinterpret_cast<act16*>(qkv), d.rows * 3 * D, st));
+        FO_TRY(ptab_head_major<TA>(d.ptab, c->pos_rows, H, ptab_h, st));
+        FO_CUDA(cudaMemsetAsync(out, 0, (size_t)d.rows * D * sizeof(TA), st));      // rows no query writes (packed gaps) read 0
+        if (d.mode == FO_ATT_OFFLINE)
+            return attention_offline<TA>(qkv, d.qkv, d.n, d.T, H, tab, d.chunk, d.left, d.ptab, ptab_h, c->pos_rows, d.pos_u,
+                                         d.pos_v, out, st);
+        if (d.mode == FO_ATT_PACKED) {
+            AttnVarlen vl;
+            vl.tiles = reinterpret_cast<const int2*>(tab);
+            vl.lens = tab + 2 * d.ntiles;
+            vl.rows = vl.lens + d.n;
+            vl.n = d.ntiles;
+            return attention_offline_packed<TA>(qkv, d.qkv, vl, d.n, d.tmax, H, d.chunk, d.left, d.ptab, ptab_h, c->pos_rows,
+                                                d.pos_u, d.pos_v, out, st);
+        }
+        AttnStream a;                     // as stream_program fills it
+        a.ids = tab;
+        a.n_frames = c->n_frames;
+        a.pe_index = c->pe_index;
+        a.n = d.n; a.t = d.t; a.H = H; a.ring_cap = c->ring_cap; a.window = c->window; a.full_chunk = c->full_chunk;
+        a.pe_wrap = c->pe_wrap; a.pos_rows = c->pos_rows;
+        a.ring_slot_stride = 2LL * H * c->ring_cap * 64;
+        a.chunk_size = c->cfg.chunk_size;
+        TA* ring_l = reinterpret_cast<TA*>(c->ring) + (long long)d.layer * c->cfg.max_sessions * a.ring_slot_stride;
+        if (d.mode == FO_ATT_STREAM) {
+            if (d.nsplit > 0) {
+                a.part = d.part;
+                a.part_bias = d.part_bias;
+                a.nsplit = d.nsplit;
+                a.part_stride = d.rows * 3 * D;
+            }
+            return attention_stream<TA>(a, qkv, d.qkv, ring_l, ptab_h, d.pos_u, d.pos_v, out, st);
+        }
+        a.cnt = tab + d.n;
+        a.off = tab + 2 * d.n;
+        a.chunks = d.group;
+        return attention_chunks<TA>(a, d.groups, qkv, d.qkv, ring_l, ptab_h, d.pos_u, d.pos_v, out, st);
+    };
+    r = run();
+    if (r == 0 && F16) r = act16_to_f32(reinterpret_cast<const act16*>(out), d.out, d.rows * D, st);
+    const cudaError_t e = cudaStreamSynchronize(st);
+    cudaFree(scratch);
+    if (r == 0 && e != cudaSuccess) { set_error("fo_debug_attention: %s", cudaGetErrorString(e)); r = FO_ERR_CUDA; }
+    return r;
+}
+
 }  // namespace
 
 // =================================================================================================
@@ -3005,6 +3081,77 @@ int fo_debug_gemm(fo_ctx* c, const float* A, const float* W, const float* bias, 
     FO_CUDA(e);
     if (ms_out) *ms_out = iters > 0 ? ms / iters : 0.f;
     return 0;
+}
+
+int fo_debug_attention(fo_ctx* c, int mode, int n, const int32_t* seq, const int32_t* cnt, const int32_t* off, int T, int gap,
+                       int chunk, int left, int t, int layer, int group, const float* qkv, const float* part, int nsplit,
+                       const float* part_bias, const float* ptab, int ptab_rows, const float* pos_u, const float* pos_v,
+                       float* out, void* stream) {
+    FO_CHECK(c && c->finalized && c->cfg.has_encoder, "fo_debug_attention: context has no finalized encoder");
+    FO_CHECK(mode >= FO_ATT_OFFLINE && mode <= FO_ATT_CHUNKS && n > 0 && seq && ptab && pos_u && pos_v && out,
+             "fo_debug_attention: bad argument");
+    FO_CHECK(ptab_rows >= c->pos_rows, "fo_debug_attention: the rel-pos table has %d rows; this context reads %d", ptab_rows,
+             c->pos_rows);
+    FO_CHECK(nsplit >= 0 && (nsplit == 0 || (mode == FO_ATT_STREAM && c->dtype == FO_BF16 && part && part_bias)),
+             "fo_debug_attention: split-K partials (with their bias) go with the stream mode of a bf16 context");
+    FO_CHECK(qkv || nsplit > 0, "fo_debug_attention: qkv is null");
+    DebugAttn d;
+    d.mode = mode; d.n = n; d.chunk = chunk; d.left = left; d.nsplit = nsplit;
+    d.qkv = qkv; d.part = part; d.part_bias = part_bias; d.ptab = ptab; d.pos_u = pos_u; d.pos_v = pos_v; d.out = out;
+    if (mode == FO_ATT_OFFLINE) {
+        FO_CHECK(T > 0 && T <= c->pos_rows, "fo_debug_attention: T = %d outside 1..%d (rel-pos rows)", T, c->pos_rows);
+        for (int b = 0; b < n; ++b) FO_CHECK(seq[b] >= 0, "fo_debug_attention: ilens[%d] < 0", b);
+        d.T = T;
+        d.rows = (long long)n * T;
+        d.tab.assign(seq, seq + n);
+    } else if (mode == FO_ATT_PACKED) {
+        FO_CHECK(gap >= 0, "fo_debug_attention: gap < 0");
+        const int tq = attention_offline_tile_rows(c->dtype == FO_BF16);
+        std::vector<int32_t> lens(n), rows(n);
+        for (int b = 0; b < n; ++b) {
+            FO_CHECK(seq[b] >= 1 && seq[b] <= c->pos_rows, "fo_debug_attention: lens[%d] = %d outside 1..%d", b, seq[b], c->pos_rows);
+            lens[b] = seq[b];
+            rows[b] = (int32_t)d.rows;
+            d.rows += seq[b] + (b + 1 < n ? gap : 0);
+            d.tmax = std::max(d.tmax, seq[b]);
+            for (int q = 0; q < cdiv(seq[b], tq); ++q) { d.tab.push_back(b); d.tab.push_back(q); }   // as fo_encode_offline_packed
+        }
+        d.ntiles = (int)d.tab.size() / 2;
+        d.tab.insert(d.tab.end(), lens.begin(), lens.end());
+        d.tab.insert(d.tab.end(), rows.begin(), rows.end());
+    } else {
+        FO_CHECK(c->ring, "fo_debug_attention: context has no streaming sessions");
+        FO_CHECK(layer >= 0 && layer < c->L, "fo_debug_attention: layer %d out of range", layer);
+        FO_CHECK(t >= 1 && t <= c->max_t && t <= STREAM_MAX_T, "fo_debug_attention: t = %d outside 1..%d (max_t)", t, c->max_t);
+        FO_CHECK(c->window + t <= c->ring_cap && c->window + t <= STREAM_CHUNKS_MAX_KEYS,
+                 "fo_debug_attention: window %d + t %d exceeds ring capacity %d or %d keys", c->window, t, c->ring_cap,
+                 STREAM_CHUNKS_MAX_KEYS);
+        FO_TRY(check_ids(c, seq, n));
+        d.t = t; d.layer = layer;
+        d.tab.assign(seq, seq + n);
+        if (mode == FO_ATT_STREAM) {
+            d.rows = (long long)n * t;
+        } else {
+            FO_CHECK(cnt && off && group >= 1, "fo_debug_attention: the chunks mode needs cnt, off and group >= 1");
+            FO_CHECK(c->window + group * t <= STREAM_CHUNKS_MAX_KEYS, "fo_debug_attention: window %d + %d chunks x %d frames exceeds %d keys",
+                     c->window, group, t, STREAM_CHUNKS_MAX_KEYS);
+            FO_CHECK(off[0] >= 0, "fo_debug_attention: off[0] < 0");
+            int kmax = 0;
+            for (int b = 0; b < n; ++b) {
+                FO_CHECK(cnt[b] >= 1 && (b == 0 || off[b] == off[b - 1] + cnt[b - 1]),
+                         "fo_debug_attention: cnt[%d] < 1 or off is not the running sum of cnt", b);
+                kmax = std::max(kmax, cnt[b]);
+                d.rows += (long long)cnt[b] * t;
+            }
+            d.group = group;
+            d.groups = cdiv(kmax, group);      // as stream_program
+            d.tab.insert(d.tab.end(), cnt, cnt + n);
+            d.tab.insert(d.tab.end(), off, off + n);
+        }
+    }
+    FO_CUDA(cudaSetDevice(c->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    return c->dtype == FO_BF16 ? debug_attention_run<act16>(c, d, st) : debug_attention_run<float>(c, d, st);
 }
 
 }  // extern "C"

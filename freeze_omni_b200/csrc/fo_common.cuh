@@ -500,6 +500,7 @@ int f32_to_bf16(const float* src, bf16* dst, long long n, cudaStream_t st);
 int f32_to_act16(const float* src, act16* dst, long long n, cudaStream_t st);
 int f32_to_weight16(const float* src, act16* dst, long long n, cudaStream_t st);   // bf16-rounded, fp16 container
 int bf16_to_f32(const bf16* src, float* dst, long long n, cudaStream_t st);
+int act16_to_f32(const act16* src, float* dst, long long n, cudaStream_t st);
 // dst[n][perm(k)] = src[n][k] style weight repacks (done once at finalize)
 template <typename TW>
 int repack_conv2(const float* w, int C, TW* out, cudaStream_t st);          // (co,ci,3,3) -> [co][(kh*3+kw)*C+ci]

@@ -413,6 +413,10 @@ __global__ void bf16_to_f32_kernel(const bf16* __restrict__ s, float* __restrict
     long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) d[i] = __bfloat162float(s[i]);
 }
+__global__ void act16_to_f32_kernel(const act16* __restrict__ s, float* __restrict__ d, long long n) {
+    long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) d[i] = __half2float(s[i]);
+}
 
 template <typename TW>
 __global__ void repack_conv2_kernel(const float* __restrict__ w, int C, TW* __restrict__ out) {
@@ -784,6 +788,13 @@ int f32_to_weight16(const float* src, act16* dst, long long n, cudaStream_t st) 
 int bf16_to_f32(const bf16* src, float* dst, long long n, cudaStream_t st) {
     if (n <= 0) return 0;
     bf16_to_f32_kernel<<<blocks_for(n, 256), 256, 0, st>>>(src, dst, n);
+    FO_LAUNCHED();
+    FO_CUDA(cudaGetLastError());
+    return 0;
+}
+int act16_to_f32(const act16* src, float* dst, long long n, cudaStream_t st) {
+    if (n <= 0) return 0;
+    act16_to_f32_kernel<<<blocks_for(n, 256), 256, 0, st>>>(src, dst, n);
     FO_LAUNCHED();
     FO_CUDA(cudaGetLastError());
     return 0;

@@ -530,3 +530,36 @@ class Engine:
         _lib.check(self.lib.fo_debug_gemm(self._h, _ptr(A), _ptr(W), _ptr(bias), _ptr(out), M, N, K, backend, int(relu),
                                           iters, C.byref(ms), self._stream()))
         return out, float(ms.value)
+
+    def debug_attention(self, mode: str, qkv: Optional[torch.Tensor], ptab: torch.Tensor, pos_u: torch.Tensor,
+                        pos_v: torch.Tensor, *, seq=None, T: int = 0, gap: int = 0, chunk: int = 0, left: int = -1, t: int = 0,
+                        layer: int = 0, cnt=None, off0: int = 0, group: int = 1, part: Optional[torch.Tensor] = None,
+                        part_bias: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """One attention launcher of the library (fo_debug_attention) on fp32 device tensors; returns out (rows, D) fp32.
+        mode "offline" (seq = ilens, T), "packed" (seq = lens, gap), "stream" (seq = session ids, t, layer; optional split-K
+        partials `part` (nsplit, rows, 3D) with `part_bias`), "chunks" (seq = ids, cnt, off0 = off[0], t, layer, group).
+        chunk / left: the offline band."""
+        m = {"offline": _lib.FO_ATT_OFFLINE, "packed": _lib.FO_ATT_PACKED, "stream": _lib.FO_ATT_STREAM,
+             "chunks": _lib.FO_ATT_CHUNKS}[mode]
+        s = _ids(seq)
+        n = len(s)
+        cn = offs = None
+        if mode == "offline":
+            rows = n * T
+        elif mode == "packed":
+            rows = int(s.sum()) + (n - 1) * gap
+        elif mode == "stream":
+            rows = n * t
+        else:
+            cn = _ids(cnt)
+            offs = np.ascontiguousarray(off0 + np.concatenate([[0], np.cumsum(cn)[:-1]]).astype(np.int32))
+            rows = int(cn.sum()) * t
+        for x in (qkv, ptab, pos_u, pos_v, part, part_bias):
+            assert x is None or (x.is_cuda and x.dtype == torch.float32 and x.is_contiguous())
+        nsplit = 0 if part is None else int(part.shape[0])
+        out = torch.empty(max(rows, 1), self.cfg.d_model, device=self.torch_device)[:rows]
+        _lib.check(self.lib.fo_debug_attention(
+            self._h, m, n, _i32p(s), None if cn is None else _i32p(cn), None if offs is None else _i32p(offs), int(T), int(gap),
+            int(chunk), int(left), int(t), int(layer), int(group), _ptr(qkv), _ptr(part), nsplit, _ptr(part_bias), _ptr(ptab),
+            int(ptab.shape[0]), _ptr(pos_u), _ptr(pos_v), _ptr(out), self._stream()))
+        return out

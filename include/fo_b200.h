@@ -312,6 +312,26 @@ int fo_debug_stack_plan(int d_model, int ffn_dim, int heads, int n_sessions, int
  * C[M,N] = A[M,K] * W[N,K]^T (+bias) in the context's dtype, fp32 in/out on device pointers. */
 int fo_debug_gemm(fo_ctx* ctx, const float* A, const float* W, const float* bias, float* C,
                   int M, int N, int K, int backend, int relu, int iters, float* ms_out, void* stream);
+/* one attention launcher of the library on caller-given tensors, exposed for kernel-level parity tests.  Runs on `stream` and
+ * returns when it is done.  All tensors are fp32 device pointers, all tables host arrays:
+ *   qkv (rows, 3D) Q | K | V as the QKV GEMM writes them: bf16 contexts convert K | V to fp16 (round to nearest, as the
+ *       activations are), Q is read as fp32 from the same array;  ptab (ptab_rows, D) the rel-pos table P_l, at least the
+ *       context's pos_rows rows (head-major copy built as fo_finalize_weights builds it);  pos_u, pos_v (D);
+ *   out (rows, D): the attention output converted to fp32; rows no query writes (packed gaps) are 0.
+ * mode FO_ATT_OFFLINE: n utterances padded to T rows (rows = n*T), seq = ilens (n) -- fo_encode_offline's attention.
+ *      FO_ATT_PACKED: n utterances of seq[b] rows back to back with `gap` unused rows between them -- fo_encode_offline_packed's.
+ *      chunk, left: the band of both offline modes.
+ *      FO_ATT_STREAM: sessions seq (n), t frames each (rows = n*t) against `layer`'s KV ring at each slot's n_frames / pe_index;
+ *      nsplit > 0 (bf16 contexts): q / k / v summed from split-K partials part [nsplit][rows][3D] + part_bias (3D), qkv unused.
+ *      FO_ATT_CHUNKS: sessions seq bring cnt[b] chunks of t frames, rows from (off[b] - off[0]) * t (off = off[0] + running sum
+ *      of cnt), `group` chunks per CTA.
+ * The streaming modes append the new K/V rows to the ring as a step does, and advance no session.  FO_ERR_ARG, nothing
+ * launched: t > max_t, window + t > ring capacity or 128, window + group * t > 128, T or a length past pos_rows, ptab_rows < pos_rows. */
+enum { FO_ATT_OFFLINE = 0, FO_ATT_PACKED = 1, FO_ATT_STREAM = 2, FO_ATT_CHUNKS = 3 };
+int fo_debug_attention(fo_ctx* ctx, int mode, int n, const int32_t* seq, const int32_t* cnt, const int32_t* off, int T, int gap,
+                       int chunk, int left, int t, int layer, int group, const float* qkv, const float* part, int nsplit,
+                       const float* part_bias, const float* ptab, int ptab_rows, const float* pos_u, const float* pos_v,
+                       float* out, void* stream);
 
 #ifdef __cplusplus
 }
