@@ -56,6 +56,7 @@ SYMBOLS = {
     "fo_session_restore": (C.c_int, [_P, _I32P, C.c_int, _P, _P]),
     "fo_fbank_stream": (C.c_int, [_P, _I32P, C.c_int, _P, C.c_int, C.c_float, _P, _P]),
     "fo_fbank_offline": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int64, C.c_float, _P, _P]),
+    "fo_fbank_offline_packed": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, C.c_float, _P, _P]),
     "fo_encode_stream": (C.c_int, [_P, _I32P, C.c_int, _P, C.c_int, _P, _P, _P]),
     "fo_encode_stream_chunks": (C.c_int, [_P, _I32P, C.c_int, C.c_int, _P, C.c_int, _P, _P, _P]),
     "fo_encode_stream_chunks_v": (C.c_int, [_P, _I32P, _I32P, C.c_int, _P, C.c_int, _P, _P, _P]),
@@ -70,6 +71,7 @@ SYMBOLS = {
     "fo_handoff_arm": (C.c_int, [_P, C.c_int, _P, C.c_int64, C.c_int64, _P, _P, _P, _P]),
     "fo_encode_offline": (C.c_int, [_P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, _P, _P, _P]),
     "fo_encode_offline_packed": (C.c_int, [_P, _P, _P, C.c_int, C.c_int, C.c_int, _P, _P, _P]),
+    "fo_encode_offline_packed_pcm": (C.c_int, [_P, _P, C.c_int, _P, C.c_int, C.c_float, C.c_int, C.c_int, _P, _P, _P, _P]),
     "fo_adapter_forward": (C.c_int, [_P, _P, _P, C.c_int, C.c_int, _P, _P, _P, _P]),
     "fo_adapter_forward2": (C.c_int, [_P, _P, _P, C.c_int, C.c_int, _P, _P, _P, _P, _P, _P]),
     "fo_stats": (C.c_int, [_P, C.POINTER(FoStats)]),

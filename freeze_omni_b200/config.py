@@ -136,6 +136,18 @@ class PathConfig:
         t3 = t2 if self.adapter_type in ("linear", "cnn") else (t2 - 1) // 2 + 1
         return np.concatenate([[0], np.cumsum(t2)]), np.concatenate([[0], np.cumsum(t3)])
 
+    def packed_audio_offsets(self, n_samples):
+        """Offsets of a packed PCM call (fo_encode_offline_packed_pcm) for utterances of ``n_samples`` samples: (frames,
+        enc_offsets, adapter_offsets), int64 arrays.  frames[i] = 1 + (n_samples[i] - frame_len) // frame_shift (kaldi
+        snip_edges: trailing samples that fill no frame are dropped); the offsets are packed_offsets(frames)."""
+        import numpy as np
+        n = np.asarray(n_samples, dtype=np.int64).reshape(-1)
+        m = np.where(n >= self.frame_len, 1 + (n - self.frame_len) // self.frame_shift, 0)
+        if m.size == 0 or (m < 7).any():
+            raise ValueError("every utterance needs >= 7 feature frames (%d samples)" % (self.frame_len + 6 * self.frame_shift))
+        eoff, aoff = self.packed_offsets(m)
+        return m, eoff, aoff
+
     def validate(self) -> None:
         """The reference exits on an inconsistent config (encoder.py:74-75,86-87,94); here a
         ValueError.  Variants whose streaming path is broken upstream are refused loudly

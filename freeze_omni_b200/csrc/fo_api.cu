@@ -188,6 +188,7 @@ struct fo_ctx {
     unsigned long long* stack_trace = nullptr;
     long long stack_launches = 0;
     int steps_pass_blocks = 0;                // option: blocks per pass of fo_stream_steps_v (0: from STEPS_PASS_BYTES)
+    int packed_pass_frames = 0;               // option: grid feature frames per pass of fo_encode_offline_packed_pcm (0: from PACKED_PASS_BYTES)
     struct ProfRec { cudaEvent_t e0, e1; int M, N, K; };
     std::vector<ProfRec> prof_events;
     // captured step graphs, keyed by the shape of the call; invalidated when a workspace moves
@@ -219,7 +220,7 @@ namespace {
 
 enum { WS_FEATS = 0, WS_C1, WS_C2, WS_XSUB, WS_EMB, WS_X, WS_H, WS_QKV, WS_ATT, WS_FFH, WS_ENC, WS_XIN, WS_ACONV, WS_AH,
        WS_Y, WS_MASK2, WS_ILENS, WS_ILENS2, WS_AMASK, WS_PCM, WS_TMP0, WS_TMP1, WS_TMP2, WS_TMP3, WS_Q32, WS_HC, WS_PART, WS_PCM2, WS_ENC2, WS_Y2, WS_AC1, WS_XIN2, WS_TMP4, WS_TMP5, WS_HP, WS_FP, WS_PACK, WS_SROWS,
-       WS_PKTAB, WS_FGRID, WS_XP, WS_COUNT };
+       WS_PKTAB, WS_FGRID, WS_XP, WS_FBTAB, WS_COUNT };
 static_assert(WS_COUNT <= (int)(sizeof(fo_ctx::ws) / sizeof(DevBuf)), "fo_ctx::ws holds every named workspace");
 
 int dev_alloc(fo_ctx* c, void** p, size_t bytes) {
@@ -1348,6 +1349,7 @@ struct PackTab {
     int rows = 0, trunk = 0, ad_rows = 0, gap = 0, tiles = 0, grid_frames = 0;
     int o_tiles = 0, o_lens = 0, o_eoff = 0, o_xrow = 0, o_grow = 0, o_flen = 0, o_foff = 0, o_frow = 0, o_gaps = 0, o_adcnt = 0,
         o_aoff = 0;
+    int o_soff = 0;                   // PCM entry only: int64 sample offsets (two words each, 8-byte aligned), else 0
     std::vector<int32_t> h;
 };
 // Packed twin of offline_program: B utterances back to back, every kernel on their rows only.
@@ -1357,16 +1359,15 @@ struct PackTab {
 //    depthwise conv restarts at each utterance.  MultiLayeredConv1d (two-sided conv) keeps k - 1 zeroed rows between
 //    utterances in the residual stream (`gap`), and the encoder rows are gathered out of it at the end.
 //  - adapter: adapter_program's packed mode.
+// The features reach the grid (WS_FGRID, spare frames zeroed) either from packed features (offline_packed_program) or straight
+// from the fbank of packed PCM (fo_encode_offline_packed_pcm); offline_packed_trunk runs everything from the grid on.
 template <typename TA>
-int offline_packed_program(fo_ctx* c, const float* feats, const PackTab& p, const int32_t* tab, int chunk, int left,
-                           float* enc_out_dev, float* y_dev, cudaStream_t st) {
-    const int D = c->D, FF = c->FF, H = c->H, F = c->F, B = p.B, M = p.trunk;
-    void *fg, *xp;
-    FO_TRY(ws_ensure(c, WS_FGRID, (size_t)p.grid_frames * F * sizeof(float), &fg));
-    FO_CUDA(cudaMemsetAsync(fg, 0, (size_t)p.grid_frames * F * sizeof(float), st));
-    FO_TRY(copy_utt_rows(feats, tab + p.o_foff, reinterpret_cast<float*>(fg), tab + p.o_frow, tab + p.o_flen, B, p.fmax, F, st));
+int offline_packed_trunk(fo_ctx* c, const float* fg, const PackTab& p, const int32_t* tab, int chunk, int left, float* enc_out_dev,
+                         float* y_dev, cudaStream_t st) {
+    const int D = c->D, FF = c->FF, H = c->H, B = p.B, M = p.trunk;
+    void* xp;
     float* xg;
-    FO_TRY(subsample_program<TA>(c, reinterpret_cast<const float*>(fg), 1, p.grid_frames, &xg, st));
+    FO_TRY(subsample_program<TA>(c, fg, 1, p.grid_frames, &xg, st));
     FO_TRY(ws_ensure(c, WS_XP, (size_t)M * D * sizeof(float), &xp));
     float* x = reinterpret_cast<float*>(xp);
     if (p.gap) FO_CUDA(cudaMemsetAsync(x, 0, (size_t)M * D * sizeof(float), st));
@@ -1419,6 +1420,24 @@ int offline_packed_program(fo_ctx* c, const float* feats, const PackTab& p, cons
         FO_TRY(adapter_program<TA>(c, enc_out_dev, nullptr, B, p.tmax, nullptr, nullptr, nullptr, out, st, nullptr, &pk));
     }
     return 0;
+}
+
+// feature grid of a packed call: grid_frames fp32 rows, zeroed (the spare frames behind each utterance stay zero)
+int packed_grid(fo_ctx* c, const PackTab& p, float** fg, cudaStream_t st) {
+    void* g;
+    FO_TRY(ws_ensure(c, WS_FGRID, (size_t)p.grid_frames * c->F * sizeof(float), &g));
+    FO_CUDA(cudaMemsetAsync(g, 0, (size_t)p.grid_frames * c->F * sizeof(float), st));
+    *fg = reinterpret_cast<float*>(g);
+    return 0;
+}
+
+template <typename TA>
+int offline_packed_program(fo_ctx* c, const float* feats, const PackTab& p, const int32_t* tab, int chunk, int left,
+                           float* enc_out_dev, float* y_dev, cudaStream_t st) {
+    float* fg;
+    FO_TRY(packed_grid(c, p, &fg, st));
+    FO_TRY(copy_utt_rows(feats, tab + p.o_foff, fg, tab + p.o_frow, tab + p.o_flen, p.B, p.fmax, c->F, st));
+    return offline_packed_trunk<TA>(c, fg, p, tab, chunk, left, enc_out_dev, y_dev, st);
 }
 
 // Arguments of fo_debug_attention once checked: the device tables (`tab`, uploaded to the entry's own scratch), the rows of
@@ -2722,30 +2741,19 @@ int fo_encode_offline(fo_ctx* c, const float* feats, const int32_t* ilens, int B
 }
 
 // ---- full utterances packed end to end ---------------------------------------------------------------------
-int fo_encode_offline_packed(fo_ctx* c, const float* feats, const int32_t* lens, int B, int chunk, int left, float* enc_out,
-                             float* adapter_out, void* stream) {
-    FO_CHECK(c && c->finalized && c->cfg.has_encoder, "fo_encode_offline_packed: context has no finalized encoder");
-    FO_CHECK(feats && lens && B > 0 && B <= 65535, "fo_encode_offline_packed: need feats, lens and 1 <= B <= 65535");
-    if (adapter_out) FO_CHECK(c->cfg.has_adapter, "adapter_out requested but the context has no adapter");
-    FO_CUDA(cudaSetDevice(c->device));
-    cudaStream_t st = (cudaStream_t)stream;
-    PackTab p;
+// PackTab of B utterances of T[b] feature frames (refusals name utterance b0 + b of the caller's call).  soff (optional, the
+// PCM entry): each utterance's first sample, appended to the table as int64.
+static int pack_tab(fo_ctx* c, const int32_t* T, int B, const char* who, int b0, const long long* soff, PackTab* pt) {
+    PackTab& p = *pt;
     p.B = B;
-    std::vector<int32_t> T(B);
-    if (is_device_ptr(lens)) {
-        FO_CUDA(cudaMemcpyAsync(T.data(), lens, (size_t)B * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-        FO_CUDA(cudaStreamSynchronize(st));
-    } else {
-        std::copy(lens, lens + B, T.begin());
-    }
     const int ns = c->cfg.has_adapter ? c->ad_nst : 0, tq = attention_offline_tile_rows(c->dtype == FO_BF16);
     p.gap = c->KM ? c->KM - 1 : 0;
     long long frames = 0, rows = 0, ad_rows = 0, grid = 0, tiles = 0;
     for (int b = 0; b < B; ++b) {
-        FO_CHECK(T[b] >= 7, "fo_encode_offline_packed: utterance %d has %d feature frames; each needs >= 7", b, T[b]);
+        FO_CHECK(T[b] >= 7, "%s: utterance %d has %d feature frames; each needs >= 7", who, b0 + b, T[b]);
         const int t2 = ((T[b] - 1) / 2 - 1) / 2;
-        FO_CHECK(t2 <= c->cfg.pos_max_len, "fo_encode_offline_packed: utterance %d has %d encoder frames, past the positional table (%d)",
-                 b, t2, c->cfg.pos_max_len);
+        FO_CHECK(t2 <= c->cfg.pos_max_len, "%s: utterance %d has %d encoder frames, past the positional table (%d)",
+                 who, b0 + b, t2, c->cfg.pos_max_len);
         frames += T[b];
         rows += t2;
         ad_rows += ad_frames(c, t2);
@@ -2754,15 +2762,17 @@ int fo_encode_offline_packed(fo_ctx* c, const float* feats, const int32_t* lens,
         p.tmax = std::max(p.tmax, t2);
         p.fmax = std::max(p.fmax, T[b]);
     }
-    FO_CHECK(grid < (1LL << 28), "fo_encode_offline_packed: %lld feature frames in one call; pass fewer utterances", frames);
+    FO_CHECK(grid < (1LL << 28), "%s: %lld feature frames in one call; pass fewer utterances", who, frames);
     p.rows = (int)rows; p.ad_rows = (int)ad_rows; p.grid_frames = (int)grid; p.tiles = (int)tiles;
     p.trunk = (int)(rows + (long long)(B - 1) * p.gap);
-    // table: tiles {b, q} | lens | eoff | xrow | grow | flen | foff | frow | gaps | adcnt | aoff
+    // table: tiles {b, q} | lens | eoff | xrow | grow | flen | foff | frow | gaps | adcnt | aoff [| soff (int64)]
     p.o_tiles = 0; p.o_lens = 2 * p.tiles; p.o_eoff = p.o_lens + B; p.o_xrow = p.o_eoff + B + 1; p.o_grow = p.o_xrow + B;
     p.o_flen = p.o_grow + B; p.o_foff = p.o_flen + B; p.o_frow = p.o_foff + B + 1; p.o_gaps = p.o_frow + B;
     p.o_adcnt = p.o_gaps + B; p.o_aoff = p.o_adcnt + (ns + 1) * B;
     std::vector<int32_t>& h = p.h;
-    h.assign(p.o_aoff + B + 1, 0);
+    p.o_soff = soff ? (p.o_aoff + B + 1 + 1) / 2 * 2 : 0;
+    h.assign(soff ? p.o_soff + 2 * B : p.o_aoff + B + 1, 0);
+    if (soff) memcpy(h.data() + p.o_soff, soff, (size_t)B * sizeof(long long));
     int32_t* tl = h.data();
     for (int b = 0, g = 0; b < B; ++b) {
         const int t2 = ((T[b] - 1) / 2 - 1) / 2;
@@ -2779,9 +2789,29 @@ int fo_encode_offline_packed(fo_ctx* c, const float* feats, const int32_t* lens,
         h[p.o_aoff + b + 1] = h[p.o_aoff + b] + ad_frames(c, t2);
         for (int q = 0; q < cdiv(t2, tq); ++q) { *tl++ = b; *tl++ = q; }
     }
+    return 0;
+}
+
+int fo_encode_offline_packed(fo_ctx* c, const float* feats, const int32_t* lens, int B, int chunk, int left, float* enc_out,
+                             float* adapter_out, void* stream) {
+    FO_CHECK(c && c->finalized && c->cfg.has_encoder, "fo_encode_offline_packed: context has no finalized encoder");
+    FO_CHECK(feats && lens && B > 0 && B <= 65535, "fo_encode_offline_packed: need feats, lens and 1 <= B <= 65535");
+    if (adapter_out) FO_CHECK(c->cfg.has_adapter, "adapter_out requested but the context has no adapter");
+    FO_CUDA(cudaSetDevice(c->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    PackTab p;
+    std::vector<int32_t> T(B);
+    if (is_device_ptr(lens)) {
+        FO_CUDA(cudaMemcpyAsync(T.data(), lens, (size_t)B * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+        FO_CUDA(cudaStreamSynchronize(st));
+    } else {
+        std::copy(lens, lens + B, T.begin());
+    }
+    FO_TRY(pack_tab(c, T.data(), B, "fo_encode_offline_packed", 0, nullptr, &p));
+    const long long frames = p.h[p.o_foff + B], rows = p.rows, ad_rows = p.ad_rows;
     void *dtab, *dfeats, *denc, *dy = nullptr;
-    FO_TRY(ws_ensure(c, WS_PKTAB, h.size() * sizeof(int32_t), &dtab));
-    FO_CUDA(cudaMemcpyAsync(dtab, h.data(), h.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    FO_TRY(ws_ensure(c, WS_PKTAB, p.h.size() * sizeof(int32_t), &dtab));
+    FO_CUDA(cudaMemcpyAsync(dtab, p.h.data(), p.h.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
     FO_TRY(in_dev(c, feats, (size_t)frames * c->F * sizeof(float), WS_FEATS, st, (const void**)&dfeats));
     const size_t enc_bytes = (size_t)rows * c->D * sizeof(float), y_bytes = (size_t)ad_rows * c->E * sizeof(float);
     FO_TRY(out_dev(c, enc_out, enc_bytes, WS_ENC, &denc));
@@ -2794,6 +2824,152 @@ int fo_encode_offline_packed(fo_ctx* c, const float* feats, const int32_t* lens,
     if (adapter_out) FO_TRY(out_done(adapter_out, dy, y_bytes, st));
     c->stats.offline_calls += 1;
     c->stats.offline_frames += rows;
+    return 0;
+}
+
+// ---- packed PCM: fbank of utterances of different lengths, and PCM -> embeddings in passes ------------------------------
+// frames of an utterance of n samples (kaldi snip_edges: the trailing samples that fill no frame are dropped); 0 below one frame
+static long long utt_frames(const fo_ctx* c, long long n) {
+    return n >= c->cfg.frame_len ? 1 + (n - c->cfg.frame_len) / c->cfg.frame_shift : 0;
+}
+
+int fo_fbank_offline_packed(fo_ctx* c, const void* pcm, int pcm_dtype, const int64_t* n_samples, int B, float scale, float* out,
+                            void* stream) {
+    FO_CHECK(c && c->finalized && c->fb_window, "fo_fbank_offline_packed: context has no finalized frontend");
+    FO_CHECK(pcm && n_samples && out && B > 0, "fo_fbank_offline_packed: need pcm, n_samples, out and B >= 1");
+    FO_CHECK(pcm_dtype == FO_F32 || pcm_dtype == FO_I16, "fo_fbank_offline_packed: pcm must be FO_F32 or FO_I16");
+    // table: sample offsets (int64) | frame offsets (B + 1, int32); the frame offsets are also the output rows
+    std::vector<int32_t> h(2 * (size_t)B + B + 1, 0);
+    long long* soff = reinterpret_cast<long long*>(h.data());
+    int32_t* foff = h.data() + 2 * (size_t)B;
+    long long samples = 0, frames = 0;
+    for (int b = 0; b < B; ++b) {
+        FO_CHECK(n_samples[b] >= c->cfg.frame_len, "fo_fbank_offline_packed: utterance %d has %lld samples, shorter than one frame (%d)",
+                 b, (long long)n_samples[b], c->cfg.frame_len);
+        soff[b] = samples;
+        samples += n_samples[b];
+        frames += utt_frames(c, n_samples[b]);
+        FO_CHECK(frames < (1LL << 31), "fo_fbank_offline_packed: more than 2^31 - 1 frames in one call; pass fewer utterances");
+        foff[b + 1] = (int32_t)frames;
+    }
+    FO_CUDA(cudaSetDevice(c->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    void* dtab;
+    FO_TRY(ws_ensure(c, WS_FBTAB, h.size() * sizeof(int32_t), &dtab));
+    FO_CUDA(cudaMemcpyAsync(dtab, h.data(), h.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    const void* dp;
+    FO_TRY(in_dev(c, pcm, (size_t)samples * (pcm_dtype == FO_I16 ? 2 : 4), WS_PCM, st, &dp));
+    const size_t out_bytes = (size_t)frames * c->F * sizeof(float);
+    void* dout;
+    FO_TRY(out_dev(c, out, out_bytes, WS_FEATS, &dout));
+    FbankVarlen vl;
+    vl.sample_off = reinterpret_cast<const long long*>(dtab);
+    vl.frame_off = reinterpret_cast<const int32_t*>(dtab) + 2 * (size_t)B;
+    vl.out_row = vl.frame_off;
+    vl.n = B;
+    vl.frames = frames;
+    FO_TRY(fbank_offline_packed(fbank_params(c), dp, pcm_dtype == FO_I16, scale, vl, (float*)dout, nullptr, st));
+    FO_TRY(out_done(out, dout, out_bytes, st));
+    return 0;
+}
+
+// fo_encode_offline_packed_pcm runs in passes over consecutive utterances: utterance i takes ceil(m_i / 4) * 4 frames of the
+// feature grid, and a pass takes utterances in call order while their grid frames fit P (option "packed_pass_frames", else
+// PACKED_PASS_BYTES over the workspace bytes of one encoder row); an utterance larger than P runs in a pass of its own.  Every
+// workspace is sized by the pass, so the device memory a call adds follows P, not the corpus.  Passes run eagerly (no graphs).
+constexpr long long PACKED_PASS_BYTES = 10LL << 30;
+
+// workspace bytes of one encoder row of a pass (4 grid frames): PCM staging and the feature grid (+ feats_out staging), conv1
+// planes and conv2 rows, sub-Linear / residual / LayerNorm / attention rows, QKV (+ fp32 Q), FFN hidden rows, encoder and
+// adapter rows -- the terms of steps_block_bytes per encoder frame
+static long long packed_row_bytes(const fo_ctx* c) {
+    const long long esz = (long long)c->esz, D = c->D;
+    long long b = 4LL * c->cfg.frame_shift * 4 + 2 * 4LL * c->F * 4;
+    b += 6LL * (c->F2 + 1) * D * esz + (long long)c->F2 * D * esz;
+    b += D * (4 + 4 + 4 + 5 * esz) + 3 * D * (esz + 4) + (long long)c->FF * esz;
+    if (c->cfg.has_adapter) b += 4 * D * (esz + 4) + (long long)c->E * 4;
+    return b;
+}
+// ... and never more grid frames than the conv2 implicit GEMM of one pass (T' (F2 + 1) rows, d_model columns) can take
+static int packed_pass_frames(const fo_ctx* c) {
+    const long long cap = std::max(4LL, gemm_tc_max_rows(c->D) / (c->F2 + 1) * 4);
+    const long long P = c->packed_pass_frames > 0 ? c->packed_pass_frames : PACKED_PASS_BYTES / packed_row_bytes(c) * 4;
+    return (int)std::max(4LL, std::min({1LL << 26, cap, P}));
+}
+
+int fo_encode_offline_packed_pcm(fo_ctx* c, const void* pcm, int pcm_dtype, const int64_t* n_samples, int B, float scale, int chunk,
+                                 int left, float* enc_out, float* adapter_out, float* feats_out, void* stream) {
+    const char* who = "fo_encode_offline_packed_pcm";
+    FO_CHECK(c && c->finalized && c->cfg.has_encoder && c->fb_window, "%s: context has no finalized encoder + frontend", who);
+    FO_CHECK(pcm && n_samples && B > 0 && B <= 65535, "%s: need pcm, n_samples and 1 <= B <= 65535", who);
+    FO_CHECK(pcm_dtype == FO_F32 || pcm_dtype == FO_I16, "%s: pcm must be FO_F32 or FO_I16", who);
+    if (adapter_out) FO_CHECK(c->cfg.has_adapter, "adapter_out requested but the context has no adapter");
+    // every utterance is checked before the first pass: m_i frames, T'_i encoder rows; offsets of the whole call
+    std::vector<int32_t> T(B);
+    std::vector<long long> soff(B + 1, 0), foff(B + 1, 0), eoff(B + 1, 0), aoff(B + 1, 0);
+    for (int b = 0; b < B; ++b) {
+        const long long m = utt_frames(c, n_samples[b]);
+        FO_CHECK(m >= 7, "%s: utterance %d has %lld samples, %lld feature frames; each needs >= 7", who, b, (long long)n_samples[b], m);
+        const long long t2 = ((m - 1) / 2 - 1) / 2;
+        FO_CHECK(t2 <= c->cfg.pos_max_len, "%s: utterance %d has %lld encoder frames, past the positional table (%d)", who, b, t2,
+                 c->cfg.pos_max_len);
+        T[b] = (int32_t)m;
+        soff[b + 1] = soff[b] + n_samples[b];
+        foff[b + 1] = foff[b] + m;
+        eoff[b + 1] = eoff[b] + t2;
+        aoff[b + 1] = aoff[b] + ad_frames(c, (int)t2);
+    }
+    FO_CUDA(cudaSetDevice(c->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    const int P = packed_pass_frames(c), F = c->F, D = c->D, E = c->E;
+    const size_t esz_pcm = pcm_dtype == FO_I16 ? 2 : 4;
+    const bool pcm_dev = is_device_ptr(pcm), enc_dev = enc_out && is_device_ptr(enc_out);
+    const bool y_dev = adapter_out && is_device_ptr(adapter_out), f_dev = feats_out && is_device_ptr(feats_out);
+    std::vector<long long> ps(B);
+    for (int b0 = 0, b1; b0 < B; b0 = b1) {
+        long long g = (T[b0] + 3) / 4 * 4;
+        for (b1 = b0 + 1; b1 < B && g + (T[b1] + 3) / 4 * 4 <= P; ++b1) g += (T[b1] + 3) / 4 * 4;
+        const int n = b1 - b0;
+        for (int b = b0; b < b1; ++b) ps[b - b0] = soff[b] - soff[b0];
+        PackTab p;
+        FO_TRY(pack_tab(c, T.data() + b0, n, who, b0, ps.data(), &p));
+        void *dtab, *dpcm, *denc, *dy = nullptr, *dfeats = nullptr;
+        FO_TRY(ws_ensure(c, WS_PKTAB, p.h.size() * sizeof(int32_t), &dtab));
+        FO_CUDA(cudaMemcpyAsync(dtab, p.h.data(), p.h.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+        const size_t pcm_bytes = (size_t)(soff[b1] - soff[b0]) * esz_pcm;
+        const char* src = (const char*)pcm + (size_t)soff[b0] * esz_pcm;
+        if (pcm_dev) {
+            dpcm = const_cast<char*>(src);
+        } else {
+            FO_TRY(ws_ensure(c, WS_PCM, pcm_bytes, &dpcm));
+            FO_CUDA(cudaMemcpyAsync(dpcm, src, pcm_bytes, cudaMemcpyHostToDevice, st));
+        }
+        const size_t enc_bytes = (size_t)p.rows * D * sizeof(float), y_bytes = (size_t)p.ad_rows * E * sizeof(float);
+        const size_t f_bytes = (size_t)(foff[b1] - foff[b0]) * F * sizeof(float);
+        if (enc_dev) denc = enc_out + eoff[b0] * D;
+        else FO_TRY(ws_ensure(c, WS_ENC, enc_bytes, &denc));
+        if (y_dev) dy = adapter_out + aoff[b0] * E;
+        else if (adapter_out) FO_TRY(ws_ensure(c, WS_Y, y_bytes, &dy));
+        if (f_dev) dfeats = feats_out + foff[b0] * F;
+        else if (feats_out) FO_TRY(ws_ensure(c, WS_FEATS, f_bytes, &dfeats));
+        const int32_t* tab = reinterpret_cast<const int32_t*>(dtab);
+        float* fg;
+        FO_TRY(packed_grid(c, p, &fg, st));
+        FbankVarlen vl;
+        vl.frame_off = tab + p.o_foff;
+        vl.sample_off = reinterpret_cast<const long long*>(tab + p.o_soff);
+        vl.out_row = tab + p.o_frow;
+        vl.n = n;
+        vl.frames = foff[b1] - foff[b0];
+        FO_TRY(fbank_offline_packed(fbank_params(c), dpcm, pcm_dtype == FO_I16, scale, vl, fg, (float*)dfeats, st));
+        FO_TRY(c->dtype == FO_BF16 ? offline_packed_trunk<act16>(c, fg, p, tab, chunk, left, (float*)denc, (float*)dy, st)
+                                   : offline_packed_trunk<float>(c, fg, p, tab, chunk, left, (float*)denc, (float*)dy, st));
+        if (enc_out && !enc_dev) FO_CUDA(cudaMemcpyAsync(enc_out + eoff[b0] * D, denc, enc_bytes, cudaMemcpyDeviceToHost, st));
+        if (adapter_out && !y_dev) FO_CUDA(cudaMemcpyAsync(adapter_out + aoff[b0] * E, dy, y_bytes, cudaMemcpyDeviceToHost, st));
+        if (feats_out && !f_dev) FO_CUDA(cudaMemcpyAsync(feats_out + foff[b0] * F, dfeats, f_bytes, cudaMemcpyDeviceToHost, st));
+    }
+    c->stats.offline_calls += 1;
+    c->stats.offline_frames += eoff[B];
     return 0;
 }
 
@@ -2906,6 +3082,11 @@ int fo_set_option(fo_ctx* c, const char* name, int64_t value) {
         FO_CHECK(value >= 0 && value <= (1 << 20), "steps_pass_blocks must be 0 (byte budget) or 1..%d blocks", 1 << 20);
         c->steps_pass_blocks = (int)value;
     }
+    else if (!strcmp(name, "packed_pass_frames")) {
+        FO_CHECK(value == 0 || (value >= 4 && value <= (1 << 26)), "packed_pass_frames must be 0 (byte budget) or 4..%d grid frames",
+                 1 << 26);
+        c->packed_pass_frames = (int)value;
+    }
     else if (!strcmp(name, "defer_reduce")) c->defer_reduce = value != 0;
     else if (!strcmp(name, "tc_persist")) gemm_tc_set_persist(value != 0);
     else if (!strcmp(name, "l2_prefetch")) c->use_prefetch = (int)(value & 3);
@@ -2939,6 +3120,7 @@ int fo_get_option(fo_ctx* c, const char* name, int64_t* value) {
     else if (!strcmp(name, "fuse_ln")) *value = c->fuse_ln;
     else if (!strcmp(name, "stack_rows")) *value = c->stack_rows;
     else if (!strcmp(name, "steps_pass_blocks")) *value = c->steps_pass_blocks;
+    else if (!strcmp(name, "packed_pass_frames")) *value = packed_pass_frames(c);    // the budget's frames when not set
     else if (!strcmp(name, "stack_launches")) *value = c->stack_launches;
     else if (!strcmp(name, "defer_reduce")) *value = c->defer_reduce;
     else if (!strcmp(name, "tc_persist_launches")) *value = gemm_tc_persist_launches();

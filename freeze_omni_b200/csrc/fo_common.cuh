@@ -289,6 +289,7 @@ void gemm_tc_set_persist(int on);          // persistent tile loop for fat short
 long long gemm_tc_persist_launches();
 void gemm_tc_force_producers(int npa, int npb);   // 0 = default
 long long gemm_tc_launches();                // tcgen05 kernel launches so far (tests check the path taken)
+long long gemm_tc_max_rows(int N);           // the most activation rows one GEMM of N output columns takes (its tile table)
 // A and W: 16-bit operands of ONE format (fp16 when is_fp16, else bf16); c_act / ln_act are written in the same type.
 int gemm_tc(const void* A, int is_fp16, const AGather& ga, const void* W, int M, int N, int K, const Epilogue& ep,
             const RowMap& rmap, const TcWorkspace& ws, cudaStream_t st, int* deferred_splits = nullptr);
@@ -314,6 +315,19 @@ int fbank_stream_blocks(const FbankParams& p, const int32_t* ids, const int32_t*
                         float* carry, float* ring, float* rows, float* feats_out, cudaStream_t st);
 int fbank_offline(const FbankParams& p, const void* pcm, int pcm_is_i16, int B, long long n_samples, float scale,
                   float* out, cudaStream_t st);
+// Utterances of different lengths back to back (fo_fbank_offline_packed, fo_encode_offline_packed_pcm): utterance b of n has
+// frame_off[b + 1] - frame_off[b] frames (kaldi snip_edges: 1 + (n_samples - frame_len) / frame_shift), its samples from
+// sample_off[b] of pcm; its frames go to rows out_row[b].. of out, and to rows frame_off[b].. of out2 (optional).  Every frame
+// is computed as fbank_offline computes it.  Device tables; frames = frame_off[n].
+struct FbankVarlen {
+    const int32_t* frame_off = nullptr;   // n + 1 prefix sums of the frame counts
+    const long long* sample_off = nullptr;
+    const int32_t* out_row = nullptr;
+    int n = 0;
+    long long frames = 0;
+};
+int fbank_offline_packed(const FbankParams& p, const void* pcm, int pcm_is_i16, float scale, const FbankVarlen& vl, float* out,
+                         float* out2, cudaStream_t st);
 
 // ---- elementwise / normalisation ----------------------------------------------------------------
 // CMVN + Conv2d(1->C,3,2) + ReLU, written as the A operand of the conv2 implicit GEMM:

@@ -39,12 +39,40 @@ __device__ __forceinline__ float warp_sum(float v) {
     return v;
 }
 
-// out row for (signal b, frame f) = out + (out_ids ? out_ids[b] : b) * out_row_stride + (out_frame0 + f) * n_mel;
-// out2 (optional, dense (B, out2_frames, n_mel)) receives the same frame at row out2_frame0 + f.
+// Which signal and frame a warp takes, where its samples start and where its mel row goes.
+//  Uniform (VL = false): B signals of frames_per_signal frames each, signal b at sample row src.row_ids[b] (or b) of
+//    src.row_stride samples; out row = out + (out_ids ? out_ids[b] : b) * out_row_stride + (out_frame0 + f) * n_mel, and out2
+//    (optional, dense (B, out2_frames, n_mel)) receives the same frame at row out2_frame0 + f.
+//  Varlen (VL = true, fbank_offline_packed): frame fr of the call belongs to the utterance b with frame_off[b] <= fr <
+//    frame_off[b + 1] (binary search of the device table), local frame f = fr - frame_off[b]; its samples start at
+//    sample_off[b] + f * frame_shift of src.base; out row = out + (out_row[b] + f) * n_mel, out2 (optional) row frame_off[b] + f.
+template <bool VL>
+__device__ __forceinline__ void fbank_frame(const FbankVarlen& vl, const SampleSrc& src, int frames_per_signal, int frame_shift,
+                                            long long fr, int& b, int& f, long long& srow, long long& s0) {
+    if constexpr (VL) {
+        int lo = 0, hi = vl.n;                             // frame_off[lo] <= fr < frame_off[hi]
+        while (hi - lo > 1) {
+            const int mid = (lo + hi) >> 1;
+            if (vl.frame_off[mid] <= fr) lo = mid;
+            else hi = mid;
+        }
+        b = lo;
+        f = (int)(fr - vl.frame_off[b]);
+        srow = 0;
+        s0 = vl.sample_off[b] + (long long)f * frame_shift;
+    } else {
+        b = (int)(fr / frames_per_signal);
+        f = (int)(fr % frames_per_signal);
+        srow = src.row_ids ? src.row_ids[b] : b;
+        s0 = (long long)f * frame_shift;
+    }
+}
+
+template <bool VL>
 __global__ void __launch_bounds__(FB_WARPS * 32)
 fbank_kernel(FbankParams p, SampleSrc src, int B, int frames_per_signal, float* __restrict__ out,
              const int32_t* __restrict__ out_ids, long long out_row_stride, int out_frame0, float* __restrict__ out2,
-             int out2_frames, int out2_frame0) {
+             int out2_frames, int out2_frame0, FbankVarlen vl) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int P = p.fft_size, M = P >> 1;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -54,11 +82,11 @@ fbank_kernel(FbankParams p, SampleSrc src, int B, int frames_per_signal, float* 
     int log2m = 0;
     while ((1 << log2m) < M) ++log2m;
 
-    const long long total = (long long)B * frames_per_signal;
+    const long long total = VL ? vl.frames : (long long)B * frames_per_signal;
     for (long long fr = (long long)blockIdx.x * FB_WARPS + warp; fr < total; fr += (long long)gridDim.x * FB_WARPS) {
-        const int b = (int)(fr / frames_per_signal), f = (int)(fr % frames_per_signal);
-        const long long srow = src.row_ids ? src.row_ids[b] : b;
-        const long long s0 = (long long)f * p.frame_shift;
+        int b, f;
+        long long srow, s0;
+        fbank_frame<VL>(vl, src, frames_per_signal, p.frame_shift, fr, b, f, srow, s0);
         // 1. samples + mean (kaldi.py:183-186)
         float part = 0.f;
         for (int i = lane; i < p.frame_len; i += 32) {
@@ -118,9 +146,15 @@ fbank_kernel(FbankParams p, SampleSrc src, int B, int frames_per_signal, float* 
         }
         __syncwarp();
         // 5. mel + log (kaldi.py:630-633)
-        const long long orow = out_ids ? out_ids[b] : b;
-        float* o = out + orow * out_row_stride + (long long)(out_frame0 + f) * p.n_mel;
-        float* o2 = out2 ? out2 + ((long long)b * out2_frames + out2_frame0 + f) * p.n_mel : nullptr;
+        float *o, *o2;
+        if constexpr (VL) {
+            o = out + ((long long)vl.out_row[b] + f) * p.n_mel;
+            o2 = out2 ? out2 + ((long long)vl.frame_off[b] + f) * p.n_mel : nullptr;
+        } else {
+            const long long orow = out_ids ? out_ids[b] : b;
+            o = out + orow * out_row_stride + (long long)(out_frame0 + f) * p.n_mel;
+            o2 = out2 ? out2 + ((long long)b * out2_frames + out2_frame0 + f) * p.n_mel : nullptr;
+        }
         for (int m = lane; m < p.n_mel; m += 32) {
             const int lo = p.mel_lo[m], hi = p.mel_hi[m];
             const float* wrow = p.mel + (long long)m * (M + 1);
@@ -210,7 +244,8 @@ int upload_twiddles(int P) {
         host[k].y = sin(-2.0 * PI * k / P);
     }
     FO_CUDA(cudaMemcpyToSymbol(c_twiddle, host, sizeof(double2) * (P / 2)));
-    FO_CUDA(cudaFuncSetAttribute(fbank_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
+    FO_CUDA(cudaFuncSetAttribute(fbank_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
+    FO_CUDA(cudaFuncSetAttribute(fbank_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
     g_twiddle_fft = P;
     return 0;
 }
@@ -234,9 +269,9 @@ int fbank_stream(const FbankParams& p, const int32_t* ids, int n, const void* pc
     SampleSrc src{carry, 0, 1.0f, (long long)(carry_n + chunk), ids};
     const long long frames = (long long)n * frames_per_chunk;
     const int grid = (int)((frames + FB_WARPS - 1) / FB_WARPS);
-    fbank_kernel<<<grid, FB_WARPS * 32, fbank_smem(p.fft_size), st>>>(
+    fbank_kernel<false><<<grid, FB_WARPS * 32, fbank_smem(p.fft_size), st>>>(
         p, src, n, frames_per_chunk, ring, ids, (long long)(ctx_frames + frames_per_chunk) * p.n_mel, ctx_frames,
-        feats_out, ctx_frames + frames_per_chunk, ctx_frames);
+        feats_out, ctx_frames + frames_per_chunk, ctx_frames, FbankVarlen());
     FO_LAUNCHED();
     FO_CUDA(cudaGetLastError());
     return 0;
@@ -254,9 +289,9 @@ int fbank_stream_blocks(const FbankParams& p, const int32_t* ids, const int32_t*
     FO_CUDA(cudaGetLastError());
     SampleSrc src{rows, 0, 1.0f, (long long)(carry_n + chunk), nullptr};
     const long long frames = (long long)blocks * frames_per_chunk;
-    fbank_kernel<<<(int)((frames + FB_WARPS - 1) / FB_WARPS), FB_WARPS * 32, fbank_smem(p.fft_size), st>>>(
+    fbank_kernel<false><<<(int)((frames + FB_WARPS - 1) / FB_WARPS), FB_WARPS * 32, fbank_smem(p.fft_size), st>>>(
         p, src, blocks, frames_per_chunk, feats_out, nullptr, (long long)(ctx_frames + frames_per_chunk) * p.n_mel, ctx_frames,
-        nullptr, 0, 0);
+        nullptr, 0, 0, FbankVarlen());
     FO_LAUNCHED();
     FO_CUDA(cudaGetLastError());
     frontend_blocks_finish_kernel<<<n, 256, 0, st>>>(ids, cnt, off, carry_n, chunk, ctx_frames, frames_per_chunk, p.n_mel, rows,
@@ -275,8 +310,21 @@ int fbank_offline(const FbankParams& p, const void* pcm, int pcm_is_i16, int B, 
     const long long frames = (long long)B * m;
     long long want = (frames + FB_WARPS - 1) / FB_WARPS;
     const int grid = (int)(want < 148 * 16 ? want : 148 * 16);      // persistent-ish: 16 CTAs per SM, grid-stride
-    fbank_kernel<<<grid, FB_WARPS * 32, fbank_smem(p.fft_size), st>>>(p, src, B, m, out, nullptr,
-                                                                      (long long)m * p.n_mel, 0, nullptr, 0, 0);
+    fbank_kernel<false><<<grid, FB_WARPS * 32, fbank_smem(p.fft_size), st>>>(p, src, B, m, out, nullptr,
+                                                                             (long long)m * p.n_mel, 0, nullptr, 0, 0, FbankVarlen());
+    FO_LAUNCHED();
+    FO_CUDA(cudaGetLastError());
+    return 0;
+}
+
+int fbank_offline_packed(const FbankParams& p, const void* pcm, int pcm_is_i16, float scale, const FbankVarlen& vl, float* out,
+                         float* out2, cudaStream_t st) {
+    if (vl.n <= 0 || vl.frames <= 0) return 0;
+    FO_TRY(upload_twiddles(p.fft_size));
+    SampleSrc src{pcm, pcm_is_i16, scale, 0, nullptr};
+    long long want = (vl.frames + FB_WARPS - 1) / FB_WARPS;
+    const int grid = (int)(want < 148 * 16 ? want : 148 * 16);      // as fbank_offline
+    fbank_kernel<true><<<grid, FB_WARPS * 32, fbank_smem(p.fft_size), st>>>(p, src, 0, 0, out, nullptr, 0, 0, out2, 0, 0, vl);
     FO_LAUNCHED();
     FO_CUDA(cudaGetLastError());
     return 0;

@@ -1075,6 +1075,7 @@ void gemm_tc_set_persist(int on) { g_persist = on; }
 long long gemm_tc_persist_launches() { return g_persist_launches; }
 void gemm_tc_force_producers(int npa, int npb) { g_forced_npa = npa; g_forced_npb = npb; }
 long long gemm_tc_launches() { return g_tc_launches; }
+long long gemm_tc_max_rows(int N) { return (long long)(MAX_TILES / ((N + 255) / 256)) * BM; }
 
 int gemm_tc(const void* A, int act_fp16, const AGather& ga, const void* W, int M, int N, int K, const Epilogue& ep,
             const RowMap& rmap, const TcWorkspace& ws, cudaStream_t st, int* deferred_splits) {

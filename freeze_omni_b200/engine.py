@@ -286,6 +286,36 @@ class Engine:
                                              self._stream()))
         return out
 
+    def _packed_pcm(self, pcms, n_samples):
+        """(packed 1-D PCM, n_samples int64) from a list of 1-D int16 / float32 tensors or arrays, or a packed 1-D one plus
+        n_samples.  A list with a CUDA tensor is packed on the engine's device, else on the host."""
+        if n_samples is not None:
+            ns = np.ascontiguousarray(np.asarray(n_samples.cpu() if isinstance(n_samples, torch.Tensor) else n_samples,
+                                                 dtype=np.int64).reshape(-1))
+            assert pcms.ndim == 1 and int(ns.sum()) == pcms.shape[0], "packed pcm must be 1-D with sum(n_samples) samples"
+            return pcms, ns
+        pcms = list(pcms)
+        assert pcms and all(p.ndim == 1 for p in pcms), "pcms must be a non-empty list of 1-D signals"
+        dts = {self._pcm_dtype(p) for p in pcms}
+        assert len(dts) == 1, "all signals must share one dtype (int16 or float32)"
+        ns = np.array([p.shape[0] for p in pcms], dtype=np.int64)
+        if any(isinstance(p, torch.Tensor) for p in pcms):
+            ts = [p if isinstance(p, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(p)) for p in pcms]
+            dev = self.torch_device if any(t.is_cuda for t in ts) else torch.device("cpu")
+            return torch.cat([t.to(dev) for t in ts]), ns
+        return np.ascontiguousarray(np.concatenate(pcms)), ns
+
+    def fbank_offline_packed(self, pcms, scale: Optional[float] = None, n_samples=None):
+        """Filterbank of utterances of different lengths in one call.  Returns (feats (sum m_i, F), frame_offsets int64 (B + 1)):
+        utterance i's frames are rows [off[i], off[i+1]), each bit-identical to fbank_offline of it alone."""
+        pcm, ns = self._packed_pcm(pcms, n_samples)
+        m = np.where(ns >= self.cfg.frame_len, 1 + (ns - self.cfg.frame_len) // self.cfg.frame_shift, 0)
+        off = np.concatenate([[0], np.cumsum(m)]).astype(np.int64)
+        out = torch.empty(int(off[-1]), self.cfg.feat_dim, device=self.torch_device)
+        _lib.check(self.lib.fo_fbank_offline_packed(self._h, _ptr(pcm), self._pcm_dtype(pcm), ns.ctypes.data, len(ns),
+                                                    self._scale(pcm, scale), _ptr(out), self._stream()))
+        return out, off
+
     # ---- streaming --------------------------------------------------------------------------------
     def out_frames(self, t_in: int) -> Tuple[int, int]:
         t = PathConfig.sub_len(t_in)
@@ -489,6 +519,24 @@ class Engine:
         _lib.check(self.lib.fo_encode_offline_packed(self._h, _ptr(feats), ln.ctypes.data, len(ln), chunk, left, _ptr(enc), _ptr(y),
                                                      self._stream()))
         return enc, y, eoff, aoff
+
+    def encode_offline_packed_pcm(self, pcms, chunk: Optional[int] = None, left: Optional[int] = None, scale: Optional[float] = None,
+                                  want_adapter: Optional[bool] = None, want_feats: bool = False, n_samples=None):
+        """PCM -> embeddings for utterances of different lengths, fbank included, in one call that runs in passes of bounded
+        memory (option packed_pass_frames).  pcms as for fbank_offline_packed.  Returns (enc, adapter rows or None, enc_offsets,
+        adapter_offsets[, feats]) as encode_offline_packed does, feats (sum m_i, F) being fbank_offline_packed's features."""
+        pcm, ns = self._packed_pcm(pcms, n_samples)
+        chunk = self.cfg.chunk_size if chunk is None else int(chunk)
+        left = self.cfg.left_chunks if left is None else int(left)
+        m, eoff, aoff = self.cfg.packed_audio_offsets(ns)
+        want_adapter = self.has_adapter if want_adapter is None else want_adapter
+        enc = torch.empty(int(eoff[-1]), self.cfg.d_model, device=self.torch_device)
+        y = torch.empty(int(aoff[-1]), self.cfg.llm_dim, device=self.torch_device) if want_adapter else None
+        feats = torch.empty(int(m.sum()), self.cfg.feat_dim, device=self.torch_device) if want_feats else None
+        _lib.check(self.lib.fo_encode_offline_packed_pcm(self._h, _ptr(pcm), self._pcm_dtype(pcm), ns.ctypes.data, len(ns),
+                                                         self._scale(pcm, scale), chunk, left, _ptr(enc), _ptr(y), _ptr(feats),
+                                                         self._stream()))
+        return (enc, y, eoff, aoff, feats) if want_feats else (enc, y, eoff, aoff)
 
     def adapter_forward(self, x: torch.Tensor, mask: Optional[torch.Tensor], cache):
         """Stateless adapter: x (B,T,D), mask (B,1,T)|(B,T) bool or None.  `cache`: None, a tensor (B,D,k-1) (single-conv

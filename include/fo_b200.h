@@ -169,6 +169,13 @@ int fo_fbank_stream(fo_ctx* ctx, const int32_t* ids, int n, const void* pcm, int
  * pcm (B, n_samples); out (B, 1 + (n_samples-frame_len)/frame_shift, feat_dim). */
 int fo_fbank_offline(fo_ctx* ctx, const void* pcm, int pcm_dtype, int B, int64_t n_samples, float scale,
                      float* out, void* stream);
+/* torchaudio.compliance.kaldi.fbank on B signals of different lengths packed end to end (a corpus without padding).
+ * pcm: sum n_samples[i] samples, FO_F32 or FO_I16, host or device; value used = sample * scale.  n_samples: HOST, B int64.
+ * Utterance i gets m_i = 1 + (n_samples[i] - frame_len) / frame_shift frames (snip_edges: trailing samples that fill no frame
+ * are dropped); out (sum m_i, feat_dim) in utterance order, every row bit-identical to fo_fbank_offline of that utterance
+ * alone.  FO_ERR_ARG, with nothing enqueued, for B <= 0, an n_samples[i] < frame_len (naming i) or a bad pcm_dtype. */
+int fo_fbank_offline_packed(fo_ctx* ctx, const void* pcm, int pcm_dtype, const int64_t* n_samples, int B, float scale,
+                            float* out, void* stream);
 
 /* ---- streaming chunk: replaces speechEncoder.infer (models/encoder/encoder.py:149-155) followed by
  * CNNSubsampling.forward(cache=..., return_cache=True) (models/adapter.py:112-157), i.e. the two
@@ -259,6 +266,22 @@ int fo_encode_offline(fo_ctx* ctx, const float* feats, const int32_t* ilens, int
  * enqueued, for B <= 0, a T_i < 7 or a T'_i past pos_max_len. */
 int fo_encode_offline_packed(fo_ctx* ctx, const float* feats, const int32_t* lens, int B, int chunk, int left,
                              float* enc_out, float* adapter_out, void* stream);
+/* PCM -> embeddings for utterances of different lengths packed end to end: torchaudio.compliance.kaldi.fbank +
+ * speechEncoder.forward (models/encoder/encoder.py:104-147) + the configured adapter per utterance, in one call.  pcm and
+ * n_samples as in fo_fbank_offline_packed; enc_out / adapter_out / chunk / left as in fo_encode_offline_packed for the frame
+ * counts m_i; feats_out (sum m_i, feat_dim) receives the features of fo_fbank_offline_packed.  Any output may be NULL; host or
+ * device.  The fbank writes each utterance's frames straight onto the packed encoder's feature grid.
+ * Passes: utterance i takes ceil(m_i / 4) * 4 grid frames, and the call runs over consecutive utterances in call order, a pass
+ * taking them while their grid frames fit the option "packed_pass_frames" (default: a 10 GiB workspace budget; never more than
+ * the conv2 GEMM of one pass takes; fo_get_option returns the frames in force); an utterance larger than that runs in a pass
+ * of its own.  So the device memory the call adds
+ * follows the budget, not the corpus.  Host PCM is uploaded one pass at a time, host outputs copied back per pass.  Each pass's
+ * rows are bit-identical to fo_fbank_offline per utterance followed by fo_encode_offline_packed over that pass's utterances.
+ * FO_ERR_ARG, with nothing enqueued, for a context without a finalized encoder, adapter_out without an adapter, B <= 0, a bad
+ * pcm_dtype, an m_i < 7 or a T'_i past pos_max_len (naming the utterance; all are checked before the first pass).
+ * Counts as one offline call. */
+int fo_encode_offline_packed_pcm(fo_ctx* ctx, const void* pcm, int pcm_dtype, const int64_t* n_samples, int B, float scale,
+                                 int chunk, int left, float* enc_out, float* adapter_out, float* feats_out, void* stream);
 
 /* ---- stateless adapter: replaces CNNSubsampling.forward (models/adapter.py:112-157) when the
  * caller owns the cache tensor.  x (B, T, d_model); mask (B, T) uint8 or NULL (all valid);

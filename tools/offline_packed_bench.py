@@ -2,9 +2,13 @@
 model in bf16 (SURVEY 8d config 4 and its ragged variant).
 
   * ragged: 256 utterances of seeded U[10, 30] s int16 audio; equal: 256 x 30 s, where the two entries do the same rows.
-  * Each leg is fbank + encoder + adapter over the 256 utterances in slices of --slice (as bench.py slices the padded batch):
-    padded = fbank_offline of the slice padded to its longest utterance, then encode_offline; packed = fbank_offline per
-    utterance into one packed feature buffer, then encode_offline_packed.  Audio on the device before timing.
+  * Each leg is fbank + encoder + adapter over the 256 utterances (audio on the device before timing):
+    padded = per slice of --slice (as bench.py slices the padded batch), fbank_offline of the slice padded to its longest
+    utterance, then encode_offline; packed = per slice, fbank_offline per utterance into one packed feature buffer, then
+    encode_offline_packed; packed_pcm = per slice, one encode_offline_packed_pcm (fbank written onto the packed grid);
+    corpus_pcm = ONE encode_offline_packed_pcm over all utterances, in passes at the default packed_pass_frames budget.
+  * Every leg has an engine of its own (same weights), so fo_stats.device_bytes after a leg is that leg's footprint:
+    weights plus the workspaces it grew (`device_bytes` per workload, read after its timed runs; the equal set runs second).
   * The legs alternate --reps times in one process after a warm-up each; best and median, audio-s per s of real audio.
   * rows: encoder rows each entry computes (padded B x T'_max per slice, packed sum T'_i); their ratio bounds the gain.
 
@@ -42,7 +46,7 @@ def timed(fn):
     return (time.perf_counter() - t0) * 1e3
 
 
-def legs(eng, cfg, seconds, slice_):
+def legs(engs, cfg, seconds, slice_):
     sr = cfg.sample_rate
     g = torch.Generator().manual_seed(11)
     pcm = [(0.05 * torch.randn(int(s * sr), generator=g) * 32768).round().clamp(-32768, 32767).to(torch.int16).cuda() for s in seconds]
@@ -61,21 +65,33 @@ def legs(eng, cfg, seconds, slice_):
         rows["padded"] += len(il) * cfg.sub_len(int(il.max()))
         rows["packed"] += int(sum(cfg.sub_len(int(t)) for t in il))
 
-    def padded():
+    def padded(eng=engs["padded"]):
         for x, il in pad:
             feats = eng.fbank_offline(x, 1.0)
             eng.encode_offline(feats, il, cfg.chunk_size, cfg.left_chunks)
 
-    def packed():
+    def packed(eng=engs["packed"]):
         for (x, il), sl in zip(pad, slices):
             feats = torch.cat([eng.fbank_offline(pcm[i][None], 1.0)[0] for i in sl])
             eng.encode_offline_packed(feats, il, cfg.chunk_size, cfg.left_chunks)
 
-    return {"padded": padded, "packed": packed}, rows
+    flat = [torch.cat([pcm[i] for i in sl]) for sl in slices]
+    counts = [np.array([pcm[i].numel() for i in sl], dtype=np.int64) for sl in slices]
+
+    def packed_pcm(eng=engs["packed_pcm"]):
+        for x, n in zip(flat, counts):
+            eng.encode_offline_packed_pcm(x, cfg.chunk_size, cfg.left_chunks, 1.0, n_samples=n)
+
+    corpus, corpus_n = torch.cat(flat), np.concatenate(counts)
+
+    def corpus_pcm(eng=engs["corpus_pcm"]):
+        eng.encode_offline_packed_pcm(corpus, cfg.chunk_size, cfg.left_chunks, 1.0, n_samples=corpus_n)
+
+    return {"padded": padded, "packed": packed, "packed_pcm": packed_pcm, "corpus_pcm": corpus_pcm}, rows
 
 
-def bench(eng, cfg, name, seconds, slice_, reps):
-    fns, rows = legs(eng, cfg, seconds, slice_)
+def bench(engs, cfg, name, seconds, slice_, reps):
+    fns, rows = legs(engs, cfg, seconds, slice_)
     times = {k: [] for k in fns}
     for fn in fns.values():
         fn()
@@ -87,8 +103,11 @@ def bench(eng, cfg, name, seconds, slice_, reps):
            "row_ratio": rows["padded"] / rows["packed"]}
     for k, v in times.items():
         best = min(v)
-        out[k] = {"ms_best": best, "ms_median": statistics.median(v), "audio_s_per_s": audio / (best * 1e-3), "ms_all": v}
+        out[k] = {"ms_best": best, "ms_median": statistics.median(v), "audio_s_per_s": audio / (best * 1e-3), "ms_all": v,
+                  "device_bytes": engs[k].stats()["device_bytes"]}
     out["speedup_best"] = out["padded"]["ms_best"] / out["packed"]["ms_best"]
+    out["packed_pcm_vs_packed_best"] = out["packed"]["ms_best"] / out["packed_pcm"]["ms_best"]
+    out["corpus_pcm_vs_packed_best"] = out["packed"]["ms_best"] / out["corpus_pcm"]["ms_best"]
     print(json.dumps({k: (v if not isinstance(v, dict) else {kk: vv for kk, vv in v.items() if kk != "ms_all"}) for k, v in out.items()}),
           flush=True)
     return out
@@ -105,12 +124,16 @@ def main():
         raise SystemExit("needs a CUDA device")
     result = {"gpu": gpu_info()}
     cfg = load_path_config("shipped")
-    eng = Engine(cfg, make_encoder_state(cfg, 0), make_adapter_state(cfg, 0), dtype=torch.bfloat16, max_sessions=2)
+    esd, asd = make_encoder_state(cfg, 0), make_adapter_state(cfg, 0)
+    engs = {k: Engine(cfg, esd, asd, dtype=torch.bfloat16, max_sessions=2) for k in ("padded", "packed", "packed_pcm", "corpus_pcm")}
+    result["packed_pass_frames"] = engs["corpus_pcm"].get_option("packed_pass_frames")
+    result["device_bytes_weights"] = {k: e.stats()["device_bytes"] for k, e in engs.items()}
     rng = np.random.default_rng(2024)
     ragged = [round(float(s), 2) for s in rng.uniform(10.0, 30.0, size=args.utterances)]
-    result["runs"] = [bench(eng, cfg, "ragged_U10_30s", ragged, args.slice, args.reps),
-                      bench(eng, cfg, "equal_30s", [30.0] * args.utterances, args.slice, args.reps)]
-    eng.close()
+    result["runs"] = [bench(engs, cfg, "ragged_U10_30s", ragged, args.slice, args.reps),
+                      bench(engs, cfg, "equal_30s", [30.0] * args.utterances, args.slice, args.reps)]
+    for e in engs.values():
+        e.close()
     result["gpu_after"] = gpu_info()
     os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
     with open(args.out, "w") as f:
