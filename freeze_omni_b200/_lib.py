@@ -62,6 +62,8 @@ SYMBOLS = {
     "fo_encode_stream_chunks_v": (C.c_int, [_P, _I32P, _I32P, C.c_int, _P, C.c_int, _P, _P, _P]),
     "fo_stream_step": (C.c_int, [_P, _I32P, C.c_int, _P, C.c_int, C.c_float, _P, _P, _P]),
     "fo_stream_steps_v": (C.c_int, [_P, _I32P, _I32P, C.c_int, _P, C.c_int, C.c_float, _P, _P, _P]),
+    "fo_fbank_stream_v": (C.c_int, [_P, _I32P, _I32P, C.c_int, _P, C.c_int, C.c_float, _P, _P]),
+    "fo_encode_stream_steps_v": (C.c_int, [_P, _I32P, _I32P, C.c_int, _P, C.c_int, _P, _P, _P]),
     "fo_debug_trace_read": (C.c_int, [_P, _P, C.c_int64, _I64P]),
     "fo_debug_plan": (C.c_int, [C.c_int64, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "fo_debug_stack_plan": (C.c_int, [C.c_int] * 9 + [C.POINTER(C.c_int)] * 5),

@@ -2589,10 +2589,12 @@ int fo_stream_step(fo_ctx* c, const int32_t* ids, int n, const void* pcm, int pc
 }
 
 // ---- recorded audio: many chunks per session, exact-streaming ----------------------------------------
-// fo_stream_steps_v runs in passes of at most P blocks (option "steps_pass_blocks", else STEPS_PASS_BYTES over the workspace
-// bytes of one block): each pass gives every session that still has chunks its next min(remaining, q) chunks, q = the
-// longest remaining count spread evenly over the passes that max(1, P / sessions left) chunks per pass would take; it then
-// runs the fbank of those blocks (fbank_stream_blocks) and the streaming program, whose attention spreads a session's chunks over groups of CTAs (Mix::group).  Every workspace is sized by the pass, so the device memory a call adds does not grow with the recording.
+// The recording entries (fo_stream_steps_v, fo_fbank_stream_v, fo_encode_stream_steps_v) run in passes of at most P blocks
+// (option "steps_pass_blocks", else STEPS_PASS_BYTES over the workspace bytes of one block): each pass gives every session that
+// still has chunks its next min(remaining, q) chunks, q = the longest remaining count spread evenly over the passes that
+// max(1, P / sessions left) chunks per pass would take.  A pass takes its blocks' features from PCM (fbank_stream_blocks) or
+// from the caller, then runs the streaming program, whose attention spreads a session's chunks over groups of CTAs (Mix::group).
+// Every workspace is sized by the pass, so the device memory a call adds does not grow with the recording.
 // Passes run eagerly: a captured graph per pass shape would multiply with recording lengths.
 constexpr long long STEPS_PASS_BYTES = 1LL << 30;
 
@@ -2608,38 +2610,46 @@ static long long steps_block_bytes(const fo_ctx* c, int t_in) {
     return b;
 }
 
-int fo_stream_steps_v(fo_ctx* c, const int32_t* ids, const int32_t* chunks, int n, const void* pcm, int pcm_dtype, float scale,
-                      float* enc_out, float* adapter_out, void* stream) {
-    FO_CHECK(c && c->finalized && c->cfg.has_encoder && c->fb_window, "fo_stream_steps_v: context has no finalized encoder + frontend");
-    FO_CHECK(pcm && (pcm_dtype == FO_F32 || pcm_dtype == FO_I16), "fo_stream_steps_v: pcm must be FO_F32 or FO_I16");
-    FO_CHECK(chunks, "fo_stream_steps_v: chunks must be a host array of n counts");
-    FO_CHECK(!c->armed.on, "fo_stream_steps_v: an LLM hand-off is armed (fo_handoff_arm); this call does not take it, and it stays "
-                           "armed for the next fo_stream_step / fo_encode_stream call");
-    FO_TRY(check_ids(c, ids, n));
-    const int t_in = c->cfg.context_frames + c->cfg.frames_per_chunk;
-    FO_TRY(stream_geometry(c, t_in));
-    FO_CHECK(!c->KM, "fo_stream_steps_v: MultiLayeredConv1d has no streaming form (models/encoder/attention.py:145-196); use fo_encode_offline");
-    if (adapter_out) FO_CHECK(c->cfg.has_adapter, "adapter_out requested but the context has no adapter");
+static int steps_pass_blocks(const fo_ctx* c, int t_in) {
+    return c->steps_pass_blocks > 0 ? c->steps_pass_blocks
+                                    : (int)std::max(1LL, std::min(1LL << 20, STEPS_PASS_BYTES / steps_block_bytes(c, t_in)));
+}
+
+static int check_steps_counts(const char* fn, const int32_t* ids, const int32_t* chunks, int n) {
+    for (int i = 0; i < n; ++i)
+        FO_CHECK(chunks[i] >= 1, "%s: session %d (id %d) has chunk count %d; counts must be >= 1", fn, i, ids[i], chunks[i]);
+    return 0;
+}
+
+// What one recording call reads and writes.  Blocks come from PCM (pcm != null) or from the caller's features (feats);
+// feats_out receives the features of PCM blocks; with `encode` the blocks run through the encoder into enc_out / adapter_out.
+struct StepsIo {
+    const void* pcm = nullptr;
+    int pcm_dtype = FO_F32;
+    float scale = 1.0f;
+    const float* feats = nullptr;
+    float* feats_out = nullptr;
+    bool encode = false;
+    float* enc_out = nullptr;
+    float* adapter_out = nullptr;
+};
+
+// The pass loop shared by the recording entries; arguments are checked by the caller, so nothing here refuses a call.
+static int steps_passes(fo_ctx* c, const int32_t* ids, const int32_t* chunks, int n, int t_in, const StepsIo& io, cudaStream_t st) {
     std::vector<long long> off(n + 1, 0);
-    for (int i = 0; i < n; ++i) {
-        FO_CHECK(chunks[i] >= 1, "fo_stream_steps_v: session %d (id %d) has chunk count %d; counts must be >= 1", i, ids[i], chunks[i]);
-        off[i + 1] = off[i] + chunks[i];
-    }
-    FO_CUDA(cudaSetDevice(c->device));
-    cudaStream_t st = (cudaStream_t)stream;
+    for (int i = 0; i < n; ++i) off[i + 1] = off[i] + chunks[i];
     if (c->copy_stream && c->async_ticket > 0) {       // as in stream_common: pipelined steps still read the shared buffers
         FO_CUDA(cudaStreamWaitEvent(st, c->ev_out[0], 0));
         if (c->async_ticket > 1) FO_CUDA(cudaStreamWaitEvent(st, c->ev_out[1], 0));
     }
-    const int T1 = (t_in - 1) / 2, t = (T1 - 1) / 2, t_out = ad_frames(c, t);
-    const int P = c->steps_pass_blocks > 0 ? c->steps_pass_blocks
-                                           : (int)std::max(1LL, std::min(1LL << 20, STEPS_PASS_BYTES / steps_block_bytes(c, t_in)));
-    const long long pcm_row = (long long)c->chunk_samples * (pcm_dtype == FO_I16 ? 2 : 4);
-    const long long enc_row = (long long)t * c->D, y_row = (long long)t_out * c->E;
-    const bool want_y = adapter_out != nullptr;
+    const int T1 = (t_in - 1) / 2, t = (T1 - 1) / 2, t_out = c->cfg.has_encoder ? ad_frames(c, t) : 0;
+    const int P = steps_pass_blocks(c, t_in);
+    const long long pcm_row = (long long)c->chunk_samples * (io.pcm_dtype == FO_I16 ? 2 : 4);
+    const long long feat_row = (long long)t_in * c->F, enc_row = (long long)t * c->D, y_row = (long long)t_out * c->E;
+    const bool want_y = io.adapter_out != nullptr;
     int sms = 148;
     FO_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->device));
-    const int gmax = std::max(1, (STREAM_CHUNKS_MAX_KEYS - c->window) / t);
+    const int gmax = std::max(1, (STREAM_CHUNKS_MAX_KEYS - c->window) / std::max(1, t));
     g_use_pdl = g_want_pdl;
     std::vector<int32_t> done(n, 0), pids, pcnt, poff, psrc;
     for (;;) {
@@ -2661,43 +2671,126 @@ int fo_stream_steps_v(fo_ctx* c, const int32_t* ids, const int32_t* chunks, int 
         }
         m.blocks = poff.back();
         m.off = poff.data();
-        // chunks per attention CTA: enough (session, head, group) CTAs to fill the SMs, each staging at most 128 keys
-        const int want = std::max(1, (sms + na * c->H - 1) / (na * c->H));
-        m.group = std::min(gmax, std::max(1, (m.kmax + want - 1) / want));
         FO_TRY(upload_ids(c, pids.data(), na, st, nullptr, 0, pcnt.data()));
         c->pf_slot_lo = *std::min_element(pids.begin(), pids.end());
         c->pf_slot_hi = *std::max_element(pids.begin(), pids.end());
-        void *dpcm, *drows, *dfeats, *denc, *dy = nullptr;
-        FO_TRY(ws_ensure(c, WS_PCM, (size_t)m.blocks * c->chunk_samples * 4, &dpcm));
-        FO_TRY(ws_ensure(c, WS_SROWS, (size_t)m.blocks * (c->carry + c->chunk_samples) * sizeof(float), &drows));
-        FO_TRY(ws_ensure(c, WS_FEATS, (size_t)m.blocks * t_in * c->F * sizeof(float), &dfeats));
-        FO_TRY(ws_ensure(c, WS_ENC, (size_t)m.blocks * enc_row * sizeof(float), &denc));
-        if (want_y) FO_TRY(ws_ensure(c, WS_Y, (size_t)m.blocks * y_row * sizeof(float), &dy));
-        for (int a = 0; a < na; ++a) {
-            const int i = psrc[a];
-            FO_CUDA(cudaMemcpyAsync((char*)dpcm + poff[a] * pcm_row, (const char*)pcm + (off[i] + done[i]) * pcm_row, pcnt[a] * pcm_row,
-                                    cudaMemcpyDefault, st));
+        void *dpcm = nullptr, *drows = nullptr, *dfeats, *denc = nullptr, *dy = nullptr;
+        if (io.pcm) {
+            FO_TRY(ws_ensure(c, WS_PCM, (size_t)m.blocks * c->chunk_samples * 4, &dpcm));
+            FO_TRY(ws_ensure(c, WS_SROWS, (size_t)m.blocks * (c->carry + c->chunk_samples) * sizeof(float), &drows));
         }
-        FO_TRY(fbank_stream_blocks(fbank_params(c), c->ids_dev, c->cnt_dev, c->off_dev, na, m.kmax, m.blocks, dpcm, pcm_dtype == FO_I16,
-                                   scale, c->cfg.frames_per_chunk, c->cfg.context_frames, c->samples, c->feat_ring, (float*)drows,
-                                   (float*)dfeats, st));
-        FO_TRY(c->dtype == FO_BF16 ? stream_program<act16>(c, na, m, (const float*)dfeats, t_in, (float*)denc, (float*)dy, st)
-                                   : stream_program<float>(c, na, m, (const float*)dfeats, t_in, (float*)denc, (float*)dy, st));
-        for (int a = 0; a < na; ++a) {
-            const int i = psrc[a];
-            const long long b0 = off[i] + done[i];
-            if (enc_out) FO_CUDA(cudaMemcpyAsync(enc_out + b0 * enc_row, (float*)denc + poff[a] * enc_row, pcnt[a] * enc_row * sizeof(float),
-                                                 cudaMemcpyDefault, st));
-            if (want_y) FO_CUDA(cudaMemcpyAsync(adapter_out + b0 * y_row, (float*)dy + poff[a] * y_row, pcnt[a] * y_row * sizeof(float),
-                                                cudaMemcpyDefault, st));
-            done[i] += pcnt[a];
+        FO_TRY(ws_ensure(c, WS_FEATS, (size_t)m.blocks * feat_row * sizeof(float), &dfeats));
+        if (io.encode) {
+            FO_TRY(ws_ensure(c, WS_ENC, (size_t)m.blocks * enc_row * sizeof(float), &denc));
+            if (want_y) FO_TRY(ws_ensure(c, WS_Y, (size_t)m.blocks * y_row * sizeof(float), &dy));
         }
+        if (io.pcm) {
+            for (int a = 0; a < na; ++a) {
+                const int i = psrc[a];
+                FO_CUDA(cudaMemcpyAsync((char*)dpcm + poff[a] * pcm_row, (const char*)io.pcm + (off[i] + done[i]) * pcm_row,
+                                        pcnt[a] * pcm_row, cudaMemcpyDefault, st));
+            }
+            FO_TRY(fbank_stream_blocks(fbank_params(c), c->ids_dev, c->cnt_dev, c->off_dev, na, m.kmax, m.blocks, dpcm,
+                                       io.pcm_dtype == FO_I16, io.scale, c->cfg.frames_per_chunk, c->cfg.context_frames, c->samples,
+                                       c->feat_ring, (float*)drows, (float*)dfeats, st));
+        } else {
+            for (int a = 0; a < na; ++a) {
+                const int i = psrc[a];
+                FO_CUDA(cudaMemcpyAsync((float*)dfeats + poff[a] * feat_row, io.feats + (off[i] + done[i]) * feat_row,
+                                        pcnt[a] * feat_row * sizeof(float), cudaMemcpyDefault, st));
+            }
+        }
+        if (io.feats_out)
+            for (int a = 0; a < na; ++a) {
+                const int i = psrc[a];
+                FO_CUDA(cudaMemcpyAsync(io.feats_out + (off[i] + done[i]) * feat_row, (float*)dfeats + poff[a] * feat_row,
+                                        pcnt[a] * feat_row * sizeof(float), cudaMemcpyDefault, st));
+            }
+        if (io.encode) {
+            // chunks per attention CTA: enough (session, head, group) CTAs to fill the SMs, each staging at most 128 keys
+            const int want = std::max(1, (sms + na * c->H - 1) / (na * c->H));
+            m.group = std::min(gmax, std::max(1, (m.kmax + want - 1) / want));
+            FO_TRY(c->dtype == FO_BF16 ? stream_program<act16>(c, na, m, (const float*)dfeats, t_in, (float*)denc, (float*)dy, st)
+                                       : stream_program<float>(c, na, m, (const float*)dfeats, t_in, (float*)denc, (float*)dy, st));
+            for (int a = 0; a < na; ++a) {
+                const int i = psrc[a];
+                const long long b0 = off[i] + done[i];
+                if (io.enc_out) FO_CUDA(cudaMemcpyAsync(io.enc_out + b0 * enc_row, (float*)denc + poff[a] * enc_row,
+                                                        pcnt[a] * enc_row * sizeof(float), cudaMemcpyDefault, st));
+                if (want_y) FO_CUDA(cudaMemcpyAsync(io.adapter_out + b0 * y_row, (float*)dy + poff[a] * y_row,
+                                                    pcnt[a] * y_row * sizeof(float), cudaMemcpyDefault, st));
+            }
+        }
+        for (int a = 0; a < na; ++a) done[psrc[a]] += pcnt[a];
     }
     if (!c->ev_sync) FO_CUDA(cudaEventCreateWithFlags(&c->ev_sync, cudaEventDisableTiming));
     FO_CUDA(cudaEventRecord(c->ev_sync, st));
-    c->stats.stream_steps += 1;
-    c->stats.session_chunks += off[n];
+    if (io.encode) {
+        c->stats.stream_steps += 1;
+        c->stats.session_chunks += off[n];
+    }
     return 0;
+}
+
+// the refusals of the encoding recording entries (fo_stream_steps_v, fo_encode_stream_steps_v)
+static int check_steps_encode(fo_ctx* c, const char* fn, const int32_t* ids, const int32_t* chunks, int n, int t_in,
+                              const float* adapter_out) {
+    FO_CHECK(chunks, "%s: chunks must be a host array of n counts", fn);
+    FO_CHECK(!c->armed.on, "%s: an LLM hand-off is armed (fo_handoff_arm); this call does not take it, and it stays "
+                           "armed for the next fo_stream_step / fo_encode_stream call", fn);
+    FO_TRY(check_ids(c, ids, n));
+    FO_TRY(stream_geometry(c, t_in));
+    FO_CHECK(!c->KM, "%s: MultiLayeredConv1d has no streaming form (models/encoder/attention.py:145-196); use fo_encode_offline", fn);
+    if (adapter_out) FO_CHECK(c->cfg.has_adapter, "adapter_out requested but the context has no adapter");
+    return check_steps_counts(fn, ids, chunks, n);
+}
+
+int fo_stream_steps_v(fo_ctx* c, const int32_t* ids, const int32_t* chunks, int n, const void* pcm, int pcm_dtype, float scale,
+                      float* enc_out, float* adapter_out, void* stream) {
+    FO_CHECK(c && c->finalized && c->cfg.has_encoder && c->fb_window, "fo_stream_steps_v: context has no finalized encoder + frontend");
+    FO_CHECK(pcm && (pcm_dtype == FO_F32 || pcm_dtype == FO_I16), "fo_stream_steps_v: pcm must be FO_F32 or FO_I16");
+    const int t_in = c->cfg.context_frames + c->cfg.frames_per_chunk;
+    FO_TRY(check_steps_encode(c, "fo_stream_steps_v", ids, chunks, n, t_in, adapter_out));
+    FO_CUDA(cudaSetDevice(c->device));
+    StepsIo io;
+    io.pcm = pcm;
+    io.pcm_dtype = pcm_dtype;
+    io.scale = scale;
+    io.encode = true;
+    io.enc_out = enc_out;
+    io.adapter_out = adapter_out;
+    return steps_passes(c, ids, chunks, n, t_in, io, (cudaStream_t)stream);
+}
+
+int fo_encode_stream_steps_v(fo_ctx* c, const int32_t* ids, const int32_t* chunks, int n, const float* feats, int t_in,
+                             float* enc_out, float* adapter_out, void* stream) {
+    FO_CHECK(c && c->finalized && c->cfg.has_encoder, "fo_encode_stream_steps_v: context has no finalized encoder");
+    FO_CHECK(feats, "fo_encode_stream_steps_v: feats must not be NULL");
+    FO_CHECK(t_in >= 7, "fo_encode_stream_steps_v: need at least 7 feature frames per chunk");
+    FO_TRY(check_steps_encode(c, "fo_encode_stream_steps_v", ids, chunks, n, t_in, adapter_out));
+    FO_CUDA(cudaSetDevice(c->device));
+    StepsIo io;
+    io.feats = feats;
+    io.encode = true;
+    io.enc_out = enc_out;
+    io.adapter_out = adapter_out;
+    return steps_passes(c, ids, chunks, n, t_in, io, (cudaStream_t)stream);
+}
+
+int fo_fbank_stream_v(fo_ctx* c, const int32_t* ids, const int32_t* chunks, int n, const void* pcm, int pcm_dtype, float scale,
+                      float* feats_out, void* stream) {
+    FO_CHECK(c && c->finalized && c->fb_window, "fo_fbank_stream_v: context has no finalized frontend");
+    FO_CHECK(pcm && (pcm_dtype == FO_F32 || pcm_dtype == FO_I16), "fo_fbank_stream_v: pcm must be FO_F32 or FO_I16");
+    FO_CHECK(chunks, "fo_fbank_stream_v: chunks must be a host array of n counts");
+    FO_TRY(check_ids(c, ids, n));
+    FO_TRY(check_steps_counts("fo_fbank_stream_v", ids, chunks, n));
+    FO_CUDA(cudaSetDevice(c->device));
+    StepsIo io;
+    io.pcm = pcm;
+    io.pcm_dtype = pcm_dtype;
+    io.scale = scale;
+    io.feats_out = feats_out;
+    return steps_passes(c, ids, chunks, n, c->cfg.context_frames + c->cfg.frames_per_chunk, io, (cudaStream_t)stream);
 }
 
 // ---- full utterance -----------------------------------------------------------------------------------
@@ -3120,6 +3213,10 @@ int fo_get_option(fo_ctx* c, const char* name, int64_t* value) {
     else if (!strcmp(name, "fuse_ln")) *value = c->fuse_ln;
     else if (!strcmp(name, "stack_rows")) *value = c->stack_rows;
     else if (!strcmp(name, "steps_pass_blocks")) *value = c->steps_pass_blocks;
+    else if (!strcmp(name, "steps_pass_blocks_in_use")) {             // P of a recording call at the context's chunking
+        FO_CHECK(c->finalized, "fo_get_option: steps_pass_blocks_in_use needs a finalized context");
+        *value = steps_pass_blocks(c, c->cfg.context_frames + c->cfg.frames_per_chunk);
+    }
     else if (!strcmp(name, "packed_pass_frames")) *value = packed_pass_frames(c);    // the budget's frames when not set
     else if (!strcmp(name, "stack_launches")) *value = c->stack_launches;
     else if (!strcmp(name, "defer_reduce")) *value = c->defer_reduce;

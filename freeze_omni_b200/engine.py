@@ -424,6 +424,44 @@ class Engine:
                                               _ptr(adapter_out) if want_adapter else None, self._stream()))
         return enc_out, (adapter_out if want_adapter else None)
 
+    def fbank_stream_v(self, ids, chunks, pcm: ArrayLike, scale: Optional[float] = None,
+                       out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """The fbank half of stream_steps_v: session ids[i] takes chunks[i] >= 1 consecutive chunks of PCM (B, samples_per_chunk),
+        B = sum(chunks), in (session, chunk) order.  Returns feats (B, t_in, F) in that order, every block with its context
+        frames, and leaves sample carry and feature ring bit-identical to chunks[i] fbank_stream calls."""
+        ids = _ids(ids)
+        n = len(ids)
+        cnt = _ids(chunks)
+        assert len(cnt) == n, "one chunk count per session"
+        B = int(cnt.sum())
+        assert tuple(pcm.shape) == (B, self.cfg.samples_per_chunk), "pcm must be (sum(chunks), samples_per_chunk)"
+        out = self._out(out, (B, self.cfg.chunk_feat_frames, self.cfg.feat_dim))
+        _lib.check(self.lib.fo_fbank_stream_v(self._h, _i32p(ids), _i32p(cnt), n, _ptr(pcm), self._pcm_dtype(pcm),
+                                              self._scale(pcm, scale), _ptr(out), self._stream()))
+        return out
+
+    def encode_stream_steps_v(self, ids, chunks, feats: ArrayLike, want_adapter: Optional[bool] = None,
+                              enc_out: Optional[torch.Tensor] = None, adapter_out: Optional[torch.Tensor] = None):
+        """The encoder half of stream_steps_v: session ids[i] advances by chunks[i] >= 1 blocks of feats (B, t_in, F), B =
+        sum(chunks), in (session, chunk) order, with no cap on the counts (encode_stream_chunks_v stops at 128 keys).  On the
+        features fbank_stream_v gave it is bit-identical to stream_steps_v.  Returns enc (B, t, D) and adapter (B, t_out, E)."""
+        ids = _ids(ids)
+        n = len(ids)
+        cnt = _ids(chunks)
+        assert len(cnt) == n, "one chunk count per session"
+        assert feats is not None and feats.ndim == 3, "feats must be (sum(chunks), t_in, F)"
+        B, t_in = int(feats.shape[0]), int(feats.shape[1])
+        assert B == int(cnt.sum()) and tuple(feats.shape) == (B, t_in, self.cfg.feat_dim)
+        assert feats.dtype in (torch.float32, np.dtype(np.float32))
+        t, t_out = self.out_frames(t_in)
+        want_adapter = self.has_adapter if want_adapter is None else want_adapter
+        enc_out = self._out(enc_out, (B, t, self.cfg.d_model))
+        if want_adapter:
+            adapter_out = self._out(adapter_out, (B, t_out, self.cfg.llm_dim))
+        _lib.check(self.lib.fo_encode_stream_steps_v(self._h, _i32p(ids), _i32p(cnt), n, _ptr(feats), t_in, _ptr(enc_out),
+                                                     _ptr(adapter_out) if want_adapter else None, self._stream()))
+        return enc_out, (adapter_out if want_adapter else None)
+
     def stream_step_async(self, ids, pcm: ArrayLike, adapter_out: torch.Tensor, scale: Optional[float] = None,
                           enc_out: Optional[torch.Tensor] = None) -> int:
         """Pipelined stream_step for pinned HOST buffers: returns a ticket; `adapter_out` (and `enc_out`) are valid after

@@ -22,6 +22,9 @@ replaying their history, instead of 1 + onset_chunks calls.  With `mixed_calls` 
 session brings its own number of blocks (Engine.encode_stream_chunks_v), so an onset tick costs one encoder step.
 State (KV rings, adapter cache, sample carry, feature ring, history ring, queued blocks) never leaves the device, unless a
 session is moved: `detach` / `attach` carry it, history rows included, to another scheduler on any GPU.
+A recorded, VAD-annotated conversation goes through `replay` in one call: `plan_gated_replay` applies the same rule on the host,
+and windows of recorded chunks run as one fbank call (Engine.fbank_stream_v) and one encoder call (Engine.encode_stream_steps_v)
+each, with the blocks and history rows gathered on the device; the sessions end as one tick per chunk would leave them.
 """
 from collections import deque
 from typing import Any, Deque, Dict, Hashable, List, NamedTuple, Optional, Tuple
@@ -76,6 +79,36 @@ def onset_statuses(n_history: int, status: str) -> List[str]:
     if status != IPU_START or n_history == 0:
         return [status]
     return [IPU_START] + [IPU_CONT] * n_history
+
+
+class ReplaySource(NamedTuple):
+    """Where a block of a gated replay comes from: recorded chunk `index` of the replayed statuses (kind 'chunk'), or slot
+    `index` of the session's history ring as it stood before them (kind 'history', oldest slot 0)."""
+    kind: str
+    index: int
+
+
+class GatedPlan(NamedTuple):
+    blocks: List[Tuple[ReplaySource, str]]    # the encoder blocks in stream order, with their labels
+    history: List[ReplaySource]               # the history ring afterwards, oldest first
+
+
+def plan_gated_replay(statuses, history_chunks: int, onset_chunks: int) -> GatedPlan:
+    """What `tick`'s gating rule makes of a session's chunks pushed one per tick with these statuses: a silent chunk (None) only
+    enters the history ring, an 'ipu_sl' onset queues the last `onset_chunks` history slots in front of its own chunk (slots
+    still zero when no silence came before, and the same slots again for a second onset with no silence in between), any other
+    status queues its chunk.  Pure function of the statuses -> testable without a GPU."""
+    assert 0 <= onset_chunks <= history_chunks
+    ring = [ReplaySource("history", h) for h in range(history_chunks)]
+    blocks: List[Tuple[ReplaySource, str]] = []
+    for j, status in enumerate(statuses):
+        cur = ReplaySource("chunk", j)
+        if status is None:
+            ring = (ring + [cur])[1:]
+            continue
+        replayed = ring[history_chunks - onset_chunks:] if status == IPU_START and onset_chunks > 0 else []
+        blocks.extend(zip(replayed + [cur], onset_statuses(len(replayed), status)))
+    return GatedPlan(blocks, ring)
 
 
 def plan_rounds(queue_lens: Dict[Hashable, int], max_batch: int) -> List[List[Hashable]]:
@@ -406,6 +439,81 @@ class StreamScheduler:
             enc, emb = self.eng.encode_stream(ids, x[:, 0], **kw)
             return enc.unsqueeze(1), (emb.unsqueeze(1) if emb is not None else None)
         return self.eng.encode_stream_chunks(ids, x, **kw)
+
+    def replay(self, recordings: Dict[Hashable, Tuple[Any, Any]], scale: Optional[float] = None) -> Dict[Hashable, List[Block]]:
+        """Recorded, VAD-annotated audio of open sessions in one call, with the blocks, labels and session state that pushing
+        it one chunk per tick would give (plan_gated_replay).  `recordings` maps a key to (pcm (c, samples_per_chunk) int16 or
+        float32, host or device, statuses (c,) of None or str); every recording has the same PCM dtype.  Returns, per session
+        that produced output, its Blocks in stream order, and logs them in `block_log` as tick does.  The recordings run in
+        windows of at most max(P, sessions) chunks, P the engine's "steps_pass_blocks_in_use": per window one fbank_stream_v
+        over every session, the encoder blocks and the new history rows gathered on the device from the window's features and
+        the history rows, and one encode_stream_steps_v over the sessions with a block in the window.  A session with a
+        pushed chunk or queued blocks is refused before anything runs: tick first.  The LLM hand-off is not offered here."""
+        recs: Dict[Hashable, Tuple[torch.Tensor, List[Optional[str]]]] = {}
+        for key, (pcm, statuses) in recordings.items():
+            if key not in self.keys:
+                raise KeyError("session %r is not open" % (key,))
+            if key in self.pending or self.queues[key]:
+                raise RuntimeError("session %r has a pushed chunk or queued blocks: tick first, then replay" % (key,))
+            pcm, statuses = torch.as_tensor(pcm), list(statuses)
+            if pcm.dtype not in (torch.int16, torch.float32):
+                raise TypeError("session %r: PCM must be int16 or float32, got %s" % (key, pcm.dtype))
+            if pcm.ndim != 2 or pcm.shape[1] != self.cfg.samples_per_chunk or pcm.shape[0] != len(statuses):
+                raise ValueError("session %r: pcm %s and %d statuses do not form (c, %d) chunks with one status each"
+                                 % (key, tuple(pcm.shape), len(statuses), self.cfg.samples_per_chunk))
+            if any(st is not None and not isinstance(st, str) for st in statuses):
+                raise TypeError("session %r: statuses must be None or str" % (key,))
+            if len(statuses):
+                recs[key] = (pcm, statuses)
+        if len({p.dtype for p, _ in recs.values()}) > 1:
+            raise TypeError("the recordings of one replay must share one PCM dtype")
+        out: Dict[Hashable, List[Block]] = {}
+        dev, H = self.eng.torch_device, self.history_chunks
+        P = self.eng.get_option("steps_pass_blocks_in_use")
+        done = {key: 0 for key in recs}
+        while True:
+            active = [key for key in recs if done[key] < len(recs[key][1])]
+            if not active:
+                return out
+            q = max(1, P // len(active))
+            counts = [min(q, len(recs[key][1]) - done[key]) for key in active]
+            pcm = torch.cat([recs[key][0][done[key]:done[key] + c].to(dev) for key, c in zip(active, counts)])
+            feats = self.eng.fbank_stream_v([self.keys[key] for key in active], counts, pcm, scale)
+            self.stats["fbank_calls"] += 1
+            # gather table: the history rows of every window session (H each), then the window's feature blocks
+            rows = torch.tensor([self.rows[key] for key in active], device=dev)
+            table = torch.cat([self._hist.index_select(0, rows).flatten(0, 1), feats])
+            src: List[int] = []
+            hist_src: List[int] = []
+            labels: List[str] = []
+            enc_keys: List[Hashable] = []
+            enc_counts: List[int] = []
+            first = len(active) * H
+            for i, (key, c) in enumerate(zip(active, counts)):
+                plan = plan_gated_replay(recs[key][1][done[key]:done[key] + c], H, self.onset_chunks)
+                row = [i * H + h for h in range(H)] + list(range(first, first + c))     # table row of history slot / chunk
+                hist_src.extend(row[s.index if s.kind == "history" else H + s.index] for s in plan.history)
+                if plan.blocks:
+                    enc_keys.append(key)
+                    enc_counts.append(len(plan.blocks))
+                    src.extend(row[s.index if s.kind == "history" else H + s.index] for s, _ in plan.blocks)
+                    labels.extend(lab for _, lab in plan.blocks)
+                first += c
+            if H:
+                self._hist.index_copy_(0, rows, table.index_select(0, torch.tensor(hist_src, device=dev)).view(len(active), H,
+                                                                                                              *feats.shape[1:]))
+            if enc_keys:
+                x = table.index_select(0, torch.tensor(src, device=dev))
+                enc, emb = self.eng.encode_stream_steps_v([self.keys[key] for key in enc_keys], enc_counts, x)
+                self.stats["encode_calls"] += 1
+                self.stats["session_steps"] += len(src)
+                owners = [key for key, c in zip(enc_keys, enc_counts) for _ in range(c)]
+                for b, (key, lab) in enumerate(zip(owners, labels)):
+                    out.setdefault(key, []).append(Block(enc[b], emb[b] if emb is not None else None, lab))
+                    if self.block_log is not None:
+                        self.block_log.append((key, x[b], lab))
+            for key, c in zip(active, counts):
+                done[key] += c
 
     def history(self, key: Hashable) -> torch.Tensor:
         return self._hist[self.rows[key]]

@@ -220,6 +220,20 @@ int fo_stream_step(fo_ctx* ctx, const int32_t* ids, int n, const void* pcm, int 
  * stays for the next step).  Ordered after outstanding fo_stream_step_async steps.  One stream step, sum(chunks) session chunks. */
 int fo_stream_steps_v(fo_ctx* ctx, const int32_t* ids, const int32_t* chunks, int n, const void* pcm, int pcm_dtype,
                       float scale, float* enc_out, float* adapter_out, void* stream);
+/* the two halves of fo_stream_steps_v, for callers that choose which blocks reach the encoder (a VAD-gated service replaying
+ * a recorded conversation: StreamScheduler.replay).  fo_fbank_stream_v: session ids[i] takes chunks[i] >= 1 consecutive chunks of
+ * PCM, laid out as in fo_stream_steps_v; feats_out (B, context + frames_per_chunk, feat_dim), B = sum(chunks), same block order,
+ * every block with its context frames; host or device, or NULL.  Features, sample carry and feature ring afterwards are
+ * bit-identical to chunks[i] successive fo_fbank_stream calls.  Needs a frontend only; no session's encoder state moves.
+ * FO_ERR_ARG, with nothing enqueued: a count < 1, a duplicate or unallocated id, a bad pcm_dtype. */
+int fo_fbank_stream_v(fo_ctx* ctx, const int32_t* ids, const int32_t* chunks, int n, const void* pcm, int pcm_dtype, float scale,
+                      float* feats_out, void* stream);
+/* fo_stream_steps_v from features: feats (B, t_in, feat_dim), B = sum(chunks), in (session, chunk) order, every block with its
+ * own context frames (as fo_fbank_stream_v returns them); no cap on the counts, the same passes, results and refusals as
+ * fo_stream_steps_v (an armed hand-off is refused and stays armed).  On the features fo_fbank_stream_v produced it is bit-identical
+ * to fo_stream_steps_v of that PCM.  One stream step, sum(chunks) session chunks. */
+int fo_encode_stream_steps_v(fo_ctx* ctx, const int32_t* ids, const int32_t* chunks, int n, const float* feats, int t_in,
+                             float* enc_out, float* adapter_out, void* stream);
 /* pipelined form for HOST buffers (a server loop that already holds the next chunk; the reference runs this loop one chunk
  * and one session at a time, bin/dialog_state_pred.py:793-814 -> models/audioLLM.py:380-387): returns once the step is enqueued.
  * The PCM upload and the read-back of enc_out / adapter_out run on two internal copy streams with double-buffered staging,
@@ -307,10 +321,11 @@ int fo_stats(fo_ctx* ctx, fo_stats_t* out);
  *       transformer layers in ONE cooperative launch (csrc/fo_stack.cu; bf16 contexts, pre-norm linear-FFN layers) instead of
  *       the per-kernel chain; the first such step builds the kernel's row-padded copy of the layer matrices (+ 2 x 12 D^2 bytes
  *       per layer, 604 MB for the shipped model).  0 = always the chain.
- *   "steps_pass_blocks" 0: blocks (session chunks) per pass of fo_stream_steps_v; 0 = as many as 1 GiB of workspace holds
- *       (720 blocks of the shipped model in bf16)
+ *   "steps_pass_blocks" 0: blocks (session chunks) per pass of fo_stream_steps_v, fo_fbank_stream_v and
+ *       fo_encode_stream_steps_v; 0 = as many as 1 GiB of workspace holds (720 blocks of the shipped model in bf16)
  *   "profile_gemm" 0/1, "debug_skip" (timing attribution), "tc_swap"/"tc_bn"/"tc_split" (-1 = cost model): development
- * get-only: "tc_launches", "tc_persist_launches", "stack_launches", "ring_cap", "max_t", "profile_gemm_us", "profile_gemm_count".
+ * get-only: "tc_launches", "tc_persist_launches", "stack_launches", "ring_cap", "max_t", "profile_gemm_us", "profile_gemm_count",
+ *   "steps_pass_blocks_in_use" (the blocks per pass "steps_pass_blocks" gives at the context's chunking).
  * Development environment variables read once per process: FO_TC_OCC, FO_TC_KB, FO_TC_KBD, FO_TC_SMAX, FO_TC_CAP, FO_TC_SKINNY (tile
  * plan of the skinny GEMMs), FO_PDL_MIN, FO_PERSIST_DBG, FO_TC_TRACE. */
 int fo_set_option(fo_ctx* ctx, const char* name, int64_t value);
