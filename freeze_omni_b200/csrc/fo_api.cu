@@ -175,6 +175,11 @@ struct fo_ctx {
         int32_t* row_start = nullptr;
     } armed;
     uint8_t* onset_dev = nullptr;
+    // an armed recording call: {caller block, onset flag} of every pass block, pass after pass (pinned, uploaded one pass at a
+    // time into WS_HOTAB); reused once ho_tab_event (the previous armed call's last upload) has completed
+    int2* ho_tab_host = nullptr;
+    long long ho_tab_cap = 0;
+    cudaEvent_t ho_tab_event = nullptr;
     int groups = 1;                           // session groups whose layer kernels run on parallel streams
     cudaStream_t grp_stream[MAX_GROUPS] = {nullptr};
     cudaEvent_t ev_fork = nullptr, ev_join[MAX_GROUPS] = {nullptr};
@@ -220,7 +225,7 @@ namespace {
 
 enum { WS_FEATS = 0, WS_C1, WS_C2, WS_XSUB, WS_EMB, WS_X, WS_H, WS_QKV, WS_ATT, WS_FFH, WS_ENC, WS_XIN, WS_ACONV, WS_AH,
        WS_Y, WS_MASK2, WS_ILENS, WS_ILENS2, WS_AMASK, WS_PCM, WS_TMP0, WS_TMP1, WS_TMP2, WS_TMP3, WS_Q32, WS_HC, WS_PART, WS_PCM2, WS_ENC2, WS_Y2, WS_AC1, WS_XIN2, WS_TMP4, WS_TMP5, WS_HP, WS_FP, WS_PACK, WS_SROWS,
-       WS_PKTAB, WS_FGRID, WS_XP, WS_FBTAB, WS_COUNT };
+       WS_PKTAB, WS_FGRID, WS_XP, WS_FBTAB, WS_HOTAB, WS_COUNT };
 static_assert(WS_COUNT <= (int)(sizeof(fo_ctx::ws) / sizeof(DevBuf)), "fo_ctx::ws holds every named workspace");
 
 int dev_alloc(fo_ctx* c, void** p, size_t bytes) {
@@ -1696,6 +1701,8 @@ int fo_destroy(fo_ctx* c) {
     if (c->snap_ids_event) cudaEventDestroy(c->snap_ids_event);
     if (c->snap_ids_host) cudaFreeHost(c->snap_ids_host);
     if (c->snap_hdr_host) cudaFreeHost(c->snap_hdr_host);
+    if (c->ho_tab_event) cudaEventDestroy(c->ho_tab_event);
+    if (c->ho_tab_host) cudaFreeHost(c->ho_tab_host);
     for (void* p : c->owned) if (p) cudaFree(p);
     for (int k = 0; k < fo_ctx::NSTAGE; ++k) {
         if (c->ids_host[k]) cudaFreeHost(c->ids_host[k]);
@@ -2470,8 +2477,9 @@ int fo_handoff_arm(fo_ctx* c, int n, void* embeds_f16, int64_t rows_per_session,
                    const uint8_t* prefix_mask, uint8_t* attn_mask, int32_t* row_start) {
     FO_CHECK(c && c->finalized && c->cfg.has_encoder && c->cfg.has_adapter, "fo_handoff_arm: context needs a finalized encoder + adapter");
     FO_CHECK(c->dtype == FO_BF16, "fo_handoff_arm: the fp16 hand-off is built for bf16 contexts");
-    // n blocks: one per session, or per (session, chunk) for fo_encode_stream_chunks
-    FO_CHECK(n > 0 && n <= c->cfg.max_sessions * STREAM_CHUNKS_MAX_KEYS && embeds_f16 && onset, "fo_handoff_arm: bad argument");
+    // n blocks: one per session, or per (session, chunk) of a multi-chunk or recording call -- the latter has no cap on the
+    // counts, so neither has n; a call of another block count refuses the arm
+    FO_CHECK(n > 0 && embeds_f16 && onset, "fo_handoff_arm: bad argument");
     FO_CHECK(prefix_len >= 0 && rows_per_session > prefix_len && rows_per_session < (1LL << 31), "fo_handoff_arm: bad row counts");
     cudaPointerAttributes pa;
     FO_CHECK(cudaPointerGetAttributes(&pa, embeds_f16) == cudaSuccess && pa.type == cudaMemoryTypeDevice && pa.device == c->device,
@@ -2632,6 +2640,7 @@ struct StepsIo {
     bool encode = false;
     float* enc_out = nullptr;
     float* adapter_out = nullptr;
+    const fo_ctx::Armed* armed = nullptr;   // the hand-off this call took (fo_handoff_arm), in place of adapter_out
 };
 
 // The pass loop shared by the recording entries; arguments are checked by the caller, so nothing here refuses a call.
@@ -2646,7 +2655,21 @@ static int steps_passes(fo_ctx* c, const int32_t* ids, const int32_t* chunks, in
     const int P = steps_pass_blocks(c, t_in);
     const long long pcm_row = (long long)c->chunk_samples * (io.pcm_dtype == FO_I16 ? 2 : 4);
     const long long feat_row = (long long)t_in * c->F, enc_row = (long long)t * c->D, y_row = (long long)t_out * c->E;
-    const bool want_y = io.adapter_out != nullptr;
+    const fo_ctx::Armed* ho = io.armed;
+    const bool want_y = io.adapter_out != nullptr || ho;
+    long long tab_pos = 0;
+    if (ho) {
+        // the pass tables of the whole call, in pinned memory: wait until the previous armed call has uploaded its own
+        if (c->ho_tab_event) FO_CUDA(cudaEventSynchronize(c->ho_tab_event));
+        else FO_CUDA(cudaEventCreateWithFlags(&c->ho_tab_event, cudaEventDisableTiming));
+        if (c->ho_tab_cap < off[n]) {
+            if (c->ho_tab_host) FO_CUDA(cudaFreeHost(c->ho_tab_host));
+            c->ho_tab_host = nullptr;
+            c->ho_tab_cap = 0;
+            FO_CUDA(cudaMallocHost((void**)&c->ho_tab_host, (size_t)off[n] * sizeof(int2)));
+            c->ho_tab_cap = off[n];
+        }
+    }
     int sms = 148;
     FO_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->device));
     const int gmax = std::max(1, (STREAM_CHUNKS_MAX_KEYS - c->window) / std::max(1, t));
@@ -2717,12 +2740,30 @@ static int steps_passes(fo_ctx* c, const int32_t* ids, const int32_t* chunks, in
                 const long long b0 = off[i] + done[i];
                 if (io.enc_out) FO_CUDA(cudaMemcpyAsync(io.enc_out + b0 * enc_row, (float*)denc + poff[a] * enc_row,
                                                         pcnt[a] * enc_row * sizeof(float), cudaMemcpyDefault, st));
-                if (want_y) FO_CUDA(cudaMemcpyAsync(io.adapter_out + b0 * y_row, (float*)dy + poff[a] * y_row,
-                                                    pcnt[a] * y_row * sizeof(float), cudaMemcpyDefault, st));
+                if (io.adapter_out) FO_CUDA(cudaMemcpyAsync(io.adapter_out + b0 * y_row, (float*)dy + poff[a] * y_row,
+                                                            pcnt[a] * y_row * sizeof(float), cudaMemcpyDefault, st));
+            }
+            if (ho) {
+                // pass block poff[a] + j is chunk done_i + j of session i, the caller's block off_i + done_i + j
+                int2* tab = c->ho_tab_host + tab_pos;
+                for (int a = 0; a < na; ++a) {
+                    const int i = psrc[a];
+                    for (int j = 0; j < pcnt[a]; ++j) {
+                        const long long d = off[i] + done[i] + j;
+                        tab[poff[a] + j] = make_int2((int)d, ho->onset[d]);
+                    }
+                }
+                void* dtab;
+                FO_TRY(ws_ensure(c, WS_HOTAB, (size_t)m.blocks * sizeof(int2), &dtab));
+                FO_CUDA(cudaMemcpyAsync(dtab, tab, (size_t)m.blocks * sizeof(int2), cudaMemcpyHostToDevice, st));
+                FO_TRY(handoff_rows((const float*)dy, (const int2*)dtab, m.blocks, t_out, c->E, ho->embeds, (int)ho->rows, (int)ho->prefix,
+                                    ho->prefix_mask, ho->attn_mask, ho->row_start, c->sat_counter, st));
+                tab_pos += m.blocks;
             }
         }
         for (int a = 0; a < na; ++a) done[psrc[a]] += pcnt[a];
     }
+    if (ho) FO_CUDA(cudaEventRecord(c->ho_tab_event, st));
     if (!c->ev_sync) FO_CUDA(cudaEventCreateWithFlags(&c->ev_sync, cudaEventDisableTiming));
     FO_CUDA(cudaEventRecord(c->ev_sync, st));
     if (io.encode) {
@@ -2732,17 +2773,35 @@ static int steps_passes(fo_ctx* c, const int32_t* ids, const int32_t* chunks, in
     return 0;
 }
 
-// the refusals of the encoding recording entries (fo_stream_steps_v, fo_encode_stream_steps_v)
+// the refusals of the encoding recording entries (fo_stream_steps_v, fo_encode_stream_steps_v).  Unlike stream_common, a refused
+// call leaves an armed hand-off armed: nothing here consumes it.
 static int check_steps_encode(fo_ctx* c, const char* fn, const int32_t* ids, const int32_t* chunks, int n, int t_in,
                               const float* adapter_out) {
     FO_CHECK(chunks, "%s: chunks must be a host array of n counts", fn);
-    FO_CHECK(!c->armed.on, "%s: an LLM hand-off is armed (fo_handoff_arm); this call does not take it, and it stays "
-                           "armed for the next fo_stream_step / fo_encode_stream call", fn);
     FO_TRY(check_ids(c, ids, n));
     FO_TRY(stream_geometry(c, t_in));
     FO_CHECK(!c->KM, "%s: MultiLayeredConv1d has no streaming form (models/encoder/attention.py:145-196); use fo_encode_offline", fn);
     if (adapter_out) FO_CHECK(c->cfg.has_adapter, "adapter_out requested but the context has no adapter");
-    return check_steps_counts(fn, ids, chunks, n);
+    FO_TRY(check_steps_counts(fn, ids, chunks, n));
+    if (c->armed.on) {
+        long long blocks = 0;
+        for (int i = 0; i < n; ++i) blocks += chunks[i];
+        const int t_out = ad_frames(c, ((t_in - 1) / 2 - 1) / 2);
+        FO_CHECK(c->armed.n == blocks, "%s: the LLM hand-off is armed for %d blocks (fo_handoff_arm), this call brings %lld; "
+                                       "it stays armed", fn, c->armed.n, blocks);
+        FO_CHECK(!adapter_out, "%s: an armed LLM hand-off replaces adapter_out: pass NULL (the hand-off stays armed)", fn);
+        FO_CHECK(c->armed.rows >= c->armed.prefix + t_out, "%s: the armed hand-off's %lld rows per block do not hold %d adapter rows "
+                 "behind a %lld-row prefix; it stays armed", fn, c->armed.rows, t_out, c->armed.prefix);
+    }
+    return 0;
+}
+
+// after check_steps_encode: the call takes the armed hand-off, if any, into `armed` (io.armed points at it)
+static void take_arm(fo_ctx* c, fo_ctx::Armed* armed, StepsIo* io) {
+    if (!c->armed.on) return;
+    *armed = c->armed;
+    c->armed.on = false;
+    io->armed = armed;
 }
 
 int fo_stream_steps_v(fo_ctx* c, const int32_t* ids, const int32_t* chunks, int n, const void* pcm, int pcm_dtype, float scale,
@@ -2759,6 +2818,8 @@ int fo_stream_steps_v(fo_ctx* c, const int32_t* ids, const int32_t* chunks, int 
     io.encode = true;
     io.enc_out = enc_out;
     io.adapter_out = adapter_out;
+    fo_ctx::Armed armed;
+    take_arm(c, &armed, &io);
     return steps_passes(c, ids, chunks, n, t_in, io, (cudaStream_t)stream);
 }
 
@@ -2774,6 +2835,8 @@ int fo_encode_stream_steps_v(fo_ctx* c, const int32_t* ids, const int32_t* chunk
     io.encode = true;
     io.enc_out = enc_out;
     io.adapter_out = adapter_out;
+    fo_ctx::Armed armed;
+    take_arm(c, &armed, &io);
     return steps_passes(c, ids, chunks, n, t_in, io, (cudaStream_t)stream);
 }
 

@@ -399,6 +399,10 @@ int subsample_mask(const int32_t* ilens, int B, int T, int T2, uint8_t* mask2, i
 // attention-mask rows + input start rows of the LLM hand-off (audioLLM.py:404-411); device pointers
 int handoff_mask(const uint8_t* onset, const uint8_t* prefix_mask, int n, int P, int t_out, int rows, uint8_t* attn_mask,
                  int32_t* row_start, cudaStream_t st);
+// the hand-off of one pass of the recording entries: pass block b's fp32 adapter rows (y) as fp16 into caller block tab[b].x,
+// its mask row and row_start from onset flag tab[b].y (tab: device, nblk entries)
+int handoff_rows(const float* y, const int2* tab, int nblk, int t_out, int E, void* embeds_f16, int rows, int P,
+                 const uint8_t* prefix_mask, uint8_t* attn_mask, int32_t* row_start, unsigned long long* sat, cudaStream_t st);
 int stride2_mask(const uint8_t* mask, int B, int T, int To, uint8_t* out, cudaStream_t st);
 
 // ---- attention -----------------------------------------------------------------------------------

@@ -733,23 +733,65 @@ template int depthwise_conv<__half>(const __half*, int, int, int, int, const flo
 
 // LLM hand-off bookkeeping (models/audioLLM.py:404-411): per session the attention-mask row over its block of the inputs_embeds
 // buffer, [prefix_mask | 1 x t_out | 0 ...] when the block opens an IPU (status 'ipu_sl': the chat prefix is part of the input) and
-// [0 x P | 1 x t_out | 0 ...] otherwise, plus the row where the session's input starts (0 / P).
-__global__ void handoff_mask_kernel(const uint8_t* __restrict__ onset, const uint8_t* __restrict__ prefix_mask, int P, int t_out,
-                                    int rows, uint8_t* __restrict__ attn_mask, int32_t* __restrict__ row_start) {
-    const int b = blockIdx.x;
-    const bool on = onset[b] != 0;
+// [0 x P | 1 x t_out | 0 ...] otherwise, plus the row where the session's input starts (0 / P).  One CTA writes block b's row.
+__device__ __forceinline__ void handoff_mask_row(bool on, const uint8_t* __restrict__ prefix_mask, int P, int t_out, int rows,
+                                                 long long b, uint8_t* __restrict__ attn_mask, int32_t* __restrict__ row_start) {
     for (int r = threadIdx.x; r < rows; r += blockDim.x) {
         uint8_t v;
         if (r < P) v = on ? (prefix_mask ? (prefix_mask[r] != 0) : 1) : 0;
         else v = r < P + t_out ? 1 : 0;
-        attn_mask[(long long)b * rows + r] = v;
+        attn_mask[b * rows + r] = v;
     }
     if (threadIdx.x == 0 && row_start) row_start[b] = on ? 0 : P;
+}
+__global__ void handoff_mask_kernel(const uint8_t* __restrict__ onset, const uint8_t* __restrict__ prefix_mask, int P, int t_out,
+                                    int rows, uint8_t* __restrict__ attn_mask, int32_t* __restrict__ row_start) {
+    handoff_mask_row(onset[blockIdx.x] != 0, prefix_mask, P, t_out, rows, blockIdx.x, attn_mask, row_start);
+}
+
+// The hand-off of a pass of the recording entries: CTA b takes pass block b's t_out fp32 adapter rows (y, contiguous per block) to
+// the caller's block tab[b].x -- rows [P, P + t_out) of embeds, as fp16 with the clamp and saturation count of the projection
+// epilogue's hand-off write -- and writes that block's mask row and row_start from its onset flag tab[b].y.
+__global__ void __launch_bounds__(256) handoff_rows_kernel(const float* __restrict__ y, const int2* __restrict__ tab, int t_out, int E,
+                                                           __half* __restrict__ embeds, int rows, int P,
+                                                           const uint8_t* __restrict__ prefix_mask, uint8_t* __restrict__ attn_mask,
+                                                           int32_t* __restrict__ row_start, unsigned long long* sat) {
+    const int2 e = tab[blockIdx.x];
+    const long long n = (long long)t_out * E;
+    const float* src = y + blockIdx.x * n;
+    __half* dst = embeds + ((long long)e.x * rows + P) * E;
+    if (n % 8 == 0 && (reinterpret_cast<uintptr_t>(dst) & 15) == 0) {
+        // 8 values per step: two 16-byte loads, one 16-byte store (src is 32-byte aligned: blocks of t_out * E floats, E % 8 == 0)
+        const float4* s4 = reinterpret_cast<const float4*>(src);
+        uint4* d4 = reinterpret_cast<uint4*>(dst);
+        for (long long i = threadIdx.x; i < n / 8; i += blockDim.x) {
+            const float4 a = s4[2 * i], b = s4[2 * i + 1];
+            count_sat4(sat, a.x, a.y, a.z, a.w);
+            count_sat4(sat, b.x, b.y, b.z, b.w);
+            d4[i] = make_uint4(pack2<__half>(a.x, a.y), pack2<__half>(a.z, a.w), pack2<__half>(b.x, b.y), pack2<__half>(b.z, b.w));
+        }
+    } else {
+        for (long long i = threadIdx.x; i < n; i += blockDim.x) {
+            const float v = src[i];
+            count_sat4(sat, v, 0.f, 0.f, 0.f);
+            dst[i] = from_f<__half>(v);
+        }
+    }
+    if (attn_mask) handoff_mask_row(e.y != 0, prefix_mask, P, t_out, rows, e.x, attn_mask, row_start);
 }
 int handoff_mask(const uint8_t* onset, const uint8_t* prefix_mask, int n, int P, int t_out, int rows, uint8_t* attn_mask,
                  int32_t* row_start, cudaStream_t st) {
     if (n <= 0) return 0;
     handoff_mask_kernel<<<n, 128, 0, st>>>(onset, prefix_mask, P, t_out, rows, attn_mask, row_start);
+    FO_LAUNCHED();
+    FO_CUDA(cudaGetLastError());
+    return 0;
+}
+int handoff_rows(const float* y, const int2* tab, int nblk, int t_out, int E, void* embeds_f16, int rows, int P,
+                 const uint8_t* prefix_mask, uint8_t* attn_mask, int32_t* row_start, unsigned long long* sat, cudaStream_t st) {
+    if (nblk <= 0) return 0;
+    handoff_rows_kernel<<<nblk, 256, 0, st>>>(y, tab, t_out, E, reinterpret_cast<__half*>(embeds_f16), rows, P, prefix_mask, attn_mask,
+                                              row_start, sat);
     FO_LAUNCHED();
     FO_CUDA(cudaGetLastError());
     return 0;

@@ -502,9 +502,12 @@ class Engine:
 
     def handoff_arm(self, n: int, embeds: torch.Tensor, prefix_len: int, onset, prefix_mask: Optional[torch.Tensor] = None,
                     attn_mask: Optional[torch.Tensor] = None, row_start: Optional[torch.Tensor] = None) -> None:
-        """Arm the NEXT encode_stream / stream_step call of n sessions (want_adapter=False) with the LLM hand-off of
-        models/audioLLM.py:383-411: adapter rows as fp16 behind the chat prefix of each session's block of `embeds`
-        (>= n, rows, llm_dim), attention-mask rows and input start rows on the device.  `onset`: n flags, status == 'ipu_sl'."""
+        """Arm the NEXT streaming call of n blocks (want_adapter=False) with the LLM hand-off of models/audioLLM.py:383-411:
+        adapter rows as fp16 behind the chat prefix of each block of `embeds` (>= n, rows, llm_dim), attention-mask rows and
+        input start rows on the device.  `onset`: n flags, status == 'ipu_sl'.  The call is encode_stream / stream_step (a block
+        per session), encode_stream_chunks[_v], or one of the recording entries stream_steps_v / encode_stream_steps_v (block
+        b is the b-th block of the call's (session, chunk) order, for any number of blocks).  encode_stream & co. consume the arm
+        whatever their outcome; a recording entry that refuses the call (another block count, adapter_out given) leaves it armed."""
         assert embeds.is_cuda and embeds.dtype == torch.float16 and embeds.is_contiguous() and embeds.dim() == 3
         assert embeds.shape[0] >= n and embeds.shape[2] == self.cfg.llm_dim
         on = np.ascontiguousarray(np.asarray(onset, dtype=np.uint8).reshape(-1))

@@ -24,7 +24,8 @@ State (KV rings, adapter cache, sample carry, feature ring, history ring, queued
 session is moved: `detach` / `attach` carry it, history rows included, to another scheduler on any GPU.
 A recorded, VAD-annotated conversation goes through `replay` in one call: `plan_gated_replay` applies the same rule on the host,
 and windows of recorded chunks run as one fbank call (Engine.fbank_stream_v) and one encoder call (Engine.encode_stream_steps_v)
-each, with the blocks and history rows gathered on the device; the sessions end as one tick per chunk would leave them.
+each, with the blocks and history rows gathered on the device; the sessions end as one tick per chunk would leave them.  With a
+Handoff, the encoder call of each window writes the blocks' LLM inputs (fp16 rows, mask rows, start rows) as a tick's does.
 """
 from collections import deque
 from typing import Any, Deque, Dict, Hashable, List, NamedTuple, Optional, Tuple
@@ -47,9 +48,10 @@ class Block(NamedTuple):
 
 
 class Handoff:
-    """Pre-allocated LLM-side buffers for `StreamScheduler.tick(handoff=...)` (models/audioLLM.py:383-411): `embeds`
-    (capacity, prefix_len + t_out, E) fp16 whose first prefix_len rows of every block hold the chat-prefix embeddings,
-    `attn_mask` (capacity, prefix_len + t_out) uint8 and `row_start` (capacity) int32.  One block per encoder step of a tick."""
+    """Pre-allocated LLM-side buffers for `StreamScheduler.tick(handoff=...)` and `StreamScheduler.replay(..., handoff=...)`
+    (models/audioLLM.py:383-411): `embeds` (capacity, prefix_len + t_out, E) fp16 whose first prefix_len rows of every block hold
+    the chat-prefix embeddings, `attn_mask` (capacity, prefix_len + t_out) uint8 and `row_start` (capacity) int32.  One block per
+    encoder step of a tick or a replay."""
 
     def __init__(self, engine, capacity: int, prefix_embeds: torch.Tensor, prefix_mask: Optional[torch.Tensor] = None):
         dev = engine.torch_device
@@ -109,6 +111,13 @@ def plan_gated_replay(statuses, history_chunks: int, onset_chunks: int) -> Gated
         replayed = ring[history_chunks - onset_chunks:] if status == IPU_START and onset_chunks > 0 else []
         blocks.extend(zip(replayed + [cur], onset_statuses(len(replayed), status)))
     return GatedPlan(blocks, ring)
+
+
+def gated_block_count(statuses, onset_chunks: int) -> int:
+    """len(plan_gated_replay(statuses, history_chunks, onset_chunks).blocks) without building the plan: every non-silent chunk is
+    one block, and an 'ipu_sl' chunk brings `onset_chunks` history slots in front of it (the ring always holds history_chunks)."""
+    statuses = list(statuses)
+    return sum(st is not None for st in statuses) + onset_chunks * statuses.count(IPU_START)
 
 
 def plan_rounds(queue_lens: Dict[Hashable, int], max_batch: int) -> List[List[Hashable]]:
@@ -440,7 +449,8 @@ class StreamScheduler:
             return enc.unsqueeze(1), (emb.unsqueeze(1) if emb is not None else None)
         return self.eng.encode_stream_chunks(ids, x, **kw)
 
-    def replay(self, recordings: Dict[Hashable, Tuple[Any, Any]], scale: Optional[float] = None) -> Dict[Hashable, List[Block]]:
+    def replay(self, recordings: Dict[Hashable, Tuple[Any, Any]], scale: Optional[float] = None,
+               handoff: Optional[Handoff] = None) -> Dict[Hashable, List[Block]]:
         """Recorded, VAD-annotated audio of open sessions in one call, with the blocks, labels and session state that pushing
         it one chunk per tick would give (plan_gated_replay).  `recordings` maps a key to (pcm (c, samples_per_chunk) int16 or
         float32, host or device, statuses (c,) of None or str); every recording has the same PCM dtype.  Returns, per session
@@ -448,7 +458,12 @@ class StreamScheduler:
         windows of at most max(P, sessions) chunks, P the engine's "steps_pass_blocks_in_use": per window one fbank_stream_v
         over every session, the encoder blocks and the new history rows gathered on the device from the window's features and
         the history rows, and one encode_stream_steps_v over the sessions with a block in the window.  A session with a
-        pushed chunk or queued blocks is refused before anything runs: tick first.  The LLM hand-off is not offered here."""
+        pushed chunk or queued blocks is refused before anything runs: tick first.
+        With a Handoff (bf16 engines), every block's LLM input is written as tick(handoff=) writes it: Block.emb and Block.mask
+        are views of `handoff.embeds` / `handoff.attn_mask` (chat prefix included for 'ipu_sl' blocks), the fp16 rows being
+        .half() of the adapter rows the replay returns without one.  Hand-off block b is the replay's b-th block: window by
+        window, and within a window session by session in stream order.  A replay with more blocks than the Handoff holds
+        is refused before anything runs."""
         recs: Dict[Hashable, Tuple[torch.Tensor, List[Optional[str]]]] = {}
         for key, (pcm, statuses) in recordings.items():
             if key not in self.keys:
@@ -469,6 +484,12 @@ class StreamScheduler:
             raise TypeError("the recordings of one replay must share one PCM dtype")
         out: Dict[Hashable, List[Block]] = {}
         dev, H = self.eng.torch_device, self.history_chunks
+        if handoff is not None:
+            # the windows split no block count: a chunk gives its blocks (onset history included) in whichever window it falls
+            total = sum(gated_block_count(st, self.onset_chunks) for _, st in recs.values())
+            if total > handoff.embeds.shape[0]:
+                raise RuntimeError("the replay gives %d blocks, more than the Handoff capacity %d" % (total, handoff.embeds.shape[0]))
+        cursor = 0
         P = self.eng.get_option("steps_pass_blocks_in_use")
         done = {key: 0 for key in recs}
         while True:
@@ -504,14 +525,33 @@ class StreamScheduler:
                                                                                                               *feats.shape[1:]))
             if enc_keys:
                 x = table.index_select(0, torch.tensor(src, device=dev))
-                enc, emb = self.eng.encode_stream_steps_v([self.keys[key] for key in enc_keys], enc_counts, x)
+                ids = [self.keys[key] for key in enc_keys]
+                if handoff is not None:
+                    # the window's blocks land in the next free blocks of the caller's buffers, as in tick's drains
+                    self.eng.handoff_arm(len(src), handoff.embeds[cursor:], handoff.prefix_len, [lab == IPU_START for lab in labels],
+                                         handoff.prefix_mask, handoff.attn_mask[cursor:], handoff.row_start[cursor:])
+                    enc, emb = self.eng.encode_stream_steps_v(ids, enc_counts, x, want_adapter=False)
+                else:
+                    enc, emb = self.eng.encode_stream_steps_v(ids, enc_counts, x)
                 self.stats["encode_calls"] += 1
                 self.stats["session_steps"] += len(src)
                 owners = [key for key, c in zip(enc_keys, enc_counts) for _ in range(c)]
+                if handoff is not None:
+                    # the views tick(handoff=) returns, cut in four calls rather than two per block: [st0:] of every
+                    # block, st0 = 0 for 'ipu_sl' (chat prefix included) and prefix_len otherwise
+                    win = slice(cursor, cursor + len(src))
+                    views = {st0: (handoff.embeds[win, st0:].unbind(0), handoff.attn_mask[win, st0:].unbind(0))
+                             for st0 in (0, handoff.prefix_len)}
                 for b, (key, lab) in enumerate(zip(owners, labels)):
-                    out.setdefault(key, []).append(Block(enc[b], emb[b] if emb is not None else None, lab))
+                    if handoff is not None:
+                        e, m = views[0 if lab == IPU_START else handoff.prefix_len]
+                        blk = Block(enc[b], e[b], lab, m[b])
+                    else:
+                        blk = Block(enc[b], emb[b] if emb is not None else None, lab)
+                    out.setdefault(key, []).append(blk)
                     if self.block_log is not None:
                         self.block_log.append((key, x[b], lab))
+                cursor += len(src)
             for key, c in zip(active, counts):
                 done[key] += c
 

@@ -215,23 +215,29 @@ int fo_stream_step(fo_ctx* ctx, const int32_t* ids, int n, const void* pcm, int 
  * (session, chunk) order as in fo_encode_stream_chunks_v; FO_F32 or FO_I16, value used = sample * scale.  enc_out (B, t, d_model),
  * adapter_out (B, t_out, llm_dim), same block order; either may be NULL.  No cap on the counts: the call runs in passes of a
  * bounded number of blocks (option "steps_pass_blocks"), so the device memory it adds does not grow with the recording.
+ * An armed hand-off (fo_handoff_arm) applies when armed for B blocks: block off_i + j is chunk j of session i, as in
+ * fo_encode_stream_chunks_v, and gets its onset flag, its fp16 rows [prefix_len, prefix_len + t_out) -- bit for bit the fp32
+ * adapter rows the call returns without the arm, rounded to fp16 (clamped to +-65504 and counted in act_saturations) --, its
+ * mask row and its row_start; adapter_out must then be NULL, enc_out still works.
  * FO_ERR_ARG, with nothing enqueued and no session touched: the geometry rules of every streaming entry, a count < 1, a
- * duplicate or unallocated id, a MultiLayeredConv1d context, and a call while a hand-off is armed (fo_handoff_arm; the arm
- * stays for the next step).  Ordered after outstanding fo_stream_step_async steps.  One stream step, sum(chunks) session chunks. */
+ * duplicate or unallocated id, a MultiLayeredConv1d context, and, while a hand-off is armed, an arm for another block count,
+ * adapter_out given or too few rows per block.  Every refusal leaves an armed hand-off armed for the next call.
+ * Ordered after outstanding fo_stream_step_async steps.  One stream step, sum(chunks) session chunks. */
 int fo_stream_steps_v(fo_ctx* ctx, const int32_t* ids, const int32_t* chunks, int n, const void* pcm, int pcm_dtype,
                       float scale, float* enc_out, float* adapter_out, void* stream);
 /* the two halves of fo_stream_steps_v, for callers that choose which blocks reach the encoder (a VAD-gated service replaying
  * a recorded conversation: StreamScheduler.replay).  fo_fbank_stream_v: session ids[i] takes chunks[i] >= 1 consecutive chunks of
  * PCM, laid out as in fo_stream_steps_v; feats_out (B, context + frames_per_chunk, feat_dim), B = sum(chunks), same block order,
  * every block with its context frames; host or device, or NULL.  Features, sample carry and feature ring afterwards are
- * bit-identical to chunks[i] successive fo_fbank_stream calls.  Needs a frontend only; no session's encoder state moves.
+ * bit-identical to chunks[i] successive fo_fbank_stream calls.  Needs a frontend only; no session's encoder state moves.  It runs
+ * no adapter, so an armed hand-off is neither applied nor consumed.
  * FO_ERR_ARG, with nothing enqueued: a count < 1, a duplicate or unallocated id, a bad pcm_dtype. */
 int fo_fbank_stream_v(fo_ctx* ctx, const int32_t* ids, const int32_t* chunks, int n, const void* pcm, int pcm_dtype, float scale,
                       float* feats_out, void* stream);
 /* fo_stream_steps_v from features: feats (B, t_in, feat_dim), B = sum(chunks), in (session, chunk) order, every block with its
- * own context frames (as fo_fbank_stream_v returns them); no cap on the counts, the same passes, results and refusals as
- * fo_stream_steps_v (an armed hand-off is refused and stays armed).  On the features fo_fbank_stream_v produced it is bit-identical
- * to fo_stream_steps_v of that PCM.  One stream step, sum(chunks) session chunks. */
+ * own context frames (as fo_fbank_stream_v returns them); no cap on the counts, the same passes, results, armed hand-off and
+ * refusals as fo_stream_steps_v.  On the features fo_fbank_stream_v produced it is bit-identical to fo_stream_steps_v of that
+ * PCM.  One stream step, sum(chunks) session chunks. */
 int fo_encode_stream_steps_v(fo_ctx* ctx, const int32_t* ids, const int32_t* chunks, int n, const float* feats, int t_in,
                              float* enc_out, float* adapter_out, void* stream);
 /* pipelined form for HOST buffers (a server loop that already holds the next chunk; the reference runs this loop one chunk
@@ -253,13 +259,17 @@ int fo_stream_step_embeds(fo_ctx* ctx, const int32_t* ids, int n, const void* pc
 /* The hand-off with the status-dependent chat prefix and the attention mask, i.e. all of
  *   if status == 'ipu_sl': inputs_embeds = cat(chat_prefix_embeds, inputs_embeds); attention_mask = cat(chat_prefix_mask, attention_mask)
  *   inputs_embeds.half()                                                                          (models/audioLLM.py:383-411)
- * Arms the NEXT fo_encode_stream / fo_stream_step call of n sessions (its adapter_out must be NULL): the t_out adapter rows of
- * session i are written as fp16 to rows [prefix_len, prefix_len + t_out) of its block of embeds_f16 (n, rows_per_session, llm_dim),
- * whose rows [0, prefix_len) the caller filled once with the chat-prefix embeddings.  onset (HOST, n bytes): 1 where the
+ * Arms the NEXT streaming call of n blocks (its adapter_out must be NULL): fo_encode_stream / fo_stream_step (one block per
+ * session), fo_encode_stream_chunks[_v], or the recording entries fo_stream_steps_v / fo_encode_stream_steps_v (any n: a block
+ * per session chunk, however long the recording).  The t_out adapter rows of block i are written as fp16 to rows
+ * [prefix_len, prefix_len + t_out) of block i of embeds_f16 (n, rows_per_session, llm_dim), whose rows [0, prefix_len) the caller
+ * filled once with the chat-prefix embeddings.  onset (HOST, n bytes): 1 where the
  * block's status is 'ipu_sl'.  attn_mask (DEVICE, n x rows_per_session bytes) row i becomes [prefix_mask | 1 x t_out | 0 ..] for an
  * onset block and [0 x prefix_len | 1 x t_out | 0 ..] otherwise (prefix_mask: DEVICE, prefix_len bytes, NULL = all ones);
- * row_start (DEVICE, n) = 0 / prefix_len.  The LLM input of session i is rows [row_start[i], prefix_len + t_out) of its block,
- * with the same slice of attn_mask (the caller prepends the past-KV mask, audioLLM.py:418-420).  bf16 contexts only. */
+ * row_start (DEVICE, n) = 0 / prefix_len.  The LLM input of block i is rows [row_start[i], prefix_len + t_out) of its block,
+ * with the same slice of attn_mask (the caller prepends the past-KV mask, audioLLM.py:418-420).  bf16 contexts only.
+ * fo_encode_stream & co. consume the arm whatever their outcome; the recording entries refuse a call whose block count differs,
+ * or that passes adapter_out, and leave the arm in place (fo_fbank_stream_v ignores it). */
 int fo_handoff_arm(fo_ctx* ctx, int n, void* embeds_f16, int64_t rows_per_session, int64_t prefix_len, const uint8_t* onset,
                    const uint8_t* prefix_mask, uint8_t* attn_mask, int32_t* row_start);
 
