@@ -35,6 +35,7 @@ SYMBOLS = {
     "fo_abi_version": (C.c_int, []),
     "fo_last_error": (C.c_char_p, []),
     "fo_create": (C.c_int, [C.POINTER(FoConfig), C.c_int, C.c_int, C.POINTER(_P)]),
+    "fo_create_on_sms": (C.c_int, [C.POINTER(FoConfig), C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(_P)]),
     "fo_destroy": (C.c_int, [_P]),
     "fo_load_tensor": (C.c_int, [_P, C.c_char_p, _P, _I64P, C.c_int]),
     "fo_finalize_weights": (C.c_int, [_P]),
@@ -65,6 +66,7 @@ SYMBOLS = {
     "fo_fbank_stream_v": (C.c_int, [_P, _I32P, _I32P, C.c_int, _P, C.c_int, C.c_float, _P, _P]),
     "fo_encode_stream_steps_v": (C.c_int, [_P, _I32P, _I32P, C.c_int, _P, C.c_int, _P, _P, _P]),
     "fo_debug_trace_read": (C.c_int, [_P, _P, C.c_int64, _I64P]),
+    "fo_debug_sm_ids": (C.c_int, [_P, C.c_int, C.c_int, _P, _P]),
     "fo_debug_plan": (C.c_int, [C.c_int64, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "fo_debug_stack_plan": (C.c_int, [C.c_int] * 9 + [C.POINTER(C.c_int)] * 5),
     "fo_stream_step_async": (C.c_int, [_P, _I32P, C.c_int, _P, C.c_int, C.c_float, _P, _P, _P, C.POINTER(C.c_int64)]),

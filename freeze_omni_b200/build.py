@@ -16,7 +16,7 @@ CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "csrc", "build")
 LIB = os.path.join(HERE, "libfo_b200.so")
 SOURCES = ["fo_api.cu", "fo_gemm_simt.cu", "fo_gemm_tc.cu", "fo_elementwise.cu", "fo_attention.cu", "fo_fbank.cu", "fo_stack.cu",
-           "fo_session.cu"]
+           "fo_session.cu", "fo_partition.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr"]
 if os.environ.get("FO_TC_TRACE_BUILD") == "1":        # in-kernel timeline stamps for tools/gemm_trace.py

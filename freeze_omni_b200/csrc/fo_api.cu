@@ -26,8 +26,9 @@
 
 namespace fo {
 
-long long g_launches = 0;
-int g_use_pdl = 1;        // launch attribute actually applied (set per step)
+std::atomic<long long> g_launches{0};
+thread_local long long t_launches = 0;
+thread_local int g_use_pdl = 1;   // launch attribute actually applied (set per step, by the thread that enqueues it)
 int g_want_pdl = 1;       // option "pdl"
 static thread_local char g_err[1024] = "";
 
@@ -216,6 +217,14 @@ struct fo_ctx {
     int snap_stage_n = 0;
     cudaStream_t cap_stream = nullptr;        // capture happens here (the caller's stream may be the legacy
                                               // default stream, which cannot be captured); replay on the caller's
+    // SMs the context's grids are sized to: its SM group (fo_create_on_sms), else the device
+    int sms = 148;
+    int smem_optin = 0, coop = 0;             // the device's opt-in shared memory per CTA, cooperative-launch support
+    void* green = nullptr;                    // the group's green context (fo_partition.cu); null: the whole device
+    cudaStream_t exec_stream = nullptr;       // with a group: the stream of the group every entry point enqueues on (OnGroup)
+    cudaEvent_t ev_enter = nullptr, ev_leave = nullptr;
+    std::string leave_err;                    // a call whose caller's stream could not be ordered after its work (OnGroup):
+                                              // the next call through OnGroup returns this as its error
     // stats
     fo_stats_t stats;
     std::mutex mu;
@@ -241,12 +250,14 @@ int dev_alloc(fo_ctx* c, void** p, size_t bytes) {
     return 0;
 }
 
+int ctx_sync(fo_ctx* c);
+
 int ws_ensure(fo_ctx* c, int which, size_t bytes, void** out) {
     DevBuf& b = c->ws[which];
     if (b.cap < bytes) {
         if (b.p) {
             // grown buffers are rare (first call at a new size); wait for users of the old one
-            FO_CUDA(cudaDeviceSynchronize());
+            FO_TRY(ctx_sync(c));
             for (auto& q : c->owned)
                 if (q == b.p) { q = nullptr; break; }
             cudaFree(b.p);
@@ -286,6 +297,61 @@ int out_done(void* user, void* dev, size_t bytes, cudaStream_t st) {
     if (user && user != dev) FO_CUDA(cudaMemcpyAsync(user, dev, bytes, cudaMemcpyDeviceToHost, st));
     return 0;
 }
+
+// every internal stream of the context: in its SM group when it has one
+int make_stream(fo_ctx* c, cudaStream_t* st) {
+    if (c->green) return sm_group_stream(c->green, st);
+    FO_CUDA(cudaStreamCreateWithFlags(st, cudaStreamNonBlocking));
+    return 0;
+}
+
+// cudaDeviceSynchronize, and the context's own streams when they live in its SM group's green context
+int ctx_sync(fo_ctx* c) {
+    FO_CUDA(cudaDeviceSynchronize());
+    if (!c->green) return 0;
+    for (cudaStream_t s : {c->exec_stream, c->cap_stream, c->copy_stream, c->upload_stream})
+        if (s) FO_CUDA(cudaStreamSynchronize(s));
+    for (int g = 0; g < fo_ctx::MAX_GROUPS; ++g) {
+        if (c->grp_stream[g]) FO_CUDA(cudaStreamSynchronize(c->grp_stream[g]));
+        if (c->mix_stream[g]) FO_CUDA(cudaStreamSynchronize(c->mix_stream[g]));
+    }
+    return 0;
+}
+
+// The stream an entry point enqueues on.  A whole-device context works on the caller's stream itself.  A context on an SM
+// group works on its execution stream in that group, ordered after what the caller enqueued on its stream before the call
+// and before what the caller enqueues after it: caller -> record -> wait -> the call's work -> record -> caller waits.
+struct OnGroup {
+    fo_ctx* c;
+    cudaStream_t user, st;
+    int err = 0;
+    OnGroup(fo_ctx* c_, void* stream) : c(c_), user((cudaStream_t)stream), st((cudaStream_t)stream) {
+        if (!c || !c->green) return;
+        if (!c->leave_err.empty()) {
+            set_error("%s", c->leave_err.c_str());
+            c->leave_err.clear();
+            err = FO_ERR_CUDA;
+            return;
+        }
+        cudaError_t e = cudaEventRecord(c->ev_enter, user);
+        if (e == cudaSuccess) e = cudaStreamWaitEvent(c->exec_stream, c->ev_enter, 0);
+        if (e != cudaSuccess) { set_error("entering the context's SM group: %s", cudaGetErrorString(e)); err = FO_ERR_CUDA; return; }
+        st = c->exec_stream;
+    }
+    ~OnGroup() {
+        if (st == user) return;
+        cudaError_t e = cudaEventRecord(c->ev_leave, st);
+        if (e == cudaSuccess) e = cudaStreamWaitEvent(user, c->ev_leave, 0);
+        if (e != cudaSuccess)
+            c->leave_err = std::string("a previous call could not order the caller's stream after its work in the context's SM group: ") +
+                           cudaGetErrorString(e);
+    }
+};
+// at the top of an entry point taking `void* stream`: from here on `stream` is the stream the call enqueues on
+#define FO_ON_GROUP(c, stream)                       \
+    OnGroup on_group_(c, stream);                    \
+    FO_TRY(on_group_.err);                           \
+    stream = (void*)on_group_.st
 
 int check_ids(fo_ctx* c, const int32_t* ids, int n) {
     FO_CHECK(ids != nullptr && n > 0, "ids must be a host array of n > 0 session ids");
@@ -671,6 +737,7 @@ FbankParams fbank_params(fo_ctx* c) {
     p.window = c->fb_window;
     p.mel = c->fb_mel;
     p.mel_lo = c->fb_lo;
+    p.sms = c->sms;
     p.mel_hi = c->fb_hi;
     return p;
 }
@@ -1058,7 +1125,8 @@ int stack_program(fo_ctx* c, int n, int t, float* x, void* qkv, float* q32, void
     static int want_trace = -1;
     if (want_trace < 0) want_trace = getenv("FO_STACK_TRACE") ? 1 : 0;
     s.trace = want_trace ? c->stack_trace : nullptr;
-    const int r = stream_stack(s, st);
+    if (!c->coop) return 1;
+    const int r = stream_stack(s, c->sms, c->smem_optin, st);
     if (r != 0) return r;
     c->stack_launches += 1;
     if (want_trace) {
@@ -1081,8 +1149,7 @@ int stack_program(fo_ctx* c, int n, int t, float* x, void* qkv, float* q32, void
             }
             fprintf(stderr, "\n  barriers of that layer, over the CTAs (ns from the phase start): ");
             {
-                int G = 0;
-                cudaDeviceGetAttribute(&G, cudaDevAttrMultiProcessorCount, c->device);
+                const int G = c->sms;
                 for (int q = 0; q < 5; ++q) {
                     const unsigned long long* a = hb.data() + 35 * c->L + 8 + 2 * G * q;
                     unsigned long long amin = ~0ULL, amax = 0, rmin = ~0ULL, rmax = 0;
@@ -1529,10 +1596,10 @@ extern "C" {
 int fo_abi_version(void) { return FO_ABI_VERSION; }
 const char* fo_last_error(void) { return g_err; }
 
-int fo_create(const fo_config* cfg, int device, int dtype, fo_ctx** out) {
-    FO_CHECK(cfg && out, "fo_create: null argument");
-    *out = nullptr;
-    FO_CHECK(dtype == FO_F32 || dtype == FO_BF16, "fo_create: dtype must be FO_F32 or FO_BF16");
+}  // extern "C"
+
+// fo_create (sm_split 0: the whole device) and fo_create_on_sms
+static int create_ctx(const fo_config* cfg, int device, int dtype, int sm_split, int sm_group, fo_ctx** out) {
     int ndev = 0;
     cudaError_t e = cudaGetDeviceCount(&ndev);
     if (e != cudaSuccess || ndev == 0) {
@@ -1556,11 +1623,19 @@ int fo_create(const fo_config* cfg, int device, int dtype, fo_ctx** out) {
     FO_CHECK(!(cfg->has_adapter && (cfg->adapter_type == 2 || (cfg->adapter_type == 0 && 4 * cfg->d_model < cfg->llm_dim))) || 4 * cfg->d_model <= 4096,
              "fo_create: the two-conv adapters normalise 4 * d_model channels; d_model must be <= 1024");
 
+    void* green = nullptr;
+    int sms = prop.multiProcessorCount;
+    if (sm_split > 0) FO_TRY(sm_group_acquire(device, sm_split, sm_group, &green, &sms));
+
     fo_ctx* c = new fo_ctx();
     c->cfg = *cfg;
     c->device = device;
     c->dtype = dtype;
     c->esz = dtype == FO_BF16 ? 2 : 4;
+    c->sms = sms;
+    c->green = green;
+    c->smem_optin = (int)prop.sharedMemPerBlockOptin;
+    c->coop = prop.cooperativeLaunch;
     memset(&c->stats, 0, sizeof(c->stats));
     c->F = cfg->feat_dim; c->F1 = (c->F - 1) / 2; c->F2 = (c->F1 - 1) / 2;
     c->D = cfg->d_model; c->H = cfg->n_heads; c->FF = cfg->ffn_dim; c->L = cfg->n_layers; c->E = cfg->llm_dim;
@@ -1645,22 +1720,22 @@ int fo_create(const fo_config* cfg, int device, int dtype, fo_ctx** out) {
             r = FO_ERR_NOMEM;
         }
     }
-    if (!r && cudaStreamCreateWithFlags(&c->cap_stream, cudaStreamNonBlocking) != cudaSuccess) {
-        set_error("fo_create: cudaStreamCreate failed");
-        r = FO_ERR_CUDA;
-    }
+    if (!r) r = make_stream(c, &c->cap_stream);
+    if (!r && c->green) r = make_stream(c, &c->exec_stream);
+    if (!r && c->green && (cudaEventCreateWithFlags(&c->ev_enter, cudaEventDisableTiming) != cudaSuccess ||
+                           cudaEventCreateWithFlags(&c->ev_leave, cudaEventDisableTiming) != cudaSuccess)) r = FO_ERR_CUDA;
     for (int g = 1; g < fo_ctx::MAX_GROUPS && !r; ++g) {
-        if (cudaStreamCreateWithFlags(&c->grp_stream[g], cudaStreamNonBlocking) != cudaSuccess ||
-            cudaEventCreateWithFlags(&c->ev_join[g], cudaEventDisableTiming) != cudaSuccess) {
+        r = make_stream(c, &c->grp_stream[g]);
+        if (!r && cudaEventCreateWithFlags(&c->ev_join[g], cudaEventDisableTiming) != cudaSuccess) {
             set_error("fo_create: group stream creation failed");
             r = FO_ERR_CUDA;
         }
     }
     if (!r && cudaEventCreateWithFlags(&c->ev_fork, cudaEventDisableTiming) != cudaSuccess) r = FO_ERR_CUDA;
     for (int g = 0; g < fo_ctx::MAX_GROUPS && !r; ++g) {
-        if (cudaStreamCreateWithFlags(&c->mix_stream[g], cudaStreamNonBlocking) != cudaSuccess ||
-            cudaEventCreateWithFlags(&c->ev_mix_fork[g], cudaEventDisableTiming) != cudaSuccess ||
-            cudaEventCreateWithFlags(&c->ev_mix_join[g], cudaEventDisableTiming) != cudaSuccess) {
+        r = make_stream(c, &c->mix_stream[g]);
+        if (!r && (cudaEventCreateWithFlags(&c->ev_mix_fork[g], cudaEventDisableTiming) != cudaSuccess ||
+            cudaEventCreateWithFlags(&c->ev_mix_join[g], cudaEventDisableTiming) != cudaSuccess)) {
             set_error("fo_create: stream creation failed");
             r = FO_ERR_CUDA;
         }
@@ -1673,13 +1748,34 @@ int fo_create(const fo_config* cfg, int device, int dtype, fo_ctx** out) {
     return 0;
 }
 
+extern "C" {
+
+int fo_create(const fo_config* cfg, int device, int dtype, fo_ctx** out) {
+    FO_CHECK(cfg && out, "fo_create: null argument");
+    *out = nullptr;
+    FO_CHECK(dtype == FO_F32 || dtype == FO_BF16, "fo_create: dtype must be FO_F32 or FO_BF16");
+    return create_ctx(cfg, device, dtype, 0, 0, out);
+}
+
+int fo_create_on_sms(const fo_config* cfg, int device, int dtype, int sm_split, int sm_group, fo_ctx** out) {
+    FO_CHECK(cfg && out, "fo_create_on_sms: null argument");
+    *out = nullptr;
+    FO_CHECK(dtype == FO_F32 || dtype == FO_BF16, "fo_create_on_sms: dtype must be FO_F32 or FO_BF16");
+    FO_CHECK(sm_split >= 1, "fo_create_on_sms: sm_split must be >= 1 (got %d)", sm_split);
+    FO_CHECK(sm_group >= 0 && sm_group < sm_split, "fo_create_on_sms: sm_group %d is outside [0, sm_split = %d)", sm_group, sm_split);
+    return create_ctx(cfg, device, dtype, sm_split, sm_group, out);
+}
+
 int fo_destroy(fo_ctx* c) {
     if (!c) return 0;
     cudaSetDevice(c->device);
-    cudaDeviceSynchronize();
+    ctx_sync(c);
     for (auto& kv : c->staged) cudaFree(kv.second.d);
     for (auto& kv : c->graphs) if (kv.second.exec) cudaGraphExecDestroy(kv.second.exec);
     if (c->cap_stream) cudaStreamDestroy(c->cap_stream);
+    if (c->exec_stream) cudaStreamDestroy(c->exec_stream);
+    if (c->ev_enter) cudaEventDestroy(c->ev_enter);
+    if (c->ev_leave) cudaEventDestroy(c->ev_leave);
     if (c->copy_stream) cudaStreamDestroy(c->copy_stream);
     if (c->upload_stream) cudaStreamDestroy(c->upload_stream);
     for (int i = 0; i < 2; ++i) {
@@ -1735,6 +1831,7 @@ int fo_finalize_weights(fo_ctx* c) {
         FO_TRY(gemm_tc_init());
         for (int g = 0; g < fo_ctx::MAX_GROUPS; ++g) {
             FO_TRY(gemm_tc_workspace(&c->tc_wsg[g]));
+            c->tc_wsg[g].sms = c->sms;
             c->owned.push_back(c->tc_wsg[g].partial);
             c->owned.push_back(c->tc_wsg[g].counters);
             c->device_bytes += (long long)c->tc_wsg[g].partial_bytes;
@@ -1766,7 +1863,7 @@ int fo_session_alloc(fo_ctx* c, int n, int32_t* ids_out) {
     std::lock_guard<std::mutex> lk(c->mu);
     FO_CHECK((int)c->free_slots.size() >= n, "fo_session_alloc: %d sessions requested, %zu slots free", n, c->free_slots.size());
     FO_CUDA(cudaSetDevice(c->device));
-    FO_CUDA(cudaDeviceSynchronize());
+    FO_TRY(ctx_sync(c));
     for (int i = 0; i < n; ++i) {
         int s = c->free_slots.back();
         c->free_slots.pop_back();
@@ -1782,7 +1879,7 @@ int fo_session_reset(fo_ctx* c, int n, const int32_t* ids) {
     FO_CHECK(c, "null context");
     FO_TRY(check_ids(c, ids, n));
     FO_CUDA(cudaSetDevice(c->device));
-    FO_CUDA(cudaDeviceSynchronize());
+    FO_TRY(ctx_sync(c));
     for (int i = 0; i < n; ++i) FO_TRY(reset_slot(c, ids[i]));
     return 0;
 }
@@ -1837,7 +1934,7 @@ static int kv_ptrs(fo_ctx* c, int32_t id, int layer, void** k, void** v, int32_t
     FO_TRY(check_ids(c, &id, 1));
     FO_CHECK(layer >= 0 && layer < c->L, "layer %d out of range", layer);
     FO_CUDA(cudaSetDevice(c->device));
-    FO_CUDA(cudaDeviceSynchronize());
+    FO_TRY(ctx_sync(c));
     FO_CUDA(cudaMemcpy(nf, c->n_frames + id, 4, cudaMemcpyDeviceToHost));
     const size_t per_kv = (size_t)c->H * c->ring_cap * 64;
     char* base = reinterpret_cast<char*>(c->ring) + (((size_t)layer * c->cfg.max_sessions + id) * 2) * per_kv * c->esz;
@@ -1866,7 +1963,7 @@ int fo_session_export_kv(fo_ctx* c, int32_t id, int layer, float* K, float* V, i
     }
     if (K) FO_TRY(out_done(K, dk, bytes, 0));
     if (V) FO_TRY(out_done(V, dv, bytes, 0));
-    FO_CUDA(cudaDeviceSynchronize());
+    FO_TRY(ctx_sync(c));
     return 0;
 }
 
@@ -1888,7 +1985,7 @@ int fo_session_import_kv(fo_ctx* c, int32_t id, int layer, const float* K, const
         FO_TRY(ring_import<float>((float*)k, c->H, c->ring_cap, nf - cache_len, cache_len, (const float*)dk, 0));
         FO_TRY(ring_import<float>((float*)v, c->H, c->ring_cap, nf - cache_len, cache_len, (const float*)dv, 0));
     }
-    FO_CUDA(cudaDeviceSynchronize());
+    FO_TRY(ctx_sync(c));
     return 0;
 }
 
@@ -1913,7 +2010,7 @@ int fo_session_export_adapter_cache_n(fo_ctx* c, int32_t id, int which, float* c
     FO_TRY(ad_cache_of(c, which, &base, &C));
     FO_TRY(check_ids(c, &id, 1));
     FO_CUDA(cudaSetDevice(c->device));
-    FO_CUDA(cudaDeviceSynchronize());
+    FO_TRY(ctx_sync(c));
     int32_t live = 0;
     FO_CUDA(cudaMemcpy(&live, c->ad_valid + id, 4, cudaMemcpyDeviceToHost));
     if (valid) *valid = live != 0;
@@ -1933,7 +2030,7 @@ int fo_session_import_adapter_cache_n(fo_ctx* c, int32_t id, int which, const fl
     FO_TRY(ad_cache_of(c, which, &base, &C));
     FO_TRY(check_ids(c, &id, 1));
     FO_CUDA(cudaSetDevice(c->device));
-    FO_CUDA(cudaDeviceSynchronize());
+    FO_TRY(ctx_sync(c));
     int32_t live = 0;
     FO_CUDA(cudaMemcpy(&live, c->ad_valid + id, 4, cudaMemcpyDeviceToHost));
     if (valid) {
@@ -1966,7 +2063,7 @@ int fo_session_export_ffn_cache(fo_ctx* c, int32_t id, int layer, float* cache) 
     FO_TRY(check_ids(c, &id, 1));
     FO_CHECK(layer >= 0 && layer < c->L, "layer %d out of range", layer);
     FO_CUDA(cudaSetDevice(c->device));
-    FO_CUDA(cudaDeviceSynchronize());
+    FO_TRY(ctx_sync(c));
     const int km1 = c->KF - 1, D = c->D;
     std::vector<float> tm((size_t)km1 * D), out((size_t)km1 * D);
     FO_CUDA(cudaMemcpy(tm.data(), c->ffn_cache + ((size_t)id * c->L + layer) * km1 * D, tm.size() * 4, cudaMemcpyDeviceToHost));
@@ -2131,6 +2228,7 @@ int fo_session_snapshot_bytes(fo_ctx* c, int64_t* bytes) {
 }
 
 int fo_session_save(fo_ctx* c, const int32_t* ids, int n, void* buf, void* stream) {
+    FO_ON_GROUP(c, stream);
     const cudaStream_t st = (cudaStream_t)stream;
     SnapArgs a;
     bool on_device;
@@ -2154,6 +2252,7 @@ int fo_session_save(fo_ctx* c, const int32_t* ids, int n, void* buf, void* strea
 }
 
 int fo_session_restore(fo_ctx* c, const int32_t* ids, int n, const void* buf, void* stream) {
+    FO_ON_GROUP(c, stream);
     const cudaStream_t st = (cudaStream_t)stream;
     SnapArgs a;
     bool on_device;
@@ -2195,6 +2294,7 @@ int fo_fbank_stream(fo_ctx* c, const int32_t* ids, int n, const void* pcm, int p
     FO_CHECK(pcm && (pcm_dtype == FO_F32 || pcm_dtype == FO_I16), "fo_fbank_stream: pcm must be FO_F32 or FO_I16");
     FO_TRY(check_ids(c, ids, n));
     FO_CUDA(cudaSetDevice(c->device));
+    FO_ON_GROUP(c, stream);
     cudaStream_t st = (cudaStream_t)stream;
     FO_TRY(upload_ids(c, ids, n, st));
     const size_t in_bytes = (size_t)n * c->chunk_samples * (pcm_dtype == FO_I16 ? 2 : 4);
@@ -2216,6 +2316,7 @@ int fo_fbank_offline(fo_ctx* c, const void* pcm, int pcm_dtype, int B, int64_t n
     FO_CHECK(pcm && out && B > 0 && (pcm_dtype == FO_F32 || pcm_dtype == FO_I16), "fo_fbank_offline: bad argument");
     FO_CHECK(n_samples >= c->cfg.frame_len, "fo_fbank_offline: signal shorter than one frame");
     FO_CUDA(cudaSetDevice(c->device));
+    FO_ON_GROUP(c, stream);
     cudaStream_t st = (cudaStream_t)stream;
     const size_t in_bytes = (size_t)B * n_samples * (pcm_dtype == FO_I16 ? 2 : 4);
     const void* dp;
@@ -2304,7 +2405,7 @@ static int run_step(fo_ctx* c, const StepArgs& a, cudaStream_t st) {
         g.warm_epoch = c->ws_epoch;
         return 0;
     }
-    const long long l0 = g_launches, e0 = c->ws_epoch, s0 = c->stack_launches;
+    const long long l0 = t_launches, e0 = c->ws_epoch, s0 = c->stack_launches;
     FO_CUDA(cudaStreamBeginCapture(c->cap_stream, cudaStreamCaptureModeRelaxed));
     int r = step_body(c, a, c->cap_stream);
     cudaGraph_t graph = nullptr;
@@ -2319,8 +2420,8 @@ static int run_step(fo_ctx* c, const StepArgs& a, cudaStream_t st) {
     cudaGraphDestroy(graph);
     if (ce != cudaSuccess) { g.exec = nullptr; set_error("cudaGraphInstantiate: %s", cudaGetErrorString(ce)); return FO_ERR_CUDA; }
     g.epoch = c->ws_epoch;
-    g.launches = g_launches - l0;                  // counted while capturing, not yet run
-    g_launches = l0;
+    g.launches = t_launches - l0;                  // counted (by this thread) while capturing, not yet run
+    g_launches -= g.launches;
     g.stacks = c->stack_launches - s0;
     FO_CUDA(cudaGraphLaunch(g.exec, st));
     g_launches += g.launches;
@@ -2412,6 +2513,7 @@ int fo_encode_stream(fo_ctx* c, const int32_t* ids, int n, const float* feats, i
     FO_CHECK(c && c->finalized && c->cfg.has_encoder, "fo_encode_stream: context has no finalized encoder");
     FO_TRY(check_ids(c, ids, n));
     FO_CUDA(cudaSetDevice(c->device));
+    FO_ON_GROUP(c, stream);
     if (feats) FO_CHECK(t_in >= 7, "fo_encode_stream: need at least 7 feature frames");
     else t_in = c->cfg.context_frames + c->cfg.frames_per_chunk;
     Mix m;
@@ -2435,6 +2537,7 @@ int fo_encode_stream_chunks(fo_ctx* c, const int32_t* ids, int n, int k, const f
                  c->window, k, t, STREAM_CHUNKS_MAX_KEYS, kmax);
     }
     FO_CUDA(cudaSetDevice(c->device));
+    FO_ON_GROUP(c, stream);
     // the uniform case of fo_encode_stream_chunks_v: every session brings k chunks
     const std::vector<int32_t> chunks(n, k);
     Mix m;
@@ -2469,6 +2572,7 @@ int fo_encode_stream_chunks_v(fo_ctx* c, const int32_t* ids, const int32_t* chun
     m.blocks = off[n];
     if (!m.uniform(n)) m.off = off.data();
     FO_CUDA(cudaSetDevice(c->device));
+    FO_ON_GROUP(c, stream);
     return stream_common(c, ids, n, m.kmax > 1 ? chunks : nullptr, m, nullptr, FO_F32, 1.0f, feats, t_in, enc_out, adapter_out,
                          (cudaStream_t)stream);
 }
@@ -2506,6 +2610,7 @@ int fo_stream_step_embeds(fo_ctx* c, const int32_t* ids, int n, const void* pcm,
     FO_CHECK(pcm && (pcm_dtype == FO_F32 || pcm_dtype == FO_I16), "fo_stream_step_embeds: pcm must be FO_F32 or FO_I16");
     FO_TRY(check_ids(c, ids, n));
     FO_CUDA(cudaSetDevice(c->device));
+    FO_ON_GROUP(c, stream);
     const int t_in = c->cfg.context_frames + c->cfg.frames_per_chunk;
     const int t = ((t_in - 1) / 2 - 1) / 2, t_out = ad_frames(c, t);
     FO_CHECK(embeds_f16 && row_offset >= 0 && rows_per_session >= row_offset + t_out && rows_per_session < (1LL << 31),
@@ -2534,10 +2639,11 @@ int fo_stream_step_async(fo_ctx* c, const int32_t* ids, int n, const void* pcm, 
     FO_TRY(check_ids(c, ids, n));
     FO_TRY(stream_geometry(c, c->cfg.context_frames + c->cfg.frames_per_chunk));
     FO_CUDA(cudaSetDevice(c->device));
+    FO_ON_GROUP(c, stream);
     cudaStream_t st = (cudaStream_t)stream;
     if (!c->copy_stream) {
-        FO_CUDA(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
-        FO_CUDA(cudaStreamCreateWithFlags(&c->upload_stream, cudaStreamNonBlocking));
+        FO_TRY(make_stream(c, &c->copy_stream));
+        FO_TRY(make_stream(c, &c->upload_stream));
         for (int i = 0; i < 2; ++i) {
             FO_CUDA(cudaEventCreateWithFlags(&c->ev_in[i], cudaEventDisableTiming));
             FO_CUDA(cudaEventCreateWithFlags(&c->ev_compute[i], cudaEventDisableTiming));
@@ -2590,6 +2696,7 @@ int fo_stream_step(fo_ctx* c, const int32_t* ids, int n, const void* pcm, int pc
     FO_CHECK(pcm && (pcm_dtype == FO_F32 || pcm_dtype == FO_I16), "fo_stream_step: pcm must be FO_F32 or FO_I16");
     FO_TRY(check_ids(c, ids, n));
     FO_CUDA(cudaSetDevice(c->device));
+    FO_ON_GROUP(c, stream);
     Mix m;
     m.blocks = m.n1 = n;
     return stream_common(c, ids, n, nullptr, m, pcm, pcm_dtype, scale, nullptr, c->cfg.context_frames + c->cfg.frames_per_chunk, enc_out,
@@ -2670,8 +2777,7 @@ static int steps_passes(fo_ctx* c, const int32_t* ids, const int32_t* chunks, in
             c->ho_tab_cap = off[n];
         }
     }
-    int sms = 148;
-    FO_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->device));
+    const int sms = c->sms;
     const int gmax = std::max(1, (STREAM_CHUNKS_MAX_KEYS - c->window) / std::max(1, t));
     g_use_pdl = g_want_pdl;
     std::vector<int32_t> done(n, 0), pids, pcnt, poff, psrc;
@@ -2811,6 +2917,7 @@ int fo_stream_steps_v(fo_ctx* c, const int32_t* ids, const int32_t* chunks, int 
     const int t_in = c->cfg.context_frames + c->cfg.frames_per_chunk;
     FO_TRY(check_steps_encode(c, "fo_stream_steps_v", ids, chunks, n, t_in, adapter_out));
     FO_CUDA(cudaSetDevice(c->device));
+    FO_ON_GROUP(c, stream);
     StepsIo io;
     io.pcm = pcm;
     io.pcm_dtype = pcm_dtype;
@@ -2830,6 +2937,7 @@ int fo_encode_stream_steps_v(fo_ctx* c, const int32_t* ids, const int32_t* chunk
     FO_CHECK(t_in >= 7, "fo_encode_stream_steps_v: need at least 7 feature frames per chunk");
     FO_TRY(check_steps_encode(c, "fo_encode_stream_steps_v", ids, chunks, n, t_in, adapter_out));
     FO_CUDA(cudaSetDevice(c->device));
+    FO_ON_GROUP(c, stream);
     StepsIo io;
     io.feats = feats;
     io.encode = true;
@@ -2848,6 +2956,7 @@ int fo_fbank_stream_v(fo_ctx* c, const int32_t* ids, const int32_t* chunks, int 
     FO_TRY(check_ids(c, ids, n));
     FO_TRY(check_steps_counts("fo_fbank_stream_v", ids, chunks, n));
     FO_CUDA(cudaSetDevice(c->device));
+    FO_ON_GROUP(c, stream);
     StepsIo io;
     io.pcm = pcm;
     io.pcm_dtype = pcm_dtype;
@@ -2864,6 +2973,7 @@ int fo_encode_offline(fo_ctx* c, const float* feats, const int32_t* ilens, int B
     const int T1 = (T - 1) / 2, T2 = (T1 - 1) / 2;
     FO_CHECK(T2 <= c->cfg.pos_max_len, "fo_encode_offline: %d encoder frames exceed the positional table (%d)", T2, c->cfg.pos_max_len);
     FO_CUDA(cudaSetDevice(c->device));
+    FO_ON_GROUP(c, stream);
     cudaStream_t st = (cudaStream_t)stream;
     const void *dfeats, *dil;
     FO_TRY(in_dev(c, feats, (size_t)B * T * c->F * sizeof(float), WS_FEATS, st, &dfeats));
@@ -2954,6 +3064,7 @@ int fo_encode_offline_packed(fo_ctx* c, const float* feats, const int32_t* lens,
     FO_CHECK(feats && lens && B > 0 && B <= 65535, "fo_encode_offline_packed: need feats, lens and 1 <= B <= 65535");
     if (adapter_out) FO_CHECK(c->cfg.has_adapter, "adapter_out requested but the context has no adapter");
     FO_CUDA(cudaSetDevice(c->device));
+    FO_ON_GROUP(c, stream);
     cudaStream_t st = (cudaStream_t)stream;
     PackTab p;
     std::vector<int32_t> T(B);
@@ -3009,6 +3120,7 @@ int fo_fbank_offline_packed(fo_ctx* c, const void* pcm, int pcm_dtype, const int
         foff[b + 1] = (int32_t)frames;
     }
     FO_CUDA(cudaSetDevice(c->device));
+    FO_ON_GROUP(c, stream);
     cudaStream_t st = (cudaStream_t)stream;
     void* dtab;
     FO_TRY(ws_ensure(c, WS_FBTAB, h.size() * sizeof(int32_t), &dtab));
@@ -3076,6 +3188,7 @@ int fo_encode_offline_packed_pcm(fo_ctx* c, const void* pcm, int pcm_dtype, cons
         aoff[b + 1] = aoff[b] + ad_frames(c, (int)t2);
     }
     FO_CUDA(cudaSetDevice(c->device));
+    FO_ON_GROUP(c, stream);
     cudaStream_t st = (cudaStream_t)stream;
     const int P = packed_pass_frames(c), F = c->F, D = c->D, E = c->E;
     const size_t esz_pcm = pcm_dtype == FO_I16 ? 2 : 4;
@@ -3134,6 +3247,7 @@ int fo_adapter_forward2(fo_ctx* c, const float* x, const uint8_t* mask, int B, i
     FO_CHECK(c && c->finalized && c->cfg.has_adapter, "fo_adapter_forward: context has no finalized adapter");
     FO_CHECK(x && y && B > 0 && T > 0, "fo_adapter_forward: bad argument");
     FO_CUDA(cudaSetDevice(c->device));
+    FO_ON_GROUP(c, stream);
     cudaStream_t st = (cudaStream_t)stream;
     const int km1 = c->KA - 1, t_out = ad_frames(c, T);
     FO_CHECK(t_out >= 1, "fo_adapter_forward: input too short");
@@ -3183,7 +3297,7 @@ int fo_adapter_forward(fo_ctx* c, const float* x, const uint8_t* mask, int B, in
 int fo_stats(fo_ctx* c, fo_stats_t* out) {
     FO_CHECK(c && out, "fo_stats: null argument");
     *out = c->stats;
-    out->kernel_launches = g_launches;
+    out->kernel_launches = g_launches.load();
     out->sessions_in_use = c->sessions_in_use;
     out->device_bytes = c->device_bytes;
     out->act_saturations = 0;
@@ -3210,7 +3324,7 @@ int fo_set_option(fo_ctx* c, const char* name, int64_t value) {
         // development builds (FO_TRACE_BUILD): value > 0 allocates room for `value` CTA records and binds the kernels to it,
         // 0 unbinds.  fo_debug_trace_read copies the records out.
         FO_CUDA(cudaSetDevice(c->device));
-        FO_CUDA(cudaDeviceSynchronize());
+        FO_TRY(ctx_sync(c));
         if (value > 0 && (unsigned int)value > c->trace_cap) {
             void* p = nullptr;
             FO_TRY(dev_alloc(c, &p, (size_t)value * 8 * sizeof(unsigned long long)));
@@ -3300,6 +3414,7 @@ int fo_get_option(fo_ctx* c, const char* name, int64_t* value) {
     else if (!strcmp(name, "tc_launches")) *value = gemm_tc_launches();
     else if (!strcmp(name, "ring_cap")) *value = c->ring_cap;
     else if (!strcmp(name, "max_t")) *value = c->max_t;
+    else if (!strcmp(name, "sm_count")) *value = c->sms;
     else { set_error("fo_get_option: unknown option '%s'", name); return FO_ERR_ARG; }
     return 0;
 }
@@ -3332,7 +3447,7 @@ int fo_debug_trace_read(fo_ctx* c, uint64_t* out, int64_t cap_records, int64_t* 
     *n_records = 0;
     if (!c->trace_cnt) return 0;
     FO_CUDA(cudaSetDevice(c->device));
-    FO_CUDA(cudaDeviceSynchronize());
+    FO_TRY(ctx_sync(c));
     unsigned int n = 0;
     FO_CUDA(cudaMemcpy(&n, c->trace_cnt, sizeof(n), cudaMemcpyDeviceToHost));
     if (n > c->trace_cap) n = c->trace_cap;
@@ -3350,6 +3465,35 @@ int fo_debug_stack_plan(int d_model, int ffn_dim, int heads, int n_sessions, int
                       rows_ffn1, rows_out);
 }
 
+int fo_debug_sm_ids(fo_ctx* c, int n_ctas, int graph, int32_t* out, void* stream) {
+    FO_CHECK(c && out && n_ctas > 0 && n_ctas <= 65535, "fo_debug_sm_ids: bad argument");
+    FO_CUDA(cudaSetDevice(c->device));
+    FO_ON_GROUP(c, stream);
+    const cudaStream_t st = (cudaStream_t)stream;
+    void* d;
+    FO_TRY(out_dev(c, out, (size_t)n_ctas * sizeof(int32_t), WS_TMP0, &d));
+    if (!graph) {
+        FO_TRY(sm_ids((int32_t*)d, n_ctas, st));
+    } else {
+        // as run_step does with a step: captured on the capture stream, instantiated, replayed on the stream of the call
+        FO_CUDA(cudaStreamBeginCapture(c->cap_stream, cudaStreamCaptureModeRelaxed));
+        const int r = sm_ids((int32_t*)d, n_ctas, c->cap_stream);
+        cudaGraph_t g = nullptr;
+        const cudaError_t ce = cudaStreamEndCapture(c->cap_stream, &g);
+        if (r != 0) { if (g) cudaGraphDestroy(g); return r; }
+        FO_CUDA(ce);
+        cudaGraphExec_t ge = nullptr;
+        const cudaError_t ie = cudaGraphInstantiate(&ge, g, 0);
+        cudaGraphDestroy(g);
+        FO_CUDA(ie);
+        const cudaError_t le = cudaGraphLaunch(ge, st);
+        const cudaError_t se = le == cudaSuccess ? cudaStreamSynchronize(st) : le;
+        cudaGraphExecDestroy(ge);
+        FO_CUDA(se);
+    }
+    return out_done(out, d, (size_t)n_ctas * sizeof(int32_t), st);
+}
+
 int fo_debug_plan(int64_t act_rows, int n_out, int K, int can_defer, int* swap, int* bn, int* split) {
     FO_CHECK(act_rows > 0 && n_out > 0 && K > 0 && K % 64 == 0 && swap && bn && split, "fo_debug_plan: bad argument");
     gemm_tc_plan(act_rows, n_out, K, can_defer, swap, bn, split);
@@ -3360,6 +3504,7 @@ int fo_debug_gemm(fo_ctx* c, const float* A, const float* W, const float* bias, 
                   int backend, int relu, int iters, float* ms_out, void* stream) {
     FO_CHECK(c && A && W && C && M > 0 && N > 0 && K > 0, "fo_debug_gemm: bad argument");
     FO_CUDA(cudaSetDevice(c->device));
+    FO_ON_GROUP(c, stream);
     cudaStream_t st = (cudaStream_t)stream;
     Epilogue ep;
     ep.bias = bias;
@@ -3492,6 +3637,7 @@ int fo_debug_attention(fo_ctx* c, int mode, int n, const int32_t* seq, const int
         }
     }
     FO_CUDA(cudaSetDevice(c->device));
+    FO_ON_GROUP(c, stream);
     cudaStream_t st = (cudaStream_t)stream;
     return c->dtype == FO_BF16 ? debug_attention_run<act16>(c, d, st) : debug_attention_run<float>(c, d, st);
 }

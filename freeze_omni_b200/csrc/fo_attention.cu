@@ -993,7 +993,7 @@ int attention_stream(const AttnStream& a, const TA* qkv, const float* q32, TA* r
         smem = (size_t)3 * prow * DK * 4 + (size_t)2 * t * DK * 4 + (size_t)t * prow * 4;
     }
     FO_CHECK(smem <= 160 * 1024, "attention_stream: window too large for shared memory");
-    static bool opted_in = false;      // past 48 KB (window + t > ~115 keys, e.g. left_chunks 31) a launch needs the opt-in
+    static std::atomic<bool> opted_in{false};      // past 48 KB (window + t > ~115 keys, e.g. left_chunks 31) a launch needs the opt-in
     if (!opted_in) {
         for (Kernel k : kernels) FO_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
         opted_in = true;
@@ -1034,7 +1034,7 @@ int attention_chunks(const AttnStream& a, int groups, const TA* qkv, const float
         kern = attention_chunks_kernel;
         smem = (size_t)(2 * rows + prow) * DK * 4 + (size_t)2 * t * DK * 4 + (size_t)t * prow * 4;
     }
-    static bool opted_in = false;      // past 48 KB a launch needs the opt-in
+    static std::atomic<bool> opted_in{false};      // past 48 KB a launch needs the opt-in
     if (!opted_in) {
         FO_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
         opted_in = true;
@@ -1086,7 +1086,7 @@ int attention_offline_any(const TA* qkv, const float* q32, int B, int T, int H, 
     if constexpr (sizeof(TA) == 2) {
         if (!ptab_h || T > pos_rows) return 1;
         const size_t smem = (size_t)2 * 3 * FK * DK * 2;      // 48 KB: double-buffered K | P | V tiles
-        static bool attr_set = false;
+        static std::atomic<bool> attr_set{false};
         if (!attr_set) {
             FO_CUDA(cudaFuncSetAttribute(attention_offline_fa_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
             FO_CUDA(cudaFuncSetAttribute(attention_offline_fa_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
@@ -1100,7 +1100,7 @@ int attention_offline_any(const TA* qkv, const float* q32, int B, int T, int H, 
                                                                                                   ptab_h, pos_rows, pos_u, pos_v, out, v);
     } else {
         const size_t smem = (size_t)3 * KT * (DK + 4) * 4 + (size_t)2 * QB * DK * 4 + (size_t)(ATT_THREADS / 32) * KT * 4;
-        static bool attr_set = false;
+        static std::atomic<bool> attr_set{false};
         if (!attr_set) {
             FO_CUDA(cudaFuncSetAttribute(attention_offline_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
             FO_CUDA(cudaFuncSetAttribute(attention_offline_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));

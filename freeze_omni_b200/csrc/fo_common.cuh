@@ -1,5 +1,6 @@
 // Shared declarations of the sm_100a kernels behind include/fo_b200.h.
 #pragma once
+#include <atomic>
 #include <cuda_runtime.h>
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
@@ -36,8 +37,9 @@ void set_error(const char* fmt, ...);
     } while (0)
 #define FO_TRY(expr) do { int _r = (expr); if (_r != 0) return _r; } while (0)
 
-extern long long g_launches;      // kernels enqueued by this library (fo_stats.kernel_launches)
-#define FO_LAUNCHED() (++fo::g_launches)
+extern std::atomic<long long> g_launches;      // kernels enqueued by this library, every thread (fo_stats.kernel_launches)
+extern thread_local long long t_launches;       // the same, by this thread (kernels counted while a graph is captured)
+#define FO_LAUNCHED() (fo::g_launches.fetch_add(1), ++fo::t_launches)
 
 __host__ __device__ inline int cdiv(int a, int b) { return (a + b - 1) / b; }
 // pe_index after j streaming steps of pe = pe % wrap + chunk_size (attention.py:107,120), in closed form since j may run into
@@ -53,7 +55,7 @@ __host__ __device__ inline int pe_after(int pe, int j, int chunk_size, int wrap)
 // while its predecessor is still draining.  FO_PDL_TRIGGER lets the successor launch as soon as every CTA of this
 // grid has started; FO_PDL_WAIT returns once the predecessor grid has completed and its memory is visible.  Every
 // thread executes FO_PDL_WAIT before it touches global memory that another kernel of the chain writes or reads.
-extern int g_use_pdl;
+extern thread_local int g_use_pdl;   // set per step by the host thread that enqueues it
 #define FO_PDL_TRIGGER() asm volatile("griddepcontrol.launch_dependents;" ::: "memory")
 #define FO_PDL_WAIT() asm volatile("griddepcontrol.wait;" ::: "memory")
 template <typename... KArgs, typename... Args>
@@ -277,11 +279,12 @@ struct TcWorkspace {
     size_t partial_bytes = 0;
     int* counters = nullptr;       // split-K arrivals per output tile
     int* ln_counters = nullptr;    // fused-LayerNorm arrivals per row block
+    int sms = 148;                 // SMs the context's grids spread over (its SM group, or the device)
 };
 struct TcTune { int swap, bn, split; };      // -1 / 0 = let the cost model decide
 int gemm_tc_init();
 int gemm_tc_workspace(TcWorkspace* ws);       // allocates; the caller frees the two device pointers
-// the tile plan the host would pick (pure host logic; fo_debug_plan exposes it to the CPU tests)
+// the tile plan the host would pick for a context on the whole device (pure host logic; fo_debug_plan exposes it to the CPU tests)
 void gemm_tc_plan(long long act_rows, int n_out, int K, int can_defer, int* swap, int* bn, int* split);
 void gemm_tc_force(const TcTune& t);
 void gemm_tc_plan_override(int N, int K, int swap, int bn, int split, int cap_kb);   // N <= 0 clears (development)
@@ -301,6 +304,7 @@ struct FbankParams {
     const float* mel;      // n_mel x (fft_size/2+1), zero outside each triangle
     const int* mel_lo;     // first non-zero fft bin per mel filter
     const int* mel_hi;     // one past the last non-zero bin
+    int sms;               // SMs of the context: the grid-stride kernels launch 16 CTAs per SM
 };
 // Streaming: per session s = ids[b]: samples = [carry[s] (frame_len-frame_shift) | new chunk], m = frames_per_chunk
 // frames; ring[s] <- [last ctx frames | new frames]; optional copy of the ring block to feats_out.
@@ -506,12 +510,20 @@ struct StackArgs {
     unsigned long long* trace = nullptr;          // development: %globaltimer of CTA 0 after every grid barrier, [L*5 + 2]
 };
 constexpr int STACK_MAX_ROWS = 16;
-// 0 = launched; 1 = shape not supported (the caller runs the per-kernel chain); < 0 error
-int stream_stack(const StackArgs& a, cudaStream_t st);
+// One cooperative launch of G CTAs, G = the SMs of the context (its SM group, or the device); smem_max = opt-in shared memory
+// per CTA.  0 = launched; 1 = shape not supported or the grid not co-resident (the caller runs the per-kernel chain); < 0 error
+int stream_stack(const StackArgs& a, int G, int smem_max, cudaStream_t st);
 // host-only: does a step of n sessions x t frames qualify on a device of `sms` SMs with smem_max bytes of shared memory per CTA,
 // and with which plan (dynamic shared memory, K chunk of the FFN2 activations, weight rows per CTA and phase); 1 = no
 int stack_plan(int D, int FF, int H, int n, int t, int window, int L, int sms, int smem_max, int* smem_bytes, int* ffn2_chunk,
                int* rows_qkv, int* rows_ffn1, int* rows_out);
+
+// ---- SM groups (fo_partition.cu): CUDA green contexts of fo_create_on_sms ---------------------------------------
+constexpr int SM_GROUP_GRANULE = 8;           // smallest group and its multiple on sm_90 and later (cuda.h, green contexts)
+// the green context of group `group` of `split` equal groups of `device`'s SMs (made at the first use, kept for the process)
+int sm_group_acquire(int device, int split, int group, void** green, int* sms);
+int sm_group_stream(void* green, cudaStream_t* st);          // a non-blocking stream whose work runs on the group's SMs
+int sm_ids(int32_t* out, int n, cudaStream_t st);            // n CTAs write their %smid (fo_debug_sm_ids)
 
 // ---- conversions -----------------------------------------------------------------------------------
 int f32_to_bf16(const float* src, bf16* dst, long long n, cudaStream_t st);

@@ -8,6 +8,9 @@
 // 1.5e-4 relative from exact arithmetic on assets/question.wav; fp64 makes the result exact to fp32
 // rounding, and B200 has full-rate FP64 pipes) -> power spectrum -> sparse triangular mel sums ->
 // log(max(., FLT_EPSILON)).  Bytes moved per frame: frame_shift samples in, n_mel floats out.
+#include <algorithm>
+#include <mutex>
+
 #include "fo_common.cuh"
 
 namespace fo {
@@ -234,7 +237,11 @@ frontend_blocks_finish_kernel(const int32_t* __restrict__ ids, const int32_t* __
     for (int i = threadIdx.x; i < carry + chunk; i += blockDim.x) samples[(long long)s * (carry + chunk) + i] = lr[i];
 }
 
+// The twiddle table is process-wide constant memory, uploaded under a lock: contexts of one process whose frame lengths need
+// different FFT sizes must not run their frontends concurrently (include/fo_b200.h, fo_create_on_sms).
 int upload_twiddles(int P) {
+    static std::mutex mu;
+    std::lock_guard<std::mutex> lk(mu);
     if (g_twiddle_fft == P) return 0;
     FO_CHECK(P >= 64 && P <= MAX_FFT && (P & (P - 1)) == 0, "fbank: FFT size %d unsupported", P);
     static double2 host[MAX_FFT / 2];
@@ -309,7 +316,7 @@ int fbank_offline(const FbankParams& p, const void* pcm, int pcm_is_i16, int B, 
     SampleSrc src{pcm, pcm_is_i16, scale, n_samples, nullptr};
     const long long frames = (long long)B * m;
     long long want = (frames + FB_WARPS - 1) / FB_WARPS;
-    const int grid = (int)(want < 148 * 16 ? want : 148 * 16);      // persistent-ish: 16 CTAs per SM, grid-stride
+    const int grid = (int)std::min<long long>(want, 16LL * p.sms);  // persistent-ish: 16 CTAs per SM of the context, grid-stride
     fbank_kernel<false><<<grid, FB_WARPS * 32, fbank_smem(p.fft_size), st>>>(p, src, B, m, out, nullptr,
                                                                              (long long)m * p.n_mel, 0, nullptr, 0, 0, FbankVarlen());
     FO_LAUNCHED();
@@ -323,7 +330,7 @@ int fbank_offline_packed(const FbankParams& p, const void* pcm, int pcm_is_i16, 
     FO_TRY(upload_twiddles(p.fft_size));
     SampleSrc src{pcm, pcm_is_i16, scale, 0, nullptr};
     long long want = (vl.frames + FB_WARPS - 1) / FB_WARPS;
-    const int grid = (int)(want < 148 * 16 ? want : 148 * 16);      // as fbank_offline
+    const int grid = (int)std::min<long long>(want, 16LL * p.sms);  // as fbank_offline
     fbank_kernel<true><<<grid, FB_WARPS * 32, fbank_smem(p.fft_size), st>>>(p, src, 0, 0, out, nullptr, 0, 0, out2, 0, 0, vl);
     FO_LAUNCHED();
     FO_CUDA(cudaGetLastError());

@@ -864,12 +864,12 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 EncodeTiledFn g_encode = nullptr;
 constexpr int MAX_TILES = 16384;
-int g_sm_count = 148;
+int g_sm_count = 148;            // the device's SMs, for fo_debug_plan (a context plans for its own: TcWorkspace::sms)
 TcTune g_forced = {-1, -1, -1};
-long long g_tc_launches = 0;
+std::atomic<long long> g_tc_launches{0};
 int g_forced_npa = 0, g_forced_npb = 0;
 int g_persist = 1;               // fat short-K GEMMs on the persistent kernel (option tc_persist)
-long long g_persist_launches = 0;
+std::atomic<long long> g_persist_launches{0};
 
 // encoded tensor maps are pure functions of (pointer, extents, box): cached so that eager launches stay cheap on the host
 struct MapKey {
@@ -963,9 +963,8 @@ int skinny_rows() {
     return v;
 }
 
-Plan choose_plan(long long act_rows, int n_out, int K, bool can_defer = false) {
+Plan choose_plan(long long act_rows, int n_out, int K, int sms, bool can_defer = false) {
     const int kblocks = K / BK;
-    const int sms = g_sm_count;
     if (act_rows <= skinny_rows()) {
         const int ta = (n_out + BM - 1) / BM;
         // two CTAs fit one SM (<= 100 KB of stages each) and hide each other's fill / epilogue: up to 2 x SMs CTAs, K split
@@ -1061,7 +1060,7 @@ int gemm_tc_workspace(TcWorkspace* ws) {
 }
 
 void gemm_tc_plan(long long act_rows, int n_out, int K, int can_defer, int* swap, int* bn, int* split) {
-    const Plan p = choose_plan(act_rows, n_out, K, can_defer != 0);
+    const Plan p = choose_plan(act_rows, n_out, K, g_sm_count, can_defer != 0);
     *swap = p.swap; *bn = p.bn; *split = p.split;
 }
 void gemm_tc_force(const TcTune& t) { g_forced = t; }
@@ -1104,9 +1103,9 @@ int gemm_tc(const void* A, int act_fp16, const AGather& ga, const void* W, int M
         }
         const int ta = (M + BM - 1) / BM;
         const bool relaxed = ta >= ta_min;
-        if (relaxed && bn == 256 && N % 128 == 0 && (long long)ta * ((N + 255) / 256) * 10 < (long long)bn128_below_w10 * g_sm_count) bn = 128;
+        if (relaxed && bn == 256 && N % 128 == 0 && (long long)ta * ((N + 255) / 256) * 10 < (long long)bn128_below_w10 * ws.sms) bn = 128;
         const int tb = (N + bn - 1) / bn;
-        if ((long long)ta * tb * 10 >= (long long)(relaxed ? min_w10 : 20) * g_sm_count) {
+        if ((long long)ta * tb * 10 >= (long long)(relaxed ? min_w10 : 20) * ws.sms) {
             TcPersistParams pp;
             memset(&pp, 0, sizeof(pp));
             pp.rows_a = M;
@@ -1141,7 +1140,7 @@ int gemm_tc(const void* A, int act_fp16, const AGather& ga, const void* W, int M
             FO_TRY(make_map(&map_act, reinterpret_cast<const bf16*>(A), ga.seg_len, ga.rows, ga.planes, BM));
             FO_TRY(make_map(&map_w, reinterpret_cast<const bf16*>(W), K, N, 1, bn));
             const size_t smem = (size_t)pp.stages * stage + strips + 1024;
-            const int grid = std::min<long long>(g_sm_count, (long long)ta * tb);
+            const int grid = std::min<long long>(ws.sms, (long long)ta * tb);
             CUtensorMap map_c32 = map_w, map_c16 = map_w;            // (placeholders when an output is absent / the epilogue stores directly)
             if (pp.tma_store) {
                 if (ep.c_f32) FO_TRY(make_out_map(&map_c32, ep.c_f32, 4, M, N, ep.ldc));
@@ -1156,7 +1155,7 @@ int gemm_tc(const void* A, int act_fp16, const AGather& ga, const void* W, int M
         }
     }
     const bool can_defer = ep.defer_reduce && deferred_splits && rmap.p1 == 0 && !ep.ln_gamma && N == ep.ldc;
-    Plan pl = choose_plan(M, N, K, can_defer);
+    Plan pl = choose_plan(M, N, K, ws.sms, can_defer);
     if (!g_plan_override.empty() && M <= skinny_rows()) {
         auto it = g_plan_override.find(PlanKey{N, K});
         if (it != g_plan_override.end()) pl = it->second;
@@ -1199,7 +1198,7 @@ int gemm_tc(const void* A, int act_fp16, const AGather& ga, const void* W, int M
         if (!cap_kb) { const char* e3 = getenv("FO_TC_CAP"); cap_kb = e3 ? atoi(e3) : (occ_cap <= 2 ? 100 : occ_cap == 3 ? 70 : 52); }
         const int cap = (int)(((pl.cap_kb > 0 ? pl.cap_kb : cap_kb) * 1024) / stage);
         if (cap >= 2) p.stages = std::min(p.stages, std::max(cap, 2));
-    } else if ((long long)ta * tb * pl.split > g_sm_count) {
+    } else if ((long long)ta * tb * pl.split > ws.sms) {
         // more CTAs than SMs: keep two resident per SM (<= ~110 KB each) so one CTA's epilogue overlaps the other's mainloop
         const int cap = (int)((110 * 1024) / stage);
         if (cap >= 3) p.stages = std::min(p.stages, cap);

@@ -32,6 +32,8 @@
 #include <stdlib.h>
 
 #include <algorithm>
+#include <map>
+#include <mutex>
 
 #include "fo_attn_core.cuh"
 
@@ -649,27 +651,30 @@ int stack_plan(int D, int FF, int H, int n, int t, int window, int L, int sms, i
     return 0;
 }
 
-int stream_stack(const StackArgs& a, cudaStream_t st) {
-    static int sm_count = 0, smem_max = 0, coop = 0;
-    if (!sm_count) {
-        int dev = 0;
-        FO_CUDA(cudaGetDevice(&dev));
-        FO_CUDA(cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev));
-        FO_CUDA(cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
-        FO_CUDA(cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, dev));
-    }
-    const int G = sm_count;
+int stream_stack(const StackArgs& a, int G, int smem_max, cudaStream_t st) {
     StackLayout lay;
     int smem = 0;
-    if (!coop || !stack_layout(a.D, a.FF, a.a.H, a.a.n, a.a.t, a.a.window, a.L, G, smem_max, &lay, &smem)) return 1;
+    if (!stack_layout(a.D, a.FF, a.a.H, a.a.n, a.a.t, a.a.window, a.L, G, smem_max, &lay, &smem)) return 1;
     static int dbg = -1;
     if (dbg < 0) { const char* e = getenv("FO_STACK_DBG"); dbg = e ? atoi(e) : 0; }
     lay.dbg = dbg;
-    static int attr_smem = 0;
-    if (smem > attr_smem) {
-        FO_CUDA(cudaFuncSetAttribute(stream_stack_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        attr_smem = smem;
+    // the kernel's shared-memory opt-in only grows, per device, under a lock: contexts of different SM counts (hence layouts)
+    // may launch from several host threads
+    {
+        static std::mutex mu;
+        static std::map<int, int> attr_smem;
+        int dev = 0;
+        FO_CUDA(cudaGetDevice(&dev));
+        std::lock_guard<std::mutex> lk(mu);
+        if (smem > attr_smem[dev]) {
+            FO_CUDA(cudaFuncSetAttribute(stream_stack_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+            attr_smem[dev] = smem;
+        }
     }
+    // the G CTAs wait on each other at the grid barriers: one must fit every SM of the group
+    int occ = 0;
+    FO_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, stream_stack_kernel, ST_THREADS, smem));
+    if (occ < 1) return 1;
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(G);
     cfg.blockDim = dim3(ST_THREADS);

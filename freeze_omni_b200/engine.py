@@ -44,7 +44,10 @@ class Engine:
     def __init__(self, cfg: PathConfig, enc_state: Optional[Dict[str, torch.Tensor]] = None,
                  adp_state: Optional[Dict[str, torch.Tensor]] = None, dtype: torch.dtype = torch.float32,
                  device: int = 0, max_sessions: int = 64, max_stream_frames: Optional[int] = None,
-                 use_cmvn: bool = True):
+                 use_cmvn: bool = True, sm_partition: Optional[Tuple[int, int]] = None):
+        """``sm_partition``: None runs the context on the whole device; ``(split, group)`` runs it on group ``group`` of
+        ``split`` equal groups of the device's SMs (fo_create_on_sms), so that contexts on other groups of the same split
+        (another encoder, an LLM beside it) run on disjoint SMs."""
         if not torch.cuda.is_available():
             raise RuntimeError("freeze_omni_b200 needs a CUDA device (sm_100a); there is no CPU fallback")
         if dtype not in (torch.float32, torch.bfloat16):
@@ -70,9 +73,14 @@ class Engine:
             post_norm=int(not cfg.normalize_before), concat_after=int(cfg.concat_after),
             ffn_multi_conv=int(cfg.ffn_type == "conv1d"))
         h = C.c_void_p()
-        _lib.check(self.lib.fo_create(C.byref(c), self.device, _lib.FO_BF16 if dtype == torch.bfloat16 else _lib.FO_F32,
-                                      C.byref(h)))
+        fo_dtype = _lib.FO_BF16 if dtype == torch.bfloat16 else _lib.FO_F32
+        if sm_partition is None:
+            _lib.check(self.lib.fo_create(C.byref(c), self.device, fo_dtype, C.byref(h)))
+        else:
+            split, group = sm_partition
+            _lib.check(self.lib.fo_create_on_sms(C.byref(c), self.device, fo_dtype, int(split), int(group), C.byref(h)))
         self._h = h
+        self.sm_count = self.get_option("sm_count")   # SMs the context's grids spread over: its group's, or the device's
         self.max_t = self.get_option("max_t")      # encoder frames per streaming chunk, capped at 8 by the library
         try:
             if self.has_encoder:
@@ -619,6 +627,13 @@ class Engine:
         _lib.check(self.lib.fo_debug_gemm(self._h, _ptr(A), _ptr(W), _ptr(bias), _ptr(out), M, N, K, backend, int(relu),
                                           iters, C.byref(ms), self._stream()))
         return out, float(ms.value)
+
+    def debug_sm_ids(self, n_ctas: int, graph: bool = False) -> torch.Tensor:
+        """The SM ids that n_ctas CTAs launched as this context launches its kernels ran on (int32, on the device); with
+        `graph` the launch is captured into a graph on the context's capture stream and replayed, as a streaming step is."""
+        out = torch.empty(n_ctas, dtype=torch.int32, device=self.torch_device)
+        _lib.check(self.lib.fo_debug_sm_ids(self._h, int(n_ctas), int(graph), _ptr(out), self._stream()))
+        return out
 
     def debug_attention(self, mode: str, qkv: Optional[torch.Tensor], ptab: torch.Tensor, pos_u: torch.Tensor,
                         pos_v: torch.Tensor, *, seq=None, T: int = 0, gap: int = 0, chunk: int = 0, left: int = -1, t: int = 0,

@@ -108,6 +108,19 @@ const char* fo_last_error(void);
 
 /* ---- lifetime: replaces speechEncoder(...) / CNNSubsampling(...) construction + .to(device) ---- */
 int fo_create(const fo_config* cfg, int device, int dtype, fo_ctx** out);
+/* fo_create on one group of the device's SMs, so that several contexts share a GPU without waiting on each other's grids
+ * (a user and a system encoder, an LLM beside them).  The device's SMs are split into sm_split equal groups of a multiple of
+ * 8 SMs (the granularity of CUDA green contexts: at least 8, in multiples of 8; 148 SMs split 2 ways give 2 x 72); the context
+ * runs on group sm_group.  The split is made once per process and device: contexts created with the same sm_split and
+ * different groups run on disjoint SMs.  Every grid, GEMM plan and the layer stack are sized to the group's SMs
+ * (fo_get_option "sm_count").  Entry points keep their stream contract: the work of a call runs on a stream of the group,
+ * after what the caller enqueued on `stream` before the call and before what it enqueues there after it.  Refused, with
+ * nothing allocated: sm_split < 1, sm_group outside [0, sm_split), groups below 8 SMs, a driver without green contexts
+ * (CUDA 12.4+).  There is no fall-back to the whole device.
+ * Shared by every context of the process: the fbank twiddle table (contexts whose frame lengths need different FFT sizes
+ * must not run their frontends at the same time) and the counters of fo_stats.kernel_launches / options "tc_launches",
+ * "tc_persist_launches" (totals over all contexts and threads). */
+int fo_create_on_sms(const fo_config* cfg, int device, int dtype, int sm_split, int sm_group, fo_ctx** out);
 int fo_destroy(fo_ctx* ctx);
 
 /* ---- weights: replaces load_state_dict (models/utils.py:11-20).  `name` is the reference's
@@ -335,7 +348,8 @@ int fo_stats(fo_ctx* ctx, fo_stats_t* out);
  *       fo_encode_stream_steps_v; 0 = as many as 1 GiB of workspace holds (720 blocks of the shipped model in bf16)
  *   "profile_gemm" 0/1, "debug_skip" (timing attribution), "tc_swap"/"tc_bn"/"tc_split" (-1 = cost model): development
  * get-only: "tc_launches", "tc_persist_launches", "stack_launches", "ring_cap", "max_t", "profile_gemm_us", "profile_gemm_count",
- *   "steps_pass_blocks_in_use" (the blocks per pass "steps_pass_blocks" gives at the context's chunking).
+ *   "steps_pass_blocks_in_use" (the blocks per pass "steps_pass_blocks" gives at the context's chunking), "sm_count" (the SMs
+ *   of the context's group, fo_create_on_sms, or of the device).
  * Development environment variables read once per process: FO_TC_OCC, FO_TC_KB, FO_TC_KBD, FO_TC_SMAX, FO_TC_CAP, FO_TC_SKINNY (tile
  * plan of the skinny GEMMs), FO_PDL_MIN, FO_PERSIST_DBG, FO_TC_TRACE. */
 int fo_set_option(fo_ctx* ctx, const char* name, int64_t value);
@@ -347,6 +361,11 @@ int fo_profile_dump(fo_ctx* ctx, char* buf, int cap);
  * record of 8 uint64 {kernel id | smid << 8 | aux << 16 | linear block id << 32, grid dims, 6 x %globaltimer ns}; this copies up to
  * cap_records of them out and restarts the log.  A regular build records nothing (n_records = 0). */
 int fo_debug_trace_read(fo_ctx* ctx, uint64_t* out, int64_t cap_records, int64_t* n_records);
+/* n_ctas CTAs launched as the context launches its kernels (on `stream`, in its SM group if it has one) write the id of the
+ * SM they ran on to out (n_ctas int32, device or host memory; a host buffer is filled when the call returns).  graph = 0: a
+ * direct launch; graph = 1: the launch captured into a CUDA graph on the context's capture stream and replayed, as a streaming
+ * step is.  Each CTA stays ~20 us, so that a launch spreads over every SM the context can reach. */
+int fo_debug_sm_ids(fo_ctx* ctx, int n_ctas, int graph, int32_t* out, void* stream);
 /* host-only: the tile plan of the tcgen05 GEMM for (activation rows, output columns, K) -- swap = weights on the UMMA-M side,
  * bn = UMMA N, split = K splits; can_defer = a consumer kernel finishes the split-K sum.  Needs no GPU (CPU tests of the plan). */
 int fo_debug_plan(int64_t act_rows, int n_out, int K, int can_defer, int* swap, int* bn, int* split);
